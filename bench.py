@@ -1,13 +1,15 @@
 #!/usr/bin/env python
 """bench.py -- pages/s of the EAST decode + LANMS + box filters + crop/resize/pad hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
 A step = one pass of the hot path over one batch of synthetic pages PER GPU (pages are independent, so
 ranks never exchange data: weak scaling, no collective on the data path; torch.distributed is used only
-for the barrier and the max-over-ranks of the timings).
+for the barrier and the max-over-ranks of the timings).  Exactly K steps are timed.  The inputs are generated from
+fixed seeds, so runs with the same arguments compute on the same data; --dump-outputs DIR writes the results of the
+last timed step there (dump_outputs) for comparing two builds output for output.
 
 Workload (BASELINE.json configs[2]): 64 synthetic 2048x2048 pages per GPU, ~2000 word quads per page
 (score map 512x512, geometry 8x512x512, page image 2048x2048x3 u8), TRBA 32x128 crop batch output.
@@ -51,15 +53,15 @@ _REAL_STDOUT = None  # set when stdout's descriptor is redirected (multi-rank ru
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: 250 for the b200 arm, a timed region of about 0.5 s at the default workload "
+                         "(2.26 ms per step on one B200); 5 for the reference arm, whose steps take seconds on the host)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--pages", type=int, default=64, help="pages per GPU per step")
     ap.add_argument("--page-size", type=int, default=2048)
     ap.add_argument("--words", type=int, default=2000)
     ap.add_argument("--cpu-pages", type=int, default=8, help="pages in the bounded cpu_baseline sample")
-    ap.add_argument("--min-timed-s", type=float, default=0.5,
-                    help="the K timed steps are repeated (rounds) until the timed region lasts at least this long")
     ap.add_argument("--corpus", type=int, default=1024, help="pages of the strong-scaling corpus run (BASELINE configs[4])")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
@@ -70,7 +72,17 @@ def parse_args():
     ap.add_argument("--reading-order", action="store_true",
                     help="also run the reading-order sort between the box filters and the crops (what Pipeline.predict "
                          "does; not part of the BASELINE metric, reported under config.reading_order)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path returned in its last timed step (rank 0's pages) as DIR/<name>.npy, "
+                         "so that two builds can be compared output for output: see dump_outputs()")
+    a = ap.parse_args()
+    if a.steps is None:
+        a.steps = 250 if a.impl == "b200" else 5
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return a
 
 
 BASELINE_SHAPES = {(1280, 500, 1): "configs[1]", (2048, 2000, 64): "configs[2]", (4096, 10000, None): "configs[3]"}
@@ -250,6 +262,42 @@ def parity_check(a, score_np, geo_np, imgs_np, res, pages=(0, 1), every=50):
             "against": "oracle/oracle.c chain (pinned to the reference's goldens), bit-exact"}
 
 
+DUMP_BYTES = 64 << 20
+DUMP_CROPS = 512
+
+
+def dump_outputs(out_dir, res):
+    """Write the results of one ms_page_batch step as <out_dir>/<name>.npy, float32 / float64 only, at most DUMP_BYTES in
+    all: every page's final boxes (rows concatenated in page order), box counts, flags and the crop list in full, a float64
+    sum of every crop of the float32 batch, and DUMP_CROPS crops of the batch chosen by a fixed seed (with their indices).
+    The inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    import torch
+
+    counts = res.box_counts.cpu().numpy()
+    boxes = res.boxes.cpu().numpy()
+    n_crops = int(res.n_crops.cpu()[0])
+    batch = res.batch[:n_crops]
+    out = {
+        "boxes": np.concatenate([boxes[p, : counts[p]] for p in range(len(counts))]),
+        "box_counts": counts.astype(np.float64),
+        "flags": res.flags.cpu().numpy().astype(np.float64),
+        "crops": res.crops[:n_crops].cpu().numpy().astype(np.float64),
+        "batch_crop_sums": torch.sum(batch, dim=(1, 2, 3), dtype=torch.float64).cpu().numpy(),
+    }
+    crop_bytes = batch[0].numel() * 4 if n_crops else 0
+    room = DUMP_BYTES - sum(v.nbytes for v in out.values())
+    if room < 0:
+        raise SystemExit(f"bench.py: the outputs of this workload exceed {DUMP_BYTES >> 20} MB; use fewer --pages")
+    k = min(n_crops, DUMP_CROPS, room // (crop_bytes + 8) if crop_bytes else 0)
+    idx = np.sort(np.random.default_rng(0).choice(n_crops, k, replace=False))
+    out["batch_sample_index"] = idx.astype(np.float64)
+    out["batch_sample"] = batch[torch.from_numpy(idx).to(batch.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    return {"dir": out_dir, "files": sorted(out), "bytes": int(sum(v.nbytes for v in out.values()))}
+
+
 def run_b200(a):
     import torch
 
@@ -321,19 +369,12 @@ def run_b200(a):
     ctx = runner.ctx
     stream = torch.cuda.current_stream()
 
-    # warm-up (also sizes the scratch arenas), timed roughly to size the rounds of the timed region
+    # warm-up (also sizes the scratch arenas)
     W = max(a.warmup, 3)
     for _ in range(W):
         res = runner.run(d_score, d_geo, d_pages)
     torch.cuda.synchronize()
     res.raise_for_flags()
-    w0, w1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    w0.record(stream)
-    res = runner.run(d_score, d_geo, d_pages)
-    w1.record(stream)
-    torch.cuda.synchronize()
-    est_ms = max(w0.elapsed_time(w1), 1e-3)
-    rounds = int(max_over_ranks(float(max(1, min(64, -(-int(a.min_timed_s * 1e3) // max(1, int(est_ms * a.steps))))))))
 
     # parity of THIS step's results with the oracle, before anything is timed
     parity = None
@@ -373,7 +414,7 @@ def run_b200(a):
         "crop": 3 * src_px + 3 * OUT_H * OUT_W * 4 * n_crops,
     }
 
-    # ---- timed region 1: inputs resident in HBM, device-timed: `rounds` x K steps ------------------------------------
+    # ---- timed region 1: inputs resident in HBM, device-timed: K steps -----------------------------------------------
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
@@ -386,18 +427,20 @@ def run_b200(a):
     torch.cuda.synchronize()
     launches0 = ctx.launches
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    n_timed = a.steps * rounds
+    n_timed = a.steps
     barrier()
     torch.cuda.synchronize()
     t_wall0 = time.perf_counter()
     ev0.record(stream)
     for _ in range(n_timed):
-        runner.run(d_score, d_geo, d_pages)
+        last = runner.run(d_score, d_geo, d_pages)
     ev1.record(stream)
     torch.cuda.synchronize()
     barrier()
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
-    launches = (ctx.launches - launches0) / rounds  # per K steps
+    launches = ctx.launches - launches0  # per K steps
+    # the runner's output buffers are overwritten by the next pass: write the last timed step's results now
+    dumped = dump_outputs(a.dump_outputs, last.raise_for_flags()) if a.dump_outputs and rank == 0 else None
     # ---- the same steps once more with the library's stage events (CUDA events between the stages on the launch
     # stream): per-stage times and the dominant kernel's duration.  Events between the stages need direct launches
     # instead of the graph replay, so this pass is a few per cent slower than the one above and is reported beside it.
@@ -422,15 +465,10 @@ def run_b200(a):
     if not a.no_e2e:
         for _ in range(2):
             runner.run_host(h_score, h_geo, h_pages)
-        torch.cuda.synchronize()
-        t0 = time.perf_counter()
-        runner.run_host(h_score, h_geo, h_pages)
-        est_e2e = time.perf_counter() - t0
-        rounds_e = int(max_over_ranks(float(max(1, min(16, -(-int(a.min_timed_s * 1e3) // max(1, int(est_e2e * 1e3 * a.steps))))))))
         barrier()
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        for _ in range(a.steps * rounds_e):
+        for _ in range(a.steps):
             rh = runner.run_host(h_score, h_geo, h_pages)
         torch.cuda.synchronize()
         t_e2e = max_over_ranks(time.perf_counter() - t0)
@@ -447,8 +485,8 @@ def run_b200(a):
             geo_bytes, geo_how = n_cand * 8 * 32, "geometry gathered from pinned host memory by the decode kernel (zero copy)"
         h2d = h_score.numel() * 4 + geo_bytes + h_pages.numel()
         d2h = P * int(counts.max()) * 36 + P * 8 + 4 + nch * 20
-        e2e = {"value": world * P * a.steps * rounds_e / t_e2e, "unit": "pages/s", "h2d_bytes_per_step": int(h2d),
-               "d2h_bytes_per_step": int(d2h), "ms_per_step": 1e3 * t_e2e / (a.steps * rounds_e), "rounds": rounds_e,
+        e2e = {"value": world * P * a.steps / t_e2e, "unit": "pages/s", "h2d_bytes_per_step": int(h2d),
+               "d2h_bytes_per_step": int(d2h), "ms_per_step": 1e3 * t_e2e / a.steps,
                "note": "ms_page_batch_host with pinned host buffers; " + geo_how +
                        "; crop batch left on the device for the recogniser"}
         # what the box can move: the same bytes as plain pinned cudaMemcpyAsync copies, all ranks at once
@@ -460,7 +498,7 @@ def run_b200(a):
         barrier()
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        reps_c = max(2, a.steps * rounds_e // 2)
+        reps_c = max(2, a.steps // 2)
         for _ in range(reps_c):
             h2d_dst.copy_(h_pages, non_blocking=True)
             sc_dst.copy_(h_score, non_blocking=True)
@@ -496,16 +534,16 @@ def run_b200(a):
         barrier()
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        for _ in range(a.steps * rounds_e):
+        for _ in range(a.steps):
             rm = runner.run_host(d_score, d_geo, h_pages)
         torch.cuda.synchronize()
         t_m = max_over_ranks(time.perf_counter() - t0)
         barrier()
         assert int(rm.n_crops[0]) == n_crops
-        e2e["maps_on_device"] = {"value": world * P * a.steps * rounds_e / t_m, "unit": "pages/s",
-                                 "ms_per_step": 1e3 * t_m / (a.steps * rounds_e),
+        e2e["maps_on_device"] = {"value": world * P * a.steps / t_m, "unit": "pages/s",
+                                 "ms_per_step": 1e3 * t_m / a.steps,
                                  "h2d_bytes_per_step": int(h_pages.numel()), "d2h_bytes_per_step": int(d2h),
-                                 "frac_of_ceiling": (world * P * a.steps * rounds_e / t_m) /
+                                 "frac_of_ceiling": (world * P * a.steps / t_m) /
                                                     (world * P * reps_c / t_c * copy_bytes / h_pages.numel())}
 
     # ---- BASELINE configs[4]: a fixed corpus strong-scaled over the ranks, results gathered on rank 0's host ---------
@@ -585,7 +623,7 @@ def run_b200(a):
     line = {
         "metric": METRIC, "value": world * P * n_timed / (ms_total * 1e-3), "unit": "pages/s", "n_gpus": world,
         "steps": a.steps, "warmup": W, "ms_per_step": ms_step, "higher_is_better": True,
-        "timed_rounds": rounds, "timed_region_ms": ms_total,
+        "timed_region_ms": ms_total,
         "scaling": "weak", "vs_baseline": None, "dtype": "f64 (NMS) / f32 (boxes) / u8 (crops)", "data": "synthetic",
         "config": {"workload": workload_name(a), "pages_per_gpu": P, "page": S, "map": M, "words_per_page": a.words,
                    "candidates_per_page": n_cand / P, "boxes_per_page": n_boxes / P, "crops_per_page": n_crops / P,
@@ -595,9 +633,9 @@ def run_b200(a):
                                       "probe (~12 per word, 24k per page) used larger words -- variants.dense_candidates "
                                       "times that load",
                    "l2": "inputs (maps + pages) of one step exceed L2 (no flush needed)",
-                   "timing": f"the {a.steps} timed steps are repeated {rounds}x back to back inside one CUDA-event bracket so "
-                             f"that the timed region lasts >= {a.min_timed_s} s; ms_per_step is the mean over all of them; "
-                             "the repeated call is replayed as a CUDA graph by the library (MS_B200_NO_GRAPHS=1: direct launches)",
+                   "timing": f"the {a.steps} timed steps run back to back inside one CUDA-event bracket; ms_per_step is "
+                             "their mean; the repeated call is replayed as a CUDA graph by the library (MS_B200_NO_GRAPHS=1: "
+                             "direct launches)",
                    "reading_order": bool(a.reading_order), "host_cpus_rank0": (len(cpus) if cpus else None),
                    "numa_node_rank0": numa_node,
                    "parallelism": f"pages sharded over {world} GPU(s), no collective"},
@@ -614,6 +652,8 @@ def run_b200(a):
                                "`value` / `ms_per_step` are the timed region itself (graph replay, what a caller gets)"},
         "clocks": sampler.summary(t_wall0, t_wall2),
     }
+    if dumped is not None:
+        line["outputs_dumped"] = dumped
     if e2e is not None:
         line["e2e"] = e2e
     if corpus is not None:

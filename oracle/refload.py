@@ -1,9 +1,9 @@
-"""Load the REAL reference hot-path modules from /root/reference by file path.
+"""Load the REAL reference hot-path modules (olegiy/manuscript-ocr v0.1.8) by file path.
 
-TEST INFRASTRUCTURE ONLY, and only usable in the build container: /root/reference does not
-exist on the GPU box, so nothing marked `gpu`, smoke() or bench.py may call this.  It is used
-by tests/golden/make_golden.py (fixture generation) and by `not gpu` tests that cross-check the
-oracle against the live reference when it happens to be present (skipped otherwise).
+The reference source tree is not part of this repository: it is looked for in oracle/_ref/ (kept out of git) or in
+the directory MANUSCRIPT_REFERENCE_ROOT names.  TEST INFRASTRUCTURE ONLY, so nothing marked `gpu`, smoke() or
+bench.py may call this.  It is used by tests/golden/make_golden*.py (fixture generation) and by `not gpu` tests that
+cross-check the oracle against the live reference when it is present (skipped otherwise).
 
 The reference package cannot be imported as a whole here (gdown / shapely / albumentations are
 not installed, SURVEY 8c), so the two self-contained modules are loaded directly:
@@ -19,7 +19,7 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("MANUSCRIPT_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("MANUSCRIPT_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 _SRC = os.path.join(REF_ROOT, "src", "manuscript")
 
 

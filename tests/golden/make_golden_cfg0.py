@@ -14,8 +14,10 @@ locality_aware_nms, expand_boxes, the EAST box filters) are then run on those ma
 
 The fixture holds the network INPUT hash, the maps (float32, exactly as the network produced them) and the reference's
 outputs, so that the GPU box -- which has neither /root/reference nor the example image -- can replay the maps through
-mb.EAST / mb.Pipeline and compare.  target_size = 640 keeps the fixture small (160 x 160 maps, < 1 MB); the example
-image itself is 4250 x 5390 and is replaced by its 640 x 640 network-input resize (stored as uint8).
+mb.EAST / mb.Pipeline and compare.  target_size = 640 keeps the fixture small (160 x 160 maps); the example
+image itself is 4250 x 5390 and is replaced by its 640 x 640 network-input resize (stored as uint8).  The geometry map
+is stored only at the pixels a quantisation-2 decode reads (geo[:, 1::2, 1::2], the centre of every 2 x 2 cell), which
+keeps the file under 1 MB; the outputs are checked to be the same with every other pixel set to zero.
 """
 import hashlib
 import importlib.util
@@ -71,8 +73,12 @@ def main():
     assert np.array_equal(oq, quads)
     assert np.array_equal(cpu.locality_aware_nms(oq, 0.2), nms)
     assert np.array_equal(cpu.east_postprocess(nms, orig_hw, target_size=TARGET), final)
+    centres = np.ascontiguousarray(geo[:, 1::2, 1::2])
+    sparse = np.zeros_like(geo)
+    sparse[:, 1::2, 1::2] = centres
+    assert np.array_equal(cpu.decode_quads_from_maps(score, sparse, thr, 4.0, 2), quads)
     np.savez_compressed(OUT, target=TARGET, orig_hw=np.array(orig_hw), resized=resized, input_sha=sha(t.numpy()),
-                        score=score, geo=geo, score_thresh=thr, n_candidates=len(quads), quads_sha=sha(quads),
+                        score=score, geo_centres=centres, score_thresh=thr, n_candidates=len(quads), quads_sha=sha(quads),
                         lanms=nms, final=final, score_min=float(score.min()), score_max=float(score.max()))
     print("score range", score.min(), score.max(), "thr", thr, "candidates", len(quads), "kept", len(nms), "final",
           len(final), "bytes", os.path.getsize(OUT))

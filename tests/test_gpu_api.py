@@ -641,15 +641,20 @@ def test_configs0_example_image_random_init_network(mb, golden_dir):
     """tests/golden/make_golden_cfg0.py ran the reference's OWN network module (detectors/_east/east.py, random init,
     seed 0, CPU) on example/ocr_example_image.jpg prepared as EAST.predict prepares it, and the reference's
     post-processing on the maps it produced (score_thresh = the map's median: random init never reaches 0.6).  Here
-    the maps are replayed through mb.EAST and mb.Pipeline: the network input made on the device is bit-identical to the
-    reference's, and candidates / kept rows / final boxes equal the reference's outputs."""
+    the maps are replayed (the geometry map at the pixels the decode reads) through mb.EAST and mb.Pipeline: the network
+    input made on the device is bit-identical to the reference's, and candidates / kept rows / final boxes equal the
+    reference's outputs."""
     import hashlib
 
     import torch
 
     g = np.load(os.path.join(golden_dir, "cfg0_example.npz"))
     target, thr = int(g["target"]), float(g["score_thresh"])
-    score, geo, resized = g["score"], g["geo"], g["resized"]
+    score, resized = g["score"], g["resized"]
+    # the fixture keeps the geometry only at the pixels a quantisation-2 decode reads (the centre of every 2x2 cell);
+    # every other pixel is zero, so a decode that reads a wrong pixel gets a wrong quad
+    geo = np.zeros((8, *score.shape), np.float32)
+    geo[:, 1::2, 1::2] = g["geo_centres"]
     seen = {}
 
     class Net:  # stands in for the reference's network: checks its input, replays the maps the real one produced

@@ -151,7 +151,8 @@ def test_decode_edge_cases():
         cpu.decode_quads_from_maps(s7, np.zeros((8, 7, 7), np.float32), 0.6, 4.0, 2)
 
 
-@pytest.mark.skipif(not refload.available(), reason="live reference only in the build container")
+@pytest.mark.skipif(not refload.available(),
+                    reason="needs the original manuscript-ocr source tree in oracle/_ref/ or MANUSCRIPT_REFERENCE_ROOT")
 def test_live_reference_random_pages():
     """Extra seeds against the live reference (stable-patched), decode -> lanms -> expand."""
     ru, rs = refload.utils(), refload.lanms_stable()
