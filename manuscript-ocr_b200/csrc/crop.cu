@@ -22,7 +22,7 @@
 //                           word box to a 32- or 64-pixel-high canvas gives): persistent, warp specialised, 4 CTAs
 //                           of 7 warps per SM.  Warp 0 (copy warp) stages the next crop's source rows with TMA bulk
 //                           copies (cp.async.bulk global->shared, one 16-byte-aligned span per row, completion on an
-//                           mbarrier) into a double-buffered stage; warp 1 (table warp) builds OpenCV's coefficient
+//                           mbarrier) into a byte-granular staging ring; warp 1 (table warp) builds OpenCV's coefficient
 //                           tables in shared memory (structure of arrays) and writes the 255-padding as constant
 //                           16-byte streaming stores; warps 2..6 (consumers) resample column strips out of shared
 //                           memory (aligned 32-bit loads + funnel shift + PRMT u8->f32, 3 or 4 taps) and store
@@ -34,35 +34,13 @@
 
 namespace {
 
-// CTA shape of the persistent kernel.  MS_CROP_PAD_WARP = 0: copy warp + table/padding warp + 5 consumer warps, 4 CTAs
-// per SM (224 threads, 72 registers).  MS_CROP_PAD_WARP = 1: copy warp + table warp + PADDING warp + 7 consumer warps,
-// 3 CTAs per SM (320 threads, 64 registers): the padding no longer serialises behind the tables in one warp.
-#ifndef MS_CROP_PAD_WARP
-#define MS_CROP_PAD_WARP 0
-#endif
-#if MS_CROP_PAD_WARP
-constexpr int kThreads = 320;
-constexpr int kCtasPerSm = 3;
-constexpr int kSlots = 4;       // crops in flight per CTA (ring slots: metadata + tables per slot, bytes from the ring)
-#else
+// CTA shape of the persistent kernel: copy warp + table/padding warp + 5 consumer warps, 4 CTAs per SM (224 threads,
+// 72 registers).
 constexpr int kThreads = 224;
 constexpr int kCtasPerSm = 4;
-#ifndef MS_CROP_SLOTS
-#define MS_CROP_SLOTS 3
-#endif
-constexpr int kSlots = MS_CROP_SLOTS;  // (4 slots: 3.5 KB less ring per CTA -- measured r2p, see profiles/README.md)
-#endif
-constexpr bool kPadWarp = MS_CROP_PAD_WARP != 0;
+constexpr int kSlots = 3;  // crops in flight per CTA (ring slots: metadata + tables per slot, bytes from the ring)
 constexpr int kSrcBuf = 40 * 1024;  // largest staged crop (bytes); the staging ring of a CTA holds at least one
 constexpr int kBandsY = 64, kCellsX = 8;  // work-list buckets per page: (row band, x cell)
-#ifndef MS_COPY_PAD_CHANNELS
-#define MS_COPY_PAD_CHANNELS 0
-#endif
-constexpr int kCopyPadChannels = MS_COPY_PAD_CHANNELS;  // float32 padding channels written by the copy warp (A/B switch)
-#ifndef MS_PAD_LAG
-#define MS_PAD_LAG 0
-#endif
-constexpr int kPadLag = MS_PAD_LAG;  // crops between building a crop's tables and writing its padding (A/B switch)
 
 // Pages are either one (n_pages, img_h, img_w, 3) tensor, or -- page_ptrs != NULL -- separate images of their own
 // sizes: page_ptrs[p] -> (page_hw[2p], page_hw[2p+1], 3) bytes.
@@ -273,7 +251,7 @@ __global__ void __launch_bounds__(256) crop_bucket_scatter_kernel(const Plan *__
 // Each consumer thread resamples a column strip (one destination column, G consecutive destination rows): with a
 // shrink factor near 2 neighbouring destination rows share their boundary source row, so a strip needs ~(2G + 1)
 // horizontal row sums instead of 3G; per-pixel arithmetic and its order are unchanged.
-constexpr int kProducerWarps = kPadWarp ? 3 : 2;
+constexpr int kProducerWarps = 2;
 constexpr int kConsumerWarps = kThreads / 32 - kProducerWarps;
 
 template <bool kWriteF32, bool kWriteU8>
@@ -292,7 +270,6 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
     // the plan array in global memory
     __shared__ int s_next[kSlots];    // copy warp -> table warp: crop index of the slot
     __shared__ int s_off[kSlots];     // copy warp -> consumers: ring offset of the crop's first row
-    __shared__ int s_pad[kSlots][2];  // copy warp -> padding warp: nw | nh << 16, y0
     __shared__ long long s_ci[kSlots];
     __shared__ int s_meta[kSlots][8];  // nw, nh, y0, pitch, misalignment of row 0, its change per row, <= 3 x taps, strip height
 
@@ -303,7 +280,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
 #pragma unroll
         for (int i = 0; i < kSlots; i++) {
             mbar_init(&s_full[i], 2);  // the copy warp (with the byte count) and the table warp
-            mbar_init(&s_empty[i], kConsumerWarps + (kPadWarp ? 1 : 0));  // + the padding warp (it read the slot's descriptor)
+            mbar_init(&s_empty[i], kConsumerWarps);
             mbar_init(&s_tick[i], 1);
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -390,8 +367,6 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
             if (lane == 0) {
                 s_next[s] = cur.ci;
                 s_off[s] = off;
-                s_pad[s][0] = cur.nwh;
-                s_pad[s][1] = cur.y0;
                 mbar_arrive(&s_tick[s]);  // release: the table warp and (through full) the consumers see both
             }
             uint32_t bytes = 0;
@@ -403,40 +378,19 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
                     const uint8_t *g = src + (size_t)r * stride;
                     const uint32_t a = (uint32_t)(reinterpret_cast<uintptr_t>(g) & 15);
                     const uint32_t sz = (a + (uint32_t)cw * 3 + 15) & ~15u;
-#if !defined(MS_EXP_NO_COPY)
                     tma_bulk_g2s(buf + (size_t)r * cur.pitch, g - a, sz, &s_full[s]);
                     bytes += sz;
-#endif
                 }
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) bytes += __shfl_xor_sync(0xffffffffu, bytes, o);
             }
             if (lane == 0) mbar_expect_tx(&s_full[s], bytes);
-            // this warp's share of the crop's padding (kCopyPadChannels of the three channels): a lone warp's stores
-            // proceed at one 128-byte line per ~25 cycles, so all the padding on the table warp made that warp the
-            // kernel's critical path (profiles/README.md, r2d experiments)
-            if (kCopyPadChannels > 0)
-                write_padding<kWriteF32, kWriteU8>(cur.nwh & 0xffff, (int)((uint32_t)cur.nwh >> 16), cur.y0, ih, iw,
-                                                   kWriteF32 ? batch + (size_t)cur.ci * 3 * plane : nullptr, nullptr, vec_ok,
-                                                   lane, 32, 3 - kCopyPadChannels, 3);
             cur = nxt;
         }
         return;
     }
     if (warp == 1) {
         // ---------------- table warp: OpenCV's axis tables, then all of the padding ----------------
-        // kPadLag > 0: the padding of a crop is written kPadLag crops later, i.e. about when the consumers write its
-        // pixels, so that a canvas reaches DRAM in one visit instead of two
-        int lag_ci[kPadLag + 1], lag_nwh[kPadLag + 1], lag_y0[kPadLag + 1];
-#pragma unroll
-        for (int i = 0; i <= kPadLag; i++) lag_ci[i] = -1, lag_nwh[i] = 0, lag_y0[i] = 0;
-        auto pad_one = [&](int pci, int nwh, int py0) {
-            if (pci >= 0)
-                write_padding<kWriteF32, kWriteU8>(nwh & 0xffff, (int)((uint32_t)nwh >> 16), py0, ih, iw,
-                                                   kWriteF32 ? batch + (size_t)pci * 3 * plane : nullptr,
-                                                   kWriteU8 ? canvas_out + (size_t)pci * 3 * plane : nullptr, vec_ok, lane,
-                                                   32, 0, kWriteF32 ? 3 - kCopyPadChannels : 3);
-        };
         for (int k = 0;; k++) {
             const int s = k % kSlots;
             mbar_wait(&s_tick[s], (uint32_t)((k / kSlots) & 1));
@@ -446,10 +400,6 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
                     s_ci[s] = -1;
                     mbar_arrive(&s_full[s]);
                 }
-#if !defined(MS_EXP_NO_PAD)
-#pragma unroll
-                for (int i = 0; i < kPadLag; i++) pad_one(lag_ci[i], lag_nwh[i], lag_y0[i]);
-#endif
                 break;
             }
             const Plan p = plans[ci];
@@ -468,32 +418,8 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
             }
             __syncwarp();  // every lane's table stores are ordered before lane 0's releasing arrive
             if (lane == 0) mbar_arrive(&s_full[s]);
-#if !defined(MS_EXP_NO_PAD)
-            if (kPadWarp) continue;
-            lag_ci[kPadLag] = ci, lag_nwh[kPadLag] = p.nw | (p.nh << 16), lag_y0[kPadLag] = p.y0;
-            pad_one(lag_ci[0], lag_nwh[0], lag_y0[0]);
-#pragma unroll
-            for (int i = 0; i < kPadLag; i++) lag_ci[i] = lag_ci[i + 1], lag_nwh[i] = lag_nwh[i + 1], lag_y0[i] = lag_y0[i + 1];
-#endif
-        }
-        return;
-    }
-
-    if (kPadWarp && warp == 2) {
-        // ---------------- padding warp: the 255-padding of every crop, as soon as the copy warp has drawn it ----------------
-        for (int k = 0;; k++) {
-            const int s = k % kSlots;
-            mbar_wait(&s_tick[s], (uint32_t)((k / kSlots) & 1));
-            const int ci = s_next[s];
-            if (ci < 0) break;
-            const int nwh = s_pad[s][0], py0 = s_pad[s][1];
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&s_empty[s]);  // the slot's descriptor has been read
-#if !defined(MS_EXP_NO_PAD)
-            write_padding<kWriteF32, kWriteU8>(nwh & 0xffff, (int)((uint32_t)nwh >> 16), py0, ih, iw,
-                                               kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr,
-                                               kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr, vec_ok, lane, 32, 0, 3);
-#endif
+            write_padding<kWriteF32, kWriteU8>(p.nw, p.nh, p.y0, ih, iw, kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr,
+                                               kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr, vec_ok, lane, 32);
         }
         return;
     }
@@ -516,24 +442,18 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
         // three x taps at most (shrink factor below 2, most word boxes): a quarter of the horizontal work less; a page
         // stride that is a multiple of 16 bytes (sstep == 0): no per-row misalignment arithmetic
         bool bad = false;
-#if defined(MS_EXP_NO_CONSUME)
-        if (false)
-#else
         if (s_meta[s][6] == 2)
             area2x2_pixels<kWriteF32, kWriteU8, kCT>(smem, stage_off, pitch, a0, sstep, ih, iw, nw, nh, y0, dstf, dstu, ct);
         else if (sstep == 0)
-#endif
             bad = s_meta[s][6] == 1 ? area4_strips<kWriteF32, kWriteU8, kCT, 3, true>(smem, stage_off, pitch, a0, 0u, tab, tab_n, ih,
                                                                                  iw, nw, nh, y0, dstf, dstu, ct, G)
                                : area4_strips<kWriteF32, kWriteU8, kCT, 4, true>(smem, stage_off, pitch, a0, 0u, tab, tab_n, ih,
                                                                                  iw, nw, nh, y0, dstf, dstu, ct, G);
-#if !defined(MS_EXP_NO_CONSUME)
         else
             bad = s_meta[s][6] == 1 ? area4_strips<kWriteF32, kWriteU8, kCT, 3>(smem, stage_off, pitch, a0, sstep, tab, tab_n, ih, iw,
                                                                            nw, nh, y0, dstf, dstu, ct, G)
                                : area4_strips<kWriteF32, kWriteU8, kCT, 4>(smem, stage_off, pitch, a0, sstep, tab, tab_n, ih, iw,
                                                                            nw, nh, y0, dstf, dstu, ct, G);
-#endif
         if (bad) redo[ci] = 1;  // a table entry with more than 4 taps: the generic kernel redoes the crop
         __syncwarp();
         if (lane == 0) mbar_arrive(&s_empty[s]);

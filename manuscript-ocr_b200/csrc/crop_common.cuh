@@ -5,25 +5,6 @@
 
 namespace {
 
-// store policy of the batch writes (experiment switch): 0 = evict-first streaming stores, 1 = default, 2 = write-through
-#ifndef MS_CROP_STORE
-#define MS_CROP_STORE 0
-#endif
-template <class T>
-__device__ __forceinline__ void ms_store(T *p, const T &v)
-{
-#if MS_CROP_STORE == 0
-    __stcs(p, v);
-#elif MS_CROP_STORE == 1
-    *p = v;
-#else
-    __stwt(p, v);
-#endif
-}
-
-#ifndef MS_CROP_WAIT_NS
-#define MS_CROP_WAIT_NS 100u
-#endif
 // ---- mbarrier + TMA bulk copy (sm_90+ PTX; SASS: SYNCS / UBLKCP) ----------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -37,8 +18,8 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes)
 }
 __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity)
 {
-    // A failed try sleeps before the next one: a waiting warp that retries every few tens of cycles takes issue slots
-    // from the warps that do the arithmetic (r2c capture: a quarter of all executed instructions were retries).
+    // A failed try sleeps (100 ns) before the next one: a waiting warp that retries every few tens of cycles takes issue
+    // slots from the warps that do the arithmetic (r2c capture: a quarter of all executed instructions were retries).
     asm volatile(
         "{\n"
         ".reg .pred p;\n"
@@ -50,7 +31,7 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity)
         "@!p bra WAIT_%=;\n"
         "DONE_%=:\n"
         "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity), "r"(MS_CROP_WAIT_NS)
+        "r"(parity), "r"(100u)
         : "memory");
 }
 __device__ __forceinline__ void tma_bulk_g2s(void *dst_smem, const void *src_gmem, uint32_t bytes, uint64_t *bar)
@@ -297,7 +278,7 @@ __device__ __forceinline__ void resample_px(const Plan &p, int dx, int dy, const
 // as constant 16-byte streaming stores by `nthreads` cooperating threads.
 template <bool kWriteF32, bool kWriteU8>
 __device__ __forceinline__ void write_padding(int nw, int nh, int y0, int ih, int iw, float *dstf, uint8_t *dstu,
-                                              int vec_ok, int tid, int nthreads, int c_begin = 0, int c_end = 3)
+                                              int vec_ok, int tid, int nthreads)
 {
     const int plane = ih * iw;
     if (kWriteF32) {
@@ -312,9 +293,9 @@ __device__ __forceinline__ void write_padding(int nw, int nh, int y0, int ih, in
             float4 *bot = reinterpret_cast<float4 *>(dstf + (size_t)(y0 + nh) * iw);
             const int plane4 = plane / 4;
             for (int i = tid; i < top4; i += nthreads)
-                for (int c = c_begin; c < c_end; c++) ms_store(top + (size_t)c * plane4 + i, one4);
+                for (int c = 0; c < 3; c++) __stcs(top + (size_t)c * plane4 + i, one4);
             for (int i = tid; i < bot4; i += nthreads)
-                for (int c = c_begin; c < c_end; c++) ms_store(bot + (size_t)c * plane4 + i, one4);
+                for (int c = 0; c < 3; c++) __stcs(bot + (size_t)c * plane4 + i, one4);
             if (tail4 > 0) {
                 // right of the pasted rectangle: a thread owns one 16-byte column (and, when the tail is narrower than
                 // the thread count, one of `split` row phases) and walks down the rows -- per row one pointer
@@ -328,7 +309,7 @@ __device__ __forceinline__ void write_padding(int nw, int nh, int y0, int ih, in
                     for (int k = col; k < tail4; k += nthreads) {  // (tails wider than the thread count: several columns)
                         float4 *p4 = at + (k - col);
                         for (int r = phase; r < nh; r += split, p4 += step)
-                            for (int c = c_begin; c < c_end; c++) ms_store(p4 + (size_t)c * plane4, one4);
+                            for (int c = 0; c < 3; c++) __stcs(p4 + (size_t)c * plane4, one4);
                     }
                 }
             }
@@ -336,18 +317,18 @@ __device__ __forceinline__ void write_padding(int nw, int nh, int y0, int ih, in
                 for (int i = tid; i < nh * fr; i += nthreads) {
                     const int r = i / fr, k = i - r * fr;
                     float *at = dstf + (size_t)(y0 + r) * iw + nw + k;
-                    for (int c = c_begin; c < c_end; c++) ms_store(at + (size_t)c * plane, one);
+                    for (int c = 0; c < 3; c++) __stcs(at + (size_t)c * plane, one);
                 }
             }
         } else {
-            for (int e = c_begin * plane + tid; e < c_end * plane; e += nthreads) {
+            for (int e = tid; e < 3 * plane; e += nthreads) {
                 int c = e / plane, rem = e - c * plane;
                 int y = rem / iw, x = rem - y * iw;
                 if (!(y >= y0 && y < y0 + nh && x < nw)) dstf[e] = one;
             }
         }
     }
-    if (kWriteU8 && c_begin == 0) {
+    if (kWriteU8) {
         for (int e = tid; e < plane; e += nthreads) {
             int y = e / iw, x = e - y * iw;
             if (!(y >= y0 && y < y0 + nh && x < nw)) {
@@ -361,10 +342,10 @@ __device__ __forceinline__ void write_padding(int nw, int nh, int y0, int ih, in
 
 template <bool kWriteF32, bool kWriteU8>
 __device__ __forceinline__ void write_padding(const Plan &p, int ih, int iw, float *dstf, uint8_t *dstu, int vec_ok,
-                                              int tid, int nthreads, int c_begin = 0, int c_end = 3)
+                                              int tid, int nthreads)
 {
     write_padding<kWriteF32, kWriteU8>(p.ok ? p.nw : 0, p.ok ? p.nh : 0, p.ok ? p.y0 : 0, ih, iw, dstf, dstu, vec_ok, tid,
-                                       nthreads, c_begin, c_end);
+                                       nthreads);
 }
 
 // u8 -> f32 without the conversion pipe: byte k of `v` is spliced under the exponent of 2^23, then 2^23 is
@@ -418,20 +399,15 @@ __device__ __forceinline__ unsigned long long bytes2_f32(uint32_t va, uint32_t s
     return f2_add(f2_pack_bits(__byte_perm(va, 0x4B000000u, sa), __byte_perm(vb, 0x4B000000u, sb)), magic);
 }
 
-#ifndef MS_CROP_PACKED
-#define MS_CROP_PACKED 1
-#endif
-
 template <int kTaps>
 __device__ __forceinline__ void hrow_area4(const unsigned char *smem_base, uint32_t o, const float4 wx, float &b0,
                                            float &b1, float &b2)
 {
-#if MS_CROP_PACKED
-    const uint32_t *smem32p = reinterpret_cast<const uint32_t *>(smem_base);
-    const uint32_t wip = o >> 2, shp = (o & 3u) * 8u;
-    const uint32_t q0 = smem32p[wip], q1 = smem32p[wip + 1], q2 = smem32p[wip + 2];
-    const uint32_t q3 = kTaps > 3 ? smem32p[wip + 3] : 0u;
-    const uint32_t u0 = __funnelshift_r(q0, q1, shp), u1 = __funnelshift_r(q1, q2, shp), u2 = __funnelshift_r(q2, q3, shp);
+    const uint32_t *smem32 = reinterpret_cast<const uint32_t *>(smem_base);
+    const uint32_t wi = o >> 2, sh = (o & 3u) * 8u;
+    const uint32_t q0 = smem32[wi], q1 = smem32[wi + 1], q2 = smem32[wi + 2];
+    const uint32_t q3 = kTaps > 3 ? smem32[wi + 3] : 0u;
+    const uint32_t u0 = __funnelshift_r(q0, q1, sh), u1 = __funnelshift_r(q1, q2, sh), u2 = __funnelshift_r(q2, q3, sh);
     // bytes: tap0 = u0.b0..b2, tap1 = u0.b3 u1.b0 u1.b1, tap2 = u1.b2 u1.b3 u2.b0, tap3 = u2.b1..b3
     float p00, p01, p02, p10, p11, p12, p20, p21, p22;
     f2_unpack(f2_mul(bytes2_f32(u0, 0x7650, u0, 0x7651), f2_pack(wx.x, wx.x)), p00, p01);  // tap 0: channels 0, 1
@@ -451,28 +427,6 @@ __device__ __forceinline__ void hrow_area4(const unsigned char *smem_base, uint3
         b1 = (p01 + p11) + p21;
         b2 = (p02 + p12) + p22;
     }
-    return;
-#endif
-    const uint32_t *smem32 = reinterpret_cast<const uint32_t *>(smem_base);
-    const uint32_t wi = o >> 2, sh = (o & 3u) * 8u;
-    const uint32_t w0 = smem32[wi], w1 = smem32[wi + 1], w2 = smem32[wi + 2];
-    const uint32_t w3 = kTaps > 3 ? smem32[wi + 3] : 0u;
-    const uint32_t v0 = __funnelshift_r(w0, w1, sh), v1 = __funnelshift_r(w1, w2, sh), v2 = __funnelshift_r(w2, w3, sh);
-    // bytes: tap0 = v0.b0..b2, tap1 = v0.b3 v1.b0 v1.b1, tap2 = v1.b2 v1.b3 v2.b0, tap3 = v2.b1..b3
-    b0 = byte_f32(v0, 0x7650) * wx.x;
-    b1 = byte_f32(v0, 0x7651) * wx.x;
-    b2 = byte_f32(v0, 0x7652) * wx.x;
-    b0 = b0 + byte_f32(v0, 0x7653) * wx.y;
-    b1 = b1 + byte_f32(v1, 0x7650) * wx.y;
-    b2 = b2 + byte_f32(v1, 0x7651) * wx.y;
-    b0 = b0 + byte_f32(v1, 0x7652) * wx.z;
-    b1 = b1 + byte_f32(v1, 0x7653) * wx.z;
-    b2 = b2 + byte_f32(v2, 0x7650) * wx.z;
-    if (kTaps > 3) {
-        b0 = b0 + byte_f32(v2, 0x7651) * wx.w;
-        b1 = b1 + byte_f32(v2, 0x7652) * wx.w;
-        b2 = b2 + byte_f32(v2, 0x7653) * wx.w;
-    }
 }
 
 // words of one crop's table set: x entries as five arrays of iw words, y entries as ih records of 8 words
@@ -483,11 +437,8 @@ __host__ __device__ inline int area_tab_words(int ih, int iw) { return area_tab_
 // consecutive columns): tab[0][i] = s0 | n << 16, tab[1..4][i] = tap weights (0 beyond n), i in [0, iw).  y entries,
 // array of 8-word records after them (a thread walks down the rows: one 16-byte load for the four weights):
 // ytab[d] = {s0 | n << 16, -, -, -, w0, w1, w2, w3} at word area_tab_ybase(iw) + 8 * d (weights 16-byte aligned).
-// (older description follows)
-// The INTER_AREA coefficient tables of one crop for the 4-tap path, structure of arrays:
-// tab[0][i] = s0 | n << 16, tab[1..4][i] = tap weights (0 beyond n); x entries occupy [0, iw), y entries
-// [iw, iw + ih) of every array.  Plan::fast guarantees n <= 4; an entry that violates it is stored with n = 0xffff
-// and makes the consumers hand the crop to the generic kernel.
+// Plan::fast guarantees n <= 4; an entry that violates it is stored with n = 0xffff and makes the consumers hand the
+// crop to the generic kernel.
 // Returns whether every x entry built by this thread has at most 3 taps (the caller combines the threads' answers).
 __device__ __forceinline__ bool build_tables(const Plan &p, uint32_t *tab, int tab_n, int iw, int tid,
                                              int nthreads = 32)
@@ -564,9 +515,9 @@ __device__ __forceinline__ void area2x2_pixels(const unsigned char *smem, uint32
         const int o0 = (s0 + 2) >> 2, o1 = (s1 + 2) >> 2, o2 = (s2 + 2) >> 2;
         const int at = (y0 + dy) * iw + dx;
         if (kWriteF32) {
-            ms_store(dstf + at, ((float)o0 - 127.5f) * inv);
-            ms_store(dstf + plane + at, ((float)o1 - 127.5f) * inv);
-            ms_store(dstf + 2 * plane + at, ((float)o2 - 127.5f) * inv);
+            __stcs(dstf + at, ((float)o0 - 127.5f) * inv);
+            __stcs(dstf + plane + at, ((float)o1 - 127.5f) * inv);
+            __stcs(dstf + 2 * plane + at, ((float)o2 - 127.5f) * inv);
         }
         if (kWriteU8) {
             dstu[(size_t)at * 3] = (unsigned char)o0;
@@ -635,9 +586,9 @@ __device__ __forceinline__ bool area4_strips(const unsigned char *smem, uint32_t
             const float f0 = rintf(sum0), f1 = rintf(sum1), f2 = rintf(sum2);
             const int at = (y0 + dy) * iw + dx;
             if (kWriteF32) {
-                ms_store(orow, (f0 - 127.5f) * inv);
-                ms_store(orow + plane, (f1 - 127.5f) * inv);
-                ms_store(orow + 2 * plane, (f2 - 127.5f) * inv);
+                __stcs(orow, (f0 - 127.5f) * inv);
+                __stcs(orow + plane, (f1 - 127.5f) * inv);
+                __stcs(orow + 2 * plane, (f2 - 127.5f) * inv);
                 orow += iw;
             }
             if (kWriteU8) {

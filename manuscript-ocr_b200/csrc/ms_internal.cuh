@@ -104,17 +104,7 @@ int ms_stage_reserve(ms_ctx *ctx, size_t bytes);
 // (griddepcontrol.wait: returns when the preceding grid has completed and its writes are visible) before it touches
 // memory, which makes the chain transitive and the results those of plain stream order.  MS_B200_NO_PDL=1: plain launches.
 #if defined(__CUDACC__)
-#ifndef MS_PDL_EARLY_TRIGGER
-#define MS_PDL_EARLY_TRIGGER 0
-#endif
-__device__ __forceinline__ void ms_pdl_wait()
-{
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-#if MS_PDL_EARLY_TRIGGER
-    // let the NEXT kernel's CTAs become resident while this one runs (they wait for this grid's completion themselves)
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
+__device__ __forceinline__ void ms_pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 inline bool ms_pdl_enabled()
 {

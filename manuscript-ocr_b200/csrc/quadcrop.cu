@@ -644,7 +644,7 @@ __global__ void __launch_bounds__(kQsThreads, 2)
             __syncwarp();
             if (lane == 0) mbar_arrive(&s_full[s]);
             write_padding<kWriteF32, kWriteU8>(p.nw, p.nh, p.y0, ih, iw, kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr,
-                                               kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr, vec_ok, lane, 32, 0, 3);
+                                               kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr, vec_ok, lane, 32);
         }
         return;
     }
