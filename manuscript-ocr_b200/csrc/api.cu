@@ -290,12 +290,6 @@ thread_local ms_ctx *ms_ctx_guard::t_inside = nullptr;
     }                                                        \
     MS_CUDA(cudaSetDevice((ctx)->device))
 
-#define MS_TRY(expr)                 \
-    do {                             \
-        int _r = (expr);             \
-        if (_r != MS_OK) return _r;  \
-    } while (0)
-
 static int flags_to_rc(int32_t f, const char *where)
 {
     if (f & MS_FLAG_INDEX_ERROR) {

@@ -20,14 +20,12 @@
 //                           staging decision -> Plan
 //   crop_resize_pad_kernel  the crops with Plan::fast (INTER_AREA with shrink factors below 3 -- what shrinking a
 //                           word box to a 32- or 64-pixel-high canvas gives): persistent, warp specialised, 4 CTAs
-//                           of 7 warps per SM.  Warp 0 (copy warp) stages the next crop's source rows with TMA bulk
-//                           copies (cp.async.bulk global->shared, one 16-byte-aligned span per row, completion on an
-//                           mbarrier) into a byte-granular staging ring; warp 1 (table warp) builds OpenCV's coefficient
-//                           tables in shared memory (structure of arrays) and writes the 255-padding as constant
-//                           16-byte streaming stores; warps 2..6 (consumers) resample column strips out of shared
-//                           memory (aligned 32-bit loads + funnel shift + PRMT u8->f32, 3 or 4 taps) and store
-//                           normalised pixels straight into the CHW batch.  full / empty mbarriers, no CTA-wide
-//                           barrier in the loop.
+//                           of 7 warps per SM.  Warp 0 is the staging-ring copy warp of crop_common.cuh (the crop's
+//                           source rows by TMA bulk copies); warp 1 (table warp) builds OpenCV's coefficient tables in
+//                           shared memory (structure of arrays) and writes the 255-padding as constant 16-byte
+//                           streaming stores; warps 2..6 (consumers) resample column strips out of shared memory
+//                           (aligned 32-bit loads + funnel shift + PRMT u8->f32, 3 or 4 taps) and store normalised
+//                           pixels straight into the CHW batch.
 //   crop_generic_kernel     every other crop (copy, INTER_LINEAR upscale, integer-ratio or long-table INTER_AREA,
 //                           rows too long for the stage): one CTA per crop from global memory, same arithmetic.
 #include "crop_common.cuh"
@@ -48,18 +46,12 @@ __device__ __forceinline__ void make_plan(const int32_t *cr, int n_pages, int im
                                           const uint8_t *pages, const uint8_t *const *page_ptrs,
                                           const int32_t *page_hw, Plan &p)
 {
+    plan_reset(p);
     p.page = cr[0];
     p.x1 = cr[1];
     p.y1 = cr[2];
     p.w = cr[3] - cr[1];
     p.h = cr[4] - cr[2];
-    p.staged = 0;
-    p.fast = 0;
-    p.pitch = 0;
-    p.stride = 0;
-    p.src = nullptr;
-    p.nw = p.nh = p.y0 = p.interp = p.isx = p.isy = 0;
-    p.scale_x = p.scale_y = 1.0;
     p.ok = p.page >= 0 && p.page < n_pages;
     if (!p.ok) return;
     const int H = page_ptrs ? page_hw[2 * p.page] : img_h, W = page_ptrs ? page_hw[2 * p.page + 1] : img_w;
@@ -195,25 +187,14 @@ __global__ void __launch_bounds__(1024) crop_bucket_scan_kernel(int32_t *__restr
     if (threadIdx.x == 0) *n_work = s_carry;
 }
 
-// What the copy warp of the persistent kernel needs of a crop, in work-list order (32 bytes, one broadcast load).
-struct __align__(16) CopyDesc {
-    const uint8_t *src;  // first source byte of the crop
-    int stride;          // bytes between source rows
-    int pitch;           // bytes between staged rows
-    int wh;              // crop size in pixels: w | h << 16 (both < 65536 for a fast crop)
-    int nwh;             // pasted size: nw | nh << 16
-    int ci;              // crop index (output slot)
-    int y0;              // first canvas row of the pasted rectangle
-};
-
-// work[cursor of the crop's bucket ++] = the crop's copy descriptor (order inside a bucket is arbitrary: it only shapes
-// the schedule)
+// work[cursor of the crop's bucket ++] = the crop's staging descriptor (order inside a bucket is arbitrary: it only
+// shapes the schedule)
 __global__ void __launch_bounds__(256) crop_bucket_scatter_kernel(const Plan *__restrict__ plans,
                                                                   const int32_t *__restrict__ page_hw, int n_pages,
                                                                   int img_h, int img_w,
                                                                   const int32_t *__restrict__ n_crops_dev,
                                                                   const int32_t *__restrict__ range, int64_t crops_cap,
-                                                                  int32_t *__restrict__ cursors, CopyDesc *__restrict__ work)
+                                                                  int32_t *__restrict__ cursors, StageDesc *__restrict__ work)
 {
     ms_pdl_wait();
     int64_t begin = range ? range[0] : 0;
@@ -223,31 +204,21 @@ __global__ void __launch_bounds__(256) crop_bucket_scatter_kernel(const Plan *__
          i += (int64_t)gridDim.x * blockDim.x) {
         const Plan p = plans[i];
         if (p.fast) {
-            CopyDesc d;
+            StageDesc d;
             d.src = p.src;
             d.stride = p.stride;
             d.pitch = p.pitch;
-            d.wh = p.w | (p.h << 16);
-            d.nwh = p.nw | (p.nh << 16);
+            d.row_bytes = 3 * p.w;
+            d.rows = p.h;
             d.ci = (int)i;
-            d.y0 = p.y0;
             work[atomicAdd(&cursors[crop_bucket(p, page_hw, img_h, img_w, n_pages)], 1)] = d;
         }
     }
 }
 
-// Warp-specialised persistent kernel for the crops with Plan::fast.  Two producer warps run ahead of the consumers:
-// warp 0 (copy warp) takes the next crop of the work list (a global ticket counter: a CTA that drew narrow words simply
-// draws more of them), reserves the crop's bytes in the CTA's staging RING, tells the table warp which crop it is and
-// issues the TMA row copies; warp 1 (table warp) builds the axis tables, signals, and then writes the crop's padding
-// (which nobody waits for).  Up to kSlots crops are in flight per CTA; a slot owns its metadata and tables, its source
-// rows take exactly the bytes they need from the ring (a narrow word does not hold a 24 KB stage), so the producers
-// can be several crops ahead of the consumers and the differences between crops average out.  full[s] completes when
-// both producers have arrived and the copied bytes have landed.  Warps 2..6 (consumers) wait on full[s], resample the
-// pasted rectangle straight into the CHW batch and release the slot (and its ring bytes) on empty[s].  No CTA-wide
-// barrier inside the loop.  History (profiles/README.md): with two fixed 24 KB stages the consumers waited on `full`
-// 24 % of their time and the copy warp on `empty` 33 % of its -- producer and consumer periods are equal on average,
-// so a two-deep pipeline stalls on every fluctuation.
+// Warp-specialised persistent kernel for the crops with Plan::fast, fed by the staging ring of crop_common.cuh.  Warp 0
+// is its copy warp; warp 1 (table warp) builds the crop's axis tables, signals, and then writes the crop's padding
+// (which nobody waits for); warps 2..6 (consumers) resample the pasted rectangle straight into the CHW batch.
 // Each consumer thread resamples a column strip (one destination column, G consecutive destination rows): with a
 // shrink factor near 2 neighbouring destination rows share their boundary source row, so a strip needs ~(2G + 1)
 // horizontal row sums instead of 3G; per-pixel arithmetic and its order are unchanged.
@@ -256,7 +227,7 @@ constexpr int kConsumerWarps = kThreads / 32 - kProducerWarps;
 
 template <bool kWriteF32, bool kWriteU8>
 __global__ void __launch_bounds__(kThreads, kCtasPerSm)
-    crop_resize_pad_kernel(const Plan *__restrict__ plans, const CopyDesc *__restrict__ work,
+    crop_resize_pad_kernel(const Plan *__restrict__ plans, const StageDesc *__restrict__ work,
                            const int32_t *__restrict__ n_work_dev, int32_t *__restrict__ ticket, int ring_bytes, int ih,
                            int iw, float *__restrict__ batch, uint8_t *__restrict__ canvas_out, int vec_ok,
                            uint8_t *__restrict__ redo)
@@ -265,148 +236,28 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
     extern __shared__ __align__(128) unsigned char smem[];  // [ring_bytes] staging ring, then kSlots table sets
     const int tab_n = area_tab_words(ih, iw);  // words of one slot's table set
     uint32_t *tabs = reinterpret_cast<uint32_t *>(smem + ring_bytes);  // [kSlots][tab_n]
-    __shared__ __align__(8) uint64_t s_full[kSlots], s_empty[kSlots], s_tick[kSlots];
-    // per slot: the crop (index, -1 = no more crops) and what the consumers need of its plan, so that they never touch
-    // the plan array in global memory
-    __shared__ int s_next[kSlots];    // copy warp -> table warp: crop index of the slot
-    __shared__ int s_off[kSlots];     // copy warp -> consumers: ring offset of the crop's first row
-    __shared__ long long s_ci[kSlots];
+    __shared__ StageSlots<kSlots> s_stage;
+    // per slot: what the consumers need of the crop's plan, so that they never touch the plan array in global memory
     __shared__ int s_meta[kSlots][8];  // nw, nh, y0, pitch, misalignment of row 0, its change per row, <= 3 x taps, strip height
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int plane = ih * iw;
-
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int i = 0; i < kSlots; i++) {
-            mbar_init(&s_full[i], 2);  // the copy warp (with the byte count) and the table warp
-            mbar_init(&s_empty[i], kConsumerWarps);
-            mbar_init(&s_tick[i], 1);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
+    stage_init(s_stage, kConsumerWarps);
 
     if (warp == 0) {
-        // ---------------- copy warp: tickets, ring space, one bulk copy per source row ----------------
-        // Software pipeline: while crop k is being copied, the descriptor of crop k+1 and the ticket of crop k+2 are in
-        // flight, so neither the atomic nor the descriptor load is on the warp's critical path.
-        const int n_work = *n_work_dev;
-        int q_off[kSlots], q_len[kSlots];  // ring intervals of the slots (len 0: free)
-#pragma unroll
-        for (int i = 0; i < kSlots; i++) q_off[i] = q_len[i] = 0;
-        int head = 0;        // where the newest crop ended
-        int oldest = 0;      // first crop (sequence number) whose slot has not been seen released
-        auto load_desc = [&](int t) {
-            CopyDesc d;
-            if (t < n_work) {
-                const uint4 *q = reinterpret_cast<const uint4 *>(work + t);
-                const uint4 a = q[0], b = q[1];
-                d.src = reinterpret_cast<const uint8_t *>(((uint64_t)a.y << 32) | a.x);
-                d.stride = (int)a.z;
-                d.pitch = (int)a.w;
-                d.wh = (int)b.x;
-                d.nwh = (int)b.y;
-                d.ci = (int)b.z;
-                d.y0 = (int)b.w;
-            } else {
-                d.src = nullptr;
-                d.stride = d.pitch = d.wh = d.nwh = d.y0 = 0;
-                d.ci = -1;
-            }
-            return d;
-        };
-        int t1 = 0;
-        if (lane == 0) t1 = atomicAdd(ticket, 1);
-        CopyDesc cur = load_desc(__shfl_sync(0xffffffffu, t1, 0));
-        if (lane == 0) t1 = atomicAdd(ticket, 1);  // ticket of crop 1
-        for (int k = 0;; k++) {
-            const int s = k % kSlots;
-            const CopyDesc nxt = load_desc(__shfl_sync(0xffffffffu, t1, 0));  // crop k+1: lands during this crop's copies
-            if (lane == 0 && cur.ci >= 0) t1 = atomicAdd(ticket, 1);           // ticket of crop k+2
-            // the slot's previous crop (k - kSlots) must be done before its metadata / tables are reused
-            while (oldest + kSlots <= k) {
-                mbar_wait(&s_empty[oldest % kSlots], (uint32_t)((oldest / kSlots) & 1));
-                q_len[oldest % kSlots] = 0;
-                oldest++;
-            }
-            if (cur.ci < 0) {  // no more crops: tell the table warp, which tells the consumers
-                if (lane == 0) {
-                    s_next[s] = -1;
-                    mbar_arrive(&s_tick[s]);
-                    mbar_arrive(&s_full[s]);
-                }
-                break;
-            }
-            const int cw = cur.wh & 0xffff, chh = (int)((uint32_t)cur.wh >> 16);
-            const int need = (cur.pitch * chh + 16 + 127) & ~127;
-            int off;
-            for (;;) {  // first fit at `head`, else at 0; else wait for the oldest crop in flight
-                auto free_at = [&](int c) {
-                    bool ok = c + need <= ring_bytes;
-#pragma unroll
-                    for (int i = 0; i < kSlots; i++) ok = ok && (q_len[i] == 0 || c + need <= q_off[i] || q_off[i] + q_len[i] <= c);
-                    return ok;
-                };
-                if (free_at(head)) {
-                    off = head;
-                    break;
-                }
-                if (free_at(0)) {
-                    off = 0;
-                    break;
-                }
-                // oldest < k here: with nothing in flight the whole ring is free and `need` fits by construction
-                mbar_wait(&s_empty[oldest % kSlots], (uint32_t)((oldest / kSlots) & 1));
-                q_len[oldest % kSlots] = 0;
-                oldest++;
-            }
-            q_off[s] = off;
-            q_len[s] = need;
-            head = off + need;
-            if (lane == 0) {
-                s_next[s] = cur.ci;
-                s_off[s] = off;
-                mbar_arrive(&s_tick[s]);  // release: the table warp and (through full) the consumers see both
-            }
-            uint32_t bytes = 0;
-            {
-                const uint8_t *src = cur.src;
-                const size_t stride = (size_t)cur.stride;
-                unsigned char *buf = smem + off;
-                for (int r = lane; r < chh; r += 32) {
-                    const uint8_t *g = src + (size_t)r * stride;
-                    const uint32_t a = (uint32_t)(reinterpret_cast<uintptr_t>(g) & 15);
-                    const uint32_t sz = (a + (uint32_t)cw * 3 + 15) & ~15u;
-                    tma_bulk_g2s(buf + (size_t)r * cur.pitch, g - a, sz, &s_full[s]);
-                    bytes += sz;
-                }
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) bytes += __shfl_xor_sync(0xffffffffu, bytes, o);
-            }
-            if (lane == 0) mbar_expect_tx(&s_full[s], bytes);
-            cur = nxt;
-        }
+        stage_copy_warp(s_stage, smem, ring_bytes, work, *n_work_dev, ticket);
         return;
     }
     if (warp == 1) {
         // ---------------- table warp: OpenCV's axis tables, then all of the padding ----------------
         for (int k = 0;; k++) {
             const int s = k % kSlots;
-            mbar_wait(&s_tick[s], (uint32_t)((k / kSlots) & 1));
-            const int ci = s_next[s];
-            if (ci < 0) {
-                if (lane == 0) {
-                    s_ci[s] = -1;
-                    mbar_arrive(&s_full[s]);
-                }
-                break;
-            }
+            const int ci = stage_wait_tick(s_stage, k);
+            if (ci < 0) break;
             const Plan p = plans[ci];
             const bool two = p.interp == 2;  // exact 2 x 2 ratio: no tables
             const bool x3 = two || __all_sync(0xffffffffu, build_tables(p, tabs + (size_t)s * tab_n, tab_n, iw, lane));
             if (lane == 0) {
-                s_ci[s] = ci;
                 s_meta[s][0] = p.nw;
                 s_meta[s][1] = p.nh;
                 s_meta[s][2] = p.y0;
@@ -417,7 +268,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
                 s_meta[s][7] = strip_height<kConsumerWarps * 32>(p.nw, p.nh);
             }
             __syncwarp();  // every lane's table stores are ordered before lane 0's releasing arrive
-            if (lane == 0) mbar_arrive(&s_full[s]);
+            if (lane == 0) mbar_arrive(&s_stage.full[s]);
             write_padding<kWriteF32, kWriteU8>(p.nw, p.nh, p.y0, ih, iw, kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr,
                                                kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr, vec_ok, lane, 32);
         }
@@ -429,13 +280,12 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
     constexpr int kCT = kConsumerWarps * 32;
     for (int k = 0;; k++) {
         const int s = k % kSlots;
-        mbar_wait(&s_full[s], (uint32_t)((k / kSlots) & 1));
-        const int64_t ci = s_ci[s];
+        const int64_t ci = stage_wait_full(s_stage, k);
         if (ci < 0) break;
         const int nw = s_meta[s][0], nh = s_meta[s][1], y0 = s_meta[s][2];
         const uint32_t pitch = (uint32_t)s_meta[s][3], a0 = (uint32_t)s_meta[s][4], sstep = (uint32_t)s_meta[s][5];
         const int G = s_meta[s][7];
-        const uint32_t stage_off = (uint32_t)s_off[s];
+        const uint32_t stage_off = (uint32_t)s_stage.off[s];
         float *dstf = kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr;
         uint8_t *dstu = kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr;
         const uint32_t *tab = tabs + (size_t)s * tab_n;
@@ -455,8 +305,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
                                : area4_strips<kWriteF32, kWriteU8, kCT, 4>(smem, stage_off, pitch, a0, sstep, tab, tab_n, ih, iw,
                                                                            nw, nh, y0, dstf, dstu, ct, G);
         if (bad) redo[ci] = 1;  // a table entry with more than 4 taps: the generic kernel redoes the crop
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&s_empty[s]);
+        stage_release(s_stage, s);
     }
 }
 
@@ -491,53 +340,21 @@ __global__ void __launch_bounds__(256) crop_generic_kernel(const Plan *__restric
     ms_pdl_wait();
     __shared__ AxisEnt s_tab[kGenericMaxTab];
     const int plane = ih * iw;
-    const float inv = 1.0f / 127.5f;
     const int todo = *list_n;
     for (int li = blockIdx.x; li < todo; li += gridDim.x) {
         const int64_t ci = list[li];
-        const Plan p = plans[ci];
+        Plan p = plans[ci];
+        if (!p.ok) p.nw = p.nh = 0;  // an invalid rectangle pastes nothing: the canvas is all padding
         float *dstf = kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr;
         uint8_t *dstu = kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr;
         write_padding<kWriteF32, kWriteU8>(p, ih, iw, dstf, dstu, vec_ok, threadIdx.x, blockDim.x);
-        const int nw = p.ok ? p.nw : 0, nh = p.ok ? p.nh : 0;
         const bool need_tab = p.ok && (p.interp == 1 || p.interp == 3);
-        const bool tab_ok = need_tab && nw + nh <= kGenericMaxTab;
+        const bool tab_ok = need_tab && p.nw + p.nh <= kGenericMaxTab;
         __syncthreads();  // the previous crop's table is no longer read
-        if (tab_ok) {
-            for (int t = threadIdx.x; t < nw + nh; t += blockDim.x) {
-                const bool isx = t < nw;
-                const int d = isx ? t : t - nw;
-                s_tab[t] = p.interp == 3 ? (isx ? area_entry(d, p.scale_x, p.w) : area_entry(d, p.scale_y, p.h))
-                                         : (isx ? linear_entry_x(d, p.scale_x, p.w) : linear_entry_y(d, p.scale_y, p.h));
-            }
-        }
+        if (tab_ok) fill_axis_table(p, s_tab);
         __syncthreads();
-        const PitchedSrc gsrc{p.src, (size_t)p.stride};
-        const int npx = nw * nh;
-        for (int t = threadIdx.x; t < npx; t += blockDim.x) {
-            const int dy = t / nw, dx = t - dy * nw;
-            AxisEnt ex = {}, ey = {};
-            if (tab_ok) {
-                ex = s_tab[dx];
-                ey = s_tab[nw + dy];
-            } else if (need_tab) {
-                ex = p.interp == 3 ? area_entry(dx, p.scale_x, p.w) : linear_entry_x(dx, p.scale_x, p.w);
-                ey = p.interp == 3 ? area_entry(dy, p.scale_y, p.h) : linear_entry_y(dy, p.scale_y, p.h);
-            }
-            unsigned char o0, o1, o2;
-            resample_px(p, dx, dy, gsrc, ex, ey, o0, o1, o2);
-            const int at = (p.y0 + dy) * iw + dx;
-            if (kWriteF32) {
-                dstf[at] = ((float)o0 - 127.5f) * inv;
-                dstf[plane + at] = ((float)o1 - 127.5f) * inv;
-                dstf[2 * plane + at] = ((float)o2 - 127.5f) * inv;
-            }
-            if (kWriteU8) {
-                dstu[(size_t)at * 3] = o0;
-                dstu[(size_t)at * 3 + 1] = o1;
-                dstu[(size_t)at * 3 + 2] = o2;
-            }
-        }
+        resample_canvas<kWriteF32, kWriteU8>(p, PitchedSrc{p.src, (size_t)p.stride}, s_tab, tab_ok, need_tab, ih, iw, dstf,
+                                             dstu);
     }
 }
 
@@ -608,7 +425,7 @@ static size_t crop_bucket_count(int n_pages)
 size_t msk_crop_scratch(int64_t crops_cap, int n_pages)
 {
     const size_t n = (size_t)(crops_cap > 0 ? crops_cap : 0);
-    return n * sizeof(Plan) + n + n * sizeof(int32_t) + n * sizeof(CopyDesc) + crop_bucket_count(n_pages) * sizeof(int32_t) + 8192;
+    return n * sizeof(Plan) + n + n * sizeof(int32_t) + n * sizeof(StageDesc) + crop_bucket_count(n_pages) * sizeof(int32_t) + 8192;
 }
 
 int msk_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w, const int32_t *crops,
@@ -642,7 +459,7 @@ int msk_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_
     Plan *plans = bump.take<Plan>((size_t)crops_cap);
     uint8_t *redo = bump.take<uint8_t>((size_t)crops_cap);
     int32_t *glist = bump.take<int32_t>((size_t)crops_cap);
-    CopyDesc *work = bump.take<CopyDesc>((size_t)crops_cap);
+    StageDesc *work = bump.take<StageDesc>((size_t)crops_cap);
     int32_t *hist = bump.take<int32_t>((size_t)n_buckets);
     int32_t *cnt = bump.take<int32_t>(4);  // generic-list length, fast-crop count, ticket counter
     if (!plans || !redo || !cnt) {
@@ -669,30 +486,18 @@ int msk_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_
     int64_t ggrid = (int64_t)ctx->num_sms * 8;
     if (ggrid > crops_cap) ggrid = crops_cap;
     const int vec_ok = ((out_w & 3) == 0 && (reinterpret_cast<uintptr_t>(batch_f32) & 15) == 0) ? 1 : 0;
-    // cudaFuncSetAttribute is a synchronous driver call (milliseconds): once per context and kernel, not per launch
-#define MS_CROP_LAUNCH(F32, U8)                                                                                        \
-    do {                                                                                                               \
-        auto kfn = crop_resize_pad_kernel<F32, U8>;                                                                    \
-        int &granted = ctx->smem_attr[(F32 ? 1 : 0) + (U8 ? 2 : 0) - 1];                                               \
-        if ((int)smem > granted) {                                                                                     \
-            MS_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                \
-            granted = (int)smem;                                                                                       \
-        }                                                                                                              \
-        ms_launch(kfn, (int)grid, kThreads, smem, st, plans, work, n_work, ticket, (int)ring, out_h, out_w, batch_f32,      \
-                                              canvas_u8, vec_ok, redo);                                               \
-        MS_LAUNCH_CHECK(ctx);                                                                                          \
-        ms_launch(crop_generic_list_kernel, (int)lgrid, 256, 0, st, plans, n_crops, range, crops_cap, redo, glist, glist_n);  \
-        MS_LAUNCH_CHECK(ctx);                                                                                          \
-        ms_launch(crop_generic_kernel<F32, U8>, (int)ggrid, 256, 0, st, plans, glist, glist_n, out_h,                        \
-                                                                 out_w, batch_f32, canvas_u8, vec_ok);                \
-    } while (0)
-    if (batch_f32 && canvas_u8)
-        MS_CROP_LAUNCH(true, true);
-    else if (batch_f32)
-        MS_CROP_LAUNCH(true, false);
-    else
-        MS_CROP_LAUNCH(false, true);
-#undef MS_CROP_LAUNCH
-    MS_LAUNCH_CHECK(ctx);
-    return MS_OK;
+    return launch_for_outputs(batch_f32, canvas_u8, [&](auto f32, auto u8) {
+        constexpr bool kF32 = decltype(f32)::value, kU8 = decltype(u8)::value;
+        constexpr ms_smem_slot slot = kF32 ? (kU8 ? MS_SMEM_CROP_BOTH : MS_SMEM_CROP_F32) : MS_SMEM_CROP_U8;
+        MS_TRY(ms_allow_smem(ctx, slot, crop_resize_pad_kernel<kF32, kU8>, (int)smem));
+        ms_launch(crop_resize_pad_kernel<kF32, kU8>, (int)grid, kThreads, smem, st, plans, work, n_work, ticket, (int)ring,
+                  out_h, out_w, batch_f32, canvas_u8, vec_ok, redo);
+        MS_LAUNCH_CHECK(ctx);
+        ms_launch(crop_generic_list_kernel, (int)lgrid, 256, 0, st, plans, n_crops, range, crops_cap, redo, glist, glist_n);
+        MS_LAUNCH_CHECK(ctx);
+        ms_launch(crop_generic_kernel<kF32, kU8>, (int)ggrid, 256, 0, st, plans, glist, glist_n, out_h, out_w, batch_f32,
+                  canvas_u8, vec_ok);
+        MS_LAUNCH_CHECK(ctx);
+        return MS_OK;
+    });
 }

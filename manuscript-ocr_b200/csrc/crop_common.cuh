@@ -1,6 +1,9 @@
-// Shared by crop.cu and quadcrop.cu: the resize-and-pad plan of one crop, OpenCV's coefficient-table entries and the
-// per-pixel resampling arithmetic (cv2.resize restated, see crop.cu), and the 255-padding writer.
+// Shared by crop.cu and quadcrop.cu: the staging ring that feeds their warp-specialised kernels, the resize-and-pad plan
+// of one crop, OpenCV's coefficient-table entries and the per-pixel resampling arithmetic (cv2.resize restated, see
+// crop.cu), and the 255-padding writer.
 #pragma once
+#include <type_traits>
+
 #include "ms_internal.cuh"
 
 namespace {
@@ -46,6 +49,195 @@ __device__ __forceinline__ void mbar_arrive(uint64_t *bar)
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
+// ---- staging ring: the producer of crop_resize_pad_kernel (crop.cu) and quad_crop_staged_kernel (quadcrop.cu) -------
+// Both kernels are persistent and warp specialised, with no CTA-wide barrier in their loop.  Warp 0 (copy warp,
+// stage_copy_warp) takes the next work item from a global ticket counter (a CTA that drew narrow words simply draws more
+// of them), reserves the item's rows in the CTA's staging RING, tells warp 1 (table warp) which item the slot holds and
+// issues one TMA bulk copy per row.  The table warp builds the item's tables and metadata and arrives on `full`; the
+// consumer warps wait on `full`, work out of shared memory and release the slot on `empty`.  Up to kSlots items are in
+// flight per CTA; a slot owns its metadata and tables, its rows take exactly the bytes they need from the ring (a narrow
+// word does not hold a 24 KB stage), so the producers can be several items ahead of the consumers and the differences
+// between items average out.  History (profiles/README.md): with two fixed 24 KB stages the consumers waited on `full`
+// 24 % of their time and the copy warp on `empty` 33 % of its -- producer and consumer periods are equal on average, so
+// a two-deep pipeline stalls on every fluctuation.
+
+// What the copy warp needs of one work item (32 bytes: two 16-byte loads).  Row r is copied as the 16-byte-aligned span
+// that covers [src + r * stride, + row_bytes), to byte r * pitch of the item's ring space.
+struct __align__(16) StageDesc {
+    const uint8_t *src;  // first byte of row 0
+    int stride;          // bytes between source rows
+    int pitch;           // bytes between staged rows (at least the widest span)
+    int row_bytes;       // bytes of one source row
+    int rows;
+    int ci;              // item index (output slot)
+};
+static_assert(sizeof(StageDesc) == 32, "the copy warp loads a descriptor as two uint4");
+
+// Per slot: `tick` completes when the copy warp has filled the slot, `full` when its bytes have landed and the table
+// warp has arrived, `empty` when every consumer warp has released it (and with it its ring bytes).
+template <int kSlots>
+struct StageSlots {
+    uint64_t full[kSlots], empty[kSlots], tick[kSlots];
+    int ci[kSlots];     // item of the slot, -1: no more work (copy warp -> table warp and consumers)
+    int off[kSlots];    // ring offset of the item's row 0
+    int pitch[kSlots];  // bytes between its staged rows
+};
+
+// sequence number k -> slot k % kSlots, which it uses for the (k / kSlots)-th time: the parity of that phase
+template <int kSlots>
+__device__ __forceinline__ uint32_t stage_parity(int k)
+{
+    return (uint32_t)((k / kSlots) & 1);
+}
+
+// called by every thread of the CTA (it ends in __syncthreads)
+template <int kSlots>
+__device__ __forceinline__ void stage_init(StageSlots<kSlots> &ss, int consumer_warps)
+{
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int i = 0; i < kSlots; i++) {
+            mbar_init(&ss.full[i], 2);  // the copy warp (with the byte count) and the table warp
+            mbar_init(&ss.empty[i], consumer_warps);
+            mbar_init(&ss.tick[i], 1);
+        }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+}
+
+// The copy warp: fills slots until the work list is exhausted, then posts the end-of-work sentinel (ci = -1).
+// Software pipeline: while item k is being copied, the descriptor of item k+1 and the ticket of item k+2 are in flight,
+// so neither the atomic nor the descriptor load is on the warp's critical path.  Ring space is allocated first fit at
+// the end of the newest item, else at 0, else after the oldest item in flight has been released.
+template <int kSlots>
+__device__ __forceinline__ void stage_copy_warp(StageSlots<kSlots> &ss, unsigned char *ring, int ring_bytes,
+                                                const StageDesc *__restrict__ work, int n_work, int32_t *ticket)
+{
+    const int lane = threadIdx.x & 31;
+    int q_off[kSlots], q_len[kSlots];  // ring intervals of the slots (len 0: free)
+#pragma unroll
+    for (int i = 0; i < kSlots; i++) q_off[i] = q_len[i] = 0;
+    int head = 0;    // where the newest item ended
+    int oldest = 0;  // first item (sequence number) whose slot has not been seen released
+    auto release_oldest = [&]() {
+        mbar_wait(&ss.empty[oldest % kSlots], stage_parity<kSlots>(oldest));
+        q_len[oldest % kSlots] = 0;
+        oldest++;
+    };
+    auto load_desc = [&](int t) {
+        StageDesc d;
+        if (t < n_work) {
+            const uint4 *q = reinterpret_cast<const uint4 *>(work + t);
+            const uint4 a = q[0], b = q[1];
+            d.src = reinterpret_cast<const uint8_t *>(((uint64_t)a.y << 32) | a.x);
+            d.stride = (int)a.z;
+            d.pitch = (int)a.w;
+            d.row_bytes = (int)b.x;
+            d.rows = (int)b.y;
+            d.ci = (int)b.z;
+        } else {
+            d.src = nullptr;
+            d.stride = d.pitch = d.row_bytes = d.rows = 0;
+            d.ci = -1;
+        }
+        return d;
+    };
+    int t1 = 0;
+    if (lane == 0) t1 = atomicAdd(ticket, 1);
+    StageDesc cur = load_desc(__shfl_sync(0xffffffffu, t1, 0));
+    if (lane == 0) t1 = atomicAdd(ticket, 1);  // ticket of item 1
+    for (int k = 0;; k++) {
+        const int s = k % kSlots;
+        const StageDesc nxt = load_desc(__shfl_sync(0xffffffffu, t1, 0));  // item k+1: lands during this item's copies
+        if (lane == 0 && cur.ci >= 0) t1 = atomicAdd(ticket, 1);            // ticket of item k+2
+        // the slot's previous item (k - kSlots) must be done before its metadata / tables are reused
+        while (oldest + kSlots <= k) release_oldest();
+        if (cur.ci < 0) {  // no more work: tell the table warp, which tells the consumers
+            if (lane == 0) {
+                ss.ci[s] = -1;
+                mbar_arrive(&ss.tick[s]);
+                mbar_arrive(&ss.full[s]);
+            }
+            return;
+        }
+        // 16 bytes of slack after the last row: the consumers' aligned 32-bit reads may run past a row's end
+        const int need = (cur.pitch * cur.rows + 16 + 127) & ~127;
+        int off;
+        for (;;) {
+            auto free_at = [&](int c) {
+                bool ok = c + need <= ring_bytes;
+#pragma unroll
+                for (int i = 0; i < kSlots; i++) ok = ok && (q_len[i] == 0 || c + need <= q_off[i] || q_off[i] + q_len[i] <= c);
+                return ok;
+            };
+            if (free_at(head)) {
+                off = head;
+                break;
+            }
+            if (free_at(0)) {
+                off = 0;
+                break;
+            }
+            // oldest < k here: with nothing in flight the whole ring is free and `need` fits by construction
+            release_oldest();
+        }
+        q_off[s] = off;
+        q_len[s] = need;
+        head = off + need;
+        if (lane == 0) {
+            ss.ci[s] = cur.ci;
+            ss.off[s] = off;
+            ss.pitch[s] = cur.pitch;
+            mbar_arrive(&ss.tick[s]);  // release: the table warp and (through full) the consumers see all three
+        }
+        uint32_t bytes = 0;
+        {
+            const size_t stride = (size_t)cur.stride;
+            unsigned char *buf = ring + off;
+            for (int r = lane; r < cur.rows; r += 32) {
+                const uint8_t *g = cur.src + (size_t)r * stride;
+                const uint32_t a = (uint32_t)(reinterpret_cast<uintptr_t>(g) & 15);
+                const uint32_t sz = (a + (uint32_t)cur.row_bytes + 15) & ~15u;
+                tma_bulk_g2s(buf + (size_t)r * cur.pitch, g - a, sz, &ss.full[s]);
+                bytes += sz;
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) bytes += __shfl_xor_sync(0xffffffffu, bytes, o);
+        }
+        if (lane == 0) mbar_expect_tx(&ss.full[s], bytes);
+        cur = nxt;
+    }
+}
+
+// The table warp: waits until the copy warp has filled slot k % kSlots and returns its item -- or -1, after passing the
+// end-of-work sentinel on to the consumers.  For an item, the table warp arrives on `full` itself when its part is done.
+template <int kSlots>
+__device__ __forceinline__ int stage_wait_tick(StageSlots<kSlots> &ss, int k)
+{
+    const int s = k % kSlots;
+    mbar_wait(&ss.tick[s], stage_parity<kSlots>(k));
+    const int ci = ss.ci[s];
+    if (ci < 0 && (threadIdx.x & 31) == 0) mbar_arrive(&ss.full[s]);
+    return ci;
+}
+
+// A consumer warp: waits until slot k % kSlots is full and returns its item (-1: no more work) ...
+template <int kSlots>
+__device__ __forceinline__ int stage_wait_full(StageSlots<kSlots> &ss, int k)
+{
+    mbar_wait(&ss.full[k % kSlots], stage_parity<kSlots>(k));
+    return ss.ci[k % kSlots];
+}
+
+// ... and hands slot s back when it is done with it
+template <int kSlots>
+__device__ __forceinline__ void stage_release(StageSlots<kSlots> &ss, int s)
+{
+    __syncwarp();
+    if ((threadIdx.x & 31) == 0) mbar_arrive(&ss.empty[s]);
+}
+
 struct Plan {
     int page, x1, y1, w, h;
     int nw, nh, y0;
@@ -59,6 +251,16 @@ struct Plan {
     const uint8_t *src;  // first source byte of the crop (row y1, column x1 of its page)
     double scale_x, scale_y;
 };
+
+// the plan of no crop: not ok, nothing pasted (all padding)
+__device__ __forceinline__ void plan_reset(Plan &p)
+{
+    p.page = p.x1 = p.y1 = p.w = p.h = 0;
+    p.nw = p.nh = p.y0 = p.interp = p.isx = p.isy = 0;
+    p.ok = p.staged = p.fast = p.pitch = p.stride = 0;
+    p.src = nullptr;
+    p.scale_x = p.scale_y = 1.0;
+}
 
 // one destination index of one axis: the OpenCV coefficient table entry
 struct AxisEnt {
@@ -273,6 +475,52 @@ __device__ __forceinline__ void resample_px(const Plan &p, int dx, int dy, const
     }
 }
 
+// The generic per-pixel path, one CTA per crop.  First the crop's coefficient-table entries in shared memory: tab[t] for
+// destination column t < nw, tab[nw + d] for destination row d (INTER_LINEAR or INTER_AREA general) ...
+__device__ __forceinline__ void fill_axis_table(const Plan &p, AxisEnt *tab)
+{
+    for (int t = threadIdx.x; t < p.nw + p.nh; t += blockDim.x) {
+        const bool isx = t < p.nw;
+        const int d = isx ? t : t - p.nw;
+        tab[t] = p.interp == 3 ? (isx ? area_entry(d, p.scale_x, p.w) : area_entry(d, p.scale_y, p.h))
+                               : (isx ? linear_entry_x(d, p.scale_x, p.w) : linear_entry_y(d, p.scale_y, p.h));
+    }
+}
+
+// ... then a thread per pasted pixel, f32 and / or u8 stores.  tab_ok: the entries are in s_tab; otherwise, when the
+// mode needs entries (need_tab), every pixel computes its own.
+template <bool kWriteF32, bool kWriteU8, class Src>
+__device__ __forceinline__ void resample_canvas(const Plan &p, const Src &src, const AxisEnt *s_tab, bool tab_ok,
+                                                bool need_tab, int ih, int iw, float *dstf, uint8_t *dstu)
+{
+    const int plane = ih * iw;
+    const float inv = 1.0f / 127.5f;
+    const int nw = p.nw, nh = p.nh, npx = nw * nh;
+    for (int t = threadIdx.x; t < npx; t += blockDim.x) {
+        const int dy = t / nw, dx = t - dy * nw;
+        AxisEnt ex = {}, ey = {};
+        if (tab_ok) {
+            ex = s_tab[dx];
+            ey = s_tab[nw + dy];
+        } else if (need_tab) {
+            ex = p.interp == 3 ? area_entry(dx, p.scale_x, p.w) : linear_entry_x(dx, p.scale_x, p.w);
+            ey = p.interp == 3 ? area_entry(dy, p.scale_y, p.h) : linear_entry_y(dy, p.scale_y, p.h);
+        }
+        unsigned char o0, o1, o2;
+        resample_px(p, dx, dy, src, ex, ey, o0, o1, o2);
+        const int at = (p.y0 + dy) * iw + dx;
+        if (kWriteF32) {
+            dstf[at] = ((float)o0 - 127.5f) * inv;
+            dstf[plane + at] = ((float)o1 - 127.5f) * inv;
+            dstf[2 * plane + at] = ((float)o2 - 127.5f) * inv;
+        }
+        if (kWriteU8) {
+            dstu[(size_t)at * 3] = o0;
+            dstu[(size_t)at * 3 + 1] = o1;
+            dstu[(size_t)at * 3 + 2] = o2;
+        }
+    }
+}
 
 // Everything outside the pasted rectangle is the 255 canvas (transforms.py:100), 1.0f after normalisation; written
 // as constant 16-byte streaming stores by `nthreads` cooperating threads.
@@ -599,6 +847,16 @@ __device__ __forceinline__ bool area4_strips(const unsigned char *smem, uint32_t
         }
     }
     return bad;
+}
+
+// The crop kernels are instantiated for the outputs they write: <kWriteF32, kWriteU8> = <true, true>, <true, false> or
+// <false, true>.  Calls launch(std::bool_constant<kWriteF32>, std::bool_constant<kWriteU8>) for the outputs present.
+template <class Launch>
+int launch_for_outputs(const float *batch_f32, const uint8_t *canvas_u8, Launch &&launch)
+{
+    if (batch_f32 && canvas_u8) return launch(std::true_type{}, std::true_type{});
+    if (batch_f32) return launch(std::true_type{}, std::false_type{});
+    return launch(std::false_type{}, std::true_type{});
 }
 
 }  // namespace

@@ -27,6 +27,23 @@ struct ms_graph_entry {
 };
 #define MS_GRAPH_SLOTS 4
 
+// The kernels launched with more dynamic shared memory than the default 48 KB allows (ms_allow_smem); the crop kernels
+// once per output instantiation: f32 batch, u8 canvas, both.
+enum ms_smem_slot {
+    MS_SMEM_CROP_F32,
+    MS_SMEM_CROP_U8,
+    MS_SMEM_CROP_BOTH,
+    MS_SMEM_QUAD_F32,
+    MS_SMEM_QUAD_U8,
+    MS_SMEM_QUAD_BOTH,
+    MS_SMEM_QUAD_STAGED_F32,
+    MS_SMEM_QUAD_STAGED_U8,
+    MS_SMEM_QUAD_STAGED_BOTH,
+    MS_SMEM_READING_ORDER,
+    MS_SMEM_READING_ORDER_LARGE,
+    MS_SMEM_SLOTS
+};
+
 struct ms_ctx {
     int device;
     int num_sms;
@@ -41,8 +58,7 @@ struct ms_ctx {
     size_t stage_bytes;
     // ms_stage_timing: ring of per-batch event sets
     int edge_factor;              // NMS neighbour-pair capacity per candidate (grown by the host entry points)
-    int smem_attr[8];             // largest dynamic shared-memory size already granted to: crop f32 / u8 / both, reading
-                                  // order, quad crop f32 / u8 / both, large-page reading order
+    int smem_granted[MS_SMEM_SLOTS];  // largest dynamic shared-memory size already granted to each kernel
     cudaStream_t copy_stream;     // H2D stream of the pipelined host entry point
     cudaEvent_t chunk_ev[2];
     cudaStream_t aux_stream;      // second half of a batch's front stages (page_batch_impl)
@@ -56,7 +72,6 @@ struct ms_ctx {
     int graphs_enabled;           // 0 with MS_B200_NO_GRAPHS=1 in the environment
     int graph_clock;
     ms_graph_entry graphs[MS_GRAPH_SLOTS];
-    int smem_attr_quad_staged[3]; // ... and to the staged quad-crop kernel f32 / u8 / both
     const int32_t *quad_cnt;      // device counters of the last rotated-crop call (ms_quad_crop_last_counts)
     cudaStream_t quad_stream;
     int quad_no_stage;            // MS_B200_QUAD_NO_STAGE=1: rotated crops by the generic kernel only (A/B runs, tests)
@@ -95,6 +110,24 @@ int ms_stage_reserve(ms_ctx *ctx, size_t bytes);
         int _rc = ms_check_cuda((call), #call);                        \
         if (_rc != MS_OK) return _rc;                                  \
     } while (0)
+
+#define MS_TRY(expr)                 \
+    do {                             \
+        int _r = (expr);             \
+        if (_r != MS_OK) return _r;  \
+    } while (0)
+
+// Lets `kernel` (slot `slot`) be launched with `bytes` of dynamic shared memory.  cudaFuncSetAttribute is a synchronous
+// driver call (milliseconds): it is made once per context and kernel, and again only for a larger size.
+template <typename Kernel>
+inline int ms_allow_smem(ms_ctx *ctx, ms_smem_slot slot, Kernel kernel, int bytes)
+{
+    if (bytes > ctx->smem_granted[slot]) {
+        MS_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+        ctx->smem_granted[slot] = bytes;
+    }
+    return MS_OK;
+}
 
 // ---- programmatic dependent launch --------------------------------------------------------------------------------
 // The front stages are ~50 short kernels, each depending on the one before it: the gap between two of them (the next

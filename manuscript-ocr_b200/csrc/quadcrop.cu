@@ -44,16 +44,6 @@ constexpr int kQsBandPitch = kQsBandBytes + 64;
 constexpr int kQsWinMax = 40 * 1024;     // largest staged source window
 constexpr int kQsRing = 64 * 1024;       // window ring of a CTA
 
-// What the copy warp needs of a staged quad (32 bytes)
-struct __align__(16) QuadDesc {
-    const uint8_t *src;  // 16-byte aligned start of the window's first row
-    int stride;          // bytes between page rows
-    int pitch;           // bytes between staged rows == bytes copied per row
-    int wh;              // window rows
-    int ci;              // quad index (output slot)
-    int pad0, pad1;
-};
-
 // oracle quad_patch_size: edge lengths in float64 from the float32 vertices
 __device__ __forceinline__ bool quad_patch_size(const float *q, int &w, int &h)
 {
@@ -134,7 +124,7 @@ __global__ void __launch_bounds__(128) quad_plan_kernel(const float *__restrict_
                                                         int min_text_size, int ih, int iw, QuadPlan *__restrict__ qplans,
                                                         Plan *__restrict__ plans, int32_t *__restrict__ sizes_out,
                                                         const uint8_t *__restrict__ pages, int img_h, int img_w,
-                                                        int stage_ok, QuadDesc *__restrict__ work,
+                                                        int stage_ok, StageDesc *__restrict__ work,
                                                         int32_t *__restrict__ n_work)
 {
     ms_pdl_wait();
@@ -142,10 +132,7 @@ __global__ void __launch_bounds__(128) quad_plan_kernel(const float *__restrict_
         const float *q = quads + i * quad_stride;
         QuadPlan qp;
         Plan p;
-        p.page = p.x1 = p.y1 = p.w = p.h = p.nw = p.nh = p.y0 = p.interp = p.isx = p.isy = 0;
-        p.ok = p.staged = p.fast = p.pitch = p.stride = 0;
-        p.src = nullptr;
-        p.scale_x = p.scale_y = 1.0;
+        plan_reset(p);
         qp.page = page_of ? page_of[i] : 0;
         qp.ok = qp.staged = 0;
         qp.wx0 = qp.wy0 = qp.ww = qp.wh = qp.mis = qp.pad0 = 0;
@@ -213,13 +200,15 @@ __global__ void __launch_bounds__(128) quad_plan_kernel(const float *__restrict_
                         qp.ww = ww;
                         qp.wh = wh;
                         qp.mis = a;
-                        QuadDesc d;
+                        // the window's rows start 16-byte aligned (the page stride is a multiple of 16): each one is
+                        // copied as exactly `pitch` bytes
+                        StageDesc d;
                         d.src = first - a;
                         d.stride = (int)stride;
                         d.pitch = pitch;
-                        d.wh = wh;
+                        d.row_bytes = pitch;
+                        d.rows = wh;
                         d.ci = (int)i;
-                        d.pad0 = d.pad1 = 0;
                         work[atomicAdd(n_work, 1)] = d;
                     }
                 }
@@ -358,39 +347,6 @@ struct WarpSrc {
     }
 };
 
-template <bool kWriteF32, bool kWriteU8, class Src>
-__device__ __forceinline__ void resample_canvas(const Plan &p, const Src &src, const AxisEnt *s_tab, bool tab_ok,
-                                                bool need_tab, int ih, int iw, float *dstf, uint8_t *dstu)
-{
-    const int plane = ih * iw;
-    const float inv = 1.0f / 127.5f;
-    const int nw = p.nw, nh = p.nh, npx = nw * nh;
-    for (int t = threadIdx.x; t < npx; t += blockDim.x) {
-        const int dy = t / nw, dx = t - dy * nw;
-        AxisEnt ex = {}, ey = {};
-        if (tab_ok) {
-            ex = s_tab[dx];
-            ey = s_tab[nw + dy];
-        } else if (need_tab) {
-            ex = p.interp == 3 ? area_entry(dx, p.scale_x, p.w) : linear_entry_x(dx, p.scale_x, p.w);
-            ey = p.interp == 3 ? area_entry(dy, p.scale_y, p.h) : linear_entry_y(dy, p.scale_y, p.h);
-        }
-        unsigned char o0, o1, o2;
-        resample_px(p, dx, dy, src, ex, ey, o0, o1, o2);
-        const int at = (p.y0 + dy) * iw + dx;
-        if (kWriteF32) {
-            dstf[at] = ((float)o0 - 127.5f) * inv;
-            dstf[plane + at] = ((float)o1 - 127.5f) * inv;
-            dstf[2 * plane + at] = ((float)o2 - 127.5f) * inv;
-        }
-        if (kWriteU8) {
-            dstu[(size_t)at * 3] = o0;
-            dstu[(size_t)at * 3 + 1] = o1;
-            dstu[(size_t)at * 3 + 2] = o2;
-        }
-    }
-}
-
 template <bool kWriteF32, bool kWriteU8>
 __global__ void __launch_bounds__(kQcThreads, 4) quad_crop_kernel(const uint8_t *__restrict__ pages, int img_h,
                                                                   int img_w, const QuadPlan *__restrict__ qplans,
@@ -430,12 +386,7 @@ __global__ void __launch_bounds__(kQcThreads, 4) quad_crop_kernel(const uint8_t 
         if (strips) {
             x3_mine = build_tables(p, soa, tab_n, iw, threadIdx.x, kQcThreads);
         } else if (tab_ok) {
-            for (int t = threadIdx.x; t < p.nw + p.nh; t += blockDim.x) {
-                const bool isx = t < p.nw;
-                const int d = isx ? t : t - p.nw;
-                s_tab[t] = p.interp == 3 ? (isx ? area_entry(d, p.scale_x, p.w) : area_entry(d, p.scale_y, p.h))
-                                         : (isx ? linear_entry_x(d, p.scale_x, p.w) : linear_entry_y(d, p.scale_y, p.h));
-            }
+            fill_axis_table(p, s_tab);
         }
         const bool x3 = __syncthreads_and(x3_mine) != 0;  // also the barrier after the tables
         const QuadPlan &qp = s_qp;
@@ -468,8 +419,9 @@ __global__ void __launch_bounds__(kQcThreads, 4) quad_crop_kernel(const uint8_t 
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// The staged kernel: persistent, warp-specialised, no CTA-wide barrier in the loop (the shape of crop_resize_pad_kernel).
-//   warp 0 (copy warp)    ticket -> descriptor -> bytes in the CTA's window ring -> one TMA bulk copy per window row
+// The staged kernel: persistent, warp-specialised, fed by the staging ring of crop_common.cuh, like
+// crop_resize_pad_kernel.
+//   warp 0 (copy warp)    the ring's copy warp: each quad's source window, one TMA bulk copy per window row
 //   warp 1 (table warp)   the resize tables of the quad, its homography and window into the slot's metadata, then all
 //                         of the canvas padding
 //   warps 2..9 (consumers) a quad's destination rows are cut into BANDS of kQsG rows; consumer warp c takes bands c,
@@ -486,16 +438,16 @@ __global__ void __launch_bounds__(kQcThreads, 4) quad_crop_kernel(const uint8_t 
 // ---------------------------------------------------------------------------------------------------------------------
 struct QsMeta {
     double m[9];
-    int ci, w, h, bw0;
-    int nw, nh, y0, x3;
-    int wx0, wy0, umaxx, umaxy;   // window origin; largest window-relative tap origin (ww - 2, wh - 2)
-    int pitch, base, pad0, pad1;  // staged row pitch; ring offset + misalignment of the window's first byte
+    int w, h, bw0, x3;
+    int nw, nh, y0;
+    int wx0, wy0, umaxx, umaxy;  // window origin; largest window-relative tap origin (ww - 2, wh - 2)
+    int pitch, base;             // staged row pitch; ring offset + misalignment of the window's first byte
 };
 
 template <bool kWriteF32, bool kWriteU8>
 __global__ void __launch_bounds__(kQsThreads, 2)
     quad_crop_staged_kernel(const QuadPlan *__restrict__ qplans, const Plan *__restrict__ plans,
-                            const QuadDesc *__restrict__ work, const int32_t *__restrict__ n_work_dev,
+                            const StageDesc *__restrict__ work, const int32_t *__restrict__ n_work_dev,
                             int32_t *__restrict__ ticket, int ih, int iw, float *__restrict__ batch,
                             uint8_t *__restrict__ canvas_out, int vec_ok, uint8_t *__restrict__ redo)
 {
@@ -504,120 +456,22 @@ __global__ void __launch_bounds__(kQsThreads, 2)
     const int tab_n = area_tab_words(ih, iw);
     unsigned char *bands = smem + kQsRing + 64;
     uint32_t *tabs = reinterpret_cast<uint32_t *>(bands + kQsCW * kQsBandPitch);
-    __shared__ __align__(8) uint64_t s_full[kQsSlots], s_empty[kQsSlots], s_tick[kQsSlots];
-    __shared__ int s_next[kQsSlots], s_off[kQsSlots], s_pitch[kQsSlots];
+    __shared__ StageSlots<kQsSlots> s_stage;
     __shared__ __align__(16) QsMeta s_meta[kQsSlots];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int plane = ih * iw;
-
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int i = 0; i < kQsSlots; i++) {
-            mbar_init(&s_full[i], 2);  // the copy warp (with the byte count) and the table warp
-            mbar_init(&s_empty[i], kQsCW);
-            mbar_init(&s_tick[i], 1);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
+    stage_init(s_stage, kQsCW);
 
     if (warp == 0) {
-        // ---------------- copy warp ----------------
-        const int n_work = *n_work_dev;
-        int q_off[kQsSlots], q_len[kQsSlots];
-#pragma unroll
-        for (int i = 0; i < kQsSlots; i++) q_off[i] = q_len[i] = 0;
-        int head = 0, oldest = 0;
-        auto load_desc = [&](int t) {
-            QuadDesc d;
-            if (t < n_work) {
-                const uint4 *q = reinterpret_cast<const uint4 *>(work + t);
-                const uint4 a = q[0], b = q[1];
-                d.src = reinterpret_cast<const uint8_t *>(((uint64_t)a.y << 32) | a.x);
-                d.stride = (int)a.z;
-                d.pitch = (int)a.w;
-                d.wh = (int)b.x;
-                d.ci = (int)b.y;
-            } else {
-                d.src = nullptr;
-                d.stride = d.pitch = d.wh = 0;
-                d.ci = -1;
-            }
-            d.pad0 = d.pad1 = 0;
-            return d;
-        };
-        int t1 = 0;
-        if (lane == 0) t1 = atomicAdd(ticket, 1);
-        QuadDesc cur = load_desc(__shfl_sync(0xffffffffu, t1, 0));
-        if (lane == 0) t1 = atomicAdd(ticket, 1);
-        for (int k = 0;; k++) {
-            const int s = k % kQsSlots;
-            const QuadDesc nxt = load_desc(__shfl_sync(0xffffffffu, t1, 0));
-            if (lane == 0 && cur.ci >= 0) t1 = atomicAdd(ticket, 1);
-            while (oldest + kQsSlots <= k) {
-                mbar_wait(&s_empty[oldest % kQsSlots], (uint32_t)((oldest / kQsSlots) & 1));
-                q_len[oldest % kQsSlots] = 0;
-                oldest++;
-            }
-            if (cur.ci < 0) {
-                if (lane == 0) {
-                    s_next[s] = -1;
-                    mbar_arrive(&s_tick[s]);
-                    mbar_arrive(&s_full[s]);
-                }
-                break;
-            }
-            const int need = (cur.pitch * cur.wh + 16 + 127) & ~127;
-            int off;
-            for (;;) {
-                auto free_at = [&](int c) {
-                    bool ok = c + need <= kQsRing;
-#pragma unroll
-                    for (int i = 0; i < kQsSlots; i++) ok = ok && (q_len[i] == 0 || c + need <= q_off[i] || q_off[i] + q_len[i] <= c);
-                    return ok;
-                };
-                if (free_at(head)) {
-                    off = head;
-                    break;
-                }
-                if (free_at(0)) {
-                    off = 0;
-                    break;
-                }
-                mbar_wait(&s_empty[oldest % kQsSlots], (uint32_t)((oldest / kQsSlots) & 1));
-                q_len[oldest % kQsSlots] = 0;
-                oldest++;
-            }
-            q_off[s] = off;
-            q_len[s] = need;
-            head = off + need;
-            if (lane == 0) {
-                s_next[s] = cur.ci;
-                s_off[s] = off;
-                s_pitch[s] = cur.pitch;
-                mbar_arrive(&s_tick[s]);
-            }
-            for (int r = lane; r < cur.wh; r += 32)
-                tma_bulk_g2s(smem + off + (size_t)r * cur.pitch, cur.src + (size_t)r * cur.stride, (uint32_t)cur.pitch,
-                             &s_full[s]);
-            if (lane == 0) mbar_expect_tx(&s_full[s], (uint32_t)(cur.pitch * cur.wh));
-            cur = nxt;
-        }
+        stage_copy_warp(s_stage, smem, kQsRing, work, *n_work_dev, ticket);
         return;
     }
     if (warp == 1) {
         // ---------------- table warp: resize tables + slot metadata, then the padding ----------------
         for (int k = 0;; k++) {
             const int s = k % kQsSlots;
-            mbar_wait(&s_tick[s], (uint32_t)((k / kQsSlots) & 1));
-            const int ci = s_next[s];
-            if (ci < 0) {
-                if (lane == 0) {
-                    s_meta[s].ci = -1;
-                    mbar_arrive(&s_full[s]);
-                }
-                break;
-            }
+            const int ci = stage_wait_tick(s_stage, k);
+            if (ci < 0) break;
             const Plan p = plans[ci];
             const bool x3 = __all_sync(0xffffffffu, build_tables(p, tabs + (size_t)s * tab_n, tab_n, iw, lane));
             if (lane < 9) s_meta[s].m[lane] = qplans[ci].m[lane];
@@ -625,7 +479,6 @@ __global__ void __launch_bounds__(kQsThreads, 2)
                 const QuadPlan *qp = qplans + ci;
                 QsMeta &me = s_meta[s];
                 const int wx0 = qp->wx0, wy0 = qp->wy0;
-                me.ci = ci;
                 me.w = qp->w;
                 me.h = qp->h;
                 me.bw0 = qp->bw0;
@@ -637,12 +490,12 @@ __global__ void __launch_bounds__(kQsThreads, 2)
                 me.wy0 = wy0;
                 me.umaxx = qp->ww - 2;
                 me.umaxy = qp->wh - 2;
-                me.pitch = s_pitch[s];
-                me.base = s_off[s] + qp->mis;  // the page stride is a multiple of 16: every row has this misalignment
-                me.pad0 = me.pad1 = 0;
+                me.pitch = s_stage.pitch[s];
+                // the page stride is a multiple of 16: every row has this misalignment
+                me.base = s_stage.off[s] + qp->mis;
             }
             __syncwarp();
-            if (lane == 0) mbar_arrive(&s_full[s]);
+            if (lane == 0) mbar_arrive(&s_stage.full[s]);
             write_padding<kWriteF32, kWriteU8>(p.nw, p.nh, p.y0, ih, iw, kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr,
                                                kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr, vec_ok, lane, 32);
         }
@@ -656,10 +509,9 @@ __global__ void __launch_bounds__(kQsThreads, 2)
     const uint32_t *smem32 = reinterpret_cast<const uint32_t *>(smem);
     for (int k = 0;; k++) {
         const int s = k % kQsSlots;
-        mbar_wait(&s_full[s], (uint32_t)((k / kQsSlots) & 1));
-        const QsMeta &me = s_meta[s];
-        const int ci = me.ci;
+        const int ci = stage_wait_full(s_stage, k);
         if (ci < 0) break;
+        const QsMeta &me = s_meta[s];
         const int w = me.w, h = me.h, nw = me.nw, nh = me.nh, y0 = me.y0;
         const double m0 = me.m[0], m1 = me.m[1], m2 = me.m[2], m3 = me.m[3], m4 = me.m[4], m5 = me.m[5], m6 = me.m[6],
                      m7 = me.m[7], m8 = me.m[8];
@@ -742,8 +594,7 @@ __global__ void __launch_bounds__(kQsThreads, 2)
             __syncwarp();  // the band buffer is rewritten by the next band
         }
         if (bad) redo[ci] = 1;  // the generic kernel redoes the quad (it rewrites the whole canvas)
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&s_empty[s]);
+        stage_release(s_stage, s);
     }
 }
 
@@ -785,14 +636,8 @@ __global__ void __launch_bounds__(256) quad_warp_kernel(const uint8_t *__restric
 size_t msk_quad_crop_scratch(int64_t n)
 {
     const size_t k = (size_t)(n > 0 ? n : 0);
-    return k * (sizeof(QuadPlan) + sizeof(Plan) + sizeof(QuadDesc) + 1 + sizeof(int32_t)) + 8192;
+    return k * (sizeof(QuadPlan) + sizeof(Plan) + sizeof(StageDesc) + 1 + sizeof(int32_t)) + 8192;
 }
-
-#define MS_TRY(expr)                 \
-    do {                             \
-        int _r = (expr);             \
-        if (_r != MS_OK) return _r;  \
-    } while (0)
 
 static int quad_args_ok(int n_pages, int img_h, int img_w, int border_mode, int border_value, const char *who)
 {
@@ -821,7 +666,7 @@ int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int
     }
     QuadPlan *qplans = bump.take<QuadPlan>((size_t)n);
     Plan *plans = bump.take<Plan>((size_t)n);
-    QuadDesc *work = bump.take<QuadDesc>((size_t)n);
+    StageDesc *work = bump.take<StageDesc>((size_t)n);
     uint8_t *redo = bump.take<uint8_t>((size_t)n);
     int32_t *list = bump.take<int32_t>((size_t)n);
     int32_t *cnt = bump.take<int32_t>(4);  // staged quads, ticket counter, fallback-list length
@@ -850,40 +695,25 @@ int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int
     int64_t grid = (int64_t)ctx->num_sms * 4;  // 40 KB stage + 12 KB tables, 64 registers: four CTAs per SM
     if (grid > n) grid = n;
     const int smem = kQcPatchBytes + 16 + kQcMaxTab * (int)sizeof(AxisEnt);
-    // cudaFuncSetAttribute is a synchronous driver call: once per context and kernel
-#define MS_QC_LAUNCH(F32, U8)                                                                                          \
-    do {                                                                                                               \
-        if (staged) {                                                                                                  \
-            auto sfn = quad_crop_staged_kernel<F32, U8>;                                                               \
-            int &sgranted = ctx->smem_attr_quad_staged[(F32 ? 1 : 0) + (U8 ? 2 : 0) - 1];                              \
-            if (smem_s > sgranted) {                                                                                   \
-                MS_CUDA(cudaFuncSetAttribute(sfn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_s));              \
-                sgranted = smem_s;                                                                                     \
-            }                                                                                                          \
-            ms_launch(sfn, ctx->num_sms * 2, kQsThreads, smem_s, st, qplans, plans, work, cnt, cnt + 1, out_h, out_w,        \
-                                                               batch_f32, canvas_u8, vec_ok, redo);                    \
-            MS_LAUNCH_CHECK(ctx);                                                                                      \
-        }                                                                                                              \
-        ms_launch(quad_fallback_list_kernel, (int)pg, 256, 0, st, qplans, n, redo, list, cnt + 2);                            \
-        MS_LAUNCH_CHECK(ctx);                                                                                          \
-        auto kfn = quad_crop_kernel<F32, U8>;                                                                          \
-        int &granted = ctx->smem_attr[4 + (F32 ? 1 : 0) + (U8 ? 2 : 0) - 1];                                           \
-        if (smem > granted) {                                                                                          \
-            MS_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));                     \
-            granted = smem;                                                                                            \
-        }                                                                                                              \
-        ms_launch(kfn, (int)grid, kQcThreads, smem, st, pages, img_h, img_w, qplans, plans, n, border_mode, border_value,     \
-                                                 out_h, out_w, batch_f32, canvas_u8, vec_ok, list, cnt + 2);          \
-    } while (0)
-    if (batch_f32 && canvas_u8)
-        MS_QC_LAUNCH(true, true);
-    else if (batch_f32)
-        MS_QC_LAUNCH(true, false);
-    else
-        MS_QC_LAUNCH(false, true);
-#undef MS_QC_LAUNCH
-    MS_LAUNCH_CHECK(ctx);
-    return MS_OK;
+    return launch_for_outputs(batch_f32, canvas_u8, [&](auto f32, auto u8) {
+        constexpr bool kF32 = decltype(f32)::value, kU8 = decltype(u8)::value;
+        if (staged) {
+            constexpr ms_smem_slot slot =
+                kF32 ? (kU8 ? MS_SMEM_QUAD_STAGED_BOTH : MS_SMEM_QUAD_STAGED_F32) : MS_SMEM_QUAD_STAGED_U8;
+            MS_TRY(ms_allow_smem(ctx, slot, quad_crop_staged_kernel<kF32, kU8>, smem_s));
+            ms_launch(quad_crop_staged_kernel<kF32, kU8>, ctx->num_sms * 2, kQsThreads, smem_s, st, qplans, plans, work, cnt,
+                      cnt + 1, out_h, out_w, batch_f32, canvas_u8, vec_ok, redo);
+            MS_LAUNCH_CHECK(ctx);
+        }
+        ms_launch(quad_fallback_list_kernel, (int)pg, 256, 0, st, qplans, n, redo, list, cnt + 2);
+        MS_LAUNCH_CHECK(ctx);
+        constexpr ms_smem_slot slot = kF32 ? (kU8 ? MS_SMEM_QUAD_BOTH : MS_SMEM_QUAD_F32) : MS_SMEM_QUAD_U8;
+        MS_TRY(ms_allow_smem(ctx, slot, quad_crop_kernel<kF32, kU8>, smem));
+        ms_launch(quad_crop_kernel<kF32, kU8>, (int)grid, kQcThreads, smem, st, pages, img_h, img_w, qplans, plans, n,
+                  border_mode, border_value, out_h, out_w, batch_f32, canvas_u8, vec_ok, list, cnt + 2);
+        MS_LAUNCH_CHECK(ctx);
+        return MS_OK;
+    });
 }
 
 // One quad's patch.  *w / *h receive the patch size (0, 0: no patch); the pixels are produced only when they fit

@@ -1526,10 +1526,7 @@ int msk_reading_order(ms_ctx *ctx, const float *boxes8, int row_stride, const in
                         (size_t)(kRoMaxBoxes + 2) * 2;
     static_assert(kRoMaxPairs * 5 + kRoMaxBoxes * 2 >= 144 * 1024 && kRoMaxBoxes == 4096,
                   "pair + level region must hold the sort / line arrays laid out in the kernel");
-    if ((int)smem > ctx->smem_attr[3]) {  // a synchronous driver call: once per context
-        MS_CUDA(cudaFuncSetAttribute(reading_order_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        ctx->smem_attr[3] = (int)smem;
-    }
+    MS_TRY(ms_allow_smem(ctx, MS_SMEM_READING_ORDER, reading_order_kernel, (int)smem));
     ms_launch(reading_order_kernel, n_pages, kRoThreads, smem, st, boxes8, row_stride, counts, cap_per_page, obox, order,
                                                            reordered, flags, gpairs16, gbox32, need_large,
                                                            need_large ? need_large + n_pages : nullptr,
@@ -1537,10 +1534,7 @@ int msk_reading_order(ms_ctx *ctx, const float *boxes8, int row_stride, const in
     MS_LAUNCH_CHECK(ctx);
     if (slots) {  // pages the first kernel could not hold (none, usually: the CTAs find no ticket and leave)
         const int smem_l = kRlSmemKeys * 12;
-        if (smem_l > ctx->smem_attr[7]) {
-            MS_CUDA(cudaFuncSetAttribute(reading_order_large_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_l));
-            ctx->smem_attr[7] = smem_l;
-        }
+        MS_TRY(ms_allow_smem(ctx, MS_SMEM_READING_ORDER_LARGE, reading_order_large_kernel, smem_l));
         ms_launch(reading_order_large_kernel, slots, kRoThreads, smem_l, st, boxes8, row_stride, counts, cap_per_page, n_pages, order,
                                                                 reordered, flags, need_large, need_large + n_pages,
                                                                 slot_mem, slot_bytes);
