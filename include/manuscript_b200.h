@@ -51,6 +51,14 @@ extern "C" {
 #define MS_FLAG_ORDER_OVERFLOW 8 /* reading order not computed on the device for this page (more than
                                     max(65536, 16 cap) intersecting box pairs): its boxes and crops are in detection order */
 
+/* element type of the recogniser batch written by the *_ex crop entry points (`batch_dtype`).  The 16-bit batches are
+ * an EXTENSION (not a reference behaviour): every value is the float32 batch value ((v - 127.5) * (1/127.5), computed in
+ * float32) rounded to nearest-even, bit for bit what torch's batch_f32.to(torch.float16 / torch.bfloat16) gives -- half
+ * the bytes written, and no cast for a recogniser that runs in 16 bits.  An unknown code is MS_ERR_INVALID. */
+#define MS_DTYPE_F32 0
+#define MS_DTYPE_F16 1
+#define MS_DTYPE_BF16 2
+
 typedef struct ms_ctx ms_ctx;
 
 /* EAST constructor parameters that shape the path (infer.py:28-43). */
@@ -233,6 +241,10 @@ MS_API int ms_word_rects(ms_ctx *ctx, const float *quads, const int32_t *counts,
 MS_API int ms_crop_resize_pad(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w,
                        const int32_t *crops, const int32_t *n_crops, int64_t crops_cap, int out_h,
                        int out_w, float *batch_f32, uint8_t *canvas_u8, void *stream);
+/* ms_crop_resize_pad with the batch (crops_cap,3,out_h,out_w) in batch_dtype (MS_DTYPE_*); batch may be NULL. */
+MS_API int ms_crop_resize_pad_ex(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w,
+                          const int32_t *crops, const int32_t *n_crops, int64_t crops_cap, int out_h, int out_w,
+                          void *batch, int batch_dtype, uint8_t *canvas_u8, void *stream);
 
 /* SURVEY 8f-4, an EXTENSION (the reference crops axis-aligned rectangles only, _pipeline.py:204-221; todo.md:1):
  * rectified crops of rotated quads.  For every quad (rows of quad_stride >= 8 floats x0,y0..x3,y3 in the order
@@ -248,6 +260,11 @@ MS_API int ms_quad_crop_resize_pad(ms_ctx *ctx, const uint8_t *pages, int n_page
                             const float *quads, int quad_stride, const int32_t *page_of, int64_t n,
                             int min_text_size, int border_mode, int border_value, int out_h, int out_w,
                             float *batch_f32, uint8_t *canvas_u8, int32_t *sizes_out, void *stream);
+/* ms_quad_crop_resize_pad with the batch (n,3,out_h,out_w) in batch_dtype (MS_DTYPE_*); batch may be NULL. */
+MS_API int ms_quad_crop_resize_pad_ex(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w,
+                               const float *quads, int quad_stride, const int32_t *page_of, int64_t n,
+                               int min_text_size, int border_mode, int border_value, int out_h, int out_w,
+                               void *batch, int batch_dtype, uint8_t *canvas_u8, int32_t *sizes_out, void *stream);
 
 /* north_star's "TPS rectification grid_sample" -- NOT a reference behaviour (the reference's TRBAModel has no
  * transformation stage, recognizers/_trba/model/model.py:338-393; SURVEY 0), "parity unpinned"; specified as the
@@ -267,6 +284,13 @@ MS_API int ms_page_batch(ms_ctx *ctx, const float *score, const float *geo, cons
                   int out_h, int out_w, int cap_boxes, float *boxes_out, int32_t *box_counts,
                   int32_t *crops_out, int64_t crops_cap, int32_t *n_crops, float *batch_f32,
                   uint8_t *canvas_u8, int32_t *flags, void *stream);
+/* ms_page_batch with the crop batch in batch_dtype (MS_DTYPE_*).  The dtype is part of the call's identity for the
+ * CUDA-graph cache: the same buffers with another dtype are a different call. */
+MS_API int ms_page_batch_ex(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
+                     int map_h, int map_w, int img_h, int img_w, const ms_east_params *p, int min_text_size,
+                     int out_h, int out_w, int cap_boxes, float *boxes_out, int32_t *box_counts,
+                     int32_t *crops_out, int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype,
+                     uint8_t *canvas_u8, int32_t *flags, void *stream);
 
 /* ms_page_batch for page images of their OWN sizes (a batch of originals: EAST.predict resizes each to target_size,
  * so the maps are uniform while the images are not).  page_ptrs (n_pages) device pointers to (h_i, w_i, 3) u8
@@ -277,6 +301,12 @@ MS_API int ms_page_batch_ragged(ms_ctx *ctx, const float *score, const float *ge
                          int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
                          int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
                          float *batch_f32, uint8_t *canvas_u8, int32_t *flags, void *stream);
+/* ms_page_batch_ragged with the crop batch in batch_dtype (MS_DTYPE_*). */
+MS_API int ms_page_batch_ragged_ex(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *const *page_ptrs,
+                            const int32_t *page_hw, int n_pages, int map_h, int map_w, const ms_east_params *p,
+                            int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
+                            int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
+                            void *batch, int batch_dtype, uint8_t *canvas_u8, int32_t *flags, void *stream);
 
 /* Same path with HOST buffers (pinned or pageable; `score` / `geo` may also be DEVICE pointers of this context's
  * device -- maps a detector left on the GPU are used in place and only the page images cross PCIe): H2D of maps + pages, the batch, D2H of boxes,
@@ -292,6 +322,13 @@ MS_API int ms_page_batch_host(ms_ctx *ctx, const float *score, const float *geo,
                        int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
                        int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
                        float *batch_f32_host, float **batch_dev_out, int32_t *flags);
+/* ms_page_batch_host with the crop batch in batch_dtype (MS_DTYPE_*): the host copy (batch_host), a caller-owned
+ * device buffer (*batch_dev_out) and the library-owned device batch are all of that element type. */
+MS_API int ms_page_batch_host_ex(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages,
+                          int n_pages, int map_h, int map_w, int img_h, int img_w, const ms_east_params *p,
+                          int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
+                          int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
+                          void *batch_host, int batch_dtype, void **batch_dev_out, int32_t *flags);
 
 /* ms_page_batch_ragged with HOST buffers: pages (n_pages) host pointers, page_hw (n_pages,2) int32 on the host;
  * outputs as ms_page_batch_host. */
@@ -300,6 +337,12 @@ MS_API int ms_page_batch_ragged_host(ms_ctx *ctx, const float *score, const floa
                               int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
                               int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
                               float *batch_f32_host, float **batch_dev_out, int32_t *flags);
+/* ms_page_batch_ragged_host with the crop batch in batch_dtype (MS_DTYPE_*), as ms_page_batch_host_ex. */
+MS_API int ms_page_batch_ragged_host_ex(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *const *pages,
+                                 const int32_t *page_hw, int n_pages, int map_h, int map_w, const ms_east_params *p,
+                                 int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
+                                 int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
+                                 void *batch_host, int batch_dtype, void **batch_dev_out, int32_t *flags);
 
 #ifdef __cplusplus
 }

@@ -460,19 +460,38 @@ extern "C" int ms_word_rects(ms_ctx *ctx, const float *quads, const int32_t *cou
                           crops_cap, n_crops, 0, 0, nullptr, bump, (cudaStream_t)stream);
 }
 
-extern "C" int ms_crop_resize_pad(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w,
-                                  const int32_t *crops, const int32_t *n_crops, int64_t crops_cap, int out_h, int out_w,
-                                  float *batch_f32, uint8_t *canvas_u8, void *stream)
+// the batch_dtype argument of an *_ex entry point
+static int dtype_ok(int batch_dtype, const char *who)
+{
+    if (ms_dtype_bytes(batch_dtype) == 0) {
+        ms_set_error("%s: unknown batch dtype %d (MS_DTYPE_F32, MS_DTYPE_F16 or MS_DTYPE_BF16)", who, batch_dtype);
+        return MS_ERR_INVALID;
+    }
+    return MS_OK;
+}
+
+extern "C" int ms_crop_resize_pad_ex(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w,
+                                     const int32_t *crops, const int32_t *n_crops, int64_t crops_cap, int out_h,
+                                     int out_w, void *batch, int batch_dtype, uint8_t *canvas_u8, void *stream)
 {
     MS_CTX(ctx);
+    MS_TRY(dtype_ok(batch_dtype, "ms_crop_resize_pad"));
     if (!pages || !crops || !n_crops) {
         ms_set_error("ms_crop_resize_pad: NULL pointer");
         return MS_ERR_INVALID;
     }
     MS_TRY(ms_arena_reserve(ctx, msk_crop_scratch(crops_cap, n_pages)));
     ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
-    return msk_crop(ctx, pages, n_pages, img_h, img_w, crops, n_crops, nullptr, crops_cap, out_h, out_w, batch_f32,
-                    canvas_u8, bump, (cudaStream_t)stream);
+    return msk_crop(ctx, pages, n_pages, img_h, img_w, crops, n_crops, nullptr, crops_cap, out_h, out_w, batch,
+                    batch_dtype, canvas_u8, bump, (cudaStream_t)stream);
+}
+
+extern "C" int ms_crop_resize_pad(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w,
+                                  const int32_t *crops, const int32_t *n_crops, int64_t crops_cap, int out_h, int out_w,
+                                  float *batch_f32, uint8_t *canvas_u8, void *stream)
+{
+    return ms_crop_resize_pad_ex(ctx, pages, n_pages, img_h, img_w, crops, n_crops, crops_cap, out_h, out_w, batch_f32,
+                                 MS_DTYPE_F32, canvas_u8, stream);
 }
 
 extern "C" int ms_detector_input(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, int target_h, int target_w,
@@ -582,8 +601,8 @@ static int page_batch_impl(ms_ctx *ctx, const float *score, const float *geo, co
                            int page_base, int n_pages, int map_h, int map_w, int img_h, int img_w,
                            const ms_east_params *p, int min_text_size, int out_h, int out_w, int cap_boxes,
                            float *boxes_out, int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
-                           int32_t *n_crops, int append, float *batch_f32, uint8_t *canvas_u8, int32_t *flags,
-                           cudaStream_t st, int geo_compact = 0, const uint8_t *const *page_ptrs = nullptr,
+                           int32_t *n_crops, int append, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                           int32_t *flags, cudaStream_t st, int geo_compact = 0, const uint8_t *const *page_ptrs = nullptr,
                            const int32_t *page_hw = nullptr)
 {
     // page_ptrs / page_hw (device, indexed by the global page number): page images of their own sizes
@@ -636,9 +655,9 @@ static int page_batch_impl(ms_ctx *ctx, const float *score, const float *geo, co
         MS_TRY(msk_word_rects(ctx, boxes_out, box_counts, n_pages, cap_boxes, hw_here, img_h, img_w, min_text_size,
                               crops_out, crops_cap, n_crops, page_base, append, range, bumpT, st));
         MS_TRY(timing_mark(ctx, 4, st));
-        if (batch_f32 || canvas_u8)
+        if (batch || canvas_u8)
             MS_TRY(msk_crop(ctx, pages_all, total_pages, img_h, img_w, crops_out, n_crops, range, crops_cap, out_h,
-                            out_w, batch_f32, canvas_u8, bumpT, st, page_ptrs, page_hw));
+                            out_w, batch, batch_dtype, canvas_u8, bumpT, st, page_ptrs, page_hw));
     } else {
         MS_TRY(timing_mark(ctx, 4, st));
     }
@@ -653,21 +672,23 @@ static int page_batch_cached(ms_ctx *ctx, const float *score, const float *geo, 
                              const uint8_t *const *page_ptrs, const int32_t *page_hw, int n_pages, int map_h, int map_w,
                              int img_h, int img_w, const ms_east_params *p, int min_text_size, int out_h, int out_w,
                              int cap_boxes, float *boxes_out, int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
-                             int32_t *n_crops, float *batch_f32, uint8_t *canvas_u8, int32_t *flags, cudaStream_t st)
+                             int32_t *n_crops, void *batch, int batch_dtype, uint8_t *canvas_u8, int32_t *flags,
+                             cudaStream_t st)
 {
     auto direct = [&](cudaStream_t s) {
         return page_batch_impl(ctx, score, geo, pages, n_pages, 0, n_pages, map_h, map_w, img_h, img_w, p, min_text_size,
-                               out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, 0, batch_f32,
-                               canvas_u8, flags, s, 0, page_ptrs, page_hw);
+                               out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, 0, batch,
+                               batch_dtype, canvas_u8, flags, s, 0, page_ptrs, page_hw);
     };
     if (!ctx->graphs_enabled || ctx->timing) return direct(st);
     ms_pb_key key;
     memset(&key, 0, sizeof(key));
-    const void *ptrs[14] = {score, geo, pages, page_ptrs, page_hw, boxes_out, box_counts, crops_out, n_crops, batch_f32,
+    const void *ptrs[14] = {score, geo, pages, page_ptrs, page_hw, boxes_out, box_counts, crops_out, n_crops, batch,
                             canvas_u8, flags, ctx->arena, nullptr};
     memcpy(key.ptr, ptrs, sizeof(ptrs));
-    const long long nums[12] = {n_pages, map_h, map_w, img_h, img_w, min_text_size, out_h, out_w, cap_boxes,
-                                (long long)crops_cap, ctx->edge_factor, (long long)ctx->arena_bytes};
+    // the batch dtype selects the crop kernels' instantiation: the same buffer in another dtype is another graph
+    const long long nums[13] = {n_pages, map_h, map_w, img_h, img_w, min_text_size, out_h, out_w, cap_boxes,
+                                (long long)crops_cap, ctx->edge_factor, (long long)ctx->arena_bytes, batch_dtype};
     memcpy(key.num, nums, sizeof(nums));
     // field by field: the caller's struct may carry indeterminate padding bytes, which must not take part in the key
     key.params.score_thresh = p->score_thresh;
@@ -731,13 +752,14 @@ static int page_batch_cached(ms_ctx *ctx, const float *score, const float *geo, 
     return rc;
 }
 
-extern "C" int ms_page_batch(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
-                             int map_h, int map_w, int img_h, int img_w, const ms_east_params *p, int min_text_size,
-                             int out_h, int out_w, int cap_boxes, float *boxes_out, int32_t *box_counts,
-                             int32_t *crops_out, int64_t crops_cap, int32_t *n_crops, float *batch_f32,
-                             uint8_t *canvas_u8, int32_t *flags, void *stream)
+extern "C" int ms_page_batch_ex(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
+                                int map_h, int map_w, int img_h, int img_w, const ms_east_params *p, int min_text_size,
+                                int out_h, int out_w, int cap_boxes, float *boxes_out, int32_t *box_counts,
+                                int32_t *crops_out, int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype,
+                                uint8_t *canvas_u8, int32_t *flags, void *stream)
 {
     MS_CTX(ctx);
+    MS_TRY(dtype_ok(batch_dtype, "ms_page_batch"));
     if (n_pages <= 0) return MS_OK;
     if (!score || !geo || !p || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
         ms_set_error("ms_page_batch: bad arguments");
@@ -745,7 +767,18 @@ extern "C" int ms_page_batch(ms_ctx *ctx, const float *score, const float *geo, 
     }
     return page_batch_cached(ctx, score, geo, pages, nullptr, nullptr, n_pages, map_h, map_w, img_h, img_w, p,
                              min_text_size, out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops,
-                             batch_f32, canvas_u8, flags, (cudaStream_t)stream);
+                             batch, batch_dtype, canvas_u8, flags, (cudaStream_t)stream);
+}
+
+extern "C" int ms_page_batch(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
+                             int map_h, int map_w, int img_h, int img_w, const ms_east_params *p, int min_text_size,
+                             int out_h, int out_w, int cap_boxes, float *boxes_out, int32_t *box_counts,
+                             int32_t *crops_out, int64_t crops_cap, int32_t *n_crops, float *batch_f32,
+                             uint8_t *canvas_u8, int32_t *flags, void *stream)
+{
+    return ms_page_batch_ex(ctx, score, geo, pages, n_pages, map_h, map_w, img_h, img_w, p, min_text_size, out_h, out_w,
+                            cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch_f32, MS_DTYPE_F32,
+                            canvas_u8, flags, stream);
 }
 
 // =========================================================================================================
@@ -1128,11 +1161,31 @@ extern "C" int ms_crop_resize_pad_host(ms_ctx *ctx, const uint8_t *page, int img
     }
     MS_TRY(ms_arena_reserve(ctx, msk_crop_scratch(n, 1)));
     ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
-    MS_TRY(msk_crop(ctx, d_page, 1, img_h, img_w, d_crops, d_n, nullptr, n, out_h, out_w, d_f, d_u, bump, st));
+    MS_TRY(msk_crop(ctx, d_page, 1, img_h, img_w, d_crops, d_n, nullptr, n, out_h, out_w, d_f, MS_DTYPE_F32, d_u, bump,
+                    st));
     if (batch_f32) MS_CUDA(cudaMemcpyAsync(batch_f32, d_f, (size_t)n * one_f, cudaMemcpyDeviceToHost, st));
     if (canvas_u8) MS_CUDA(cudaMemcpyAsync(canvas_u8, d_u, (size_t)n * one_u, cudaMemcpyDeviceToHost, st));
     MS_CUDA(cudaStreamSynchronize(st));
     return MS_OK;
+}
+
+extern "C" int ms_page_batch_ragged_ex(ms_ctx *ctx, const float *score, const float *geo,
+                                       const uint8_t *const *page_ptrs, const int32_t *page_hw, int n_pages, int map_h,
+                                       int map_w, const ms_east_params *p, int min_text_size, int out_h, int out_w,
+                                       int cap_boxes, float *boxes_out, int32_t *box_counts, int32_t *crops_out,
+                                       int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype,
+                                       uint8_t *canvas_u8, int32_t *flags, void *stream)
+{
+    MS_CTX(ctx);
+    MS_TRY(dtype_ok(batch_dtype, "ms_page_batch_ragged"));
+    if (n_pages <= 0) return MS_OK;
+    if (!score || !geo || !p || !page_ptrs || !page_hw || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
+        ms_set_error("ms_page_batch_ragged: bad arguments");
+        return MS_ERR_INVALID;
+    }
+    return page_batch_cached(ctx, score, geo, nullptr, page_ptrs, page_hw, n_pages, map_h, map_w, 0, 0, p, min_text_size,
+                             out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch,
+                             batch_dtype, canvas_u8, flags, (cudaStream_t)stream);
 }
 
 extern "C" int ms_page_batch_ragged(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *const *page_ptrs,
@@ -1141,36 +1194,31 @@ extern "C" int ms_page_batch_ragged(ms_ctx *ctx, const float *score, const float
                                     int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
                                     float *batch_f32, uint8_t *canvas_u8, int32_t *flags, void *stream)
 {
-    MS_CTX(ctx);
-    if (n_pages <= 0) return MS_OK;
-    if (!score || !geo || !p || !page_ptrs || !page_hw || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
-        ms_set_error("ms_page_batch_ragged: bad arguments");
-        return MS_ERR_INVALID;
-    }
-    return page_batch_cached(ctx, score, geo, nullptr, page_ptrs, page_hw, n_pages, map_h, map_w, 0, 0, p, min_text_size,
-                             out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch_f32,
-                             canvas_u8, flags, (cudaStream_t)stream);
+    return ms_page_batch_ragged_ex(ctx, score, geo, page_ptrs, page_hw, n_pages, map_h, map_w, p, min_text_size, out_h,
+                                   out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch_f32,
+                                   MS_DTYPE_F32, canvas_u8, flags, stream);
 }
 
-extern "C" int ms_page_batch_host(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
-                                  int map_h, int map_w, int img_h, int img_w, const ms_east_params *p,
-                                  int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
-                                  int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
-                                  float *batch_f32_host, float **batch_dev_out, int32_t *flags)
+extern "C" int ms_page_batch_host_ex(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages,
+                                     int n_pages, int map_h, int map_w, int img_h, int img_w, const ms_east_params *p,
+                                     int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
+                                     int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
+                                     void *batch_host, int batch_dtype, void **batch_dev_out, int32_t *flags)
 {
     MS_CTX(ctx);
+    MS_TRY(dtype_ok(batch_dtype, "ms_page_batch_host"));
     if (n_pages <= 0) return MS_OK;
     if (!score || !geo || !p || !boxes_out || !box_counts || !flags || cap_boxes <= 0 || map_h <= 0 || map_w <= 0) {
         ms_set_error("ms_page_batch_host: bad arguments");
         return MS_ERR_INVALID;
     }
     const bool want_crops = pages != nullptr && crops_out != nullptr && n_crops != nullptr && crops_cap > 0;
-    const bool want_batch = want_crops && (batch_f32_host || batch_dev_out);
+    const bool want_batch = want_crops && (batch_host || batch_dev_out);
     // *batch_dev_out != NULL on entry: a caller-owned device buffer of crops_cap crops that receives the batch
-    float *caller_batch = (want_batch && batch_dev_out) ? *batch_dev_out : nullptr;
+    void *caller_batch = (want_batch && batch_dev_out) ? *batch_dev_out : nullptr;
     const size_t plane = (size_t)map_h * map_w;
     const size_t page_bytes = (size_t)img_h * img_w * 3;
-    const size_t one_f = (size_t)3 * out_h * out_w * sizeof(float);
+    const size_t one_f = (size_t)3 * out_h * out_w * ms_dtype_bytes(batch_dtype);  // bytes of one crop of the batch
     // The decode reads the geometry only at the candidate cells (a few per cent of the tensor).  When the caller's
     // geometry lives in pinned host memory the kernel gathers it straight from there over PCIe (zero copy) instead
     // of uploading the tensor; pageable buffers are uploaded.
@@ -1204,7 +1252,7 @@ extern "C" int ms_page_batch_host(ms_ctx *ctx, const float *score, const float *
     uint8_t *d_pages = want_crops ? sb.take<uint8_t>(n_pages * page_bytes) : nullptr;
     int32_t *d_crops = want_crops ? sb.take<int32_t>((size_t)crops_cap * 5) : nullptr;
     int32_t *d_nc = want_crops ? sb.take<int32_t>(1) : nullptr;
-    float *d_batch = !want_batch ? nullptr : caller_batch ? caller_batch : sb.take<float>((size_t)crops_cap * 3 * out_h * out_w);
+    void *d_batch = !want_batch ? nullptr : caller_batch ? caller_batch : sb.take<char>((size_t)crops_cap * one_f);
     if (!d_flags || (want_crops && !d_nc) || (want_batch && !d_batch)) {
         ms_set_error("ms_page_batch_host: staging too small");
         return MS_ERR_CAPACITY;
@@ -1248,7 +1296,7 @@ extern "C" int ms_page_batch_host(ms_ctx *ctx, const float *score, const float *
         MS_TRY(page_batch_impl(ctx, d_score + (size_t)p0 * plane, geo_chunk, d_pages, n_pages, p0,
                                np, map_h, map_w, img_h, img_w, p, min_text_size, out_h, out_w, cap_boxes,
                                d_boxes + (size_t)p0 * cap_boxes * 9, d_cnt + p0, d_crops, crops_cap, d_nc, 1, d_batch,
-                               nullptr, d_flags + p0, st, geo_compact));
+                               batch_dtype, nullptr, d_flags + p0, st, geo_compact));
     }
     MS_CUDA(cudaMemcpyAsync(box_counts, d_cnt, (size_t)n_pages * 4, cudaMemcpyDeviceToHost, st));
     MS_CUDA(cudaMemcpyAsync(flags, d_flags, (size_t)n_pages * 4, cudaMemcpyDeviceToHost, st));
@@ -1257,9 +1305,9 @@ extern "C" int ms_page_batch_host(ms_ctx *ctx, const float *score, const float *
     int32_t all = 0;
     for (int i = 0; i < n_pages; i++) all |= flags[i];
     if (grow_edge_factor(ctx, all))
-        return ms_page_batch_host(ctx, score, geo, pages, n_pages, map_h, map_w, img_h, img_w, p, min_text_size, out_h,
-                                  out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch_f32_host,
-                                  batch_dev_out, flags);
+        return ms_page_batch_host_ex(ctx, score, geo, pages, n_pages, map_h, map_w, img_h, img_w, p, min_text_size,
+                                     out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops,
+                                     batch_host, batch_dtype, batch_dev_out, flags);
     // the boxes come back page by page, only the rows each page has (counts are known now): 36 bytes per box instead
     // of cap_boxes rows per page; a page's copy runs up to the following pages' rows when they are adjacent anyway
     {
@@ -1276,8 +1324,8 @@ extern "C" int ms_page_batch_host(ms_ctx *ctx, const float *score, const float *
         if (nc > crops_cap) nc = crops_cap;
         if (nc > 0) {
             MS_CUDA(cudaMemcpyAsync(crops_out, d_crops, (size_t)nc * 20, cudaMemcpyDeviceToHost, st));
-            if (batch_f32_host)
-                MS_CUDA(cudaMemcpyAsync(batch_f32_host, d_batch, (size_t)nc * one_f, cudaMemcpyDeviceToHost, st));
+            if (batch_host)
+                MS_CUDA(cudaMemcpyAsync(batch_host, d_batch, (size_t)nc * one_f, cudaMemcpyDeviceToHost, st));
         }
     }
     MS_CUDA(cudaStreamSynchronize(st));
@@ -1285,13 +1333,26 @@ extern "C" int ms_page_batch_host(ms_ctx *ctx, const float *score, const float *
     return MS_OK;
 }
 
+extern "C" int ms_page_batch_host(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
+                                  int map_h, int map_w, int img_h, int img_w, const ms_east_params *p,
+                                  int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
+                                  int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
+                                  float *batch_f32_host, float **batch_dev_out, int32_t *flags)
+{
+    return ms_page_batch_host_ex(ctx, score, geo, pages, n_pages, map_h, map_w, img_h, img_w, p, min_text_size, out_h,
+                                 out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch_f32_host,
+                                 MS_DTYPE_F32, reinterpret_cast<void **>(batch_dev_out), flags);
+}
+
 // ---- SURVEY 8f-4: rectified crops of rotated quads (an extension; see quadcrop.cu) ------------------------------------
-extern "C" int ms_quad_crop_resize_pad(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w,
-                                       const float *quads, int quad_stride, const int32_t *page_of, int64_t n,
-                                       int min_text_size, int border_mode, int border_value, int out_h, int out_w,
-                                       float *batch_f32, uint8_t *canvas_u8, int32_t *sizes_out, void *stream)
+extern "C" int ms_quad_crop_resize_pad_ex(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w,
+                                          const float *quads, int quad_stride, const int32_t *page_of, int64_t n,
+                                          int min_text_size, int border_mode, int border_value, int out_h, int out_w,
+                                          void *batch, int batch_dtype, uint8_t *canvas_u8, int32_t *sizes_out,
+                                          void *stream)
 {
     MS_CTX(ctx);
+    MS_TRY(dtype_ok(batch_dtype, "ms_quad_crop_resize_pad"));
     if (n < 0 || (n > 0 && (!pages || !quads))) {
         ms_set_error("ms_quad_crop_resize_pad: bad arguments");
         return MS_ERR_INVALID;
@@ -1300,7 +1361,17 @@ extern "C" int ms_quad_crop_resize_pad(ms_ctx *ctx, const uint8_t *pages, int n_
     MS_TRY(ms_arena_reserve(ctx, msk_quad_crop_scratch(n)));
     ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
     return msk_quad_crop(ctx, pages, n_pages, img_h, img_w, quads, quad_stride, page_of, n, min_text_size, border_mode,
-                         border_value, out_h, out_w, batch_f32, canvas_u8, sizes_out, bump, (cudaStream_t)stream);
+                         border_value, out_h, out_w, batch, batch_dtype, canvas_u8, sizes_out, bump, (cudaStream_t)stream);
+}
+
+extern "C" int ms_quad_crop_resize_pad(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w,
+                                       const float *quads, int quad_stride, const int32_t *page_of, int64_t n,
+                                       int min_text_size, int border_mode, int border_value, int out_h, int out_w,
+                                       float *batch_f32, uint8_t *canvas_u8, int32_t *sizes_out, void *stream)
+{
+    return ms_quad_crop_resize_pad_ex(ctx, pages, n_pages, img_h, img_w, quads, quad_stride, page_of, n, min_text_size,
+                                      border_mode, border_value, out_h, out_w, batch_f32, MS_DTYPE_F32, canvas_u8,
+                                      sizes_out, stream);
 }
 
 extern "C" int ms_quad_crop_last_counts(ms_ctx *ctx, int32_t *counts)
@@ -1351,7 +1422,7 @@ extern "C" int ms_quad_crop_resize_pad_host(ms_ctx *ctx, const uint8_t *page, in
     MS_TRY(ms_arena_reserve(ctx, msk_quad_crop_scratch(n)));
     ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
     MS_TRY(msk_quad_crop(ctx, d_page, 1, img_h, img_w, d_quads, 8, nullptr, n, min_text_size, border_mode, border_value,
-                         out_h, out_w, d_f, d_u, d_sizes, bump, st));
+                         out_h, out_w, d_f, MS_DTYPE_F32, d_u, d_sizes, bump, st));
     if (batch_f32) MS_CUDA(cudaMemcpyAsync(batch_f32, d_f, (size_t)n * one_f, cudaMemcpyDeviceToHost, st));
     if (canvas_u8) MS_CUDA(cudaMemcpyAsync(canvas_u8, d_u, (size_t)n * one_u, cudaMemcpyDeviceToHost, st));
     if (sizes_out) MS_CUDA(cudaMemcpyAsync(sizes_out, d_sizes, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
@@ -1393,13 +1464,15 @@ extern "C" int ms_warp_quad_host(ms_ctx *ctx, const uint8_t *page, int img_h, in
 // ---- page images of their own sizes (a batch of originals, as EAST.predict + Pipeline.predict see them) ------------------
 // Host buffers: pages[i] -> (page_hw[2i], page_hw[2i+1], 3) u8.  Maps are uploaded whole, the images one by one into a
 // packed staging buffer (256-byte aligned starts); one pass, no chunk pipelining.
-extern "C" int ms_page_batch_ragged_host(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *const *pages,
-                                         const int32_t *page_hw, int n_pages, int map_h, int map_w,
-                                         const ms_east_params *p, int min_text_size, int out_h, int out_w, int cap_boxes,
-                                         float *boxes_out, int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
-                                         int32_t *n_crops, float *batch_f32_host, float **batch_dev_out, int32_t *flags)
+extern "C" int ms_page_batch_ragged_host_ex(ms_ctx *ctx, const float *score, const float *geo,
+                                            const uint8_t *const *pages, const int32_t *page_hw, int n_pages, int map_h,
+                                            int map_w, const ms_east_params *p, int min_text_size, int out_h, int out_w,
+                                            int cap_boxes, float *boxes_out, int32_t *box_counts, int32_t *crops_out,
+                                            int64_t crops_cap, int32_t *n_crops, void *batch_host, int batch_dtype,
+                                            void **batch_dev_out, int32_t *flags)
 {
     MS_CTX(ctx);
+    MS_TRY(dtype_ok(batch_dtype, "ms_page_batch_ragged_host"));
     if (n_pages <= 0) return MS_OK;
     if (!score || !geo || !p || !pages || !page_hw || !boxes_out || !box_counts || !flags || !crops_out || !n_crops ||
         cap_boxes <= 0 || map_h <= 0 || map_w <= 0 || crops_cap <= 0) {
@@ -1414,10 +1487,10 @@ extern "C" int ms_page_batch_ragged_host(ms_ctx *ctx, const float *score, const 
         }
         img_total += al256((size_t)page_hw[2 * i] * page_hw[2 * i + 1] * 3);
     }
-    const bool want_batch = batch_f32_host || batch_dev_out;
-    float *caller_batch = batch_dev_out ? *batch_dev_out : nullptr;  // caller-owned device buffer (see ms_page_batch_host)
+    const bool want_batch = batch_host || batch_dev_out;
+    void *caller_batch = batch_dev_out ? *batch_dev_out : nullptr;  // caller-owned device buffer (see ms_page_batch_host)
     const size_t plane = (size_t)map_h * map_w;
-    const size_t one_f = (size_t)3 * out_h * out_w * sizeof(float);
+    const size_t one_f = (size_t)3 * out_h * out_w * ms_dtype_bytes(batch_dtype);  // bytes of one crop of the batch
     size_t need = al256(n_pages * plane * 4) + al256(n_pages * plane * 32) + al256((size_t)n_pages * cap_boxes * 36) +
                   4 * al256((size_t)n_pages * 8) + img_total + al256((size_t)crops_cap * 20) + 8192;
     if (want_batch && !caller_batch) need += al256((size_t)crops_cap * one_f);
@@ -1432,7 +1505,7 @@ extern "C" int ms_page_batch_ragged_host(ms_ctx *ctx, const float *score, const 
     int32_t *d_hw = sb.take<int32_t>((size_t)n_pages * 2);
     int32_t *d_crops = sb.take<int32_t>((size_t)crops_cap * 5);
     int32_t *d_nc = sb.take<int32_t>(1);
-    float *d_batch = !want_batch ? nullptr : caller_batch ? caller_batch : sb.take<float>((size_t)crops_cap * 3 * out_h * out_w);
+    void *d_batch = !want_batch ? nullptr : caller_batch ? caller_batch : sb.take<char>((size_t)crops_cap * one_f);
     uint8_t *d_img = sb.take<uint8_t>(img_total);
     if (!d_img || (want_batch && !d_batch)) {
         ms_set_error("ms_page_batch_ragged_host: staging too small");
@@ -1453,8 +1526,8 @@ extern "C" int ms_page_batch_ragged_host(ms_ctx *ctx, const float *score, const 
     MS_CUDA(cudaMemcpyAsync(d_geo, geo, n_pages * plane * 32, cudaMemcpyHostToDevice, st));
     MS_CUDA(cudaStreamSynchronize(st));  // h_ptrs is pageable host memory on this frame
     MS_TRY(page_batch_impl(ctx, d_score, d_geo, nullptr, n_pages, 0, n_pages, map_h, map_w, 0, 0, p, min_text_size, out_h,
-                           out_w, cap_boxes, d_boxes, d_cnt, d_crops, crops_cap, d_nc, 0, d_batch, nullptr, d_flags, st, 0,
-                           d_ptrs, d_hw));
+                           out_w, cap_boxes, d_boxes, d_cnt, d_crops, crops_cap, d_nc, 0, d_batch, batch_dtype, nullptr,
+                           d_flags, st, 0, d_ptrs, d_hw));
     MS_CUDA(cudaMemcpyAsync(box_counts, d_cnt, (size_t)n_pages * 4, cudaMemcpyDeviceToHost, st));
     MS_CUDA(cudaMemcpyAsync(flags, d_flags, (size_t)n_pages * 4, cudaMemcpyDeviceToHost, st));
     MS_CUDA(cudaMemcpyAsync(boxes_out, d_boxes, (size_t)n_pages * cap_boxes * 36, cudaMemcpyDeviceToHost, st));
@@ -1463,18 +1536,29 @@ extern "C" int ms_page_batch_ragged_host(ms_ctx *ctx, const float *score, const 
     int32_t all = 0;
     for (int i = 0; i < n_pages; i++) all |= flags[i];
     if (grow_edge_factor(ctx, all))
-        return ms_page_batch_ragged_host(ctx, score, geo, pages, page_hw, n_pages, map_h, map_w, p, min_text_size, out_h,
-                                         out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops,
-                                         batch_f32_host, batch_dev_out, flags);
+        return ms_page_batch_ragged_host_ex(ctx, score, geo, pages, page_hw, n_pages, map_h, map_w, p, min_text_size,
+                                            out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops,
+                                            batch_host, batch_dtype, batch_dev_out, flags);
     MS_TRY(flags_to_rc(all, "page_batch_ragged"));
     int64_t nc = *n_crops;
     if (nc > crops_cap) nc = crops_cap;
     if (nc > 0) {
         MS_CUDA(cudaMemcpyAsync(crops_out, d_crops, (size_t)nc * 20, cudaMemcpyDeviceToHost, st));
-        if (batch_f32_host)
-            MS_CUDA(cudaMemcpyAsync(batch_f32_host, d_batch, (size_t)nc * one_f, cudaMemcpyDeviceToHost, st));
+        if (batch_host)
+            MS_CUDA(cudaMemcpyAsync(batch_host, d_batch, (size_t)nc * one_f, cudaMemcpyDeviceToHost, st));
         MS_CUDA(cudaStreamSynchronize(st));
     }
     if (batch_dev_out) *batch_dev_out = d_batch;
     return MS_OK;
+}
+
+extern "C" int ms_page_batch_ragged_host(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *const *pages,
+                                         const int32_t *page_hw, int n_pages, int map_h, int map_w,
+                                         const ms_east_params *p, int min_text_size, int out_h, int out_w, int cap_boxes,
+                                         float *boxes_out, int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
+                                         int32_t *n_crops, float *batch_f32_host, float **batch_dev_out, int32_t *flags)
+{
+    return ms_page_batch_ragged_host_ex(ctx, score, geo, pages, page_hw, n_pages, map_h, map_w, p, min_text_size, out_h,
+                                        out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops,
+                                        batch_f32_host, MS_DTYPE_F32, reinterpret_cast<void **>(batch_dev_out), flags);
 }

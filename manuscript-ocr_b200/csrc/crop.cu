@@ -11,9 +11,10 @@
 //                 or the float decimation-table path, accumulated in OpenCV's order
 //   same size:    copy
 // then paste at (x0=0, y0=(ih-new_h)//2) on a 255 canvas, (v - 127.5) * (1/127.5) in f32, HWC -> CHW.
+// The batch is float32, or (an extension) float16 / bfloat16: the same f32 value rounded to nearest-even.
 //
-// HBM roofline: per crop 3*w*h source bytes read + 3*ih*iw*4 bytes written (49 152 B at 32x128): the
-// kernel is write dominated.
+// HBM roofline: per crop 3*w*h source bytes read + 3*ih*iw*sizeof(element) bytes written (49 152 B at 32x128 in
+// float32, 24 576 B in 16 bits): the kernel is write dominated.
 //
 // Kernels:
 //   crop_plan_kernel        thread per crop: the float64 sizing arithmetic of transforms.py:91-98, interpolation mode,
@@ -225,11 +226,11 @@ __global__ void __launch_bounds__(256) crop_bucket_scatter_kernel(const Plan *__
 constexpr int kProducerWarps = 2;
 constexpr int kConsumerWarps = kThreads / 32 - kProducerWarps;
 
-template <bool kWriteF32, bool kWriteU8>
+template <class T, bool kWriteU8>
 __global__ void __launch_bounds__(kThreads, kCtasPerSm)
     crop_resize_pad_kernel(const Plan *__restrict__ plans, const StageDesc *__restrict__ work,
                            const int32_t *__restrict__ n_work_dev, int32_t *__restrict__ ticket, int ring_bytes, int ih,
-                           int iw, float *__restrict__ batch, uint8_t *__restrict__ canvas_out, int vec_ok,
+                           int iw, T *__restrict__ batch, uint8_t *__restrict__ canvas_out, int vec_ok,
                            uint8_t *__restrict__ redo)
 {
     ms_pdl_wait();
@@ -269,7 +270,7 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
             }
             __syncwarp();  // every lane's table stores are ordered before lane 0's releasing arrive
             if (lane == 0) mbar_arrive(&s_stage.full[s]);
-            write_padding<kWriteF32, kWriteU8>(p.nw, p.nh, p.y0, ih, iw, kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr,
+            write_padding<T, kWriteU8>(p.nw, p.nh, p.y0, ih, iw, kHasBatch<T> ? batch + (size_t)ci * 3 * plane : nullptr,
                                                kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr, vec_ok, lane, 32);
         }
         return;
@@ -286,23 +287,23 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm)
         const uint32_t pitch = (uint32_t)s_meta[s][3], a0 = (uint32_t)s_meta[s][4], sstep = (uint32_t)s_meta[s][5];
         const int G = s_meta[s][7];
         const uint32_t stage_off = (uint32_t)s_stage.off[s];
-        float *dstf = kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr;
+        T *dstf = kHasBatch<T> ? batch + (size_t)ci * 3 * plane : nullptr;
         uint8_t *dstu = kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr;
         const uint32_t *tab = tabs + (size_t)s * tab_n;
         // three x taps at most (shrink factor below 2, most word boxes): a quarter of the horizontal work less; a page
         // stride that is a multiple of 16 bytes (sstep == 0): no per-row misalignment arithmetic
         bool bad = false;
         if (s_meta[s][6] == 2)
-            area2x2_pixels<kWriteF32, kWriteU8, kCT>(smem, stage_off, pitch, a0, sstep, ih, iw, nw, nh, y0, dstf, dstu, ct);
+            area2x2_pixels<T, kWriteU8, kCT>(smem, stage_off, pitch, a0, sstep, ih, iw, nw, nh, y0, dstf, dstu, ct);
         else if (sstep == 0)
-            bad = s_meta[s][6] == 1 ? area4_strips<kWriteF32, kWriteU8, kCT, 3, true>(smem, stage_off, pitch, a0, 0u, tab, tab_n, ih,
+            bad = s_meta[s][6] == 1 ? area4_strips<T, kWriteU8, kCT, 3, true>(smem, stage_off, pitch, a0, 0u, tab, tab_n, ih,
                                                                                  iw, nw, nh, y0, dstf, dstu, ct, G)
-                               : area4_strips<kWriteF32, kWriteU8, kCT, 4, true>(smem, stage_off, pitch, a0, 0u, tab, tab_n, ih,
+                               : area4_strips<T, kWriteU8, kCT, 4, true>(smem, stage_off, pitch, a0, 0u, tab, tab_n, ih,
                                                                                  iw, nw, nh, y0, dstf, dstu, ct, G);
         else
-            bad = s_meta[s][6] == 1 ? area4_strips<kWriteF32, kWriteU8, kCT, 3>(smem, stage_off, pitch, a0, sstep, tab, tab_n, ih, iw,
+            bad = s_meta[s][6] == 1 ? area4_strips<T, kWriteU8, kCT, 3>(smem, stage_off, pitch, a0, sstep, tab, tab_n, ih, iw,
                                                                            nw, nh, y0, dstf, dstu, ct, G)
-                               : area4_strips<kWriteF32, kWriteU8, kCT, 4>(smem, stage_off, pitch, a0, sstep, tab, tab_n, ih, iw,
+                               : area4_strips<T, kWriteU8, kCT, 4>(smem, stage_off, pitch, a0, sstep, tab, tab_n, ih, iw,
                                                                            nw, nh, y0, dstf, dstu, ct, G);
         if (bad) redo[ci] = 1;  // a table entry with more than 4 taps: the generic kernel redoes the crop
         stage_release(s_stage, s);
@@ -330,11 +331,11 @@ __global__ void __launch_bounds__(256) crop_generic_list_kernel(const Plan *__re
 // coefficient tables in shared memory, then one thread per destination pixel.
 constexpr int kGenericMaxTab = 1024;  // table entries kept in shared memory (longer axes recompute per pixel)
 
-template <bool kWriteF32, bool kWriteU8>
+template <class T, bool kWriteU8>
 __global__ void __launch_bounds__(256) crop_generic_kernel(const Plan *__restrict__ plans,
                                                            const int32_t *__restrict__ list,
                                                            const int32_t *__restrict__ list_n, int ih, int iw,
-                                                           float *__restrict__ batch,
+                                                           T *__restrict__ batch,
                                                            uint8_t *__restrict__ canvas_out, int vec_ok)
 {
     ms_pdl_wait();
@@ -345,15 +346,15 @@ __global__ void __launch_bounds__(256) crop_generic_kernel(const Plan *__restric
         const int64_t ci = list[li];
         Plan p = plans[ci];
         if (!p.ok) p.nw = p.nh = 0;  // an invalid rectangle pastes nothing: the canvas is all padding
-        float *dstf = kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr;
+        T *dstf = kHasBatch<T> ? batch + (size_t)ci * 3 * plane : nullptr;
         uint8_t *dstu = kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr;
-        write_padding<kWriteF32, kWriteU8>(p, ih, iw, dstf, dstu, vec_ok, threadIdx.x, blockDim.x);
+        write_padding<T, kWriteU8>(p, ih, iw, dstf, dstu, vec_ok, threadIdx.x, blockDim.x);
         const bool need_tab = p.ok && (p.interp == 1 || p.interp == 3);
         const bool tab_ok = need_tab && p.nw + p.nh <= kGenericMaxTab;
         __syncthreads();  // the previous crop's table is no longer read
         if (tab_ok) fill_axis_table(p, s_tab);
         __syncthreads();
-        resample_canvas<kWriteF32, kWriteU8>(p, PitchedSrc{p.src, (size_t)p.stride}, s_tab, tab_ok, need_tab, ih, iw, dstf,
+        resample_canvas<T, kWriteU8>(p, PitchedSrc{p.src, (size_t)p.stride}, s_tab, tab_ok, need_tab, ih, iw, dstf,
                                              dstu);
     }
 }
@@ -429,12 +430,12 @@ size_t msk_crop_scratch(int64_t crops_cap, int n_pages)
 }
 
 int msk_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w, const int32_t *crops,
-             const int32_t *n_crops, const int32_t *range, int64_t crops_cap, int out_h, int out_w, float *batch_f32,
-             uint8_t *canvas_u8, ms_bump bump, cudaStream_t st, const uint8_t *const *page_ptrs, const int32_t *page_hw)
+             const int32_t *n_crops, const int32_t *range, int64_t crops_cap, int out_h, int out_w, void *batch,
+             int batch_dtype, uint8_t *canvas_u8, ms_bump bump, cudaStream_t st, const uint8_t *const *page_ptrs, const int32_t *page_hw)
 {
     if (crops_cap <= 0 || n_pages <= 0) return MS_OK;
     const bool ragged = page_ptrs != nullptr && page_hw != nullptr;
-    if (out_h <= 0 || out_w <= 0 || (!ragged && (img_h <= 0 || img_w <= 0 || !pages)) || (!batch_f32 && !canvas_u8)) {
+    if (out_h <= 0 || out_w <= 0 || (!ragged && (img_h <= 0 || img_w <= 0 || !pages)) || (!batch && !canvas_u8)) {
         ms_set_error("crop: bad arguments");
         return MS_ERR_INVALID;
     }
@@ -485,17 +486,18 @@ int msk_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_
     // one CTA per listed crop, many in flight: a generic crop reads global memory byte by byte and is latency bound
     int64_t ggrid = (int64_t)ctx->num_sms * 8;
     if (ggrid > crops_cap) ggrid = crops_cap;
-    const int vec_ok = ((out_w & 3) == 0 && (reinterpret_cast<uintptr_t>(batch_f32) & 15) == 0) ? 1 : 0;
-    return launch_for_outputs(batch_f32, canvas_u8, [&](auto f32, auto u8) {
-        constexpr bool kF32 = decltype(f32)::value, kU8 = decltype(u8)::value;
-        constexpr ms_smem_slot slot = kF32 ? (kU8 ? MS_SMEM_CROP_BOTH : MS_SMEM_CROP_F32) : MS_SMEM_CROP_U8;
-        MS_TRY(ms_allow_smem(ctx, slot, crop_resize_pad_kernel<kF32, kU8>, (int)smem));
-        ms_launch(crop_resize_pad_kernel<kF32, kU8>, (int)grid, kThreads, smem, st, plans, work, n_work, ticket, (int)ring,
-                  out_h, out_w, batch_f32, canvas_u8, vec_ok, redo);
+    return launch_for_outputs(batch, batch_dtype, canvas_u8, [&](auto bt, auto u8) {
+        using T = typename decltype(bt)::type;
+        constexpr bool kU8 = decltype(u8)::value;
+        T *out = static_cast<T *>(batch);
+        const int vec_ok = batch_vec_ok<T>(batch, out_w);
+        MS_TRY(ms_allow_smem(ctx, batch_slot<T, kU8>(MS_SMEM_CROP_U8), crop_resize_pad_kernel<T, kU8>, (int)smem));
+        ms_launch(crop_resize_pad_kernel<T, kU8>, (int)grid, kThreads, smem, st, plans, work, n_work, ticket, (int)ring,
+                  out_h, out_w, out, canvas_u8, vec_ok, redo);
         MS_LAUNCH_CHECK(ctx);
         ms_launch(crop_generic_list_kernel, (int)lgrid, 256, 0, st, plans, n_crops, range, crops_cap, redo, glist, glist_n);
         MS_LAUNCH_CHECK(ctx);
-        ms_launch(crop_generic_kernel<kF32, kU8>, (int)ggrid, 256, 0, st, plans, glist, glist_n, out_h, out_w, batch_f32,
+        ms_launch(crop_generic_kernel<T, kU8>, (int)ggrid, 256, 0, st, plans, glist, glist_n, out_h, out_w, out,
                   canvas_u8, vec_ok);
         MS_LAUNCH_CHECK(ctx);
         return MS_OK;

@@ -2,11 +2,40 @@
 // of one crop, OpenCV's coefficient-table entries and the per-pixel resampling arithmetic (cv2.resize restated, see
 // crop.cu), and the 255-padding writer.
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include <type_traits>
 
 #include "ms_internal.cuh"
 
 namespace {
+
+// ---- batch element types -----------------------------------------------------------------------------------------
+// The crop kernels are instantiated for the element type of the network-input batch they write: float, __half,
+// __nv_bfloat16, or NoBatch (only the u8 canvas is written).  Every value is normalised in float32 and then converted
+// with round-to-nearest-even, so a 16-bit batch is bit for bit the float32 batch cast with torch's .to(dtype).
+struct NoBatch {};
+template <class T>
+constexpr bool kHasBatch = !std::is_same<T, NoBatch>::value;
+
+template <class T>
+__device__ __forceinline__ T to_batch(float v);
+template <>
+__device__ __forceinline__ float to_batch<float>(float v) { return v; }
+template <>
+__device__ __forceinline__ __half to_batch<__half>(float v) { return __float2half_rn(v); }
+template <>
+__device__ __forceinline__ __nv_bfloat16 to_batch<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+__device__ __forceinline__ uint32_t batch_bits(__half v) { return __half_as_ushort(v); }
+__device__ __forceinline__ uint32_t batch_bits(__nv_bfloat16 v) { return __bfloat16_as_ushort(v); }
+
+// one normalised batch value ((v - 127.5) / 127.5 as the reference's f32 expression), streaming store
+template <class T>
+__device__ __forceinline__ void store_norm(T *p, float v)
+{
+    __stcs(p, to_batch<T>((v - 127.5f) * (1.0f / 127.5f)));
+}
 
 // ---- mbarrier + TMA bulk copy (sm_90+ PTX; SASS: SYNCS / UBLKCP) ----------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -487,11 +516,11 @@ __device__ __forceinline__ void fill_axis_table(const Plan &p, AxisEnt *tab)
     }
 }
 
-// ... then a thread per pasted pixel, f32 and / or u8 stores.  tab_ok: the entries are in s_tab; otherwise, when the
-// mode needs entries (need_tab), every pixel computes its own.
-template <bool kWriteF32, bool kWriteU8, class Src>
+// ... then a thread per pasted pixel, batch (element type T) and / or u8 stores.  tab_ok: the entries are in s_tab;
+// otherwise, when the mode needs entries (need_tab), every pixel computes its own.
+template <class T, bool kWriteU8, class Src>
 __device__ __forceinline__ void resample_canvas(const Plan &p, const Src &src, const AxisEnt *s_tab, bool tab_ok,
-                                                bool need_tab, int ih, int iw, float *dstf, uint8_t *dstu)
+                                                bool need_tab, int ih, int iw, T *dstf, uint8_t *dstu)
 {
     const int plane = ih * iw;
     const float inv = 1.0f / 127.5f;
@@ -509,10 +538,10 @@ __device__ __forceinline__ void resample_canvas(const Plan &p, const Src &src, c
         unsigned char o0, o1, o2;
         resample_px(p, dx, dy, src, ex, ey, o0, o1, o2);
         const int at = (p.y0 + dy) * iw + dx;
-        if (kWriteF32) {
-            dstf[at] = ((float)o0 - 127.5f) * inv;
-            dstf[plane + at] = ((float)o1 - 127.5f) * inv;
-            dstf[2 * plane + at] = ((float)o2 - 127.5f) * inv;
+        if constexpr (kHasBatch<T>) {
+            dstf[at] = to_batch<T>(((float)o0 - 127.5f) * inv);
+            dstf[plane + at] = to_batch<T>(((float)o1 - 127.5f) * inv);
+            dstf[2 * plane + at] = to_batch<T>(((float)o2 - 127.5f) * inv);
         }
         if (kWriteU8) {
             dstu[(size_t)at * 3] = o0;
@@ -522,24 +551,38 @@ __device__ __forceinline__ void resample_canvas(const Plan &p, const Src &src, c
     }
 }
 
+// Batch elements per 16-byte vector store: 4 float, 8 __half / __nv_bfloat16.  The padding writer's vector path needs
+// out_w to be a multiple of it and a 16-byte-aligned batch (the host's vec_ok).
+template <class T>
+constexpr int kBatchVec = sizeof(T) == 2 ? 8 : 4;
+
 // Everything outside the pasted rectangle is the 255 canvas (transforms.py:100), 1.0f after normalisation; written
 // as constant 16-byte streaming stores by `nthreads` cooperating threads.
-template <bool kWriteF32, bool kWriteU8>
-__device__ __forceinline__ void write_padding(int nw, int nh, int y0, int ih, int iw, float *dstf, uint8_t *dstu,
+template <class T, bool kWriteU8>
+__device__ __forceinline__ void write_padding(int nw, int nh, int y0, int ih, int iw, T *dstf, uint8_t *dstu,
                                               int vec_ok, int tid, int nthreads)
 {
     const int plane = ih * iw;
-    if (kWriteF32) {
-        const float one = (255.0f - 127.5f) * (1.0f / 127.5f);
+    if constexpr (kHasBatch<T>) {
+        constexpr int kV = kBatchVec<T>;
+        const T one = to_batch<T>((255.0f - 127.5f) * (1.0f / 127.5f));
         if (vec_ok) {
-            const float4 one4 = make_float4(one, one, one, one);
-            const int nw4 = (nw + 3) & ~3;
-            const int top4 = y0 * iw / 4, bot4 = (ih - y0 - nh) * iw / 4, tail4 = (iw - nw4) / 4;
+            // kV copies of `one` in 16 bytes
+            float4 one4;
+            if constexpr (sizeof(T) == 4) {
+                one4 = make_float4(one, one, one, one);
+            } else {
+                const uint32_t b = batch_bits(one);
+                const float v2 = __uint_as_float(b | (b << 16));
+                one4 = make_float4(v2, v2, v2, v2);
+            }
+            const int nw4 = (nw + kV - 1) & ~(kV - 1);
+            const int top4 = y0 * iw / kV, bot4 = (ih - y0 - nh) * iw / kV, tail4 = (iw - nw4) / kV;
             const int fr = nw4 - nw;  // scalar fringe [nw, nw4)
             // the pasted rectangle sits at the same place in every channel: one index computation, a store per channel
             float4 *top = reinterpret_cast<float4 *>(dstf);
             float4 *bot = reinterpret_cast<float4 *>(dstf + (size_t)(y0 + nh) * iw);
-            const int plane4 = plane / 4;
+            const int plane4 = plane / kV;
             for (int i = tid; i < top4; i += nthreads)
                 for (int c = 0; c < 3; c++) __stcs(top + (size_t)c * plane4 + i, one4);
             for (int i = tid; i < bot4; i += nthreads)
@@ -553,7 +596,7 @@ __device__ __forceinline__ void write_padding(int nw, int nh, int y0, int ih, in
                 const int col = tid % tail4, phase = tid / tail4;
                 if (phase < split) {
                     float4 *at = reinterpret_cast<float4 *>(dstf + (size_t)(y0 + phase) * iw + nw4) + col;
-                    const size_t step = (size_t)split * iw / 4;
+                    const size_t step = (size_t)split * iw / kV;
                     for (int k = col; k < tail4; k += nthreads) {  // (tails wider than the thread count: several columns)
                         float4 *p4 = at + (k - col);
                         for (int r = phase; r < nh; r += split, p4 += step)
@@ -564,7 +607,7 @@ __device__ __forceinline__ void write_padding(int nw, int nh, int y0, int ih, in
             if (fr > 0) {
                 for (int i = tid; i < nh * fr; i += nthreads) {
                     const int r = i / fr, k = i - r * fr;
-                    float *at = dstf + (size_t)(y0 + r) * iw + nw + k;
+                    T *at = dstf + (size_t)(y0 + r) * iw + nw + k;
                     for (int c = 0; c < 3; c++) __stcs(at + (size_t)c * plane, one);
                 }
             }
@@ -588,12 +631,12 @@ __device__ __forceinline__ void write_padding(int nw, int nh, int y0, int ih, in
     }
 }
 
-template <bool kWriteF32, bool kWriteU8>
-__device__ __forceinline__ void write_padding(const Plan &p, int ih, int iw, float *dstf, uint8_t *dstu, int vec_ok,
+template <class T, bool kWriteU8>
+__device__ __forceinline__ void write_padding(const Plan &p, int ih, int iw, T *dstf, uint8_t *dstu, int vec_ok,
                                               int tid, int nthreads)
 {
-    write_padding<kWriteF32, kWriteU8>(p.ok ? p.nw : 0, p.ok ? p.nh : 0, p.ok ? p.y0 : 0, ih, iw, dstf, dstu, vec_ok, tid,
-                                       nthreads);
+    write_padding<T, kWriteU8>(p.ok ? p.nw : 0, p.ok ? p.nh : 0, p.ok ? p.y0 : 0, ih, iw, dstf, dstu, vec_ok, tid,
+                               nthreads);
 }
 
 // u8 -> f32 without the conversion pipe: byte k of `v` is spliced under the exponent of 2^23, then 2^23 is
@@ -741,13 +784,12 @@ __device__ __forceinline__ int strip_height(int nw, int nh)
 // INTER_AREA with both scale factors exactly 2 (cv2's integer fast path: (sum of the 2 x 2 block + 2) >> 2), source rows
 // staged like area4_strips'; a thread per destination pixel.  A word box exactly twice the canvas height is common
 // (2.5 % of the benchmark's crops), and its rounding differs from the float-table path, so it has its own routine.
-template <bool kWriteF32, bool kWriteU8, int kCT>
+template <class T, bool kWriteU8, int kCT>
 __device__ __forceinline__ void area2x2_pixels(const unsigned char *smem, uint32_t stage_off, uint32_t pitch, uint32_t a0,
-                                               uint32_t sstep, int ih, int iw, int nw, int nh, int y0, float *dstf,
+                                               uint32_t sstep, int ih, int iw, int nw, int nh, int y0, T *dstf,
                                                uint8_t *dstu, int ct)
 {
     const int plane = ih * iw;
-    const float inv = 1.0f / 127.5f;
     const uint32_t magic = 0xFFFFFFFFu / (uint32_t)nw + 1u;
     for (int t = ct; t < nw * nh; t += kCT) {
         const int dy = nw == 1 ? t : (int)__umulhi((uint32_t)t, magic), dx = t - dy * nw;
@@ -762,10 +804,10 @@ __device__ __forceinline__ void area2x2_pixels(const unsigned char *smem, uint32
         }
         const int o0 = (s0 + 2) >> 2, o1 = (s1 + 2) >> 2, o2 = (s2 + 2) >> 2;
         const int at = (y0 + dy) * iw + dx;
-        if (kWriteF32) {
-            __stcs(dstf + at, ((float)o0 - 127.5f) * inv);
-            __stcs(dstf + plane + at, ((float)o1 - 127.5f) * inv);
-            __stcs(dstf + 2 * plane + at, ((float)o2 - 127.5f) * inv);
+        if constexpr (kHasBatch<T>) {
+            store_norm(dstf + at, (float)o0);
+            store_norm(dstf + plane + at, (float)o1);
+            store_norm(dstf + 2 * plane + at, (float)o2);
         }
         if (kWriteU8) {
             dstu[(size_t)at * 3] = (unsigned char)o0;
@@ -777,16 +819,15 @@ __device__ __forceinline__ void area2x2_pixels(const unsigned char *smem, uint32
 
 // kAligned: the caller guarantees sstep == 0 (source row stride a multiple of 16 bytes: every staged row has the same
 // misalignment a0), so the per-row misalignment arithmetic disappears.
-template <bool kWriteF32, bool kWriteU8, int kCT, int kTaps, bool kAligned = false>
+template <class T, bool kWriteU8, int kCT, int kTaps, bool kAligned = false>
 __device__ __forceinline__ bool area4_strips(const unsigned char *smem, uint32_t stage_off, uint32_t pitch, uint32_t a0,
                                              uint32_t sstep, const uint32_t *tab, int tab_n, int ih, int iw, int nw,
-                                             int nh, int y0, float *dstf, uint8_t *dstu, int ct, int G_in = 0,
+                                             int nh, int y0, T *dstf, uint8_t *dstu, int ct, int G_in = 0,
                                              int dy_lo = 0, int dy_hi = -1)
 {
     // [dy_lo, dy_hi): the destination rows to produce (default: all nh of them); the staged rows are addressed by
     // their absolute source row either way
     const int plane = ih * iw;
-    const float inv = 1.0f / 127.5f;
     const int G = G_in > 0 ? G_in : strip_height<kCT>(nw, nh);
     if (dy_hi < 0) dy_hi = nh;
     const int nitems = ((dy_hi - dy_lo + G - 1) / G) * nw;
@@ -802,7 +843,7 @@ __device__ __forceinline__ bool area4_strips(const unsigned char *smem, uint32_t
         int last_r = -1;
         float b0 = 0.f, b1 = 0.f, b2 = 0.f;
         const int dy_first = dy_lo + grp * G, dy_end = min(dy_hi, dy_first + G);
-        float *orow = kWriteF32 ? dstf + (size_t)(y0 + dy_first) * iw + dx : nullptr;  // walks down the strip's rows
+        T *orow = kHasBatch<T> ? dstf + (size_t)(y0 + dy_first) * iw + dx : nullptr;  // walks down the strip's rows
         for (int dy = dy_first; dy < dy_end; dy++) {
             const uint32_t *yrec = tab + area_tab_ybase(iw) + 8 * dy;
             const uint32_t py = yrec[0];
@@ -833,10 +874,10 @@ __device__ __forceinline__ bool area4_strips(const unsigned char *smem, uint32_t
             // cvRound (half to even), kept as floats: the weights sum to 1 within rounding -> [0, 255]
             const float f0 = rintf(sum0), f1 = rintf(sum1), f2 = rintf(sum2);
             const int at = (y0 + dy) * iw + dx;
-            if (kWriteF32) {
-                __stcs(orow, (f0 - 127.5f) * inv);
-                __stcs(orow + plane, (f1 - 127.5f) * inv);
-                __stcs(orow + 2 * plane, (f2 - 127.5f) * inv);
+            if constexpr (kHasBatch<T>) {
+                store_norm(orow, f0);
+                store_norm(orow + plane, f1);
+                store_norm(orow + 2 * plane, f2);
                 orow += iw;
             }
             if (kWriteU8) {
@@ -849,14 +890,46 @@ __device__ __forceinline__ bool area4_strips(const unsigned char *smem, uint32_t
     return bad;
 }
 
-// The crop kernels are instantiated for the outputs they write: <kWriteF32, kWriteU8> = <true, true>, <true, false> or
-// <false, true>.  Calls launch(std::bool_constant<kWriteF32>, std::bool_constant<kWriteU8>) for the outputs present.
+// The crop kernels are instantiated for the outputs they write: <T, kWriteU8> with T the batch element type (float,
+// __half, __nv_bfloat16) with or without the u8 canvas, or <NoBatch, true>.  Calls
+// launch(BatchType<T>{}, std::bool_constant<kWriteU8>{}) for the outputs present; an unknown batch_dtype is
+// MS_ERR_INVALID.
+template <class T>
+struct BatchType {
+    using type = T;
+};
+
 template <class Launch>
-int launch_for_outputs(const float *batch_f32, const uint8_t *canvas_u8, Launch &&launch)
+int launch_for_outputs(const void *batch, int batch_dtype, const uint8_t *canvas_u8, Launch &&launch)
 {
-    if (batch_f32 && canvas_u8) return launch(std::true_type{}, std::true_type{});
-    if (batch_f32) return launch(std::true_type{}, std::false_type{});
-    return launch(std::false_type{}, std::true_type{});
+    if (!batch) return launch(BatchType<NoBatch>{}, std::true_type{});
+    switch (batch_dtype) {
+    case MS_DTYPE_F32:
+        return canvas_u8 ? launch(BatchType<float>{}, std::true_type{}) : launch(BatchType<float>{}, std::false_type{});
+    case MS_DTYPE_F16:
+        return canvas_u8 ? launch(BatchType<__half>{}, std::true_type{}) : launch(BatchType<__half>{}, std::false_type{});
+    case MS_DTYPE_BF16:
+        return canvas_u8 ? launch(BatchType<__nv_bfloat16>{}, std::true_type{})
+                         : launch(BatchType<__nv_bfloat16>{}, std::false_type{});
+    }
+    ms_set_error("crop: unknown batch dtype %d", batch_dtype);
+    return MS_ERR_INVALID;
+}
+
+// The shared-memory slot of one output instantiation, in the order of a slot group of ms_smem_slot (`first` = the
+// group's u8-only slot): u8, f32, f32 + u8, f16, f16 + u8, bf16, bf16 + u8.
+template <class T, bool kWriteU8>
+constexpr ms_smem_slot batch_slot(ms_smem_slot first)
+{
+    const int t = std::is_same<T, float>::value ? 0 : std::is_same<T, __half>::value ? 1 : 2;
+    return (ms_smem_slot)(first + (kHasBatch<T> ? 1 + 2 * t + (kWriteU8 ? 1 : 0) : 0));
+}
+
+// vec_ok of write_padding for a batch of element type T
+template <class T>
+int batch_vec_ok(const void *batch, int out_w)
+{
+    return (out_w % kBatchVec<T> == 0 && (reinterpret_cast<uintptr_t>(batch) & 15) == 0) ? 1 : 0;
 }
 
 }  // namespace

@@ -14,7 +14,7 @@
 // One recorded ms_page_batch call (all arguments) and, from its second occurrence on, the CUDA graph of its launches.
 struct ms_pb_key {
     const void *ptr[14];
-    long long num[12];
+    long long num[13];
     ms_east_params params;
 };
 struct ms_graph_entry {
@@ -28,17 +28,30 @@ struct ms_graph_entry {
 #define MS_GRAPH_SLOTS 4
 
 // The kernels launched with more dynamic shared memory than the default 48 KB allows (ms_allow_smem); the crop kernels
-// once per output instantiation: f32 batch, u8 canvas, both.
+// once per output instantiation, in groups of seven (batch_slot, crop_common.cuh): u8 canvas only, then each batch
+// element type (f32, f16, bf16) without and with the u8 canvas.
 enum ms_smem_slot {
-    MS_SMEM_CROP_F32,
     MS_SMEM_CROP_U8,
-    MS_SMEM_CROP_BOTH,
-    MS_SMEM_QUAD_F32,
+    MS_SMEM_CROP_F32,
+    MS_SMEM_CROP_F32_U8,
+    MS_SMEM_CROP_F16,
+    MS_SMEM_CROP_F16_U8,
+    MS_SMEM_CROP_BF16,
+    MS_SMEM_CROP_BF16_U8,
     MS_SMEM_QUAD_U8,
-    MS_SMEM_QUAD_BOTH,
-    MS_SMEM_QUAD_STAGED_F32,
+    MS_SMEM_QUAD_F32,
+    MS_SMEM_QUAD_F32_U8,
+    MS_SMEM_QUAD_F16,
+    MS_SMEM_QUAD_F16_U8,
+    MS_SMEM_QUAD_BF16,
+    MS_SMEM_QUAD_BF16_U8,
     MS_SMEM_QUAD_STAGED_U8,
-    MS_SMEM_QUAD_STAGED_BOTH,
+    MS_SMEM_QUAD_STAGED_F32,
+    MS_SMEM_QUAD_STAGED_F32_U8,
+    MS_SMEM_QUAD_STAGED_F16,
+    MS_SMEM_QUAD_STAGED_F16_U8,
+    MS_SMEM_QUAD_STAGED_BF16,
+    MS_SMEM_QUAD_STAGED_BF16_U8,
     MS_SMEM_READING_ORDER,
     MS_SMEM_READING_ORDER_LARGE,
     MS_SMEM_SLOTS
@@ -99,6 +112,11 @@ struct ms_bump {
 };
 
 void ms_set_error(const char *fmt, ...);
+// bytes of one batch element of an MS_DTYPE_* code; 0 for an unknown code
+inline size_t ms_dtype_bytes(int dtype)
+{
+    return dtype == MS_DTYPE_F32 ? 4 : (dtype == MS_DTYPE_F16 || dtype == MS_DTYPE_BF16) ? 2 : 0;
+}
 int ms_check_cuda(cudaError_t e, const char *what);
 // bump allocator over ctx->arena; ms_arena_reserve grows it (synchronises the device when it does)
 int ms_arena_reserve(ms_ctx *ctx, size_t bytes);
@@ -211,9 +229,10 @@ int msk_reading_order(ms_ctx *ctx, const float *boxes8, int row_stride, const in
                       int cap_per_page, int32_t *order, float *reordered, int32_t *flags, ms_bump bump, cudaStream_t st);
 size_t msk_reading_order_scratch(int n_pages, int cap_per_page);
 // crop.cu
+// batch: (crops_cap, 3, out_h, out_w) of batch_dtype (MS_DTYPE_*), or NULL
 int msk_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w, const int32_t *crops,
-             const int32_t *n_crops, const int32_t *range, int64_t crops_cap, int out_h, int out_w, float *batch_f32,
-             uint8_t *canvas_u8, ms_bump bump, cudaStream_t st, const uint8_t *const *page_ptrs = nullptr,
+             const int32_t *n_crops, const int32_t *range, int64_t crops_cap, int out_h, int out_w, void *batch,
+             int batch_dtype, uint8_t *canvas_u8, ms_bump bump, cudaStream_t st, const uint8_t *const *page_ptrs = nullptr,
              const int32_t *page_hw = nullptr);  // page_ptrs / page_hw (device): pages of their own sizes
 // tps.cu
 int msk_tps_rectify(ms_ctx *ctx, const float *input, const float *c_prime, const float *inv_delta_c, const float *p_hat_t,
@@ -224,8 +243,8 @@ size_t msk_crop_scratch(int64_t crops_cap, int n_pages);
 // quadcrop.cu
 int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w, const float *quads,
                   int quad_stride, const int32_t *page_of, int64_t n, int min_text_size, int border_mode,
-                  int border_value, int out_h, int out_w, float *batch_f32, uint8_t *canvas_u8, int32_t *sizes_out,
-                  ms_bump bump, cudaStream_t st);
+                  int border_value, int out_h, int out_w, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                  int32_t *sizes_out, ms_bump bump, cudaStream_t st);
 size_t msk_quad_crop_scratch(int64_t n);
 int msk_quad_warp(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, const float *quad_dev, int border_mode,
                   int border_value, uint8_t *patch_dev, size_t patch_cap, int *w, int *h, ms_bump bump, cudaStream_t st);

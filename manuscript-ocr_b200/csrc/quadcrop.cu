@@ -1,4 +1,5 @@
-// Rectified crops of rotated word quads -> resize-and-pad -> normalise -> CHW float32 batch (SURVEY 8f-4).
+// Rectified crops of rotated word quads -> resize-and-pad -> normalise -> CHW float32 / float16 / bfloat16 batch
+// (SURVEY 8f-4).
 //
 // NOT a reference behaviour: the reference crops the axis-aligned bounding rectangle of every polygon
 // (_pipeline.py:204-221) and lists the rotated crop as future work (todo.md:1).  The operation is defined through the
@@ -347,12 +348,12 @@ struct WarpSrc {
     }
 };
 
-template <bool kWriteF32, bool kWriteU8>
+template <class T, bool kWriteU8>
 __global__ void __launch_bounds__(kQcThreads, 4) quad_crop_kernel(const uint8_t *__restrict__ pages, int img_h,
                                                                   int img_w, const QuadPlan *__restrict__ qplans,
                                                                   const Plan *__restrict__ plans, int64_t n,
                                                                   int replicate, int bval, int ih, int iw,
-                                                                  float *__restrict__ batch,
+                                                                  T *__restrict__ batch,
                                                                   uint8_t *__restrict__ canvas_out, int vec_ok,
                                                                   const int32_t *__restrict__ list,
                                                                   const int32_t *__restrict__ list_n)
@@ -374,9 +375,9 @@ __global__ void __launch_bounds__(kQcThreads, 4) quad_crop_kernel(const uint8_t 
         __syncthreads();  // the previous quad's plan, patch and tables are no longer read
         if (threadIdx.x == 0) s_qp = qplans[ci];
         const Plan p = plans[ci];
-        float *dstf = kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr;
+        T *dstf = kHasBatch<T> ? batch + (size_t)ci * 3 * plane : nullptr;
         uint8_t *dstu = kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr;
-        write_padding<kWriteF32, kWriteU8>(p, ih, iw, dstf, dstu, vec_ok, threadIdx.x, blockDim.x);
+        write_padding<T, kWriteU8>(p, ih, iw, dstf, dstu, vec_ok, threadIdx.x, blockDim.x);
         if (!p.ok) continue;  // uniform across the CTA
         // crop.cu's 4-tap INTER_AREA path applies to a staged patch shrunk by factors below 3
         const bool strips = p.staged && soa_fits && p.interp == 3 && p.scale_x < 2.999 && p.scale_y < 2.999;
@@ -398,22 +399,22 @@ __global__ void __launch_bounds__(kQcThreads, 4) quad_crop_kernel(const uint8_t 
             bool redo = !strips;
             if (strips)
                 redo = __syncthreads_or(
-                    x3 ? area4_strips<kWriteF32, kWriteU8, kQcThreads, 3>(qc_smem, 0u, (uint32_t)pitch, 0u, 0u, soa, tab_n, ih,
+                    x3 ? area4_strips<T, kWriteU8, kQcThreads, 3>(qc_smem, 0u, (uint32_t)pitch, 0u, 0u, soa, tab_n, ih,
                                                                           iw, p.nw, p.nh, p.y0, dstf, dstu, threadIdx.x)
-                       : area4_strips<kWriteF32, kWriteU8, kQcThreads, 4>(qc_smem, 0u, (uint32_t)pitch, 0u, 0u, soa, tab_n, ih,
+                       : area4_strips<T, kWriteU8, kQcThreads, 4>(qc_smem, 0u, (uint32_t)pitch, 0u, 0u, soa, tab_n, ih,
                                                                           iw, p.nw, p.nh, p.y0, dstf, dstu, threadIdx.x));
             if (redo) {
                 if (strips) {  // an entry with more than 4 taps after all: per-pixel entries, no table
-                    resample_canvas<kWriteF32, kWriteU8>(p, PitchedSrc{qc_patch, pitch}, s_tab, false, need_tab, ih, iw,
+                    resample_canvas<T, kWriteU8>(p, PitchedSrc{qc_patch, pitch}, s_tab, false, need_tab, ih, iw,
                                                          dstf, dstu);
                 } else {
-                    resample_canvas<kWriteF32, kWriteU8>(p, PitchedSrc{qc_patch, pitch}, s_tab, tab_ok, need_tab, ih,
+                    resample_canvas<T, kWriteU8>(p, PitchedSrc{qc_patch, pitch}, s_tab, tab_ok, need_tab, ih,
                                                          iw, dstf, dstu);
                 }
             }
         } else {
             const WarpSrc src{&qp, pg};
-            resample_canvas<kWriteF32, kWriteU8>(p, src, s_tab, tab_ok, need_tab, ih, iw, dstf, dstu);
+            resample_canvas<T, kWriteU8>(p, src, s_tab, tab_ok, need_tab, ih, iw, dstf, dstu);
         }
     }
 }
@@ -444,11 +445,11 @@ struct QsMeta {
     int pitch, base;             // staged row pitch; ring offset + misalignment of the window's first byte
 };
 
-template <bool kWriteF32, bool kWriteU8>
+template <class T, bool kWriteU8>
 __global__ void __launch_bounds__(kQsThreads, 2)
     quad_crop_staged_kernel(const QuadPlan *__restrict__ qplans, const Plan *__restrict__ plans,
                             const StageDesc *__restrict__ work, const int32_t *__restrict__ n_work_dev,
-                            int32_t *__restrict__ ticket, int ih, int iw, float *__restrict__ batch,
+                            int32_t *__restrict__ ticket, int ih, int iw, T *__restrict__ batch,
                             uint8_t *__restrict__ canvas_out, int vec_ok, uint8_t *__restrict__ redo)
 {
     ms_pdl_wait();
@@ -496,7 +497,7 @@ __global__ void __launch_bounds__(kQsThreads, 2)
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(&s_stage.full[s]);
-            write_padding<kWriteF32, kWriteU8>(p.nw, p.nh, p.y0, ih, iw, kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr,
+            write_padding<T, kWriteU8>(p.nw, p.nh, p.y0, ih, iw, kHasBatch<T> ? batch + (size_t)ci * 3 * plane : nullptr,
                                                kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr, vec_ok, lane, 32);
         }
         return;
@@ -520,7 +521,7 @@ __global__ void __launch_bounds__(kQsThreads, 2)
         const uint32_t umaxx = (uint32_t)me.umaxx, umaxy = (uint32_t)me.umaxy;
         const uint32_t ppitch = (uint32_t)w * 3u;  // patch rows in the band buffer
         const uint32_t *tab = tabs + (size_t)s * tab_n;
-        float *dstf = kWriteF32 ? batch + (size_t)ci * 3 * plane : nullptr;
+        T *dstf = kHasBatch<T> ? batch + (size_t)ci * 3 * plane : nullptr;
         uint8_t *dstu = kWriteU8 ? canvas_out + (size_t)ci * 3 * plane : nullptr;
         // this lane's two columns of a 64-column coordinate block
         const double ax0 = m0 * lane, ay0 = m3 * lane, aw0 = m6 * lane;
@@ -582,14 +583,14 @@ __global__ void __launch_bounds__(kQsThreads, 2)
             const uint32_t soff = band_off - (uint32_t)r0 * ppitch;
             // (the strip height as a literal: the strip loop is unrolled for it)
             if (Gs == 2)
-                bad = (me.x3 ? area4_strips<kWriteF32, kWriteU8, 32, 3, true>(smem, soff, ppitch, 0u, 0u, tab, tab_n, ih, iw, nw, nh,
+                bad = (me.x3 ? area4_strips<T, kWriteU8, 32, 3, true>(smem, soff, ppitch, 0u, 0u, tab, tab_n, ih, iw, nw, nh,
                                                                             y0, dstf, dstu, lane, 2, dyA, dyB)
-                             : area4_strips<kWriteF32, kWriteU8, 32, 4, true>(smem, soff, ppitch, 0u, 0u, tab, tab_n, ih, iw, nw, nh,
+                             : area4_strips<T, kWriteU8, 32, 4, true>(smem, soff, ppitch, 0u, 0u, tab, tab_n, ih, iw, nw, nh,
                                                                             y0, dstf, dstu, lane, 2, dyA, dyB)) || bad;
             else
-                bad = (me.x3 ? area4_strips<kWriteF32, kWriteU8, 32, 3, true>(smem, soff, ppitch, 0u, 0u, tab, tab_n, ih, iw, nw, nh,
+                bad = (me.x3 ? area4_strips<T, kWriteU8, 32, 3, true>(smem, soff, ppitch, 0u, 0u, tab, tab_n, ih, iw, nw, nh,
                                                                             y0, dstf, dstu, lane, 4, dyA, dyB)
-                             : area4_strips<kWriteF32, kWriteU8, 32, 4, true>(smem, soff, ppitch, 0u, 0u, tab, tab_n, ih, iw, nw, nh,
+                             : area4_strips<T, kWriteU8, 32, 4, true>(smem, soff, ppitch, 0u, 0u, tab, tab_n, ih, iw, nw, nh,
                                                                             y0, dstf, dstu, lane, 4, dyA, dyB)) || bad;
             __syncwarp();  // the band buffer is rewritten by the next band
         }
@@ -654,12 +655,12 @@ static int quad_args_ok(int n_pages, int img_h, int img_w, int border_mode, int 
 
 int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w, const float *quads,
                   int quad_stride, const int32_t *page_of, int64_t n, int min_text_size, int border_mode,
-                  int border_value, int out_h, int out_w, float *batch_f32, uint8_t *canvas_u8, int32_t *sizes_out,
-                  ms_bump bump, cudaStream_t st)
+                  int border_value, int out_h, int out_w, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                  int32_t *sizes_out, ms_bump bump, cudaStream_t st)
 {
     if (n <= 0) return MS_OK;
     MS_TRY(quad_args_ok(n_pages, img_h, img_w, border_mode, border_value, "quad_crop"));
-    if (out_h <= 0 || out_w <= 0 || quad_stride < 8 || (!batch_f32 && !canvas_u8) ||
+    if (out_h <= 0 || out_w <= 0 || quad_stride < 8 || (!batch && !canvas_u8) ||
         (int64_t)out_h * out_w > (1 << 20)) {
         ms_set_error("quad_crop: bad arguments");
         return MS_ERR_INVALID;
@@ -690,27 +691,26 @@ int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int
     ms_launch(quad_plan_kernel, (int)pg, 128, 0, st, quads, quad_stride, page_of, n, n_pages, min_text_size, out_h, out_w,
                                              qplans, plans, sizes_out, pages, img_h, img_w, stage_ok, work, cnt);
     MS_LAUNCH_CHECK(ctx);
-    const int vec_ok = ((out_w & 3) == 0 && (reinterpret_cast<uintptr_t>(batch_f32) & 15) == 0) ? 1 : 0;
     const bool staged = stage_ok != 0;
     int64_t grid = (int64_t)ctx->num_sms * 4;  // 40 KB stage + 12 KB tables, 64 registers: four CTAs per SM
     if (grid > n) grid = n;
     const int smem = kQcPatchBytes + 16 + kQcMaxTab * (int)sizeof(AxisEnt);
-    return launch_for_outputs(batch_f32, canvas_u8, [&](auto f32, auto u8) {
-        constexpr bool kF32 = decltype(f32)::value, kU8 = decltype(u8)::value;
+    return launch_for_outputs(batch, batch_dtype, canvas_u8, [&](auto bt, auto u8) {
+        using T = typename decltype(bt)::type;
+        constexpr bool kU8 = decltype(u8)::value;
+        T *out = static_cast<T *>(batch);
+        const int vec_ok = batch_vec_ok<T>(batch, out_w);
         if (staged) {
-            constexpr ms_smem_slot slot =
-                kF32 ? (kU8 ? MS_SMEM_QUAD_STAGED_BOTH : MS_SMEM_QUAD_STAGED_F32) : MS_SMEM_QUAD_STAGED_U8;
-            MS_TRY(ms_allow_smem(ctx, slot, quad_crop_staged_kernel<kF32, kU8>, smem_s));
-            ms_launch(quad_crop_staged_kernel<kF32, kU8>, ctx->num_sms * 2, kQsThreads, smem_s, st, qplans, plans, work, cnt,
-                      cnt + 1, out_h, out_w, batch_f32, canvas_u8, vec_ok, redo);
+            MS_TRY(ms_allow_smem(ctx, batch_slot<T, kU8>(MS_SMEM_QUAD_STAGED_U8), quad_crop_staged_kernel<T, kU8>, smem_s));
+            ms_launch(quad_crop_staged_kernel<T, kU8>, ctx->num_sms * 2, kQsThreads, smem_s, st, qplans, plans, work, cnt,
+                      cnt + 1, out_h, out_w, out, canvas_u8, vec_ok, redo);
             MS_LAUNCH_CHECK(ctx);
         }
         ms_launch(quad_fallback_list_kernel, (int)pg, 256, 0, st, qplans, n, redo, list, cnt + 2);
         MS_LAUNCH_CHECK(ctx);
-        constexpr ms_smem_slot slot = kF32 ? (kU8 ? MS_SMEM_QUAD_BOTH : MS_SMEM_QUAD_F32) : MS_SMEM_QUAD_U8;
-        MS_TRY(ms_allow_smem(ctx, slot, quad_crop_kernel<kF32, kU8>, smem));
-        ms_launch(quad_crop_kernel<kF32, kU8>, (int)grid, kQcThreads, smem, st, pages, img_h, img_w, qplans, plans, n,
-                  border_mode, border_value, out_h, out_w, batch_f32, canvas_u8, vec_ok, list, cnt + 2);
+        MS_TRY(ms_allow_smem(ctx, batch_slot<T, kU8>(MS_SMEM_QUAD_U8), quad_crop_kernel<T, kU8>, smem));
+        ms_launch(quad_crop_kernel<T, kU8>, (int)grid, kQcThreads, smem, st, pages, img_h, img_w, qplans, plans, n,
+                  border_mode, border_value, out_h, out_w, out, canvas_u8, vec_ok, list, cnt + 2);
         MS_LAUNCH_CHECK(ctx);
         return MS_OK;
     });

@@ -10,6 +10,7 @@ from ._cabi import (  # noqa: F401
     CABIError,
     Context,
     EastParams,
+    batch_dtype_code,
     library_path,
     load_library,
 )

@@ -22,6 +22,10 @@ MS_FLAG_INDEX_ERROR = 2
 MS_FLAG_EDGE_OVERFLOW = 4
 MS_FLAG_ORDER_OVERFLOW = 8
 
+MS_DTYPE_F32 = 0
+MS_DTYPE_F16 = 1
+MS_DTYPE_BF16 = 2
+
 
 class CABIError(RuntimeError):
     def __init__(self, code, msg):
@@ -110,7 +114,30 @@ SIGNATURES = {
                                        _vp, _vp, _i64, _vp, _vp, C.POINTER(_vp), _vp]),
     "ms_page_batch_host": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i, _i, _vp,
                                 _vp, _vp, _i64, _vp, _vp, C.POINTER(_vp), _vp]),
+    # the same entry points with the batch in an MS_DTYPE_* element type (void *batch, int batch_dtype)
+    "ms_crop_resize_pad_ex": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i64, _i, _i, _vp, _i, _vp, _vp]),
+    "ms_quad_crop_resize_pad_ex": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _vp, _i64, _i, _i, _i, _i, _i, _vp, _i, _vp,
+                                        _vp, _vp]),
+    "ms_page_batch_ex": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i, _i, _vp, _vp,
+                              _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
+    "ms_page_batch_ragged_ex": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i, _i, _vp,
+                                     _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
+    "ms_page_batch_host_ex": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i, _i, _vp,
+                                   _vp, _vp, _i64, _vp, _vp, _i, C.POINTER(_vp), _vp]),
+    "ms_page_batch_ragged_host_ex": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i, _i,
+                                          _vp, _vp, _vp, _i64, _vp, _vp, _i, C.POINTER(_vp), _vp]),
 }
+
+
+def batch_dtype_code(dtype):
+    """torch.float32 / torch.float16 / torch.bfloat16 -> MS_DTYPE_F32 / _F16 / _BF16 (the `batch_dtype` argument of
+    the *_ex entry points).  Any other dtype raises ValueError."""
+    import torch
+
+    codes = {torch.float32: MS_DTYPE_F32, torch.float16: MS_DTYPE_F16, torch.bfloat16: MS_DTYPE_BF16}
+    if dtype not in codes:
+        raise ValueError(f"the recogniser batch can be float32, float16 or bfloat16, not {dtype}")
+    return codes[dtype]
 
 _lib = None
 _lock = threading.Lock()

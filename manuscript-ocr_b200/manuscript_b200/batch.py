@@ -14,7 +14,7 @@ from dataclasses import dataclass
 import numpy as np
 
 from ._cabi import (MS_FLAG_CAND_OVERFLOW, MS_FLAG_EDGE_OVERFLOW, MS_FLAG_INDEX_ERROR, MS_FLAG_ORDER_OVERFLOW, CABIError,
-                    Context, EastParams, check)
+                    Context, EastParams, batch_dtype_code, check)
 
 
 def shard_pages(n_pages, world_size, rank):
@@ -40,7 +40,7 @@ class PageBatchResult:
     box_counts: object   # (P,) int32
     crops: object        # (crops_cap, 5) int32 rows [page, x1, y1, x2, y2), first n_crops valid
     n_crops: object      # () / (1,) int32
-    batch: object        # (crops_cap | n_crops, 3, h, w) f32 CUDA tensor (None if not requested)
+    batch: object        # (crops_cap | n_crops, 3, h, w) CUDA tensor of the runner's batch_dtype (None if not requested)
     flags: object        # (P,) int32 MS_FLAG_* bits
 
     def page_boxes(self, p):
@@ -83,10 +83,13 @@ def _raise_for_flags(flags, allow_order_overflow=False):
 
 
 class PageBatch:
-    """Reusable runner for one GPU.  Output buffers are allocated once per shape and reused."""
+    """Reusable runner for one GPU.  Output buffers are allocated once per shape and reused.
+
+    batch_dtype: element type of the crop batch, torch.float32 (default), torch.float16 or torch.bfloat16.  A 16-bit
+    batch is written by the crop kernels directly and equals the float32 batch cast with .to(batch_dtype)."""
 
     def __init__(self, device=0, params=None, min_text_size=5, out_hw=(32, 128), cap_boxes=4096, crops_cap=None,
-                 want_batch=True):
+                 want_batch=True, batch_dtype=None):
         import torch
 
         if not torch.cuda.is_available():
@@ -100,6 +103,8 @@ class PageBatch:
         self.cap_boxes = int(cap_boxes)
         self.crops_cap = crops_cap
         self.want_batch = bool(want_batch)
+        self.batch_dtype = torch.float32 if batch_dtype is None else batch_dtype
+        self._dtype_code = batch_dtype_code(self.batch_dtype)
         self._bufs = {}
         self._host = {}
         self._ragged_tables = {}
@@ -118,7 +123,7 @@ class PageBatch:
                 crops=torch.zeros((cap, 5), dtype=torch.int32, device=dev),
                 n_crops=torch.zeros((1,), dtype=torch.int32, device=dev),
                 flags=torch.zeros((n_pages,), dtype=torch.int32, device=dev),
-                batch=(torch.empty((cap, 3, self.out_h, self.out_w), dtype=torch.float32, device=dev)
+                batch=(torch.empty((cap, 3, self.out_h, self.out_w), dtype=self.batch_dtype, device=dev)
                        if self.want_batch else None),
                 cap=cap,
             )
@@ -158,12 +163,12 @@ class PageBatch:
         stream = torch.cuda.current_stream(self.device).cuda_stream
         lib = self.ctx.lib
         with torch.cuda.device(self.device):
-            check(lib.ms_page_batch(
+            check(lib.ms_page_batch_ex(
                 self.ctx.handle, score.data_ptr(), geo.data_ptr(), pages.data_ptr() if pages is not None else None,
                 P, H, W, img_h, img_w, C.byref(self.params), self.min_text_size, self.out_h, self.out_w,
                 self.cap_boxes, b["boxes"].data_ptr(), b["counts"].data_ptr(), b["crops"].data_ptr(), b["cap"],
-                b["n_crops"].data_ptr(), b["batch"].data_ptr() if b["batch"] is not None else None, None,
-                b["flags"].data_ptr(), C.c_void_p(stream)))
+                b["n_crops"].data_ptr(), b["batch"].data_ptr() if b["batch"] is not None else None, self._dtype_code,
+                None, b["flags"].data_ptr(), C.c_void_p(stream)))
         return PageBatchResult(b["boxes"], b["counts"], b["crops"], b["n_crops"], b["batch"], b["flags"])
 
     def run_ragged(self, score, geo, pages, sync=False, allow_order_overflow=False):
@@ -203,11 +208,11 @@ class PageBatch:
         b = self._device_bufs(P)
         stream = torch.cuda.current_stream(self.device).cuda_stream
         with torch.cuda.device(self.device):
-            check(self.ctx.lib.ms_page_batch_ragged(
+            check(self.ctx.lib.ms_page_batch_ragged_ex(
                 self.ctx.handle, score.data_ptr(), geo.data_ptr(), ptrs.data_ptr(), hw.data_ptr(), P, H, W,
                 C.byref(self.params), self.min_text_size, self.out_h, self.out_w, self.cap_boxes, b["boxes"].data_ptr(),
                 b["counts"].data_ptr(), b["crops"].data_ptr(), b["cap"], b["n_crops"].data_ptr(),
-                b["batch"].data_ptr() if b["batch"] is not None else None, None, b["flags"].data_ptr(),
+                b["batch"].data_ptr() if b["batch"] is not None else None, self._dtype_code, None, b["flags"].data_ptr(),
                 C.c_void_p(stream)))
         res = PageBatchResult(b["boxes"], b["counts"], b["crops"], b["n_crops"], b["batch"], b["flags"])
         res._keepalive = (keep, ptrs, hw)  # the kernels read them after this call returns
@@ -229,10 +234,10 @@ class PageBatch:
         hw = np.array([[im.shape[0], im.shape[1]] for im in imgs], np.int32)
         h = self._host_bufs(P)
         dev_batch = C.c_void_p(h["batch"].data_ptr() if self.want_batch else None)
-        rc = self.ctx.lib.ms_page_batch_ragged_host(
+        rc = self.ctx.lib.ms_page_batch_ragged_host_ex(
             self.ctx.handle, s.ctypes.data, g.ctypes.data, ptrs, hw.ctypes.data, P, H, W, C.byref(self.params),
             self.min_text_size, self.out_h, self.out_w, self.cap_boxes, h["boxes"].data_ptr(), h["counts"].data_ptr(),
-            h["crops"].data_ptr(), h["cap"], h["n_crops"].data_ptr(), None,
+            h["crops"].data_ptr(), h["cap"], h["n_crops"].data_ptr(), None, self._dtype_code,
             C.byref(dev_batch) if self.want_batch else None, h["flags"].data_ptr())
         if check_flags or rc not in (0, -3, -4):
             check(rc)
@@ -256,7 +261,7 @@ class PageBatch:
                 n_crops=torch.zeros((1,), dtype=torch.int32, **pin),
                 flags=torch.zeros((n_pages,), dtype=torch.int32, **pin),
                 # the crop batch stays on the device; the runner owns it (never freed under a live view)
-                batch=(torch.empty((cap, 3, self.out_h, self.out_w), dtype=torch.float32, device=self.device)
+                batch=(torch.empty((cap, 3, self.out_h, self.out_w), dtype=self.batch_dtype, device=self.device)
                        if self.want_batch else None),
                 cap=cap,
             )
@@ -308,11 +313,11 @@ class PageBatch:
         h = self._host_bufs(P)
         dev_batch = C.c_void_p(h["batch"].data_ptr() if self.want_batch else None)
         lib = self.ctx.lib
-        rc = lib.ms_page_batch_host(
+        rc = lib.ms_page_batch_host_ex(
             self.ctx.handle, s.ctypes.data, g.ctypes.data, pg.ctypes.data if pg is not None else None, P, H, W,
             img_h, img_w, C.byref(self.params), self.min_text_size, self.out_h, self.out_w, self.cap_boxes,
             h["boxes"].data_ptr(), h["counts"].data_ptr(), h["crops"].data_ptr(), h["cap"], h["n_crops"].data_ptr(),
-            None, C.byref(dev_batch) if self.want_batch else None, h["flags"].data_ptr())
+            None, self._dtype_code, C.byref(dev_batch) if self.want_batch else None, h["flags"].data_ptr())
         if check_flags:
             check(rc)
         elif rc not in (0, -3, -4):

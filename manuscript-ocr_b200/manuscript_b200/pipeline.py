@@ -13,6 +13,9 @@ Three routes through predict(), all with the reference's results:
   crop batch are computed on the device from the detector's polygons.
 * HOST CROPS -- a foreign recogniser gets the list of uint8 crops it expects (plain slices of the page image), in the
   reading order computed on the device.
+
+With this package's TRBA, the device routes (and rotated_crops) write the recogniser batch in the TRBA's batch_dtype
+(float32 by default); a foreign recogniser still gets uint8 slices.
 """
 import ctypes as C
 import time
@@ -20,7 +23,7 @@ import time
 import numpy as np
 
 from . import ops
-from ._cabi import check
+from ._cabi import batch_dtype_code, check
 from .batch import PageBatch
 from .east import EAST, words_from_boxes
 from .imaging import read_image, visualize_page
@@ -91,11 +94,11 @@ class Pipeline:
     # ---- route 1: everything between the image upload and the recogniser network on the device ---------------------
     def _fused_runner(self):
         det, rec = self.detector, self.recognizer
-        key = (det.device, det.cap_boxes, rec.img_h, rec.img_w, int(self.min_text_size))
+        key = (det.device, det.cap_boxes, rec.img_h, rec.img_w, int(self.min_text_size), rec.batch_dtype)
         if self._runner is None or self._runner_key != key:
             self._runner = PageBatch(device=det.device.index or 0, params=det._params(sort_reading_order=1),
                                      min_text_size=int(self.min_text_size), out_hw=(rec.img_h, rec.img_w),
-                                     cap_boxes=det.cap_boxes)
+                                     cap_boxes=det.cap_boxes, batch_dtype=rec.batch_dtype)
             self._runner_key = key
         self._runner.params = det._params(sort_reading_order=1)
         return self._runner
@@ -174,14 +177,14 @@ class Pipeline:
         page_dev = torch.from_numpy(np.ascontiguousarray(rgb)).to(rec.device)
         quads_dev = torch.from_numpy(np.ascontiguousarray(quads)).to(rec.device)
         n = len(words)
-        batch = torch.empty((n, 3, rec.img_h, rec.img_w), dtype=torch.float32, device=rec.device)
+        batch = torch.empty((n, 3, rec.img_h, rec.img_w), dtype=rec.batch_dtype, device=rec.device)
         sizes = torch.zeros((n, 2), dtype=torch.int32, device=rec.device)
         stream = torch.cuda.current_stream(rec.device).cuda_stream
         with torch.cuda.device(rec.device):
-            check(rec.ctx.lib.ms_quad_crop_resize_pad(
+            check(rec.ctx.lib.ms_quad_crop_resize_pad_ex(
                 rec.ctx.handle, page_dev.data_ptr(), 1, int(rgb.shape[0]), int(rgb.shape[1]), quads_dev.data_ptr(), 8,
-                None, n, int(self.min_text_size), 0, 0, rec.img_h, rec.img_w, batch.data_ptr(), None, sizes.data_ptr(),
-                C.c_void_p(stream)))
+                None, n, int(self.min_text_size), 0, 0, rec.img_h, rec.img_w, batch.data_ptr(),
+                batch_dtype_code(rec.batch_dtype), None, sizes.data_ptr(), C.c_void_p(stream)))
         valid = (sizes[:, 0] > 0).cpu().numpy()
         keep = torch.from_numpy(np.flatnonzero(valid)).to(rec.device)
         kept_batch = batch.index_select(0, keep)

@@ -9,6 +9,10 @@ must return a list of {"text", "confidence"} dicts (or (text, confidence) tuples
 The batch is assembled on the device and stays there: a list of host crops is packed into one atlas, uploaded once,
 and resampled by one launch of the crop kernels straight into the (n,3,h,w) float32 tensor the network reads -- where
 the reference does one cv2.resize and one `.to(device)` per image (__init__.py:288).
+
+batch_dtype=torch.float16 / torch.bfloat16 (an extension) makes the crop kernels write the batch in 16 bits: exactly
+the float32 batch cast with `.to(batch_dtype)`, at half the bytes and without the cast.  It is for a network that runs
+in that dtype; the caller owns the model's dtype (from_pretrained's reference network is float32 and stays so).
 """
 import ctypes as C
 import os
@@ -16,13 +20,13 @@ from pathlib import Path
 
 import numpy as np
 
-from ._cabi import Context, check
+from ._cabi import Context, batch_dtype_code, check
 
 DEFAULT_DIR = Path.home() / ".manuscript" / "trba" / "exp_1_baseline"  # recognizers/_trba/__init__.py:24-36
 
 
 class TRBA:
-    def __init__(self, model=None, img_h=64, img_w=256, device=0, batch_size=32):
+    def __init__(self, model=None, img_h=64, img_w=256, device=0, batch_size=32, batch_dtype=None):
         # 64x256 is the reference class default (recognizers/_trba/__init__.py:150-151); configs/config.json
         # uses 32x128 -- both are supported
         import torch
@@ -34,6 +38,8 @@ class TRBA:
         self.model = model
         self.img_h, self.img_w = int(img_h), int(img_w)
         self.batch_size = int(batch_size)
+        self.batch_dtype = torch.float32 if batch_dtype is None else batch_dtype
+        self._dtype_code = batch_dtype_code(self.batch_dtype)
         self._ctx = None
 
     @classmethod
@@ -41,7 +47,9 @@ class TRBA:
         """What the reference's `TRBA()` does (recognizers/_trba/__init__.py:120-168, 207-231): the released weights
         and config from ~/.manuscript/trba/exp_1_baseline/ (put there by the reference's downloader; this package has no
         network code) inside the reference's own TRBA, whose network then runs on the batches assembled here.
-        FileNotFoundError when the checkpoint is missing, ImportError when the reference package is not installed."""
+        FileNotFoundError when the checkpoint is missing, ImportError when the reference package is not installed.
+        The reference network is float32: a batch_dtype other than torch.float32 needs a model converted by the
+        caller."""
         weights = Path(model_path) if model_path is not None else DEFAULT_DIR / "weights.pth"
         if not weights.exists():
             raise FileNotFoundError(f"Model checkpoint not found: {weights} (the reference downloads it on first use; "
@@ -94,32 +102,34 @@ class TRBA:
 
     def crops_to_batch(self, page_dev, crops_dev, n, out=None):
         """The device-resident step: page_dev (H, W, 3) or (P, H, W, 3) u8 CUDA tensor, crops_dev (>= n, 5) int32 CUDA
-        rows [page, x1, y1, x2, y2) -> (n, 3, img_h, img_w) f32 CUDA tensor (ms_crop_resize_pad; nothing touches
-        the host)."""
+        rows [page, x1, y1, x2, y2) -> (n, 3, img_h, img_w) CUDA tensor of batch_dtype (ms_crop_resize_pad_ex;
+        nothing touches the host)."""
         torch = self.torch
         if out is None:
-            out = torch.empty((n, 3, self.img_h, self.img_w), dtype=torch.float32, device=self.device)
+            out = torch.empty((n, 3, self.img_h, self.img_w), dtype=self.batch_dtype, device=self.device)
+        elif out.dtype != self.batch_dtype:
+            raise ValueError(f"out is {out.dtype}, this TRBA writes {self.batch_dtype}")
         if n == 0:
             return out
         pages = page_dev if page_dev.dim() == 4 else page_dev[None]
         n_dev = torch.tensor([n], dtype=torch.int32, device=self.device)
         stream = torch.cuda.current_stream(self.device).cuda_stream
         with torch.cuda.device(self.device):
-            check(self.ctx.lib.ms_crop_resize_pad(self.ctx.handle, pages.data_ptr(), int(pages.shape[0]),
-                                                  int(pages.shape[1]), int(pages.shape[2]), crops_dev.data_ptr(),
-                                                  n_dev.data_ptr(), n, self.img_h, self.img_w, out.data_ptr(), None,
-                                                  C.c_void_p(stream)))
+            check(self.ctx.lib.ms_crop_resize_pad_ex(self.ctx.handle, pages.data_ptr(), int(pages.shape[0]),
+                                                     int(pages.shape[1]), int(pages.shape[2]), crops_dev.data_ptr(),
+                                                     n_dev.data_ptr(), n, self.img_h, self.img_w, out.data_ptr(),
+                                                     self._dtype_code, None, C.c_void_p(stream)))
         return out
 
     def preprocess(self, images):
-        """List of (h,w,3) uint8 crops -> (n,3,img_h,img_w) float32 CUDA tensor: what the reference builds with
+        """List of (h,w,3) uint8 crops -> (n,3,img_h,img_w) CUDA tensor of batch_dtype: what the reference builds with
         one cv2.resize + .to(device) per image followed by torch.stack.  One upload (the packed atlas), one launch,
         no download."""
         torch = self.torch
         imgs = [self._as_rgb(im) for im in images]
         n = len(imgs)
         if n == 0:
-            return torch.empty((0, 3, self.img_h, self.img_w), dtype=torch.float32, device=self.device)
+            return torch.empty((0, 3, self.img_h, self.img_w), dtype=self.batch_dtype, device=self.device)
         # pack the crops into one atlas so that a single kernel launch resamples all of them
         wmax = max(im.shape[1] for im in imgs)
         htot = sum(im.shape[0] for im in imgs)
@@ -146,7 +156,7 @@ class TRBA:
         return results
 
     def predict_batch(self, batch, **model_kwargs):
-        """batch (n,3,h,w) f32 on the device -> list of {"text", "confidence"}."""
+        """batch (n,3,h,w) of batch_dtype on the device -> list of {"text", "confidence"}."""
         if self.model is None:
             raise RuntimeError("TRBA(model=...) is required")
         out = self.model(batch, **model_kwargs)
