@@ -310,7 +310,8 @@ MS_API int ms_page_batch_ragged_ex(ms_ctx *ctx, const float *score, const float 
 
 /* Same path with HOST buffers (pinned or pageable; `score` / `geo` may also be DEVICE pointers of this context's
  * device -- maps a detector left on the GPU are used in place and only the page images cross PCIe): H2D of maps + pages, the batch, D2H of boxes,
- * counts, crop list and (optionally, if batch_f32_host != NULL) the crop batch.  When
+ * counts, crop list and (optionally, if batch_f32_host != NULL) the crop batch.  Of boxes_out (n_pages*cap_boxes,9)
+ * only rows [0, box_counts[p]) of each page p are defined.  When
  * batch_dev_out != NULL the crop batch stays on the device (as the reference leaves it on `self.device`,
  * recognizers/_trba/__init__.py:288):
  *   *batch_dev_out != NULL on entry  -> a CALLER-OWNED device buffer of crops_cap crops; the batch is written there;
@@ -331,7 +332,7 @@ MS_API int ms_page_batch_host_ex(ms_ctx *ctx, const float *score, const float *g
                           void *batch_host, int batch_dtype, void **batch_dev_out, int32_t *flags);
 
 /* ms_page_batch_ragged with HOST buffers: pages (n_pages) host pointers, page_hw (n_pages,2) int32 on the host;
- * outputs as ms_page_batch_host. */
+ * outputs as ms_page_batch_host (of boxes_out, only rows [0, box_counts[p]) of each page p are defined). */
 MS_API int ms_page_batch_ragged_host(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *const *pages,
                               const int32_t *page_hw, int n_pages, int map_h, int map_w, const ms_east_params *p,
                               int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,

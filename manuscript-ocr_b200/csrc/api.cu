@@ -217,7 +217,7 @@ static int timing_mark(ms_ctx *ctx, int idx, cudaStream_t st)
     return MS_OK;
 }
 
-static int grow(ms_ctx *ctx, char **buf, size_t *have, size_t want, const char *what)
+static int grow(char **buf, size_t *have, size_t want, const char *what)
 {
     if (want <= *have) return MS_OK;
     // growing frees memory that queued work may still use: drain the device first
@@ -237,46 +237,60 @@ static int grow(ms_ctx *ctx, char **buf, size_t *have, size_t want, const char *
         return MS_ERR_CUDA;
     }
     *have = sz;
-    (void)ctx;
     return MS_OK;
 }
 
 int ms_arena_reserve(ms_ctx *ctx, size_t bytes)
 {
     if (bytes > ctx->arena_bytes) ctx->quad_cnt = nullptr;  // the counters of the last rotated-crop call go with the old arena
-    return grow(ctx, &ctx->arena, &ctx->arena_bytes, bytes, "arena");
+    return grow(&ctx->arena, &ctx->arena_bytes, bytes, "arena");
 }
-int ms_stage_reserve(ms_ctx *ctx, size_t bytes) { return grow(ctx, &ctx->stage, &ctx->stage_bytes, bytes, "stage"); }
+int ms_stage_reserve(ms_ctx *ctx, size_t bytes) { return grow(&ctx->stage, &ctx->stage_bytes, bytes, "stage"); }
+
+// the whole scratch arena as `bump`, grown to at least `bytes` first
+static int arena_bump(ms_ctx *ctx, size_t bytes, ms_bump &bump)
+{
+    MS_TRY(ms_arena_reserve(ctx, bytes));
+    bump = ms_bump{ctx->arena, 0, ctx->arena_bytes};
+    return MS_OK;
+}
+
+// The device staging of a host entry point: carve(ms_bump &) takes the call's buffers from the bump.  A first pass
+// over an empty bump measures them, the stage grows to that size, and a second pass hands them out.
+template <typename Carve>
+static int stage_carve(ms_ctx *ctx, const char *who, Carve &&carve)
+{
+    ms_bump probe{nullptr, 0, 0};
+    carve(probe);
+    MS_TRY(ms_stage_reserve(ctx, probe.off));
+    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
+    carve(sb);
+    if (sb.off > sb.cap) {
+        ms_set_error("%s: staging too small", who);
+        return MS_ERR_CAPACITY;
+    }
+    return MS_OK;
+}
 
 static inline size_t al256(size_t b) { return (b + 255) & ~size_t(255); }
 
 // Entry guard: a context is single-threaded by contract (one scratch arena); the guard turns a violation into an error.
-// Re-entrant on the same thread (the *_host entry points call themselves again after growing a capacity).
 struct ms_ctx_guard {
     ms_ctx *c = nullptr;
-    bool owner = false;
-    static thread_local ms_ctx *t_inside;
     int enter(ms_ctx *ctx, const char *fn)
     {
-        if (t_inside == ctx) return MS_OK;  // nested call of this thread
         if (__atomic_exchange_n(&ctx->busy, 1, __ATOMIC_ACQUIRE) != 0) {
             ms_set_error("%s: this ms_ctx is in use by another thread (one context per thread)", fn);
             return MS_ERR_INVALID;
         }
         c = ctx;
-        owner = true;
-        t_inside = ctx;
         return MS_OK;
     }
     ~ms_ctx_guard()
     {
-        if (owner) {
-            t_inside = nullptr;
-            __atomic_store_n(&c->busy, 0, __ATOMIC_RELEASE);
-        }
+        if (c) __atomic_store_n(&c->busy, 0, __ATOMIC_RELEASE);
     }
 };
-thread_local ms_ctx *ms_ctx_guard::t_inside = nullptr;
 
 #define MS_CTX(ctx)                                          \
     if (!(ctx)) {                                            \
@@ -328,8 +342,8 @@ extern "C" int ms_decode_quads(ms_ctx *ctx, const float *score, const float *geo
         return MS_ERR_INVALID;
     }
     if (quantization < 1) quantization = 1;  // utils.py:347 only quantises when > 1
-    MS_TRY(ms_arena_reserve(ctx, msk_decode_scratch(n_pages, map_h, map_w, quantization)));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_decode_scratch(n_pages, map_h, map_w, quantization), bump));
     return msk_decode(ctx, score, geo, n_pages, map_h, map_w, score_thresh, scale, quantization, quads_out,
                       cap_per_page, counts, flags, bump, (cudaStream_t)stream);
 }
@@ -345,8 +359,8 @@ extern "C" int ms_decode_rbox(ms_ctx *ctx, const float *score, const float *geo5
         return MS_ERR_INVALID;
     }
     if (quantization < 1) quantization = 1;
-    MS_TRY(ms_arena_reserve(ctx, msk_decode_scratch(n_pages, map_h, map_w, quantization)));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_decode_scratch(n_pages, map_h, map_w, quantization), bump));
     return msk_decode(ctx, score, geo5, n_pages, map_h, map_w, score_thresh, scale, quantization, quads_out, cap_per_page,
                       counts, flags, bump, (cudaStream_t)stream, 0, 1);
 }
@@ -360,8 +374,8 @@ extern "C" int ms_lanms(ms_ctx *ctx, const float *quads, const int32_t *counts, 
         ms_set_error("ms_lanms: bad arguments");
         return MS_ERR_INVALID;
     }
-    MS_TRY(ms_arena_reserve(ctx, msk_lanms_scratch(n_pages, cap_per_page, ctx->edge_factor)));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_lanms_scratch(n_pages, cap_per_page, ctx->edge_factor), bump));
     return msk_lanms(ctx, quads, counts, n_pages, cap_per_page, iou_threshold, quads_out, counts_out, flags, bump,
                      (cudaStream_t)stream);
 }
@@ -376,8 +390,8 @@ extern "C" int ms_east_boxes(ms_ctx *ctx, const float *quads, const int32_t *cou
         ms_set_error("ms_east_boxes: bad arguments");
         return MS_ERR_INVALID;
     }
-    MS_TRY(ms_arena_reserve(ctx, msk_east_boxes_scratch(n_pages, cap_per_page)));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_east_boxes_scratch(n_pages, cap_per_page), bump));
     return msk_east_boxes(ctx, quads, counts, n_pages, cap_per_page, p, orig_hw, quads_out, cap_per_page, counts_out,
                           nullptr, bump, (cudaStream_t)stream);
 }
@@ -391,8 +405,8 @@ extern "C" int ms_reading_order(ms_ctx *ctx, const float *quads, const int32_t *
         ms_set_error("ms_reading_order: bad arguments");
         return MS_ERR_INVALID;
     }
-    MS_TRY(ms_arena_reserve(ctx, msk_reading_order_scratch(n_pages, cap_per_page)));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_reading_order_scratch(n_pages, cap_per_page), bump));
     return msk_reading_order(ctx, quads, 9, counts, n_pages, cap_per_page, order, quads_out, flags, bump,
                              (cudaStream_t)stream);
 }
@@ -410,23 +424,21 @@ extern "C" int ms_reading_order_host(ms_ctx *ctx, const float *polys8, int64_t n
         return MS_ERR_CAPACITY;
     }
     const int cap = (int)n;
-    MS_TRY(ms_stage_reserve(ctx, al256((size_t)n * 32) + al256((size_t)n * 4) + 1024));
-    MS_TRY(ms_arena_reserve(ctx, msk_reading_order_scratch(1, cap)));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    float *d_p = sb.take<float>((size_t)n * 8);
-    int32_t *d_o = sb.take<int32_t>((size_t)n);
-    int32_t *d_i = sb.take<int32_t>(2);
-    if (!d_i) {
-        ms_set_error("ms_reading_order_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    float *d_p;
+    int32_t *d_o, *d_i;
+    MS_TRY(stage_carve(ctx, "ms_reading_order_host", [&](ms_bump &sb) {
+        d_p = sb.take<float>((size_t)n * 8);
+        d_o = sb.take<int32_t>((size_t)n);
+        d_i = sb.take<int32_t>(2);
+    }));
     cudaStream_t st = ctx->own_stream;
     int32_t *h = reinterpret_cast<int32_t *>(ctx->pinned);
     h[0] = cap;
     h[1] = 0;
     MS_CUDA(cudaMemcpyAsync(d_i, h, 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     MS_CUDA(cudaMemcpyAsync(d_p, polys8, (size_t)n * 32, cudaMemcpyHostToDevice, st));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_reading_order_scratch(1, cap), bump));
     MS_TRY(msk_reading_order(ctx, d_p, 8, d_i, 1, cap, d_o, nullptr, d_i + 1, bump, st));
     MS_CUDA(cudaMemcpyAsync(order, d_o, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
     MS_CUDA(cudaMemcpyAsync(h + 4, d_i + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -454,8 +466,8 @@ extern "C" int ms_word_rects(ms_ctx *ctx, const float *quads, const int32_t *cou
         ms_set_error("ms_word_rects: bad arguments");
         return MS_ERR_INVALID;
     }
-    MS_TRY(ms_arena_reserve(ctx, word_rects_scratch_full(n_pages, cap_per_page)));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, word_rects_scratch_full(n_pages, cap_per_page), bump));
     return msk_word_rects(ctx, quads, counts, n_pages, cap_per_page, img_hw, img_h, img_w, min_text_size, crops_out,
                           crops_cap, n_crops, 0, 0, nullptr, bump, (cudaStream_t)stream);
 }
@@ -480,8 +492,8 @@ extern "C" int ms_crop_resize_pad_ex(ms_ctx *ctx, const uint8_t *pages, int n_pa
         ms_set_error("ms_crop_resize_pad: NULL pointer");
         return MS_ERR_INVALID;
     }
-    MS_TRY(ms_arena_reserve(ctx, msk_crop_scratch(crops_cap, n_pages)));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_crop_scratch(crops_cap, n_pages), bump));
     return msk_crop(ctx, pages, n_pages, img_h, img_w, crops, n_crops, nullptr, crops_cap, out_h, out_w, batch,
                     batch_dtype, canvas_u8, bump, (cudaStream_t)stream);
 }
@@ -547,49 +559,85 @@ static size_t tail_scratch(int n_pages, int cap_c, int64_t crops_cap, int total_
 // Pages below this count run their front stages as one sequence; from it on as two concurrent halves (see below).
 #define MS_SPLIT_MIN_PAGES 16
 
-// decode -> LANMS -> expand + EAST filters (-> reading order) of n_pages pages on stream st; boxes into boxes_out /
-// box_counts.  marks: record the stage-timing events (the half that runs on the caller's stream does).
-static int front_half(ms_ctx *ctx, const float *score, const float *geo, int n_pages, int map_h, int map_w, int img_h,
-                      int img_w, const ms_east_params *p, int q, int cap_c, int cap_boxes, const int32_t *hw_here,
-                      float *boxes_out, int32_t *box_counts, int32_t *flags, ms_bump bump, cudaStream_t st,
-                      int geo_compact, bool marks)
+static int pb_quant(const pb_call &c) { return c.params.quantization < 1 ? 1 : c.params.quantization; }
+
+// A call with parameters *p and every other field zero.  The parameters are copied field by field: the caller's struct
+// may carry indeterminate padding bytes, and a call is compared bytewise as a graph key (page_batch_cached).
+static void pb_init(pb_call &c, const ms_east_params *p)
 {
-    float *qa = bump.take<float>((size_t)n_pages * cap_c * 9);  // candidates
-    float *qb = bump.take<float>((size_t)n_pages * cap_c * 9);  // NMS output
-    int32_t *ca = bump.take<int32_t>(n_pages);
-    int32_t *cb = bump.take<int32_t>(n_pages);
+    memset(&c, 0, sizeof(c));
+    c.params.score_thresh = p->score_thresh;
+    c.params.scale = p->scale;
+    c.params.quantization = p->quantization;
+    c.params.iou_threshold = p->iou_threshold;
+    c.params.expand_ratio_w = p->expand_ratio_w;
+    c.params.expand_ratio_h = p->expand_ratio_h;
+    c.params.target_size = p->target_size;
+    c.params.axis_aligned_output = p->axis_aligned_output;
+    c.params.remove_area_anomalies = p->remove_area_anomalies;
+    c.params.anomaly_sigma_threshold = p->anomaly_sigma_threshold;
+    c.params.anomaly_min_box_count = p->anomaly_min_box_count;
+    c.params.sort_reading_order = p->sort_reading_order;
+}
+
+// the per-page arrays of a call from page `base` on
+struct pb_pages {
+    const float *score, *geo;
+    const int32_t *hw;
+    float *boxes;
+    int32_t *counts, *flags;
+};
+static pb_pages pb_at(const pb_call &c, int base)
+{
+    const size_t plane = (size_t)c.map_h * c.map_w;
+    const size_t gplane = c.geo_compact ? (size_t)(c.map_h / pb_quant(c)) * c.map_w : plane;
+    return {c.score + base * plane, c.geo + base * 8 * gplane, c.page_hw ? c.page_hw + 2 * (size_t)base : nullptr,
+            c.boxes_out + (size_t)base * c.cap_boxes * 9, c.box_counts + base, c.flags + base};
+}
+
+// decode -> LANMS -> expand + EAST filters (-> reading order) of pages [base, base + n) of call c on stream st, boxes
+// into the call's boxes_out / box_counts.  marks: record the stage-timing events (the half that runs on the caller's
+// stream does).
+static int front_half(ms_ctx *ctx, const pb_call &c, int base, int n, ms_bump bump, cudaStream_t st, bool marks)
+{
+    const ms_east_params *p = &c.params;
+    const int q = pb_quant(c), cap_c = cand_cap(c.map_h, c.map_w, q);
+    const pb_pages pg = pb_at(c, base);
+    float *qa = bump.take<float>((size_t)n * cap_c * 9);  // candidates
+    float *qb = bump.take<float>((size_t)n * cap_c * 9);  // NMS output
+    int32_t *ca = bump.take<int32_t>(n);
+    int32_t *cb = bump.take<int32_t>(n);
     if (!cb) {
         ms_set_error("ms_page_batch: arena too small");
         return MS_ERR_CAPACITY;
     }
-    MS_TRY(msk_decode(ctx, score, geo, n_pages, map_h, map_w, p->score_thresh, p->scale, q, qa, cap_c, ca, flags, bump,
-                      st, geo_compact));
+    MS_TRY(msk_decode(ctx, pg.score, pg.geo, n, c.map_h, c.map_w, p->score_thresh, p->scale, q, qa, cap_c, ca, pg.flags,
+                      bump, st, c.geo_compact));
     if (marks) MS_TRY(timing_mark(ctx, 1, st));
-    MS_TRY(msk_lanms(ctx, qa, ca, n_pages, cap_c, p->iou_threshold, qb, cb, flags, bump, st));
+    MS_TRY(msk_lanms(ctx, qa, ca, n, cap_c, p->iou_threshold, qb, cb, pg.flags, bump, st));
     // expand + EAST filters; boxes are scaled to the page images' size (infer.py:134-147: the original image), or target_size
     if (marks) MS_TRY(timing_mark(ctx, 2, st));
     if (p->sort_reading_order) {
         // filtered boxes -> scratch, then into boxes_out in reading order (the order the crops are produced in)
-        float *tmp = bump.take<float>((size_t)n_pages * cap_boxes * 9);
-        int32_t *ord = bump.take<int32_t>((size_t)n_pages * cap_boxes);
+        float *tmp = bump.take<float>((size_t)n * c.cap_boxes * 9);
+        int32_t *ord = bump.take<int32_t>((size_t)n * c.cap_boxes);
         if (!ord) {
             ms_set_error("ms_page_batch: arena too small");
             return MS_ERR_CAPACITY;
         }
-        MS_TRY(msk_east_boxes(ctx, qb, cb, n_pages, cap_c, p, hw_here, tmp, cap_boxes, box_counts, flags, bump, st,
-                              img_h, img_w));
-        MS_TRY(msk_reading_order(ctx, tmp, 9, box_counts, n_pages, cap_boxes, ord, boxes_out, flags, bump, st));
+        MS_TRY(msk_east_boxes(ctx, qb, cb, n, cap_c, p, pg.hw, tmp, c.cap_boxes, pg.counts, pg.flags, bump, st, c.img_h,
+                              c.img_w));
+        MS_TRY(msk_reading_order(ctx, tmp, 9, pg.counts, n, c.cap_boxes, ord, pg.boxes, pg.flags, bump, st));
     } else {
-        MS_TRY(msk_east_boxes(ctx, qb, cb, n_pages, cap_c, p, hw_here, boxes_out, cap_boxes, box_counts, flags, bump,
-                              st, img_h, img_w));
+        MS_TRY(msk_east_boxes(ctx, qb, cb, n, cap_c, p, pg.hw, pg.boxes, c.cap_boxes, pg.counts, pg.flags, bump, st,
+                              c.img_h, c.img_w));
     }
     return MS_OK;
 }
 
-// One chunk of pages through the whole path.  `pages_all` / `total_pages` describe the page-image tensor the crop
-// rows index into; this call handles pages [page_base, page_base + n_pages) of it, whose maps start at score / geo
-// and whose boxes go to boxes_out / box_counts / flags (already offset by the caller).  append != 0 adds this
-// chunk's crops after the *n_crops rows already listed.
+// Pages [page_base, page_base + n_pages) of call c through the whole path; the crop rows index all c.n_pages pages of
+// the call (c.pages, or c.page_ptrs / c.page_hw: device images of their own sizes).  append != 0 adds this chunk's
+// crops after the *n_crops rows already listed.
 //
 // The front stages of a batch of MS_SPLIT_MIN_PAGES pages or more run as TWO CONCURRENT HALVES (pages are independent):
 // the first on the caller's stream, the second on the context's auxiliary stream, forked and joined with events (under
@@ -597,44 +645,30 @@ static int front_half(ms_ctx *ctx, const float *score, const float *geo, int n_p
 // (or one cluster) per page walking a serial recurrence, or lanes waiting on dependent loads -- and leave most of the
 // SMs' issue slots free; the other half's kernels fill them.  The crop rectangles and the crop kernel then run once
 // over all pages.  MS_B200_NO_SPLIT=1 keeps one sequence.
-static int page_batch_impl(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages_all, int total_pages,
-                           int page_base, int n_pages, int map_h, int map_w, int img_h, int img_w,
-                           const ms_east_params *p, int min_text_size, int out_h, int out_w, int cap_boxes,
-                           float *boxes_out, int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
-                           int32_t *n_crops, int append, void *batch, int batch_dtype, uint8_t *canvas_u8,
-                           int32_t *flags, cudaStream_t st, int geo_compact = 0, const uint8_t *const *page_ptrs = nullptr,
-                           const int32_t *page_hw = nullptr)
+static int page_batch_impl(ms_ctx *ctx, const pb_call &c, int page_base, int n_pages, int append, cudaStream_t st)
 {
-    // page_ptrs / page_hw (device, indexed by the global page number): page images of their own sizes
-    const bool ragged = page_ptrs != nullptr && page_hw != nullptr;
-    const int32_t *hw_here = ragged ? page_hw + 2 * (size_t)page_base : nullptr;  // this chunk's pages
-    const bool want_crops = (pages_all != nullptr || ragged) && crops_out != nullptr && n_crops != nullptr && crops_cap > 0;
-    const int q = p->quantization < 1 ? 1 : p->quantization;
-    const int cap_c = cand_cap(map_h, map_w, q);
+    const bool ragged = c.page_ptrs != nullptr && c.page_hw != nullptr;
+    const bool want_crops = (c.pages != nullptr || ragged) && c.crops_out != nullptr && c.n_crops != nullptr && c.crops_cap > 0;
+    const int q = pb_quant(c);
+    const int cap_c = cand_cap(c.map_h, c.map_w, q);
     const bool split = ctx->split_front && n_pages >= MS_SPLIT_MIN_PAGES && st != ctx->aux_stream;
     const int nA = split ? n_pages / 2 : n_pages, nB = n_pages - nA;
-    const size_t szA = front_scratch(nA, map_h, map_w, q, cap_c, ctx->edge_factor, cap_boxes);
-    const size_t szB = split ? front_scratch(nB, map_h, map_w, q, cap_c, ctx->edge_factor, cap_boxes) : 0;
-    const size_t szT = tail_scratch(n_pages, cap_c, want_crops ? crops_cap : 0, total_pages);
+    const size_t szA = front_scratch(nA, c.map_h, c.map_w, q, cap_c, ctx->edge_factor, c.cap_boxes);
+    const size_t szB = split ? front_scratch(nB, c.map_h, c.map_w, q, cap_c, ctx->edge_factor, c.cap_boxes) : 0;
+    const size_t szT = tail_scratch(n_pages, cap_c, want_crops ? c.crops_cap : 0, c.n_pages);
     // (one sequence: the tail reuses the front stages' scratch; two halves: A | B | tail side by side)
     MS_TRY(ms_arena_reserve(ctx, split ? szA + szB + szT + 1024 : (szA > szT ? szA : szT) + 1024));
     ms_bump bumpA{ctx->arena, 0, split ? szA : ctx->arena_bytes};
     ms_bump bumpT{split ? ctx->arena + szA + szB : ctx->arena, 0, split ? ctx->arena_bytes - szA - szB : ctx->arena_bytes};
-    MS_CUDA(cudaMemsetAsync(flags, 0, (size_t)n_pages * sizeof(int32_t), st));
+    const pb_pages pg = pb_at(c, page_base);
+    MS_CUDA(cudaMemsetAsync(pg.flags, 0, (size_t)n_pages * sizeof(int32_t), st));
     MS_TRY(timing_mark(ctx, 0, st));
     if (split) {
-        const size_t plane = (size_t)map_h * map_w;
-        const size_t gplane = geo_compact ? (size_t)(map_h / q) * map_w : plane;
         ms_bump bumpB{ctx->arena + szA, 0, szB};
         MS_CUDA(cudaEventRecord(ctx->split_ev[0], st));
         MS_CUDA(cudaStreamWaitEvent(ctx->aux_stream, ctx->split_ev[0], 0));
-        int rc = front_half(ctx, score, geo, nA, map_h, map_w, img_h, img_w, p, q, cap_c, cap_boxes, hw_here, boxes_out,
-                            box_counts, flags, bumpA, st, geo_compact, true);
-        if (rc == MS_OK)
-            rc = front_half(ctx, score + (size_t)nA * plane, geo + (size_t)nA * 8 * gplane, nB, map_h, map_w, img_h, img_w,
-                            p, q, cap_c, cap_boxes, hw_here ? hw_here + 2 * (size_t)nA : nullptr,
-                            boxes_out + (size_t)nA * cap_boxes * 9, box_counts + nA, flags + nA, bumpB, ctx->aux_stream,
-                            geo_compact, false);
+        int rc = front_half(ctx, c, page_base, nA, bumpA, st, true);
+        if (rc == MS_OK) rc = front_half(ctx, c, page_base + nA, nB, bumpB, ctx->aux_stream, false);
         // always join (a capture must not end with the auxiliary stream still forked)
         const int rj = ms_check_cuda(cudaEventRecord(ctx->split_ev[1], ctx->aux_stream), "cudaEventRecord");
         const int rw = ms_check_cuda(cudaStreamWaitEvent(st, ctx->split_ev[1], 0), "cudaStreamWaitEvent");
@@ -642,8 +676,7 @@ static int page_batch_impl(ms_ctx *ctx, const float *score, const float *geo, co
         if (rj != MS_OK) return rj;
         if (rw != MS_OK) return rw;
     } else {
-        MS_TRY(front_half(ctx, score, geo, n_pages, map_h, map_w, img_h, img_w, p, q, cap_c, cap_boxes, hw_here, boxes_out,
-                          box_counts, flags, bumpA, st, geo_compact, true));
+        MS_TRY(front_half(ctx, c, page_base, n_pages, bumpA, st, true));
     }
     MS_TRY(timing_mark(ctx, 3, st));
     int32_t *range = bumpT.take<int32_t>(2);
@@ -652,12 +685,12 @@ static int page_batch_impl(ms_ctx *ctx, const float *score, const float *geo, co
         return MS_ERR_CAPACITY;
     }
     if (want_crops) {
-        MS_TRY(msk_word_rects(ctx, boxes_out, box_counts, n_pages, cap_boxes, hw_here, img_h, img_w, min_text_size,
-                              crops_out, crops_cap, n_crops, page_base, append, range, bumpT, st));
+        MS_TRY(msk_word_rects(ctx, pg.boxes, pg.counts, n_pages, c.cap_boxes, pg.hw, c.img_h, c.img_w, c.min_text_size,
+                              c.crops_out, c.crops_cap, c.n_crops, page_base, append, range, bumpT, st));
         MS_TRY(timing_mark(ctx, 4, st));
-        if (batch || canvas_u8)
-            MS_TRY(msk_crop(ctx, pages_all, total_pages, img_h, img_w, crops_out, n_crops, range, crops_cap, out_h,
-                            out_w, batch, batch_dtype, canvas_u8, bumpT, st, page_ptrs, page_hw));
+        if (c.batch || c.canvas_u8)
+            MS_TRY(msk_crop(ctx, c.pages, c.n_pages, c.img_h, c.img_w, c.crops_out, c.n_crops, range, c.crops_cap,
+                            c.out_h, c.out_w, c.batch, c.batch_dtype, c.canvas_u8, bumpT, st, c.page_ptrs, c.page_hw));
     } else {
         MS_TRY(timing_mark(ctx, 4, st));
     }
@@ -668,41 +701,17 @@ static int page_batch_impl(ms_ctx *ctx, const float *score, const float *geo, co
 // ms_page_batch / ms_page_batch_ragged: direct launches the first time a call is seen, graph capture (on the
 // context's own stream, nothing executes) at its second occurrence, replay on the caller's stream from then on.
 // Stage timing needs the events between the stages, so it always launches directly.
-static int page_batch_cached(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages,
-                             const uint8_t *const *page_ptrs, const int32_t *page_hw, int n_pages, int map_h, int map_w,
-                             int img_h, int img_w, const ms_east_params *p, int min_text_size, int out_h, int out_w,
-                             int cap_boxes, float *boxes_out, int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
-                             int32_t *n_crops, void *batch, int batch_dtype, uint8_t *canvas_u8, int32_t *flags,
-                             cudaStream_t st)
+static int page_batch_cached(ms_ctx *ctx, const pb_call &c, cudaStream_t st)
 {
-    auto direct = [&](cudaStream_t s) {
-        return page_batch_impl(ctx, score, geo, pages, n_pages, 0, n_pages, map_h, map_w, img_h, img_w, p, min_text_size,
-                               out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, 0, batch,
-                               batch_dtype, canvas_u8, flags, s, 0, page_ptrs, page_hw);
-    };
+    auto direct = [&](cudaStream_t s) { return page_batch_impl(ctx, c, 0, c.n_pages, 0, s); };
     if (!ctx->graphs_enabled || ctx->timing) return direct(st);
+    // the stream is not part of the key: a graph is replayed on the caller's stream
     ms_pb_key key;
     memset(&key, 0, sizeof(key));
-    const void *ptrs[14] = {score, geo, pages, page_ptrs, page_hw, boxes_out, box_counts, crops_out, n_crops, batch,
-                            canvas_u8, flags, ctx->arena, nullptr};
-    memcpy(key.ptr, ptrs, sizeof(ptrs));
-    // the batch dtype selects the crop kernels' instantiation: the same buffer in another dtype is another graph
-    const long long nums[13] = {n_pages, map_h, map_w, img_h, img_w, min_text_size, out_h, out_w, cap_boxes,
-                                (long long)crops_cap, ctx->edge_factor, (long long)ctx->arena_bytes, batch_dtype};
-    memcpy(key.num, nums, sizeof(nums));
-    // field by field: the caller's struct may carry indeterminate padding bytes, which must not take part in the key
-    key.params.score_thresh = p->score_thresh;
-    key.params.scale = p->scale;
-    key.params.quantization = p->quantization;
-    key.params.iou_threshold = p->iou_threshold;
-    key.params.expand_ratio_w = p->expand_ratio_w;
-    key.params.expand_ratio_h = p->expand_ratio_h;
-    key.params.target_size = p->target_size;
-    key.params.axis_aligned_output = p->axis_aligned_output;
-    key.params.remove_area_anomalies = p->remove_area_anomalies;
-    key.params.anomaly_sigma_threshold = p->anomaly_sigma_threshold;
-    key.params.anomaly_min_box_count = p->anomaly_min_box_count;
-    key.params.sort_reading_order = p->sort_reading_order;
+    memcpy(&key.call, &c, sizeof(c));
+    key.arena = ctx->arena;
+    key.arena_bytes = ctx->arena_bytes;
+    key.edge_factor = ctx->edge_factor;
     ms_graph_entry *e = nullptr;
     for (int i = 0; i < MS_GRAPH_SLOTS; i++)
         if (ctx->graphs[i].used && memcmp(&ctx->graphs[i].key, &key, sizeof(key)) == 0) e = &ctx->graphs[i];
@@ -720,7 +729,7 @@ static int page_batch_cached(ms_ctx *ctx, const float *score, const float *geo, 
             const int rc = direct(cap);
             cudaGraph_t g = nullptr;
             const cudaError_t ce = cudaStreamEndCapture(cap, &g);
-            const bool same_arena = ctx->arena == (char *)key.ptr[12] && (long long)ctx->arena_bytes == key.num[11];
+            const bool same_arena = ctx->arena == key.arena && ctx->arena_bytes == key.arena_bytes;
             if (rc == MS_OK && ce == cudaSuccess && g && same_arena &&
                 cudaGraphInstantiate(&e->exec, g, 0) == cudaSuccess) {
                 e->launches = ctx->launches - l0;
@@ -765,9 +774,14 @@ extern "C" int ms_page_batch_ex(ms_ctx *ctx, const float *score, const float *ge
         ms_set_error("ms_page_batch: bad arguments");
         return MS_ERR_INVALID;
     }
-    return page_batch_cached(ctx, score, geo, pages, nullptr, nullptr, n_pages, map_h, map_w, img_h, img_w, p,
-                             min_text_size, out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops,
-                             batch, batch_dtype, canvas_u8, flags, (cudaStream_t)stream);
+    pb_call c;
+    pb_init(c, p);
+    c.score = score; c.geo = geo; c.pages = pages;
+    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w; c.img_h = img_h; c.img_w = img_w;
+    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
+    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
+    c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
+    return page_batch_cached(ctx, c, (cudaStream_t)stream);
 }
 
 extern "C" int ms_page_batch(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
@@ -816,23 +830,20 @@ static int decode_host_impl(ms_ctx *ctx, const float *score, const float *geo, i
     int capd = cand_cap(map_h, map_w, quantization);
     if (cap < capd) capd = (int)cap;
     if (capd < 1) capd = 1;
-    size_t need = al256(plane * 4) + al256(plane * 4 * planes) + al256((size_t)capd * 36) + 1024;
-    MS_TRY(ms_stage_reserve(ctx, need));
-    MS_TRY(ms_arena_reserve(ctx, msk_decode_scratch(1, map_h, map_w, quantization)));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    float *d_score = sb.take<float>(plane);
-    float *d_geo = sb.take<float>(plane * planes);
-    float *d_out = sb.take<float>((size_t)capd * 9);
-    int32_t *d_cnt = sb.take<int32_t>(2);
-    if (!d_cnt) {
-        ms_set_error("ms_decode_quads_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    float *d_score, *d_geo, *d_out;
+    int32_t *d_cnt;
+    MS_TRY(stage_carve(ctx, "ms_decode_quads_host", [&](ms_bump &sb) {
+        d_score = sb.take<float>(plane);
+        d_geo = sb.take<float>(plane * planes);
+        d_out = sb.take<float>((size_t)capd * 9);
+        d_cnt = sb.take<int32_t>(2);
+    }));
     cudaStream_t st = ctx->own_stream;
     MS_CUDA(cudaMemcpyAsync(d_score, score, plane * 4, cudaMemcpyHostToDevice, st));
     MS_CUDA(cudaMemcpyAsync(d_geo, geo, plane * 4 * planes, cudaMemcpyHostToDevice, st));
     MS_CUDA(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(int32_t), st));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_decode_scratch(1, map_h, map_w, quantization), bump));
     MS_TRY(msk_decode(ctx, d_score, d_geo, 1, map_h, map_w, score_thresh, scale, quantization, d_out, capd, d_cnt,
                       d_cnt + 1, bump, st, 0, rbox));
     int32_t *h = reinterpret_cast<int32_t *>(ctx->pinned);
@@ -863,32 +874,27 @@ extern "C" int ms_lanms_host(ms_ctx *ctx, const float *boxes, int64_t n, double 
         return MS_ERR_INVALID;
     }
     const int cap = (int)n;
-    int32_t *h = reinterpret_cast<int32_t *>(ctx->pinned);
-    float *d_out = nullptr;
-    for (;;) {
-        MS_TRY(ms_stage_reserve(ctx, 2 * al256((size_t)n * 36) + 1024));
-        MS_TRY(ms_arena_reserve(ctx, msk_lanms_scratch(1, cap, ctx->edge_factor)));
-        ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-        float *d_in = sb.take<float>((size_t)n * 9);
+    float *d_in, *d_out;
+    int32_t *d_cnt;
+    MS_TRY(stage_carve(ctx, "ms_lanms_host", [&](ms_bump &sb) {
+        d_in = sb.take<float>((size_t)n * 9);
         d_out = sb.take<float>((size_t)n * 9);
-        int32_t *d_cnt = sb.take<int32_t>(3);
-        if (!d_cnt) {
-            ms_set_error("ms_lanms_host: staging too small");
-            return MS_ERR_CAPACITY;
-        }
-        cudaStream_t st = ctx->own_stream;
+        d_cnt = sb.take<int32_t>(3);
+    }));
+    cudaStream_t st = ctx->own_stream;
+    int32_t *h = reinterpret_cast<int32_t *>(ctx->pinned);
+    do {
         h[0] = cap;
         h[1] = 0;
         h[2] = 0;
         MS_CUDA(cudaMemcpyAsync(d_cnt, h, 3 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         MS_CUDA(cudaMemcpyAsync(d_in, boxes, (size_t)n * 36, cudaMemcpyHostToDevice, st));
-        ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+        ms_bump bump;
+        MS_TRY(arena_bump(ctx, msk_lanms_scratch(1, cap, ctx->edge_factor), bump));
         MS_TRY(msk_lanms(ctx, d_in, d_cnt, 1, cap, iou_threshold, d_out, d_cnt + 1, d_cnt + 2, bump, st));
         MS_CUDA(cudaMemcpyAsync(h + 4, d_cnt, 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         MS_CUDA(cudaStreamSynchronize(st));
-        if (!grow_edge_factor(ctx, h[6])) break;
-    }
-    cudaStream_t st = ctx->own_stream;
+    } while (grow_edge_factor(ctx, h[6]));
     MS_TRY(flags_to_rc(h[6], "locality_aware_nms"));
     const int m = h[5];
     if (m > 0) {
@@ -913,27 +919,26 @@ extern "C" int ms_standard_nms_host(ms_ctx *ctx, const double *polys, const doub
         ms_set_error("ms_standard_nms_host: n too large");
         return MS_ERR_INVALID;
     }
-    MS_TRY(ms_stage_reserve(ctx, al256((size_t)n * 64) + al256((size_t)n * 8) + al256((size_t)n * 4) + 1024));
-    MS_TRY(ms_arena_reserve(ctx, msk_standard_nms_scratch((int)n, ctx->edge_factor)));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    double *d_p = sb.take<double>((size_t)n * 8);
-    double *d_s = sb.take<double>((size_t)n);
-    int32_t *d_keep = sb.take<int32_t>((size_t)n);
-    int32_t *d_cnt = sb.take<int32_t>(2);
-    if (!d_cnt) {
-        ms_set_error("ms_standard_nms_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    double *d_p, *d_s;
+    int32_t *d_keep, *d_cnt;
+    MS_TRY(stage_carve(ctx, "ms_standard_nms_host", [&](ms_bump &sb) {
+        d_p = sb.take<double>((size_t)n * 8);
+        d_s = sb.take<double>((size_t)n);
+        d_keep = sb.take<int32_t>((size_t)n);
+        d_cnt = sb.take<int32_t>(2);
+    }));
     cudaStream_t st = ctx->own_stream;
-    MS_CUDA(cudaMemcpyAsync(d_p, polys, (size_t)n * 64, cudaMemcpyHostToDevice, st));
-    MS_CUDA(cudaMemcpyAsync(d_s, scores, (size_t)n * 8, cudaMemcpyHostToDevice, st));
-    MS_CUDA(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(int32_t), st));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
-    MS_TRY(msk_standard_nms(ctx, d_p, d_s, (int)n, iou_threshold, d_keep, d_cnt, d_cnt + 1, bump, st));
     int32_t *h = reinterpret_cast<int32_t *>(ctx->pinned);
-    MS_CUDA(cudaMemcpyAsync(h, d_cnt, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    MS_CUDA(cudaStreamSynchronize(st));
-    if (grow_edge_factor(ctx, h[1])) return ms_standard_nms_host(ctx, polys, scores, n, iou_threshold, keep_idx, k_out);
+    do {
+        MS_CUDA(cudaMemcpyAsync(d_p, polys, (size_t)n * 64, cudaMemcpyHostToDevice, st));
+        MS_CUDA(cudaMemcpyAsync(d_s, scores, (size_t)n * 8, cudaMemcpyHostToDevice, st));
+        MS_CUDA(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(int32_t), st));
+        ms_bump bump;
+        MS_TRY(arena_bump(ctx, msk_standard_nms_scratch((int)n, ctx->edge_factor), bump));
+        MS_TRY(msk_standard_nms(ctx, d_p, d_s, (int)n, iou_threshold, d_keep, d_cnt, d_cnt + 1, bump, st));
+        MS_CUDA(cudaMemcpyAsync(h, d_cnt, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        MS_CUDA(cudaStreamSynchronize(st));
+    } while (grow_edge_factor(ctx, h[1]));
     MS_TRY(flags_to_rc(h[1], "standard_nms"));
     const int k = h[0];
     if (k > 0) {
@@ -964,15 +969,12 @@ extern "C" int ms_polygon_iou_host(ms_ctx *ctx, const double *subj, const double
         return MS_ERR_INVALID;
     }
     if (n == 0) return MS_OK;
-    MS_TRY(ms_stage_reserve(ctx, 2 * al256((size_t)n * 64) + al256((size_t)n * 8) + 1024));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    double *d_a = sb.take<double>((size_t)n * 8);
-    double *d_b = sb.take<double>((size_t)n * 8);
-    double *d_o = sb.take<double>((size_t)n);
-    if (!d_o) {
-        ms_set_error("ms_polygon_iou_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    double *d_a, *d_b, *d_o;
+    MS_TRY(stage_carve(ctx, "ms_polygon_iou_host", [&](ms_bump &sb) {
+        d_a = sb.take<double>((size_t)n * 8);
+        d_b = sb.take<double>((size_t)n * 8);
+        d_o = sb.take<double>((size_t)n);
+    }));
     cudaStream_t st = ctx->own_stream;
     MS_CUDA(cudaMemcpyAsync(d_a, subj, (size_t)n * 64, cudaMemcpyHostToDevice, st));
     MS_CUDA(cudaMemcpyAsync(d_b, clip, (size_t)n * 64, cudaMemcpyHostToDevice, st));
@@ -991,15 +993,13 @@ extern "C" int ms_test_iou_proved_host(ms_ctx *ctx, const double *subj, const do
         return MS_ERR_INVALID;
     }
     if (n == 0) return MS_OK;
-    MS_TRY(ms_stage_reserve(ctx, 2 * al256((size_t)n * 64) + al256((size_t)n) + 1024));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    double *d_a = sb.take<double>((size_t)n * 8);
-    double *d_b = sb.take<double>((size_t)n * 8);
-    uint8_t *d_o = sb.take<uint8_t>((size_t)n);
-    if (!d_o) {
-        ms_set_error("ms_test_iou_proved_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    double *d_a, *d_b;
+    uint8_t *d_o;
+    MS_TRY(stage_carve(ctx, "ms_test_iou_proved_host", [&](ms_bump &sb) {
+        d_a = sb.take<double>((size_t)n * 8);
+        d_b = sb.take<double>((size_t)n * 8);
+        d_o = sb.take<uint8_t>((size_t)n);
+    }));
     cudaStream_t st = ctx->own_stream;
     MS_CUDA(cudaMemcpyAsync(d_a, subj, (size_t)n * 64, cudaMemcpyHostToDevice, st));
     MS_CUDA(cudaMemcpyAsync(d_b, clip, (size_t)n * 64, cudaMemcpyHostToDevice, st));
@@ -1018,14 +1018,11 @@ extern "C" int ms_expand_boxes_host(ms_ctx *ctx, const float *quads, int64_t n, 
         return MS_ERR_INVALID;
     }
     if (n == 0) return MS_OK;
-    MS_TRY(ms_stage_reserve(ctx, 2 * al256((size_t)n * 36) + 1024));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    float *d_in = sb.take<float>((size_t)n * 9);
-    float *d_out = sb.take<float>((size_t)n * 9);
-    if (!d_out) {
-        ms_set_error("ms_expand_boxes_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    float *d_in, *d_out;
+    MS_TRY(stage_carve(ctx, "ms_expand_boxes_host", [&](ms_bump &sb) {
+        d_in = sb.take<float>((size_t)n * 9);
+        d_out = sb.take<float>((size_t)n * 9);
+    }));
     cudaStream_t st = ctx->own_stream;
     MS_CUDA(cudaMemcpyAsync(d_in, quads, (size_t)n * 36, cudaMemcpyHostToDevice, st));
     MS_TRY(msk_expand(ctx, d_in, n, expand_w, expand_h, d_out, st));
@@ -1049,16 +1046,13 @@ extern "C" int ms_east_boxes_host(ms_ctx *ctx, const float *quads, int64_t n, co
         return MS_ERR_INVALID;
     }
     const int cap = (int)n;
-    MS_TRY(ms_stage_reserve(ctx, 2 * al256((size_t)n * 36) + 1024));
-    MS_TRY(ms_arena_reserve(ctx, msk_east_boxes_scratch(1, cap)));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    float *d_in = sb.take<float>((size_t)n * 9);
-    float *d_out = sb.take<float>((size_t)n * 9);
-    int32_t *d_i = sb.take<int32_t>(4);
-    if (!d_i) {
-        ms_set_error("ms_east_boxes_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    float *d_in, *d_out;
+    int32_t *d_i;
+    MS_TRY(stage_carve(ctx, "ms_east_boxes_host", [&](ms_bump &sb) {
+        d_in = sb.take<float>((size_t)n * 9);
+        d_out = sb.take<float>((size_t)n * 9);
+        d_i = sb.take<int32_t>(4);
+    }));
     cudaStream_t st = ctx->own_stream;
     int32_t *h = reinterpret_cast<int32_t *>(ctx->pinned);
     h[0] = cap;
@@ -1067,7 +1061,8 @@ extern "C" int ms_east_boxes_host(ms_ctx *ctx, const float *quads, int64_t n, co
     h[3] = orig_w;
     MS_CUDA(cudaMemcpyAsync(d_i, h, 4 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     MS_CUDA(cudaMemcpyAsync(d_in, quads, (size_t)n * 36, cudaMemcpyHostToDevice, st));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_east_boxes_scratch(1, cap), bump));
     MS_TRY(msk_east_boxes(ctx, d_in, d_i, 1, cap, p, d_i + 2, d_out, cap, d_i + 1, nullptr, bump, st));
     MS_CUDA(cudaMemcpyAsync(h + 8, d_i + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     MS_CUDA(cudaStreamSynchronize(st));
@@ -1089,15 +1084,14 @@ extern "C" int ms_word_rects_host(ms_ctx *ctx, const float *polys8, int64_t n, i
         return MS_ERR_INVALID;
     }
     if (n == 0) return MS_OK;
-    MS_TRY(ms_stage_reserve(ctx, al256((size_t)n * 32) + al256((size_t)n * 16) + al256((size_t)n) + 1024));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    float *d_p = sb.take<float>((size_t)n * 8);
-    int32_t *d_r = sb.take<int32_t>((size_t)n * 4);
-    uint8_t *d_v = sb.take<uint8_t>((size_t)n);
-    if (!d_v) {
-        ms_set_error("ms_word_rects_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    float *d_p;
+    int32_t *d_r;
+    uint8_t *d_v;
+    MS_TRY(stage_carve(ctx, "ms_word_rects_host", [&](ms_bump &sb) {
+        d_p = sb.take<float>((size_t)n * 8);
+        d_r = sb.take<int32_t>((size_t)n * 4);
+        d_v = sb.take<uint8_t>((size_t)n);
+    }));
     cudaStream_t st = ctx->own_stream;
     MS_CUDA(cudaMemcpyAsync(d_p, polys8, (size_t)n * 32, cudaMemcpyHostToDevice, st));
     MS_TRY(msk_word_rects_flat(ctx, d_p, n, img_h, img_w, min_text_size, d_r, d_v, st));
@@ -1135,21 +1129,17 @@ extern "C" int ms_crop_resize_pad_host(ms_ctx *ctx, const uint8_t *page, int img
     }
     const size_t page_bytes = (size_t)img_h * img_w * 3;
     const size_t one_f = (size_t)3 * out_h * out_w * sizeof(float), one_u = (size_t)3 * out_h * out_w;
-    size_t need = al256(page_bytes) + al256((size_t)n * 16) + al256((size_t)n * 20) + 1024;
-    if (batch_f32) need += al256((size_t)n * one_f);
-    if (canvas_u8) need += al256((size_t)n * one_u);
-    MS_TRY(ms_stage_reserve(ctx, need));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    uint8_t *d_page = sb.take<uint8_t>(page_bytes);
-    int32_t *d_rects = sb.take<int32_t>((size_t)n * 4);
-    int32_t *d_crops = sb.take<int32_t>((size_t)n * 5);
-    int32_t *d_n = sb.take<int32_t>(1);
-    float *d_f = batch_f32 ? sb.take<float>((size_t)n * 3 * out_h * out_w) : nullptr;
-    uint8_t *d_u = canvas_u8 ? sb.take<uint8_t>((size_t)n * one_u) : nullptr;
-    if (!d_n || (batch_f32 && !d_f) || (canvas_u8 && !d_u)) {
-        ms_set_error("ms_crop_resize_pad_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    uint8_t *d_page, *d_u;
+    int32_t *d_rects, *d_crops, *d_n;
+    float *d_f;
+    MS_TRY(stage_carve(ctx, "ms_crop_resize_pad_host", [&](ms_bump &sb) {
+        d_page = sb.take<uint8_t>(page_bytes);
+        d_rects = sb.take<int32_t>((size_t)n * 4);
+        d_crops = sb.take<int32_t>((size_t)n * 5);
+        d_n = sb.take<int32_t>(1);
+        d_f = batch_f32 ? sb.take<float>((size_t)n * 3 * out_h * out_w) : nullptr;
+        d_u = canvas_u8 ? sb.take<uint8_t>((size_t)n * one_u) : nullptr;
+    }));
     cudaStream_t st = ctx->own_stream;
     MS_CUDA(cudaMemcpyAsync(d_page, page, page_bytes, cudaMemcpyHostToDevice, st));
     MS_CUDA(cudaMemcpyAsync(d_rects, rects, (size_t)n * 16, cudaMemcpyHostToDevice, st));
@@ -1159,8 +1149,8 @@ extern "C" int ms_crop_resize_pad_host(ms_ctx *ctx, const uint8_t *page, int img
         ms_launch(ms_rects_to_crops_kernel, grid, 256, 0, st, d_rects, n, d_crops, d_n);
         MS_LAUNCH_CHECK(ctx);
     }
-    MS_TRY(ms_arena_reserve(ctx, msk_crop_scratch(n, 1)));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_crop_scratch(n, 1), bump));
     MS_TRY(msk_crop(ctx, d_page, 1, img_h, img_w, d_crops, d_n, nullptr, n, out_h, out_w, d_f, MS_DTYPE_F32, d_u, bump,
                     st));
     if (batch_f32) MS_CUDA(cudaMemcpyAsync(batch_f32, d_f, (size_t)n * one_f, cudaMemcpyDeviceToHost, st));
@@ -1183,9 +1173,14 @@ extern "C" int ms_page_batch_ragged_ex(ms_ctx *ctx, const float *score, const fl
         ms_set_error("ms_page_batch_ragged: bad arguments");
         return MS_ERR_INVALID;
     }
-    return page_batch_cached(ctx, score, geo, nullptr, page_ptrs, page_hw, n_pages, map_h, map_w, 0, 0, p, min_text_size,
-                             out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch,
-                             batch_dtype, canvas_u8, flags, (cudaStream_t)stream);
+    pb_call c;
+    pb_init(c, p);
+    c.score = score; c.geo = geo; c.page_ptrs = page_ptrs; c.page_hw = page_hw;
+    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w;
+    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
+    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
+    c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
+    return page_batch_cached(ctx, c, (cudaStream_t)stream);
 }
 
 extern "C" int ms_page_batch_ragged(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *const *page_ptrs,
@@ -1197,6 +1192,48 @@ extern "C" int ms_page_batch_ragged(ms_ctx *ctx, const float *score, const float
     return ms_page_batch_ragged_ex(ctx, score, geo, page_ptrs, page_hw, n_pages, map_h, map_w, p, min_text_size, out_h,
                                    out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch_f32,
                                    MS_DTYPE_F32, canvas_u8, flags, stream);
+}
+
+// Read-back of a host page batch queued on the context's own stream, from device call d to the caller's buffers in h.
+// *again: a page overflowed the NMS pair capacity, which has grown, and the batch has to run again.  Otherwise the
+// boxes come back (per page, the rows up to the largest count) and, when every page is clean, the crop list and batch.
+static int pb_host_read_back(ms_ctx *ctx, const pb_call &h, const pb_call &d, void **batch_dev_out, const char *who,
+                             bool *again)
+{
+    cudaStream_t st = ctx->own_stream;
+    const int n_pages = d.n_pages;
+    MS_CUDA(cudaMemcpyAsync(h.box_counts, d.box_counts, (size_t)n_pages * 4, cudaMemcpyDeviceToHost, st));
+    MS_CUDA(cudaMemcpyAsync(h.flags, d.flags, (size_t)n_pages * 4, cudaMemcpyDeviceToHost, st));
+    if (d.n_crops) MS_CUDA(cudaMemcpyAsync(h.n_crops, d.n_crops, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    MS_CUDA(cudaStreamSynchronize(st));
+    int32_t all = 0;
+    int max_cnt = 0;
+    for (int i = 0; i < n_pages; i++) {
+        all |= h.flags[i];
+        max_cnt = h.box_counts[i] > max_cnt ? h.box_counts[i] : max_cnt;
+    }
+    *again = grow_edge_factor(ctx, all);
+    if (*again) return MS_OK;
+    // 36 bytes per box instead of cap_boxes rows per page; a page's copy runs up to the following pages' rows when they
+    // are adjacent anyway
+    if (max_cnt > d.cap_boxes) max_cnt = d.cap_boxes;
+    const size_t pitch = (size_t)d.cap_boxes * 36;
+    if (max_cnt > 0)
+        MS_CUDA(cudaMemcpy2DAsync(h.boxes_out, pitch, d.boxes_out, pitch, (size_t)max_cnt * 36, (size_t)n_pages,
+                                  cudaMemcpyDeviceToHost, st));
+    const int rc = flags_to_rc(all, who);
+    const int64_t nc = d.n_crops ? (*h.n_crops < d.crops_cap ? *h.n_crops : d.crops_cap) : 0;
+    if (rc == MS_OK && nc > 0) {
+        MS_CUDA(cudaMemcpyAsync(h.crops_out, d.crops_out, (size_t)nc * 20, cudaMemcpyDeviceToHost, st));
+        if (h.batch) {
+            const size_t one = (size_t)3 * d.out_h * d.out_w * ms_dtype_bytes(d.batch_dtype);  // bytes of one crop
+            MS_CUDA(cudaMemcpyAsync(h.batch, d.batch, (size_t)nc * one, cudaMemcpyDeviceToHost, st));
+        }
+    }
+    MS_CUDA(cudaStreamSynchronize(st));
+    if (rc != MS_OK) return rc;
+    if (batch_dev_out) *batch_dev_out = d.batch;
+    return MS_OK;
 }
 
 extern "C" int ms_page_batch_host_ex(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages,
@@ -1212,6 +1249,13 @@ extern "C" int ms_page_batch_host_ex(ms_ctx *ctx, const float *score, const floa
         ms_set_error("ms_page_batch_host: bad arguments");
         return MS_ERR_INVALID;
     }
+    pb_call c;  // the caller's buffers
+    pb_init(c, p);
+    c.score = score; c.geo = geo; c.pages = pages;
+    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w; c.img_h = img_h; c.img_w = img_w;
+    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
+    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
+    c.batch = batch_host; c.batch_dtype = batch_dtype; c.flags = flags;
     const bool want_crops = pages != nullptr && crops_out != nullptr && n_crops != nullptr && crops_cap > 0;
     const bool want_batch = want_crops && (batch_host || batch_dev_out);
     // *batch_dev_out != NULL on entry: a caller-owned device buffer of crops_cap crops that receives the batch
@@ -1238,98 +1282,63 @@ extern "C" int ms_page_batch_host_ex(ms_ctx *ctx, const float *score, const floa
         } else
             cudaGetLastError();
     }
-    size_t need = (score_dev ? 256 : al256(n_pages * plane * 4)) + (geo_mapped ? 256 : al256(n_pages * plane * 32)) +
-                  al256((size_t)n_pages * cap_boxes * 36) + 2 * al256((size_t)n_pages * 4) + 4096;
-    if (want_crops) need += al256(n_pages * page_bytes) + al256((size_t)crops_cap * 20) + 256;
-    if (want_batch && !caller_batch) need += al256((size_t)crops_cap * one_f);
-    MS_TRY(ms_stage_reserve(ctx, need));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    float *d_score = score_dev ? const_cast<float *>(score_dev) : sb.take<float>(n_pages * plane);
-    float *d_geo = geo_mapped ? nullptr : sb.take<float>(n_pages * plane * 8);
-    float *d_boxes = sb.take<float>((size_t)n_pages * cap_boxes * 9);
-    int32_t *d_cnt = sb.take<int32_t>(n_pages);
-    int32_t *d_flags = sb.take<int32_t>(n_pages);
-    uint8_t *d_pages = want_crops ? sb.take<uint8_t>(n_pages * page_bytes) : nullptr;
-    int32_t *d_crops = want_crops ? sb.take<int32_t>((size_t)crops_cap * 5) : nullptr;
-    int32_t *d_nc = want_crops ? sb.take<int32_t>(1) : nullptr;
-    void *d_batch = !want_batch ? nullptr : caller_batch ? caller_batch : sb.take<char>((size_t)crops_cap * one_f);
-    if (!d_flags || (want_crops && !d_nc) || (want_batch && !d_batch)) {
-        ms_set_error("ms_page_batch_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    // With quantisation q > 1 the decode reads geometry only at rows y % q == q / 2 (utils.py:347-376), so only those
+    // rows cross PCIe: one strided 2-D DMA per chunk into a compact (P, 8, H / q, W) tensor.
+    const int q = pb_quant(c);
+    pb_call d = c;  // the same call on device staging
+    d.geo_compact = (!geo_mapped && q > 1 && map_h % q == 0) ? 1 : 0;
+    const size_t gplane = d.geo_compact ? (size_t)(map_h / q) * map_w : plane;
+    float *d_score, *d_geo;
+    uint8_t *d_pages;
+    MS_TRY(stage_carve(ctx, "ms_page_batch_host", [&](ms_bump &sb) {
+        d_score = score_dev ? const_cast<float *>(score_dev) : sb.take<float>(n_pages * plane);
+        d_geo = geo_mapped ? nullptr : sb.take<float>(n_pages * plane * 8);
+        d.boxes_out = sb.take<float>((size_t)n_pages * cap_boxes * 9);
+        d.box_counts = sb.take<int32_t>(n_pages);
+        d.flags = sb.take<int32_t>(n_pages);
+        d_pages = want_crops ? sb.take<uint8_t>(n_pages * page_bytes) : nullptr;
+        d.crops_out = want_crops ? sb.take<int32_t>((size_t)crops_cap * 5) : nullptr;
+        d.n_crops = want_crops ? sb.take<int32_t>(1) : nullptr;
+        d.batch = !want_batch ? nullptr : caller_batch ? caller_batch : sb.take<char>((size_t)crops_cap * one_f);
+    }));
+    d.score = d_score;
+    d.geo = geo_mapped ? geo_mapped : d_geo;
+    d.pages = d_pages;
     // Pipeline: pages are independent, so the batch is cut into chunks; the copy stream uploads chunk c+1 (maps +
     // page images) while the compute stream runs chunk c.  PCIe is the floor of this entry point: 22 MB per
     // 2048x2048 page against a few tens of microseconds of kernels.
     cudaStream_t st = ctx->own_stream, cs = ctx->copy_stream;
-    // With quantisation q > 1 the decode reads geometry only at rows y % q == q / 2 (utils.py:347-376), so only those
-    // rows cross PCIe: one strided 2-D DMA per chunk into a compact (P, 8, H / q, W) tensor.
-    const int q = p->quantization < 1 ? 1 : p->quantization;
-    const int geo_compact = (!geo_mapped && q > 1 && map_h % q == 0) ? 1 : 0;
-    const size_t gplane = geo_compact ? (size_t)(map_h / q) * map_w : plane;
     int chunk = (n_pages + 7) / 8;
     if (chunk < 1) chunk = 1;
     if (chunk > 8) chunk = 8;
-    if (want_crops) MS_CUDA(cudaMemsetAsync(d_nc, 0, sizeof(int32_t), st));
-    int k = 0;
-    for (int p0 = 0; p0 < n_pages; p0 += chunk, k++) {
-        const int np = n_pages - p0 < chunk ? n_pages - p0 : chunk;
-        cudaEvent_t ev = ctx->chunk_ev[k & 1];
-        // the event of chunk k-2 was consumed by the compute stream before chunk k-1 was queued; reuse is safe
-        if (!score_dev)
-            MS_CUDA(cudaMemcpyAsync(d_score + (size_t)p0 * plane, score + (size_t)p0 * plane, np * plane * 4,
-                                    cudaMemcpyHostToDevice, cs));
-        if (geo_mapped) {
-            // nothing to upload
-        } else if (geo_compact)
-            MS_CUDA(cudaMemcpy2DAsync(d_geo + (size_t)p0 * gplane * 8, (size_t)map_w * 4,
-                                      geo + (size_t)p0 * plane * 8 + (size_t)(q / 2) * map_w, (size_t)q * map_w * 4,
-                                      (size_t)map_w * 4, (size_t)np * 8 * (map_h / q), cudaMemcpyHostToDevice, cs));
-        else
-            MS_CUDA(cudaMemcpyAsync(d_geo + (size_t)p0 * plane * 8, geo + (size_t)p0 * plane * 8, np * plane * 32,
-                                    cudaMemcpyHostToDevice, cs));
-        if (want_crops)
-            MS_CUDA(cudaMemcpyAsync(d_pages + (size_t)p0 * page_bytes, pages + (size_t)p0 * page_bytes,
-                                    np * page_bytes, cudaMemcpyHostToDevice, cs));
-        MS_CUDA(cudaEventRecord(ev, cs));
-        MS_CUDA(cudaStreamWaitEvent(st, ev, 0));
-        const float *geo_chunk = geo_mapped ? geo_mapped + (size_t)p0 * plane * 8 : d_geo + (size_t)p0 * gplane * 8;
-        MS_TRY(page_batch_impl(ctx, d_score + (size_t)p0 * plane, geo_chunk, d_pages, n_pages, p0,
-                               np, map_h, map_w, img_h, img_w, p, min_text_size, out_h, out_w, cap_boxes,
-                               d_boxes + (size_t)p0 * cap_boxes * 9, d_cnt + p0, d_crops, crops_cap, d_nc, 1, d_batch,
-                               batch_dtype, nullptr, d_flags + p0, st, geo_compact));
-    }
-    MS_CUDA(cudaMemcpyAsync(box_counts, d_cnt, (size_t)n_pages * 4, cudaMemcpyDeviceToHost, st));
-    MS_CUDA(cudaMemcpyAsync(flags, d_flags, (size_t)n_pages * 4, cudaMemcpyDeviceToHost, st));
-    if (want_crops) MS_CUDA(cudaMemcpyAsync(n_crops, d_nc, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    MS_CUDA(cudaStreamSynchronize(st));
-    int32_t all = 0;
-    for (int i = 0; i < n_pages; i++) all |= flags[i];
-    if (grow_edge_factor(ctx, all))
-        return ms_page_batch_host_ex(ctx, score, geo, pages, n_pages, map_h, map_w, img_h, img_w, p, min_text_size,
-                                     out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops,
-                                     batch_host, batch_dtype, batch_dev_out, flags);
-    // the boxes come back page by page, only the rows each page has (counts are known now): 36 bytes per box instead
-    // of cap_boxes rows per page; a page's copy runs up to the following pages' rows when they are adjacent anyway
-    {
-        int max_cnt = 0;
-        for (int i = 0; i < n_pages; i++) max_cnt = box_counts[i] > max_cnt ? box_counts[i] : max_cnt;
-        if (max_cnt > cap_boxes) max_cnt = cap_boxes;
-        if (max_cnt > 0)
-            MS_CUDA(cudaMemcpy2DAsync(boxes_out, (size_t)cap_boxes * 36, d_boxes, (size_t)cap_boxes * 36, (size_t)max_cnt * 36,
-                                      (size_t)n_pages, cudaMemcpyDeviceToHost, st));
-    }
-    MS_TRY(flags_to_rc(all, "page_batch"));
-    if (want_crops) {
-        int64_t nc = *n_crops;
-        if (nc > crops_cap) nc = crops_cap;
-        if (nc > 0) {
-            MS_CUDA(cudaMemcpyAsync(crops_out, d_crops, (size_t)nc * 20, cudaMemcpyDeviceToHost, st));
-            if (batch_host)
-                MS_CUDA(cudaMemcpyAsync(batch_host, d_batch, (size_t)nc * one_f, cudaMemcpyDeviceToHost, st));
+    for (bool again = true; again;) {
+        if (want_crops) MS_CUDA(cudaMemsetAsync(d.n_crops, 0, sizeof(int32_t), st));
+        int k = 0;
+        for (int p0 = 0; p0 < n_pages; p0 += chunk, k++) {
+            const int np = n_pages - p0 < chunk ? n_pages - p0 : chunk;
+            cudaEvent_t ev = ctx->chunk_ev[k & 1];
+            // the event of chunk k-2 was consumed by the compute stream before chunk k-1 was queued; reuse is safe
+            if (!score_dev)
+                MS_CUDA(cudaMemcpyAsync(d_score + (size_t)p0 * plane, score + (size_t)p0 * plane, np * plane * 4,
+                                        cudaMemcpyHostToDevice, cs));
+            if (geo_mapped) {
+                // nothing to upload
+            } else if (d.geo_compact)
+                MS_CUDA(cudaMemcpy2DAsync(d_geo + (size_t)p0 * gplane * 8, (size_t)map_w * 4,
+                                          geo + (size_t)p0 * plane * 8 + (size_t)(q / 2) * map_w, (size_t)q * map_w * 4,
+                                          (size_t)map_w * 4, (size_t)np * 8 * (map_h / q), cudaMemcpyHostToDevice, cs));
+            else
+                MS_CUDA(cudaMemcpyAsync(d_geo + (size_t)p0 * plane * 8, geo + (size_t)p0 * plane * 8, np * plane * 32,
+                                        cudaMemcpyHostToDevice, cs));
+            if (want_crops)
+                MS_CUDA(cudaMemcpyAsync(d_pages + (size_t)p0 * page_bytes, pages + (size_t)p0 * page_bytes,
+                                        np * page_bytes, cudaMemcpyHostToDevice, cs));
+            MS_CUDA(cudaEventRecord(ev, cs));
+            MS_CUDA(cudaStreamWaitEvent(st, ev, 0));
+            MS_TRY(page_batch_impl(ctx, d, p0, np, 1, st));
         }
+        MS_TRY(pb_host_read_back(ctx, c, d, batch_dev_out, "page_batch", &again));
     }
-    MS_CUDA(cudaStreamSynchronize(st));
-    if (batch_dev_out) *batch_dev_out = d_batch;
     return MS_OK;
 }
 
@@ -1358,8 +1367,8 @@ extern "C" int ms_quad_crop_resize_pad_ex(ms_ctx *ctx, const uint8_t *pages, int
         return MS_ERR_INVALID;
     }
     if (n == 0) return MS_OK;
-    MS_TRY(ms_arena_reserve(ctx, msk_quad_crop_scratch(n)));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_quad_crop_scratch(n), bump));
     return msk_quad_crop(ctx, pages, n_pages, img_h, img_w, quads, quad_stride, page_of, n, min_text_size, border_mode,
                          border_value, out_h, out_w, batch, batch_dtype, canvas_u8, sizes_out, bump, (cudaStream_t)stream);
 }
@@ -1402,25 +1411,21 @@ extern "C" int ms_quad_crop_resize_pad_host(ms_ctx *ctx, const uint8_t *page, in
     if (n == 0) return MS_OK;
     const size_t page_bytes = (size_t)img_h * img_w * 3;
     const size_t one_f = (size_t)3 * out_h * out_w * sizeof(float), one_u = (size_t)3 * out_h * out_w;
-    size_t need = al256(page_bytes) + al256((size_t)n * 32) + al256((size_t)n * 8) + 1024;
-    if (batch_f32) need += al256((size_t)n * one_f);
-    if (canvas_u8) need += al256((size_t)n * one_u);
-    MS_TRY(ms_stage_reserve(ctx, need));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    uint8_t *d_page = sb.take<uint8_t>(page_bytes);
-    float *d_quads = sb.take<float>((size_t)n * 8);
-    int32_t *d_sizes = sb.take<int32_t>((size_t)n * 2);
-    float *d_f = batch_f32 ? sb.take<float>((size_t)n * 3 * out_h * out_w) : nullptr;
-    uint8_t *d_u = canvas_u8 ? sb.take<uint8_t>((size_t)n * one_u) : nullptr;
-    if (!d_sizes || (batch_f32 && !d_f) || (canvas_u8 && !d_u)) {
-        ms_set_error("ms_quad_crop_resize_pad_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    uint8_t *d_page, *d_u;
+    float *d_quads, *d_f;
+    int32_t *d_sizes;
+    MS_TRY(stage_carve(ctx, "ms_quad_crop_resize_pad_host", [&](ms_bump &sb) {
+        d_page = sb.take<uint8_t>(page_bytes);
+        d_quads = sb.take<float>((size_t)n * 8);
+        d_sizes = sb.take<int32_t>((size_t)n * 2);
+        d_f = batch_f32 ? sb.take<float>((size_t)n * 3 * out_h * out_w) : nullptr;
+        d_u = canvas_u8 ? sb.take<uint8_t>((size_t)n * one_u) : nullptr;
+    }));
     cudaStream_t st = ctx->own_stream;
     MS_CUDA(cudaMemcpyAsync(d_page, page, page_bytes, cudaMemcpyHostToDevice, st));
     MS_CUDA(cudaMemcpyAsync(d_quads, quads, (size_t)n * 32, cudaMemcpyHostToDevice, st));
-    MS_TRY(ms_arena_reserve(ctx, msk_quad_crop_scratch(n)));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, msk_quad_crop_scratch(n), bump));
     MS_TRY(msk_quad_crop(ctx, d_page, 1, img_h, img_w, d_quads, 8, nullptr, n, min_text_size, border_mode, border_value,
                          out_h, out_w, d_f, MS_DTYPE_F32, d_u, d_sizes, bump, st));
     if (batch_f32) MS_CUDA(cudaMemcpyAsync(batch_f32, d_f, (size_t)n * one_f, cudaMemcpyDeviceToHost, st));
@@ -1439,20 +1444,18 @@ extern "C" int ms_warp_quad_host(ms_ctx *ctx, const uint8_t *page, int img_h, in
         return MS_ERR_INVALID;
     }
     const size_t page_bytes = (size_t)img_h * img_w * 3;
-    MS_TRY(ms_stage_reserve(ctx, al256(page_bytes) + al256(32) + al256((size_t)patch_cap) + 1024));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    uint8_t *d_page = sb.take<uint8_t>(page_bytes);
-    float *d_quad = sb.take<float>(8);
-    uint8_t *d_patch = sb.take<uint8_t>((size_t)patch_cap + 1);
-    if (!d_patch) {
-        ms_set_error("ms_warp_quad_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    uint8_t *d_page, *d_patch;
+    float *d_quad;
+    MS_TRY(stage_carve(ctx, "ms_warp_quad_host", [&](ms_bump &sb) {
+        d_page = sb.take<uint8_t>(page_bytes);
+        d_quad = sb.take<float>(8);
+        d_patch = sb.take<uint8_t>((size_t)patch_cap + 1);
+    }));
     cudaStream_t st = ctx->own_stream;
     MS_CUDA(cudaMemcpyAsync(d_page, page, page_bytes, cudaMemcpyHostToDevice, st));
     MS_CUDA(cudaMemcpyAsync(d_quad, quad, 32, cudaMemcpyHostToDevice, st));
-    MS_TRY(ms_arena_reserve(ctx, 8192));
-    ms_bump bump{ctx->arena, 0, ctx->arena_bytes};
+    ms_bump bump;
+    MS_TRY(arena_bump(ctx, 8192, bump));
     MS_TRY(msk_quad_warp(ctx, d_page, img_h, img_w, d_quad, border_mode, border_value, d_patch, (size_t)patch_cap, w, h,
                          bump, st));
     const size_t bytes = (size_t)(*w) * (*h) * 3;
@@ -1487,68 +1490,57 @@ extern "C" int ms_page_batch_ragged_host_ex(ms_ctx *ctx, const float *score, con
         }
         img_total += al256((size_t)page_hw[2 * i] * page_hw[2 * i + 1] * 3);
     }
+    pb_call c;  // the caller's buffers
+    pb_init(c, p);
+    c.score = score; c.geo = geo; c.page_ptrs = pages; c.page_hw = page_hw;
+    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w;
+    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
+    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
+    c.batch = batch_host; c.batch_dtype = batch_dtype; c.flags = flags;
     const bool want_batch = batch_host || batch_dev_out;
     void *caller_batch = batch_dev_out ? *batch_dev_out : nullptr;  // caller-owned device buffer (see ms_page_batch_host)
     const size_t plane = (size_t)map_h * map_w;
     const size_t one_f = (size_t)3 * out_h * out_w * ms_dtype_bytes(batch_dtype);  // bytes of one crop of the batch
-    size_t need = al256(n_pages * plane * 4) + al256(n_pages * plane * 32) + al256((size_t)n_pages * cap_boxes * 36) +
-                  4 * al256((size_t)n_pages * 8) + img_total + al256((size_t)crops_cap * 20) + 8192;
-    if (want_batch && !caller_batch) need += al256((size_t)crops_cap * one_f);
-    MS_TRY(ms_stage_reserve(ctx, need));
-    ms_bump sb{ctx->stage, 0, ctx->stage_bytes};
-    float *d_score = sb.take<float>(n_pages * plane);
-    float *d_geo = sb.take<float>(n_pages * plane * 8);
-    float *d_boxes = sb.take<float>((size_t)n_pages * cap_boxes * 9);
-    int32_t *d_cnt = sb.take<int32_t>(n_pages);
-    int32_t *d_flags = sb.take<int32_t>(n_pages);
-    const uint8_t **d_ptrs = sb.take<const uint8_t *>(n_pages);
-    int32_t *d_hw = sb.take<int32_t>((size_t)n_pages * 2);
-    int32_t *d_crops = sb.take<int32_t>((size_t)crops_cap * 5);
-    int32_t *d_nc = sb.take<int32_t>(1);
-    void *d_batch = !want_batch ? nullptr : caller_batch ? caller_batch : sb.take<char>((size_t)crops_cap * one_f);
-    uint8_t *d_img = sb.take<uint8_t>(img_total);
-    if (!d_img || (want_batch && !d_batch)) {
-        ms_set_error("ms_page_batch_ragged_host: staging too small");
-        return MS_ERR_CAPACITY;
-    }
+    pb_call d = c;  // the same call on device staging
+    float *d_score, *d_geo;
+    const uint8_t **d_ptrs;
+    int32_t *d_hw;
+    uint8_t *d_img;
+    MS_TRY(stage_carve(ctx, "ms_page_batch_ragged_host", [&](ms_bump &sb) {
+        d_score = sb.take<float>(n_pages * plane);
+        d_geo = sb.take<float>(n_pages * plane * 8);
+        d.boxes_out = sb.take<float>((size_t)n_pages * cap_boxes * 9);
+        d.box_counts = sb.take<int32_t>(n_pages);
+        d.flags = sb.take<int32_t>(n_pages);
+        d_ptrs = sb.take<const uint8_t *>(n_pages);
+        d_hw = sb.take<int32_t>((size_t)n_pages * 2);
+        d.crops_out = sb.take<int32_t>((size_t)crops_cap * 5);
+        d.n_crops = sb.take<int32_t>(1);
+        d.batch = !want_batch ? nullptr : caller_batch ? caller_batch : sb.take<char>((size_t)crops_cap * one_f);
+        d_img = sb.take<uint8_t>(img_total);
+    }));
+    d.score = d_score;
+    d.geo = d_geo;
+    d.page_ptrs = d_ptrs;
+    d.page_hw = d_hw;
     cudaStream_t st = ctx->own_stream;
     std::vector<const uint8_t *> h_ptrs(n_pages);
-    size_t off = 0;
-    for (int i = 0; i < n_pages; i++) {
-        const size_t bytes = (size_t)page_hw[2 * i] * page_hw[2 * i + 1] * 3;
-        h_ptrs[i] = d_img + off;
-        MS_CUDA(cudaMemcpyAsync(d_img + off, pages[i], bytes, cudaMemcpyHostToDevice, st));
-        off += al256(bytes);
+    for (bool again = true; again;) {
+        size_t off = 0;
+        for (int i = 0; i < n_pages; i++) {
+            const size_t bytes = (size_t)page_hw[2 * i] * page_hw[2 * i + 1] * 3;
+            h_ptrs[i] = d_img + off;
+            MS_CUDA(cudaMemcpyAsync(d_img + off, pages[i], bytes, cudaMemcpyHostToDevice, st));
+            off += al256(bytes);
+        }
+        MS_CUDA(cudaMemcpyAsync(d_ptrs, h_ptrs.data(), (size_t)n_pages * sizeof(void *), cudaMemcpyHostToDevice, st));
+        MS_CUDA(cudaMemcpyAsync(d_hw, page_hw, (size_t)n_pages * 8, cudaMemcpyHostToDevice, st));
+        MS_CUDA(cudaMemcpyAsync(d_score, score, n_pages * plane * 4, cudaMemcpyHostToDevice, st));
+        MS_CUDA(cudaMemcpyAsync(d_geo, geo, n_pages * plane * 32, cudaMemcpyHostToDevice, st));
+        MS_CUDA(cudaStreamSynchronize(st));  // h_ptrs is pageable host memory on this frame
+        MS_TRY(page_batch_impl(ctx, d, 0, n_pages, 0, st));
+        MS_TRY(pb_host_read_back(ctx, c, d, batch_dev_out, "page_batch_ragged", &again));
     }
-    MS_CUDA(cudaMemcpyAsync(d_ptrs, h_ptrs.data(), (size_t)n_pages * sizeof(void *), cudaMemcpyHostToDevice, st));
-    MS_CUDA(cudaMemcpyAsync(d_hw, page_hw, (size_t)n_pages * 8, cudaMemcpyHostToDevice, st));
-    MS_CUDA(cudaMemcpyAsync(d_score, score, n_pages * plane * 4, cudaMemcpyHostToDevice, st));
-    MS_CUDA(cudaMemcpyAsync(d_geo, geo, n_pages * plane * 32, cudaMemcpyHostToDevice, st));
-    MS_CUDA(cudaStreamSynchronize(st));  // h_ptrs is pageable host memory on this frame
-    MS_TRY(page_batch_impl(ctx, d_score, d_geo, nullptr, n_pages, 0, n_pages, map_h, map_w, 0, 0, p, min_text_size, out_h,
-                           out_w, cap_boxes, d_boxes, d_cnt, d_crops, crops_cap, d_nc, 0, d_batch, batch_dtype, nullptr,
-                           d_flags, st, 0, d_ptrs, d_hw));
-    MS_CUDA(cudaMemcpyAsync(box_counts, d_cnt, (size_t)n_pages * 4, cudaMemcpyDeviceToHost, st));
-    MS_CUDA(cudaMemcpyAsync(flags, d_flags, (size_t)n_pages * 4, cudaMemcpyDeviceToHost, st));
-    MS_CUDA(cudaMemcpyAsync(boxes_out, d_boxes, (size_t)n_pages * cap_boxes * 36, cudaMemcpyDeviceToHost, st));
-    MS_CUDA(cudaMemcpyAsync(n_crops, d_nc, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    MS_CUDA(cudaStreamSynchronize(st));
-    int32_t all = 0;
-    for (int i = 0; i < n_pages; i++) all |= flags[i];
-    if (grow_edge_factor(ctx, all))
-        return ms_page_batch_ragged_host_ex(ctx, score, geo, pages, page_hw, n_pages, map_h, map_w, p, min_text_size,
-                                            out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops,
-                                            batch_host, batch_dtype, batch_dev_out, flags);
-    MS_TRY(flags_to_rc(all, "page_batch_ragged"));
-    int64_t nc = *n_crops;
-    if (nc > crops_cap) nc = crops_cap;
-    if (nc > 0) {
-        MS_CUDA(cudaMemcpyAsync(crops_out, d_crops, (size_t)nc * 20, cudaMemcpyDeviceToHost, st));
-        if (batch_host)
-            MS_CUDA(cudaMemcpyAsync(batch_host, d_batch, (size_t)nc * one_f, cudaMemcpyDeviceToHost, st));
-        MS_CUDA(cudaStreamSynchronize(st));
-    }
-    if (batch_dev_out) *batch_dev_out = d_batch;
     return MS_OK;
 }
 

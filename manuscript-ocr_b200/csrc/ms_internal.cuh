@@ -11,19 +11,40 @@
 
 #define MS_NUM_SMS_B200 148
 
-// One recorded ms_page_batch call (all arguments) and, from its second occurrence on, the CUDA graph of its launches.
-struct ms_pb_key {
-    const void *ptr[14];
-    long long num[13];
+// Everything that defines one page-batch call (api.cu).  Per-page arrays point at the call's page 0 and are
+// page-strided: score (n_pages, map_h, map_w), geo (n_pages, 8, map_h / q or map_h, map_w), boxes_out (n_pages,
+// cap_boxes, 9), box_counts / flags (n_pages), page_hw (n_pages, 2).  pages (n_pages, img_h, img_w, 3) u8 or, for
+// images of their own sizes, page_ptrs + page_hw.  The host entry points describe the caller's host buffers in one
+// pb_call and the device staging in a copy of it.
+struct pb_call {
+    const float *score, *geo;
+    const uint8_t *pages;
+    const uint8_t *const *page_ptrs;
+    const int32_t *page_hw;
+    int n_pages, map_h, map_w, img_h, img_w, min_text_size, out_h, out_w, cap_boxes;
+    int64_t crops_cap;
     ms_east_params params;
+    float *boxes_out;
+    int32_t *box_counts, *crops_out, *n_crops;
+    void *batch;
+    int batch_dtype;
+    uint8_t *canvas_u8;
+    int32_t *flags;
+    int geo_compact;  // geo holds only the rows the decode reads, y % q == q / 2 (q = params.quantization)
 };
+// A recorded ms_page_batch call and what its launches point into or were sized by; compared bytewise.
+struct ms_pb_key {
+    pb_call call;
+    const char *arena;
+    size_t arena_bytes;
+    int edge_factor;
+};
+// ... and, from its second occurrence on, the CUDA graph of its launches.
 struct ms_graph_entry {
     ms_pb_key key;
     int used, failed;
     cudaGraphExec_t exec;
     int64_t launches;  // kernels per replay (for ms_launch_count)
-    char *arena;       // the scratch arena the graph's kernels point into
-    size_t arena_bytes;
 };
 #define MS_GRAPH_SLOTS 4
 
