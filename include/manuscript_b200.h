@@ -202,6 +202,16 @@ MS_API int ms_warp_quad_host(ms_ctx *ctx, const uint8_t *page, int img_h, int im
 MS_API int ms_detector_input(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, int target_h, int target_w,
                       float *out_f32, uint8_t *out_u8, void *stream);
 
+/* infer.py:301-305 (as ms_detector_input) for n_pages pages of their own sizes in one call: page_ptrs (n_pages) device
+ * pointers to (h_i,w_i,3) u8 RGB images and page_hw (n_pages,2) int32 on the device -- the tables ms_page_batch_ragged
+ * takes -> out (n_pages,3,target_h,target_w) in out_dtype (MS_DTYPE_*).  Every page is bit for bit what
+ * ms_detector_input makes of it.  MS_DTYPE_F16 / MS_DTYPE_BF16 (an EXTENSION) are that float32 value rounded to
+ * nearest-even, bit for bit out_f32.to(torch.float16 / torch.bfloat16); nothing is normalised in 16 bits.  Page sizes
+ * are device data: a page with h <= 0, w <= 0 or a NULL pointer is not read and its input is written as zeros.  NULL
+ * tables or output, n_pages <= 0, a non-positive target or an unknown dtype is MS_ERR_INVALID. */
+MS_API int ms_detector_input_batch(ms_ctx *ctx, const uint8_t *const *page_ptrs, const int32_t *page_hw, int n_pages,
+                                   int target_h, int target_w, void *out, int out_dtype, void *stream);
+
 /* utils.py:328 for n_pages maps.  score (n_pages,map_h,map_w), geo (n_pages,8,map_h,map_w).
  * quads_out (n_pages*cap_per_page,9); counts (n_pages) int32; flags (n_pages) int32 (OR-ed). */
 MS_API int ms_decode_quads(ms_ctx *ctx, const float *score, const float *geo, int n_pages, int map_h, int map_w,

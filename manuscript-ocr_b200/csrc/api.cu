@@ -510,7 +510,25 @@ extern "C" int ms_detector_input(ms_ctx *ctx, const uint8_t *page, int img_h, in
                                  float *out_f32, uint8_t *out_u8, void *stream)
 {
     MS_CTX(ctx);
-    return msk_detector_input(ctx, page, img_h, img_w, target_h, target_w, out_f32, out_u8, (cudaStream_t)stream);
+    ms_bump bump;  // the arguments are checked by msk_detector_input
+    MS_TRY(arena_bump(ctx, msk_detector_input_scratch(1, target_h, target_w), bump));
+    return msk_detector_input(ctx, nullptr, nullptr, page, img_h, img_w, 1, target_h, target_w, out_f32, MS_DTYPE_F32,
+                              out_u8, bump, (cudaStream_t)stream);
+}
+
+extern "C" int ms_detector_input_batch(ms_ctx *ctx, const uint8_t *const *page_ptrs, const int32_t *page_hw,
+                                       int n_pages, int target_h, int target_w, void *out, int out_dtype, void *stream)
+{
+    MS_CTX(ctx);
+    MS_TRY(dtype_ok(out_dtype, "ms_detector_input_batch"));
+    if (!page_ptrs || !page_hw || !out) {
+        ms_set_error("ms_detector_input_batch: NULL tables or output");
+        return MS_ERR_INVALID;
+    }
+    ms_bump bump;  // the sizes are checked by msk_detector_input
+    MS_TRY(arena_bump(ctx, msk_detector_input_scratch(n_pages, target_h, target_w), bump));
+    return msk_detector_input(ctx, page_ptrs, page_hw, nullptr, 0, 0, n_pages, target_h, target_w, out, out_dtype,
+                              nullptr, bump, (cudaStream_t)stream);
 }
 
 extern "C" int ms_tps_rectify(ms_ctx *ctx, const float *input, const float *c_prime, const float *inv_delta_c,

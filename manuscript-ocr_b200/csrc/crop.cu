@@ -361,59 +361,196 @@ __global__ void __launch_bounds__(256) crop_generic_kernel(const Plan *__restric
 
 // ---- detector input (the caller side of the path, EAST.predict infer.py:301-305) ---------------------------------
 // cv2.resize(img, (T, T)) -- INTER_LINEAR on uint8 (11-bit fixed-point coefficients, aspect NOT preserved), then
-// torchvision ToTensor (x / 255) and Normalize(0.5, 0.5) ((x - 0.5) / 0.5), written as the (3, T, T) float32 network
-// input.  Same arithmetic as resample_px's linear branch (the oracle's orc_resize_linear_u8c3, pinned to cv2 for
-// shrinking and enlarging); a thread per destination pixel, the source page is read through L2.  This is what lets
-// the page cross PCIe once: the original image is uploaded, the resized detector input is made on the device.
-__global__ void __launch_bounds__(256) detector_input_kernel(const uint8_t *__restrict__ page, int H, int W, int th,
-                                                             int tw, float *__restrict__ out_f32,
-                                                             uint8_t *__restrict__ out_u8)
+// torchvision ToTensor (x / 255) and Normalize(0.5, 0.5) ((x - 0.5) / 0.5), written as the (P, 3, th, tw) network input
+// in float32, or that float32 value rounded to nearest-even in 16 bits.  Same arithmetic as resample_px's linear branch
+// (the oracle's orc_resize_linear_u8c3, pinned to cv2 for shrinking and enlarging).  This is what lets a page cross
+// PCIe once: the original image is uploaded, the resized detector input is made on the device.
+//
+// HBM roofline: per page the distinct source rows the y table names (3 * w bytes each) read, 3 * th * tw * element size
+// written.  64 scans of ~2500 x 3500 at T = 1280: ~1.5 GB read, 1.26 GB written in float32.
+//
+// Kernels:
+//   detector_input_plan_kernel  thread per axis entry: every page's source, size and OpenCV x / y tables, once per page
+//   detector_input_batch_kernel a warp per chunk of an output row: lanes resample consecutive pixels (the source rows
+//                               read through L1), then each thread stores 4 (float32) or 8 (16-bit) consecutive pixels
+//                               of every plane as one 16-byte vector
+struct DetPage {
+    const uint8_t *src;
+    int h, w;  // 0 x 0: the page is not read and its input is all zeros
+    int same;  // the page already has the target size: cv2.resize returns a copy
+};
+
+// The page is table entry p, or -- page_ptrs == NULL -- the one page passed by value (ms_detector_input).
+__global__ void __launch_bounds__(256) detector_input_plan_kernel(const uint8_t *const *__restrict__ page_ptrs,
+                                                                  const int32_t *__restrict__ page_hw,
+                                                                  const uint8_t *one, int one_h, int one_w,
+                                                                  int n_pages, int th, int tw, DetPage *__restrict__ pages,
+                                                                  AxisEnt *__restrict__ tabs)
 {
     ms_pdl_wait();
-    const double scale_x = 1.0 / ((double)tw / (double)W), scale_y = 1.0 / ((double)th / (double)H);
-    const bool same = (th == H && tw == W);  // cv2.resize returns a copy
+    const int per = tw + th;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < (int64_t)n_pages * per;
+         i += (int64_t)gridDim.x * blockDim.x) {
+        const int p = (int)(i / per), t = (int)(i - (int64_t)p * per);
+        const uint8_t *src = page_ptrs ? page_ptrs[p] : one;
+        int H = page_ptrs ? page_hw[2 * p] : one_h, W = page_ptrs ? page_hw[2 * p + 1] : one_w;
+        if (!src || H <= 0 || W <= 0) H = W = 0;
+        const bool same = H == th && W == tw;
+        if (t == 0) pages[p] = DetPage{src, H, W, same ? 1 : 0};
+        if (H == 0) continue;
+        AxisEnt e = {};
+        if (same) {  // the copy reads destination row d from source row d
+            if (t >= tw) e.s0 = e.n = t - tw;
+        } else if (t < tw)
+            e = linear_entry_x(t, 1.0 / ((double)tw / (double)W), W);
+        else
+            e = linear_entry_y(t - tw, 1.0 / ((double)th / (double)H), H);
+        tabs[i] = e;
+    }
+}
+
+constexpr int kDetThreads = 256;
+
+// A warp makes chunks of 32 * kV consecutive pixels of an output row: lane l resamples pixels l, l + 32, ... (neighbouring
+// lanes read neighbouring source bytes, through L1), the values go through the warp's slice of shared memory, and lane l
+// stores pixels [l * kV, l * kV + kV) of each plane as one 16-byte vector.
+template <class T, bool kWriteU8>
+__global__ void __launch_bounds__(kDetThreads) detector_input_batch_kernel(const DetPage *__restrict__ pages,
+                                                                           const AxisEnt *__restrict__ tabs, int n_pages,
+                                                                           int th, int tw, T *__restrict__ out,
+                                                                           uint8_t *__restrict__ out_u8, int vec_ok)
+{
+    ms_pdl_wait();
+    constexpr int kV = kBatchVec<T>, kChunk = 32 * kV, kWarps = kDetThreads / 32;
+    constexpr int kElt = kHasBatch<T> ? (int)sizeof(T) : 1;
+    __shared__ __align__(16) unsigned char s_tr[kWarps][3][kChunk * kElt];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int per = tw + th, chunks = (tw + kChunk - 1) / kChunk;
     const size_t plane = (size_t)th * tw;
-    const PitchedSrc src{page, (size_t)W * 3};
-    Plan p;
-    p.interp = same ? 0 : 1;
-    p.isx = p.isy = 0;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < plane; i += (size_t)gridDim.x * blockDim.x) {
-        const int dy = (int)(i / tw), dx = (int)(i - (size_t)dy * tw);
-        AxisEnt ex = {}, ey = {};
-        if (!same) {
-            ex = linear_entry_x(dx, scale_x, W);
-            ey = linear_entry_y(dy, scale_y, H);
+    // (page, row, chunk) tasks, fewer than 2^31 (the host checks), dealt out warp by warp over the grid (1-8 % faster
+    // on a B200 than a contiguous run of rows per CTA, which keeps more of a page's x table in L1; profiles/README.md)
+    const int tasks = n_pages * th * chunks;
+    for (int task = blockIdx.x * kWarps + warp; task < tasks; task += gridDim.x * kWarps) {
+        const int item = task / chunks;
+        const int p = item / th, dy = item - p * th;
+        const int x0 = (task - item * chunks) * kChunk;
+        const DetPage pg = pages[p];
+        const AxisEnt *xt = tabs + (size_t)p * per;
+        T *orow = kHasBatch<T> ? out + (size_t)p * 3 * plane + (size_t)dy * tw : nullptr;
+        uint8_t *urow = kWriteU8 ? out_u8 + ((size_t)p * plane + (size_t)dy * tw) * 3 : nullptr;
+        // the row's two source rows as rows 0 and 1 of one pitched source
+        PitchedSrc src{nullptr, 0};
+        AxisEnt ey = {};
+        if (pg.h > 0) {
+            ey = xt[tw + dy];
+            const size_t stride = (size_t)pg.w * 3;
+            src = PitchedSrc{pg.src + (size_t)ey.s0 * stride, (size_t)(ey.n - ey.s0) * stride};
+            ey.s0 = 0;
+            ey.n = 1;
         }
-        unsigned char o0, o1, o2;
-        resample_px(p, dx, dy, src, ex, ey, o0, o1, o2);
-        if (out_f32) {
-            out_f32[i] = ((float)o0 / 255.0f - 0.5f) / 0.5f;
-            out_f32[plane + i] = ((float)o1 / 255.0f - 0.5f) / 0.5f;
-            out_f32[2 * plane + i] = ((float)o2 / 255.0f - 0.5f) / 0.5f;
+        Plan pl;
+        pl.interp = pg.same ? 0 : 1;
+        pl.isx = pl.isy = 0;
+        T *tr = kHasBatch<T> ? reinterpret_cast<T *>(&s_tr[warp][0][0]) : nullptr;
+#pragma unroll 1  // rolled: 48 registers, 5 CTAs per SM (unrolled, 60: bfloat16 9 % slower, profiles/README.md)
+        for (int k = 0; k < kV; k++) {
+            const int dx = x0 + k * 32 + lane;
+            unsigned char o0 = 0, o1 = 0, o2 = 0;
+            if (dx < tw && pg.h > 0) {
+                AxisEnt ex = {};
+                if (!pg.same) {
+                    const int4 q = __ldg(reinterpret_cast<const int4 *>(xt + dx));  // s0, n, nfirst, nmid
+                    ex.s0 = q.x;
+                    ex.n = q.y;
+                    ex.nfirst = q.z;
+                    ex.nmid = q.w;
+                }
+                resample_px(pl, dx, 0, src, ex, ey, o0, o1, o2);
+            }
+            if constexpr (kHasBatch<T>) {
+                const float f[3] = {pg.h > 0 ? ((float)o0 / 255.0f - 0.5f) / 0.5f : 0.f,
+                                    pg.h > 0 ? ((float)o1 / 255.0f - 0.5f) / 0.5f : 0.f,
+                                    pg.h > 0 ? ((float)o2 / 255.0f - 0.5f) / 0.5f : 0.f};
+#pragma unroll
+                for (int c = 0; c < 3; c++) {
+                    if (vec_ok)
+                        tr[c * kChunk + k * 32 + lane] = to_batch<T>(f[c]);
+                    else if (dx < tw)
+                        orow[c * plane + dx] = to_batch<T>(f[c]);
+                }
+            }
+            if (kWriteU8 && dx < tw) {
+                urow[(size_t)dx * 3] = o0;
+                urow[(size_t)dx * 3 + 1] = o1;
+                urow[(size_t)dx * 3 + 2] = o2;
+            }
         }
-        if (out_u8) {
-            out_u8[i * 3] = o0;
-            out_u8[i * 3 + 1] = o1;
-            out_u8[i * 3 + 2] = o2;
+        if constexpr (kHasBatch<T>) {
+            if (vec_ok) {  // tw % kV == 0 and a 16-byte-aligned output: every lane's kV pixels are whole and aligned
+                __syncwarp();
+                if (x0 + lane * kV < tw)
+#pragma unroll
+                    for (int c = 0; c < 3; c++)
+                        __stcs(reinterpret_cast<float4 *>(orow + c * plane + x0 + lane * kV),
+                               *reinterpret_cast<const float4 *>(&s_tr[warp][c][lane * kV * kElt]));
+                __syncwarp();  // the slice is reused by the warp's next chunk
+            }
         }
     }
 }
 
 }  // namespace
 
-int msk_detector_input(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, int target_h, int target_w,
-                       float *out_f32, uint8_t *out_u8, cudaStream_t st)
+// 0 for sizes msk_detector_input rejects.  The one-page ms_detector_input uses the context's scratch arena as well (the
+// first call, or a larger target, grows it: one cudaMalloc after a device synchronisation).
+size_t msk_detector_input_scratch(int n_pages, int target_h, int target_w)
 {
-    if (!page || img_h <= 0 || img_w <= 0 || target_h <= 0 || target_w <= 0 || (!out_f32 && !out_u8)) {
+    if (n_pages <= 0 || target_h <= 0 || target_w <= 0 || (int64_t)target_h + target_w >= ((int64_t)1 << 30)) return 0;
+    return (size_t)n_pages * sizeof(DetPage) + (size_t)n_pages * (size_t)(target_h + target_w) * sizeof(AxisEnt) + 1024;
+}
+
+int msk_detector_input(ms_ctx *ctx, const uint8_t *const *page_ptrs, const int32_t *page_hw, const uint8_t *one,
+                       int one_h, int one_w, int n_pages, int target_h, int target_w, void *out, int out_dtype,
+                       uint8_t *out_u8, ms_bump bump, cudaStream_t st)
+{
+    const bool tables = page_ptrs != nullptr && page_hw != nullptr;
+    if (n_pages <= 0 || target_h <= 0 || target_w <= 0 || (!out && !out_u8) ||
+        (!tables && (!one || one_h <= 0 || one_w <= 0 || n_pages != 1))) {
         ms_set_error("detector_input: bad arguments");
         return MS_ERR_INVALID;
     }
-    const size_t n = (size_t)target_h * target_w;
-    size_t grid = (n + 255) / 256;
-    if (grid > (size_t)ctx->num_sms * 16) grid = (size_t)ctx->num_sms * 16;
-    ms_launch(detector_input_kernel, (int)grid, 256, 0, st, page, img_h, img_w, target_h, target_w, out_f32, out_u8);
+    // the kernel counts (page, row, column chunk) tasks in 32 bits; its chunks are at least 32 pixels wide, so this
+    // bounds the task count
+    if ((int64_t)n_pages * target_h * ((target_w + 31) / 32) >= ((int64_t)1 << 31) ||
+        (int64_t)target_h + target_w >= ((int64_t)1 << 30)) {
+        ms_set_error("detector_input: %d pages of %d x %d are too many pixels for one call", n_pages, target_h, target_w);
+        return MS_ERR_INVALID;
+    }
+    DetPage *pages = bump.take<DetPage>((size_t)n_pages);
+    AxisEnt *tabs = bump.take<AxisEnt>((size_t)n_pages * (target_h + target_w));
+    if (!pages || !tabs) {
+        ms_set_error("detector_input: scratch too small");
+        return MS_ERR_CAPACITY;
+    }
+    const int64_t entries = (int64_t)n_pages * (target_h + target_w);
+    int64_t pgrid = (entries + 255) / 256;
+    if (pgrid > (int64_t)ctx->num_sms * 8) pgrid = (int64_t)ctx->num_sms * 8;
+    ms_launch(detector_input_plan_kernel, (int)pgrid, 256, 0, st, tables ? page_ptrs : nullptr, page_hw, one, one_h,
+              one_w, n_pages, target_h, target_w, pages, tabs);
     MS_LAUNCH_CHECK(ctx);
-    return MS_OK;
+    return launch_for_outputs(out, out_dtype, out_u8, [&](auto bt, auto u8) {
+        using T = typename decltype(bt)::type;
+        constexpr bool kU8 = decltype(u8)::value;
+        // one wave of CTAs (the kernel loops over its tasks)
+        int per_sm = 1;
+        MS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, detector_input_batch_kernel<T, kU8>, kDetThreads, 0));
+        const int64_t wave = (int64_t)ctx->num_sms * (per_sm > 0 ? per_sm : 1);
+        const int64_t grid = (int64_t)n_pages * target_h < wave ? (int64_t)n_pages * target_h : wave;
+        ms_launch(detector_input_batch_kernel<T, kU8>, (int)grid, kDetThreads, 0, st, pages, tabs, n_pages, target_h,
+                  target_w, static_cast<T *>(out), out_u8, batch_vec_ok<T>(out, target_w));
+        MS_LAUNCH_CHECK(ctx);
+        return MS_OK;
+    });
 }
 
 // scratch that depends on the page count as well: the work-list buckets

@@ -258,8 +258,12 @@ int msk_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_
 // tps.cu
 int msk_tps_rectify(ms_ctx *ctx, const float *input, const float *c_prime, const float *inv_delta_c, const float *p_hat_t,
                     int batch, int n_fid, int chans, int in_h, int in_w, int out_h, int out_w, float *out, cudaStream_t st);
-int msk_detector_input(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, int target_h, int target_w,
-                       float *out_f32, uint8_t *out_u8, cudaStream_t st);
+// detector input of n_pages pages: page_ptrs / page_hw (device tables) or, when they are NULL, the one page `one`
+// (one_h, one_w).  out (n_pages, 3, target_h, target_w) of out_dtype and / or out_u8 (n_pages, target_h, target_w, 3)
+int msk_detector_input(ms_ctx *ctx, const uint8_t *const *page_ptrs, const int32_t *page_hw, const uint8_t *one,
+                       int one_h, int one_w, int n_pages, int target_h, int target_w, void *out, int out_dtype,
+                       uint8_t *out_u8, ms_bump bump, cudaStream_t st);
+size_t msk_detector_input_scratch(int n_pages, int target_h, int target_w);
 size_t msk_crop_scratch(int64_t crops_cap, int n_pages);
 // quadcrop.cu
 int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w, const float *quads,

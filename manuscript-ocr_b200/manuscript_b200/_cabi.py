@@ -100,6 +100,7 @@ SIGNATURES = {
     "ms_quad_crop_resize_pad": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _vp, _i64, _i, _i, _i, _i, _i, _vp, _vp, _vp,
                                      _vp]),
     "ms_detector_input": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "ms_detector_input_batch": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _i, _vp]),
     "ms_tps_rectify": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "ms_decode_quads": (_i, [_vp, _vp, _vp, _i, _i, _i, _f, _d, _i, _vp, _i, _vp, _vp, _vp]),
     "ms_lanms": (_i, [_vp, _vp, _vp, _i, _i, _d, _vp, _vp, _vp, _vp]),

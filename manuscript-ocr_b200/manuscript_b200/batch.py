@@ -86,10 +86,14 @@ class PageBatch:
     """Reusable runner for one GPU.  Output buffers are allocated once per shape and reused.
 
     batch_dtype: element type of the crop batch, torch.float32 (default), torch.float16 or torch.bfloat16.  A 16-bit
-    batch is written by the crop kernels directly and equals the float32 batch cast with .to(batch_dtype)."""
+    batch is written by the crop kernels directly and equals the float32 batch cast with .to(batch_dtype).
+
+    crops_cap: crop rows of the buffers (default n_pages * cap_boxes); it may be changed between calls, and the next
+    call reallocates.  max_buffer_sets: keep the device buffers of at most this many page counts, dropping the least
+    recently used (default: one set per page count seen)."""
 
     def __init__(self, device=0, params=None, min_text_size=5, out_hw=(32, 128), cap_boxes=4096, crops_cap=None,
-                 want_batch=True, batch_dtype=None):
+                 want_batch=True, batch_dtype=None, max_buffer_sets=None):
         import torch
 
         if not torch.cuda.is_available():
@@ -105,6 +109,7 @@ class PageBatch:
         self.want_batch = bool(want_batch)
         self.batch_dtype = torch.float32 if batch_dtype is None else batch_dtype
         self._dtype_code = batch_dtype_code(self.batch_dtype)
+        self.max_buffer_sets = max_buffer_sets
         self._bufs = {}
         self._host = {}
         self._ragged_tables = {}
@@ -113,9 +118,14 @@ class PageBatch:
     def _device_bufs(self, n_pages):
         torch = self.torch
         key = n_pages
-        b = self._bufs.get(key)
+        cap = self.crops_cap if self.crops_cap is not None else n_pages * self.cap_boxes
+        b = self._bufs.pop(key, None)  # re-inserted below: the dict is kept in least-recently-used order
+        if b is not None and b["cap"] != cap:
+            b = None
         if b is None:
-            cap = self.crops_cap if self.crops_cap is not None else n_pages * self.cap_boxes
+            if self.max_buffer_sets is not None:
+                while len(self._bufs) >= self.max_buffer_sets:
+                    del self._bufs[next(iter(self._bufs))]
             dev = self.device
             b = dict(
                 boxes=torch.empty((n_pages, self.cap_boxes, 9), dtype=torch.float32, device=dev),
@@ -127,7 +137,7 @@ class PageBatch:
                        if self.want_batch else None),
                 cap=cap,
             )
-            self._bufs[key] = b
+        self._bufs[key] = b
         return b
 
     def run(self, score, geo, pages=None, sync=False):

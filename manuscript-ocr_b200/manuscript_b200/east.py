@@ -7,6 +7,11 @@ caller as any callable / nn.Module returning {"score": (1,1,H,W), "geometry": (1
 in the CUDA kernels of this package: the ORIGINAL image is uploaded once, the resized + normalised network input is made
 on the device (ms_detector_input = cv2.resize INTER_LINEAR + ToTensor + Normalize, infer.py:301-305), and the maps never
 leave the device (the reference's `.cpu().numpy()` at infer.py:312-313 is gone).
+
+Many pages at once: upload_batch puts a list of images into one device buffer, and network_inputs makes all their
+network inputs with one ms_detector_input_batch launch.  input_dtype=torch.float16 / torch.bfloat16 (an extension) makes
+the network input 16-bit: exactly the float32 input cast with `.to(input_dtype)`.  The caller owns the network's dtype;
+maps that come back in another dtype are converted to float32 for the post-processing.
 """
 import ctypes as C
 import time
@@ -14,7 +19,7 @@ from pathlib import Path
 
 import numpy as np
 
-from ._cabi import MS_FLAG_EDGE_OVERFLOW, EastParams, check
+from ._cabi import MS_FLAG_EDGE_OVERFLOW, EastParams, batch_dtype_code, check
 from .batch import PageBatch, _raise_for_flags
 from .imaging import read_image, visualize_page
 from .reading_order import reorder_words
@@ -56,7 +61,7 @@ class EAST:
     def __init__(self, model=None, target_size=1280, expand_ratio_w=0.9, expand_ratio_h=0.9, score_thresh=0.6,
                  iou_threshold=0.2, score_geo_scale=0.25, quantization=2, axis_aligned_output=True,
                  remove_area_anomalies=True, anomaly_sigma_threshold=5.0, anomaly_min_box_count=30, device=0,
-                 cap_boxes=8192):
+                 cap_boxes=8192, input_dtype=None):
         import torch
 
         if not torch.cuda.is_available():
@@ -76,10 +81,15 @@ class EAST:
         self.anomaly_sigma_threshold = anomaly_sigma_threshold
         self.anomaly_min_box_count = anomaly_min_box_count
         self.cap_boxes = int(cap_boxes)
+        self.input_dtype = torch.float32 if input_dtype is None else input_dtype
+        self._input_code = batch_dtype_code(self.input_dtype)
         self._runner = PageBatch(device=self.device.index or 0, params=self._params(), cap_boxes=cap_boxes,
                                  want_batch=False)
         self._page_buf = {}   # (h, w) -> persistent device image: stable addresses let repeated calls replay a CUDA graph
         self._input_buf = None
+        self._batch_buf = {}  # tuple of image shapes -> (device buffer, page views): see upload_batch
+        self._tables = {}     # page views -> their device pointer / size tables
+        self._inputs_buf = None
 
     @classmethod
     def from_pretrained(cls, weights_path=None, **kwargs):
@@ -172,11 +182,76 @@ class EAST:
         buf.copy_(torch.from_numpy(a), non_blocking=True)
         return buf
 
+    def upload_batch(self, images):
+        """List of (H_i, W_i, 3) uint8 RGB host arrays -> list of device views of the same images, one host-to-device copy
+        of pixels per page.  All pages live in one device buffer, each at a 16-byte-aligned offset (the crop kernels stage
+        such pages' rows by TMA); the buffer is kept per list of shapes, so a serving loop over batches of the same shapes
+        reuses the same addresses and the page batch replays its CUDA graph."""
+        torch = self.torch
+        arrs = []
+        for img in images:
+            a = np.asarray(img)
+            if a.ndim != 3 or a.shape[2] != 3 or a.dtype != np.uint8:
+                raise ValueError(f"EAST expects (H, W, 3) uint8 RGB images, got shape {a.shape} dtype {a.dtype}")
+            arrs.append(np.ascontiguousarray(a))
+        key = tuple(a.shape[:2] for a in arrs)
+        entry = self._batch_buf.get(key)
+        if entry is None:
+            offs, total = [], 0
+            for a in arrs:
+                offs.append(total)
+                total += (a.nbytes + 15) & ~15
+            if len(self._batch_buf) >= 4:
+                self._batch_buf.clear()
+                self._tables.clear()
+            buf = torch.empty((max(total, 16),), dtype=torch.uint8, device=self.device)
+            views = [buf[o:o + a.nbytes].view(a.shape) for o, a in zip(offs, arrs)]
+            entry = self._batch_buf[key] = (buf, views)
+        for v, a in zip(entry[1], arrs):
+            v.copy_(torch.from_numpy(a), non_blocking=True)
+        return list(entry[1])
+
+    def _page_tables(self, pages_dev):
+        """(pointer table, (P, 2) int32 size table) on the device for a list of device images, kept per list"""
+        torch = self.torch
+        for pg in pages_dev:
+            if not (pg.is_cuda and pg.dtype == torch.uint8 and pg.dim() == 3 and pg.shape[2] == 3 and pg.is_contiguous()):
+                raise ValueError("pages must be contiguous (H, W, 3) uint8 CUDA tensors")
+        sig = tuple((pg.data_ptr(), int(pg.shape[0]), int(pg.shape[1])) for pg in pages_dev)
+        t = self._tables.get(sig)
+        if t is None:
+            if len(self._tables) >= 8:
+                self._tables.clear()
+            t = self._tables[sig] = (torch.tensor([v[0] for v in sig], dtype=torch.int64).to(self.device),
+                                     torch.tensor([[v[1], v[2]] for v in sig], dtype=torch.int32).to(self.device))
+        return t
+
+    def network_inputs(self, pages_dev):
+        """infer.py:301-305 for a list of P device images of their own sizes in one launch (ms_detector_input_batch):
+        -> (P, 3, T, T) CUDA tensor of input_dtype, page i bit-identical to network_input(pages_dev[i]) (cast with
+        .to(input_dtype)).  The tensor is owned by this detector and overwritten by its next call."""
+        torch = self.torch
+        T, P = self.target_size, len(pages_dev)
+        if P == 0:
+            raise ValueError("network_inputs needs at least one page")
+        ptrs, hw = self._page_tables(pages_dev)
+        shape = (P, 3, T, T)
+        if self._inputs_buf is None or tuple(self._inputs_buf.shape) != shape or self._inputs_buf.dtype != self.input_dtype:
+            self._inputs_buf = torch.empty(shape, dtype=self.input_dtype, device=self.device)
+        r = self._runner
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            check(r.ctx.lib.ms_detector_input_batch(r.ctx.handle, ptrs.data_ptr(), hw.data_ptr(), P, T, T,
+                                                    self._inputs_buf.data_ptr(), self._input_code, C.c_void_p(stream)))
+        return self._inputs_buf
+
     def network_input(self, page_dev):
-        """infer.py:301-305 on the device: (H, W, 3) u8 CUDA tensor -> (1, 3, T, T) f32, bit-identical to
-        cv2.resize(img, (T, T)) -> ToTensor -> Normalize(0.5, 0.5)."""
+        """infer.py:301-305 on the device: (H, W, 3) u8 CUDA tensor -> (1, 3, T, T) of input_dtype, bit-identical to
+        cv2.resize(img, (T, T)) -> ToTensor -> Normalize(0.5, 0.5) (cast with .to(input_dtype))."""
         torch = self.torch
         T = self.target_size
+        if self.input_dtype != torch.float32:
+            return self.network_inputs([page_dev])
         if self._input_buf is None or self._input_buf.shape[-1] != T:
             self._input_buf = torch.empty((1, 3, T, T), dtype=torch.float32, device=self.device)
         r = self._runner
@@ -194,7 +269,16 @@ class EAST:
                                "package (use boxes_from_maps / predict_from_maps when the maps already exist)")
         with self.torch.no_grad():
             out = self.model(self.network_input(page_dev))
-        return out["score"][0], out["geometry"][0]
+        return out["score"][0].float(), out["geometry"][0].float()
+
+    def maps_from_device_pages(self, pages_dev):
+        """List of P device images -> (score (P,1,H',W'), geometry (P,8,H',W')) float32 CUDA tensors: one
+        network_inputs launch and one call of the network on the (P, 3, T, T) input."""
+        if self.model is None:
+            raise RuntimeError("EAST(model=...) is required for predict()")
+        with self.torch.no_grad():
+            out = self.model(self.network_inputs(pages_dev))
+        return out["score"].float(), out["geometry"].float()
 
     def predict_from_maps(self, score_map, geo_map, orig_hw, sort_reading_order=False):
         words = words_from_boxes(self.boxes_from_maps(score_map, geo_map, orig_hw))

@@ -14,6 +14,9 @@ Three routes through predict(), all with the reference's results:
 * HOST CROPS -- a foreign recogniser gets the list of uint8 crops it expects (plain slices of the page image), in the
   reading order computed on the device.
 
+process_batch on the fused route works on chunks of pages: one upload buffer, one detector-input launch, one network
+call and one ms_page_batch_ragged call per chunk, and recogniser batches that span pages ("fused_batch").
+
 With this package's TRBA, the device routes (and rotated_crops) write the recogniser batch in the TRBA's batch_dtype
 (float32 by default); a foreign recogniser still gets uint8 slices.
 """
@@ -58,7 +61,8 @@ def host_crop_rects(boxes, img_h, img_w, min_text_size):
     """_pipeline.py:125-137 + 204-221 for (K, >=8) float boxes, vectorised: int32 truncation, size filter, clamped
     slice bounds with Python's slice semantics.  Returns (rects (K,4) int32 [x1,y1,x2,y2), valid (K,) bool).  Used to
     map the device's crop list back to words; the two are compared on every call."""
-    b = np.asarray(boxes, dtype=np.float32).reshape(len(boxes), -1)[:, :8]
+    b = np.asarray(boxes, dtype=np.float32)
+    b = b.reshape(len(b), -1)[:, :8] if len(b) else np.zeros((0, 8), np.float32)
     poly = b.astype(np.int32)  # np.array(polygon, dtype=np.int32): truncation towards zero
     xs, ys = poly[:, 0::2], poly[:, 1::2]
     x_min, x_max, y_min, y_max = xs.min(1), xs.max(1), ys.min(1), ys.max(1)
@@ -77,6 +81,9 @@ def host_crop_rects(boxes, img_h, img_w, min_text_size):
     return np.stack([x1, y1, x2, y2], axis=1).astype(np.int32), valid
 
 
+_BATCH_CROPS_CAP0 = 8192  # first crop capacity of process_batch's page batch (grown to what a chunk needs)
+
+
 class Pipeline:
     def __init__(self, detector=None, recognizer=None, min_text_size=5, rotated_crops=False):
         # _pipeline.py:52-54: missing parts are built from the released weights (EAST() / TRBA() in the reference);
@@ -87,63 +94,113 @@ class Pipeline:
         # EXTENSION (SURVEY 8f-4, reference todo.md:1): rectify every word quad with a perspective warp instead of
         # cutting its bounding rectangle.  Off by default = the reference's behaviour.
         self.rotated_crops = bool(rotated_crops)
-        self._runner = None
-        self._runner_key = None
-        self.last_route = None  # "fused" | "device_crops" | "host_crops" | "detect_only" (introspection for tests / bench)
+        self._runners = {}  # False: the one-page route's PageBatch, True: the batched route's, each with its key
+        # "fused" | "fused_batch" | "device_crops" | "host_crops" | "detect_only" (introspection for tests / bench)
+        self.last_route = None
 
     # ---- route 1: everything between the image upload and the recogniser network on the device ---------------------
-    def _fused_runner(self):
+    def _fused_runner(self, batch=False):
+        """The PageBatch of the one-page route, or (batch=True) of process_batch's: its crop buffer holds the chunk's
+        crops (_BATCH_CROPS_CAP0 rows at first, grown to a power of two when a chunk needs more) instead of cap_boxes
+        per page, and it keeps the buffers of at most two chunk sizes (the full chunk and the last one)."""
         det, rec = self.detector, self.recognizer
         key = (det.device, det.cap_boxes, rec.img_h, rec.img_w, int(self.min_text_size), rec.batch_dtype)
-        if self._runner is None or self._runner_key != key:
-            self._runner = PageBatch(device=det.device.index or 0, params=det._params(sort_reading_order=1),
-                                     min_text_size=int(self.min_text_size), out_hw=(rec.img_h, rec.img_w),
-                                     cap_boxes=det.cap_boxes, batch_dtype=rec.batch_dtype)
-            self._runner_key = key
-        self._runner.params = det._params(sort_reading_order=1)
-        return self._runner
+        entry = self._runners.get(batch)
+        if entry is None or entry[0] != key:
+            kw = dict(crops_cap=_BATCH_CROPS_CAP0, max_buffer_sets=2) if batch else {}
+            entry = self._runners[batch] = (key, PageBatch(
+                device=det.device.index or 0, params=det._params(sort_reading_order=1),
+                min_text_size=int(self.min_text_size), out_hw=(rec.img_h, rec.img_w), cap_boxes=det.cap_boxes,
+                batch_dtype=rec.batch_dtype, **kw))
+        entry[1].params = det._params(sort_reading_order=1)
+        return entry[1]
+
+    @staticmethod
+    def _host_boxes(res, n_pages):
+        """Each page's final boxes as numpy (K_p, 9), from one device-to-host copy"""
+        counts = res.box_counts.cpu().numpy()
+        kmax = int(counts.max()) if n_pages else 0
+        boxes = res.boxes[:n_pages, :kmax].cpu().numpy()         # D2H: P x K_max x 36 bytes
+        return [boxes[p, :int(counts[p])] for p in range(n_pages)]
 
     def _predict_fused(self, img, profile):
-        det, rec = self.detector, self.recognizer
-        torch = det.torch
         t0 = time.time()
-        page_dev = det.upload(img)                              # the one H2D copy of pixels
-        score, geo = det.maps_from_device_page(page_dev)        # network input + maps stay on the device
-        runner = self._fused_runner()
-        res = runner.run_ragged(score[None] if score.dim() == 2 else score, geo[None], [page_dev], sync=True,
-                                allow_order_overflow=True)
-        k = int(res.box_counts[0])
-        n = int(res.n_crops[0])
-        boxes = res.boxes[0, :k].cpu().numpy()                  # D2H: K x 36 bytes
-        if len(res.order_overflow_pages()):
+        page_dev = self.detector.upload(img)                    # the one H2D copy of pixels
+        score, geo = self.detector.maps_from_device_page(page_dev)  # network input + maps stay on the device
+        res = self._fused_runner().run_ragged(score[None] if score.dim() == 2 else score, geo[None], [page_dev],
+                                              sync=True, allow_order_overflow=True)
+        return self._fused_pages(res, self._host_boxes(res, 1), [img], [page_dev], t0, profile)[0]
+
+    def _predict_fused_batch(self, imgs, profile):
+        """The fused route for a chunk of pages: one upload buffer, one detector-input launch, one network call, one
+        page batch, and recogniser batches cut from the one crop batch."""
+        t0 = time.time()
+        pages_dev = self.detector.upload_batch(imgs)            # one H2D copy of pixels per page
+        score, geo = self.detector.maps_from_device_pages(pages_dev)
+        runner = self._fused_runner(batch=True)
+        while True:
+            res = runner.run_ragged(score, geo, pages_dev, sync=True, allow_order_overflow=True)
+            boxes = self._host_boxes(res, len(imgs))
+            need = sum(int(host_crop_rects(b, im.shape[0], im.shape[1], self.min_text_size)[1].sum())
+                       for b, im in zip(boxes, imgs))
+            if need <= runner.crops_cap:
+                break
+            # the crop list stopped at crops_cap: run the chunk again with room for all of its crops
+            runner.crops_cap = 1 << (need - 1).bit_length()
+        return self._fused_pages(res, boxes, imgs, pages_dev, t0, profile)
+
+    def _fused_page(self, img, boxes, crops, overflow, page_dev, profile):
+        """One page of a fused page batch: its final boxes (K, 9) and its rows of the crop list.  Returns the Page and
+        its words that take the crops' texts, in crop order (None when the page was finished on the host)."""
+        if overflow:
             # more boxes (or intersecting pairs) than the device reading-order kernel holds: the boxes came back in
             # detection order; order them with the host restatement and cut the crops from the uploaded page
             page = Page(blocks=[Block(words=words_from_boxes(boxes))])
             self.last_route = "fused+host_order"
-            return self._finish_from_page(page, img, profile, page_dev=page_dev)
-        crops = res.crops[:n].cpu().numpy()                     # D2H: n x 20 bytes
-        if profile:
-            print(f"Detection + crops (device): {time.time() - t0:.3f}s")
+            return self._finish_from_page(page, img, profile, page_dev=page_dev), None
         words = words_from_boxes(boxes)                         # already in reading order (_pipeline.py:105-123)
         page = Page(blocks=[Block(words=words)])
         rects, valid = host_crop_rects(boxes, img.shape[0], img.shape[1], self.min_text_size)
-        if int(valid.sum()) != n or not np.array_equal(rects[valid], crops[:, 1:]):
+        if int(valid.sum()) != len(crops) or not np.array_equal(rects[valid], crops[:, 1:]):
             raise RuntimeError("crop list of the device and the word boxes disagree")
-        if n:
+        return page, [words[j] for j in np.flatnonzero(valid).tolist()]
+
+    def _fused_pages(self, res, boxes, imgs, pages_dev, t0, profile):
+        """Pages of a fused page batch (res; boxes: each page's final boxes on the host), with the texts of the
+        recogniser run over the crop batch in chunks of rec.batch_size, which may span pages."""
+        rec = self.recognizer
+        torch = rec.torch
+        n = int(res.n_crops[0])
+        crops = res.crops[:n].cpu().numpy()                     # D2H: n x 20 bytes
+        overflow = set(res.order_overflow_pages().tolist())
+        pages, targets, rows = [], [], []
+        for p, img in enumerate(imgs):
+            mine = np.flatnonzero(crops[:, 0] == p)              # the page's rows: the list is in (page, box) order
+            page, words = self._fused_page(img, boxes[p], crops[mine], p in overflow, pages_dev[p], profile)
+            pages.append(page)
+            if words is not None:
+                targets.extend(words)
+                rows.append(mine)
+        if profile:
+            print(f"Detection + crops (device): {time.time() - t0:.3f}s")
+        rows = np.concatenate(rows) if rows else np.zeros(0, np.int64)
+        if len(rows):
             t0 = time.time()
-            results = []
             batch = res.batch[:n]                               # a view of the batch the crop kernel wrote
-            for i in range(0, n, rec.batch_size):               # recognizers/_trba/__init__.py:382: chunks of 32
+            if len(rows) != n:                                  # a page finished on the host left rows out
+                batch = batch.index_select(0, torch.from_numpy(rows).to(batch.device))
+            results = []
+            for i in range(0, len(rows), rec.batch_size):       # recognizers/_trba/__init__.py:382: chunks of 32
                 results.extend(rec.model(batch[i:i + rec.batch_size]))
             if profile:
                 torch.cuda.synchronize()
                 print(f"Recognition: {time.time() - t0:.3f}s")
-            for j, result in zip(np.flatnonzero(valid).tolist(), results):
+            for word, result in zip(targets, results):
                 text, conf = _text_and_confidence(result)
-                d = words[j].__dict__  # Word has no validate_assignment (nor has the reference's): plain attribute writes
+                d = word.__dict__  # Word has no validate_assignment (nor has the reference's): plain attribute writes
                 d["text"], d["recognition_confidence"] = text, conf
-                words[j].__pydantic_fields_set__.update(("text", "recognition_confidence"))
-        return page
+                word.__pydantic_fields_set__.update(("text", "recognition_confidence"))
+        return pages
 
     # ---- routes 2 and 3: a Page from any detector ---------------------------------------------------------------------
     def _ordered_crop_rects(self, page, img_h, img_w):
@@ -223,14 +280,20 @@ class Pipeline:
         return results
 
     # ---- the reference's public surface ---------------------------------------------------------------------------
+    def _fused_ok(self, recognize_text):
+        return (recognize_text and not self.rotated_crops and isinstance(self.detector, EAST)
+                and isinstance(self.recognizer, TRBA) and self.detector.model is not None
+                and self.recognizer.model is not None and self.detector.device == self.recognizer.device)
+
+    @staticmethod
+    def _is_rgb_u8(img):
+        return isinstance(img, np.ndarray) and img.ndim == 3 and img.shape[2] == 3 and img.dtype == np.uint8
+
     def predict(self, image, recognize_text=True, vis=False, profile=False):
         t_start = time.time()
-        fused = (recognize_text and not self.rotated_crops and isinstance(self.detector, EAST)
-                 and isinstance(self.recognizer, TRBA) and self.detector.model is not None
-                 and self.recognizer.model is not None and self.detector.device == self.recognizer.device)
-        if fused:
+        if self._fused_ok(recognize_text):
             img = read_image(image)
-            if isinstance(img, np.ndarray) and img.ndim == 3 and img.shape[2] == 3 and img.dtype == np.uint8:
+            if self._is_rgb_u8(img):
                 self.last_route = "fused"
                 page = self._predict_fused(img, profile)
                 if profile:
@@ -273,13 +336,38 @@ class Pipeline:
             return page, visualize_page(image_array, page, show_order=True)
         return page
 
-    def process_batch(self, images, recognize_text=True, vis=False, profile=False):
+    def process_batch(self, images, recognize_text=True, vis=False, profile=False, max_pages=32):
         """_pipeline.py:178-191 (whose body calls a `self.process` that does not exist in the reference, so it can only
-        raise AttributeError there): the evident intent, one predict per image, Pages only."""
-        results = []
-        for img in images:
-            res = self.predict(img, recognize_text=recognize_text, vis=vis, profile=profile)
-            results.append(res[0] if vis else res)
+        raise AttributeError there): the evident intent, one predict per image, Pages only.
+
+        On the fused route (this package's EAST and TRBA, recognize_text, no rotated_crops) with every image an
+        (H, W, 3) uint8 RGB array, the images are processed in chunks of at most `max_pages` (which bounds the memory of
+        the (P, 3, T, T) network input): one upload buffer, one detector-input launch, one detector network call and one
+        page batch per chunk, and recogniser batches of rec.batch_size crops that may span pages (last_route
+        "fused_batch").  The Pages are exactly [predict(img) for img in images] -- words, polygons, confidences and
+        texts -- for a recogniser whose output for a row does not depend on the other rows of its batch (and a detector
+        network that treats the rows of its input independently).  The images are read chunk by chunk; a chunk with an
+        image that is not uint8 RGB, and every image off the fused route, runs predict per image.  The page batch of
+        this route holds the crops the chunk needs (not cap_boxes per page) and the buffers of at most two chunk sizes."""
+        max_pages = int(max_pages)
+        if max_pages < 1:
+            raise ValueError(f"max_pages must be at least 1, got {max_pages}")
+        images = list(images)
+        fused = self._fused_ok(recognize_text)
+        results, routes = [], set()
+        for i in range(0, len(images), max_pages):
+            chunk = images[i:i + max_pages]
+            imgs = [read_image(im) for im in chunk] if fused else None  # read chunk by chunk, not all at once
+            if fused and all(self._is_rgb_u8(im) for im in imgs):
+                results.extend(self._predict_fused_batch(imgs, profile))
+                routes.add("fused_batch")
+                continue
+            for img in chunk:
+                res = self.predict(img, recognize_text=recognize_text, vis=vis, profile=profile)
+                results.append(res[0] if vis else res)
+                routes.add(self.last_route)
+        if routes == {"fused_batch"}:
+            self.last_route = "fused_batch"
         return results
 
     def get_text(self, page):
