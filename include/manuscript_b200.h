@@ -145,6 +145,20 @@ MS_API int ms_polygon_iou_host(ms_ctx *ctx, const double *subj, const double *cl
 MS_API int ms_test_iou_proved_host(ms_ctx *ctx, const double *subj, const double *clip, int64_t n, double thr,
                             uint8_t *out);
 
+/* TEST-ONLY (not a reference interface): the device functions that size a crop and build its cv2.resize coefficient
+ * tables, evaluated on the device.  wh (n_plans,2) int32 (w, h) -> plans_out (n_plans,8) int32: nw, nh, y0, interp
+ * (0 copy, 1 INTER_LINEAR, 2 INTER_AREA integer ratio, 3 INTER_AREA general), isx, isy, 1 if the plan alone admits
+ * the persistent crop kernel (INTER_AREA general with shrink factors below 2.999, or exactly 2 x 2), 0 -- of the
+ * ResizeAndPadA plan at an out_h x out_w canvas.  axes (n_axes,3) int32 (ssize, dsize, mode) -> entries_out, 8 int32
+ * words per destination index, the axes one after another (at most entries_cap entries): mode 0 / 1 the INTER_AREA
+ * x tables / y records of the persistent kernel (x: word d = s0 | n << 16 and word (1 + k) * dsize + d = weight of
+ * tap k, within the axis' 8 * dsize words; y: word 8d = s0 | n << 16, words 8d + 4.. = the tap weights), mode 2 the
+ * INTER_AREA entry of the generic kernel {s0, n, nfirst, nmid, first, middle and last weight (f32), 0}, mode 3 / 4
+ * the INTER_LINEAR x / y entry {s0, edge flag (x) or second row (y), 11-bit coefficients c0, c1, 0, 0, 0, 0}. */
+MS_API int ms_test_resize_tables_host(ms_ctx *ctx, int out_h, int out_w, const int32_t *wh, int64_t n_plans,
+                               int32_t *plans_out, const int32_t *axes, int64_t n_axes, int32_t *entries_out,
+                               int64_t entries_cap);
+
 /* replaces expand_boxes, detectors/_east/utils.py:384 (called infer.py:340). */
 MS_API int ms_expand_boxes_host(ms_ctx *ctx, const float *quads, int64_t n, double expand_w, double expand_h,
                          float *out);
@@ -179,6 +193,12 @@ MS_API int ms_crop_resize_pad_host(ms_ctx *ctx, const uint8_t *page, int img_h, 
  * counts[0] quads taken by the staged (TMA window) kernel, counts[1] quads served by the generic kernel (not
  * stageable, or handed back by the staged kernel).  Waits for the call's stream work. */
 MS_API int ms_quad_crop_last_counts(ms_ctx *ctx, int32_t *counts);
+
+/* DIAGNOSTIC (tests): how the crops of this context's LAST axis-aligned crop call (ms_crop_resize_pad*, or the crop
+ * stage of a page batch) were served -- counts[0] crops listed for the persistent TMA kernel, counts[1] crops listed
+ * for the generic kernel (not stageable, another interpolation, invalid, or handed back by the persistent kernel).
+ * Waits for the call's stream work. */
+MS_API int ms_crop_last_counts(ms_ctx *ctx, int32_t *counts);
 
 /* ms_quad_crop_resize_pad for one page with HOST buffers: quads (n,8) f32, sizes_out (n,2) int32 or NULL. */
 MS_API int ms_quad_crop_resize_pad_host(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, const float *quads,

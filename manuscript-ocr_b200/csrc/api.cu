@@ -242,7 +242,10 @@ static int grow(char **buf, size_t *have, size_t want, const char *what)
 
 int ms_arena_reserve(ms_ctx *ctx, size_t bytes)
 {
-    if (bytes > ctx->arena_bytes) ctx->quad_cnt = nullptr;  // the counters of the last rotated-crop call go with the old arena
+    if (bytes > ctx->arena_bytes) {  // the counters of the last rotated- and axis-crop calls go with the old arena
+        ctx->quad_cnt = nullptr;
+        ctx->crop_cnt = nullptr;
+    }
     return grow(&ctx->arena, &ctx->arena_bytes, bytes, "arena");
 }
 int ms_stage_reserve(ms_ctx *ctx, size_t bytes) { return grow(&ctx->stage, &ctx->stage_bytes, bytes, "stage"); }
@@ -1027,6 +1030,58 @@ extern "C" int ms_test_iou_proved_host(ms_ctx *ctx, const double *subj, const do
     return MS_OK;
 }
 
+extern "C" int ms_test_resize_tables_host(ms_ctx *ctx, int out_h, int out_w, const int32_t *wh, int64_t n_plans,
+                                          int32_t *plans_out, const int32_t *axes, int64_t n_axes, int32_t *entries_out,
+                                          int64_t entries_cap)
+{
+    MS_CTX(ctx);
+    if (n_plans < 0 || n_axes < 0 || entries_cap < 0 || (n_plans > 0 && (!wh || !plans_out || out_h <= 0 || out_w <= 0)) ||
+        (n_axes > 0 && (!axes || !entries_out))) {
+        ms_set_error("ms_test_resize_tables_host: bad arguments");
+        return MS_ERR_INVALID;
+    }
+    for (int64_t i = 0; i < n_plans; i++)
+        if (wh[2 * i] <= 0 || wh[2 * i + 1] <= 0) {
+            ms_set_error("ms_test_resize_tables_host: crop %lld is %d x %d", (long long)i, wh[2 * i], wh[2 * i + 1]);
+            return MS_ERR_INVALID;
+        }
+    // the axes with the index of their first entry
+    std::vector<int32_t> ax((size_t)n_axes * 4);
+    int64_t total = 0;
+    for (int64_t a = 0; a < n_axes; a++) {
+        const int32_t ssize = axes[3 * a], dsize = axes[3 * a + 1], mode = axes[3 * a + 2];
+        if (ssize <= 0 || dsize <= 0 || mode < 0 || mode > 4 || ssize >= 65536) {
+            ms_set_error("ms_test_resize_tables_host: axis %lld (%d -> %d, mode %d)", (long long)a, ssize, dsize, mode);
+            return MS_ERR_INVALID;
+        }
+        ax[4 * a] = ssize, ax[4 * a + 1] = dsize, ax[4 * a + 2] = mode, ax[4 * a + 3] = (int32_t)total;
+        total += dsize;
+        if (total > entries_cap || total >= ((int64_t)1 << 31)) {
+            ms_set_error("ms_test_resize_tables_host: the axes have more than %lld entries", (long long)entries_cap);
+            return MS_ERR_CAPACITY;
+        }
+    }
+    if (n_plans == 0 && n_axes == 0) return MS_OK;
+    int32_t *d_wh, *d_plans, *d_axes, *d_ent;
+    MS_TRY(stage_carve(ctx, "ms_test_resize_tables_host", [&](ms_bump &sb) {
+        d_wh = sb.take<int32_t>((size_t)n_plans * 2);
+        d_plans = sb.take<int32_t>((size_t)n_plans * 8);
+        d_axes = sb.take<int32_t>((size_t)n_axes * 4);
+        d_ent = sb.take<int32_t>((size_t)total * 8);
+    }));
+    cudaStream_t st = ctx->own_stream;
+    if (n_plans > 0) MS_CUDA(cudaMemcpyAsync(d_wh, wh, (size_t)n_plans * 8, cudaMemcpyHostToDevice, st));
+    if (n_axes > 0) {
+        MS_CUDA(cudaMemcpyAsync(d_axes, ax.data(), (size_t)n_axes * 16, cudaMemcpyHostToDevice, st));
+        MS_CUDA(cudaMemsetAsync(d_ent, 0, (size_t)total * 32, st));
+    }
+    MS_TRY(msk_test_resize_tables(ctx, out_h, out_w, d_wh, n_plans, d_plans, d_axes, n_axes, d_ent, st));
+    if (n_plans > 0) MS_CUDA(cudaMemcpyAsync(plans_out, d_plans, (size_t)n_plans * 32, cudaMemcpyDeviceToHost, st));
+    if (n_axes > 0) MS_CUDA(cudaMemcpyAsync(entries_out, d_ent, (size_t)total * 32, cudaMemcpyDeviceToHost, st));
+    MS_CUDA(cudaStreamSynchronize(st));
+    return MS_OK;
+}
+
 extern "C" int ms_expand_boxes_host(ms_ctx *ctx, const float *quads, int64_t n, double expand_w, double expand_h,
                                     float *out)
 {
@@ -1413,6 +1468,21 @@ extern "C" int ms_quad_crop_last_counts(ms_ctx *ctx, int32_t *counts)
     MS_CUDA(cudaStreamSynchronize(ctx->quad_stream));
     counts[0] = h[0];
     counts[1] = h[2];
+    return MS_OK;
+}
+
+extern "C" int ms_crop_last_counts(ms_ctx *ctx, int32_t *counts)
+{
+    MS_CTX(ctx);
+    if (!counts || !ctx->crop_cnt) {
+        ms_set_error("ms_crop_last_counts: no axis-crop call on this context yet");
+        return MS_ERR_INVALID;
+    }
+    int32_t *h = reinterpret_cast<int32_t *>(ctx->pinned);
+    MS_CUDA(cudaMemcpyAsync(h, ctx->crop_cnt, 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->crop_stream));
+    MS_CUDA(cudaStreamSynchronize(ctx->crop_stream));
+    counts[0] = h[1];  // crops listed for the persistent kernel
+    counts[1] = h[0];  // crops listed for the generic kernel (including those handed back)
     return MS_OK;
 }
 

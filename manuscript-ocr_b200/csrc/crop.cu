@@ -80,10 +80,7 @@ __device__ __forceinline__ void make_plan(const int32_t *cr, int n_pages, int im
         p.staged = 1;
         p.pitch = pitch;
     }
-    // a decimation window shorter than 3 source pixels touches at most 4 of them: every table entry has <= 4 taps
-    // ... and the exact 2 x 2 integer ratio has its own staged routine
-    p.fast = p.staged && p.w < 65536 && p.h < 65536 &&
-             ((p.interp == 3 && p.scale_x < 2.999 && p.scale_y < 2.999) || (p.interp == 2 && p.isx == 2 && p.isy == 2));
+    p.fast = p.staged && p.w < 65536 && p.h < 65536 && plan_fast_shape(p);
 }
 
 // plans for all crops (thread per crop): the float64 sizing arithmetic of transforms.py:91-98 runs here, off the
@@ -359,6 +356,53 @@ __global__ void __launch_bounds__(256) crop_generic_kernel(const Plan *__restric
     }
 }
 
+// ---- test-only (ms_test_resize_tables_host): the plan and table device functions, evaluated as the kernels call them ----
+// plans_out[i] (8 words) = nw, nh, y0, interp, isx, isy, plan_fast_shape, 0 of plan_resize(wh[i]) at an out_h x out_w
+// canvas.  Axis a = axes[4a..4a+3] = ssize, dsize, mode, first entry; its dsize entries are 8 words each from word
+// 8 * first of entries_out, in the layout of the mode:
+//   0  build_tables' x tables (INTER_AREA, crop_resize_pad_kernel): the axis as a crop of width ssize, table stride iw =
+//      dsize -- word d packed s0 | n << 16, word (1 + k) * dsize + d tap weight k (the rest of the axis' words untouched)
+//   1  build_tables' y records: word 8d packed s0 | n << 16, words 8d + 4 .. 8d + 7 the tap weights
+//   2  area_entry as fill_axis_table calls it (crop_generic_kernel): the AxisEnt
+//   3  linear_entry_x, 4  linear_entry_y: the AxisEnt
+static_assert(sizeof(AxisEnt) == 32, "an AxisEnt is one 8-word entry");
+__global__ void __launch_bounds__(128) resize_tables_test_kernel(int out_h, int out_w, const int32_t *__restrict__ wh,
+                                                                 int64_t n_plans, int32_t *__restrict__ plans_out,
+                                                                 const int32_t *__restrict__ axes, int64_t n_axes,
+                                                                 int32_t *__restrict__ entries_out)
+{
+    ms_pdl_wait();
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_plans; i += stride) {
+        Plan p;
+        plan_reset(p);
+        plan_resize(wh[2 * i], wh[2 * i + 1], out_h, out_w, p);
+        int32_t *o = plans_out + 8 * i;
+        o[0] = p.nw, o[1] = p.nh, o[2] = p.y0, o[3] = p.interp, o[4] = p.isx, o[5] = p.isy;
+        o[6] = plan_fast_shape(p) ? 1 : 0;
+        o[7] = 0;
+    }
+    for (int64_t a = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; a < n_axes; a += stride) {
+        const int ssize = axes[4 * a], dsize = axes[4 * a + 1], mode = axes[4 * a + 2];
+        int32_t *out = entries_out + 8 * (int64_t)axes[4 * a + 3];
+        const double scale = 1.0 / ((double)dsize / (double)ssize);  // plan_resize's scale_x / scale_y
+        if (mode <= 1) {
+            Plan p;
+            plan_reset(p);
+            p.w = p.h = ssize;
+            p.scale_x = p.scale_y = scale;
+            (mode == 0 ? p.nw : p.nh) = dsize;
+            build_tables(p, reinterpret_cast<uint32_t *>(out), 0, mode == 0 ? dsize : 0, 0, 1);
+            continue;
+        }
+        for (int d = 0; d < dsize; d++) {
+            const AxisEnt e = mode == 2 ? area_entry(d, scale, ssize)
+                                        : (mode == 3 ? linear_entry_x(d, scale, ssize) : linear_entry_y(d, scale, ssize));
+            *reinterpret_cast<AxisEnt *>(out + 8 * d) = e;
+        }
+    }
+}
+
 // ---- detector input (the caller side of the path, EAST.predict infer.py:301-305) ---------------------------------
 // cv2.resize(img, (T, T)) -- INTER_LINEAR on uint8 (11-bit fixed-point coefficients, aspect NOT preserved), then
 // torchvision ToTensor (x / 255) and Normalize(0.5, 0.5) ((x - 0.5) / 0.5), written as the (P, 3, th, tw) network input
@@ -605,6 +649,8 @@ int msk_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_
         return MS_ERR_CAPACITY;
     }
     int32_t *glist_n = cnt, *n_work = cnt + 1, *ticket = cnt + 2;
+    ctx->crop_cnt = cnt;  // ms_crop_last_counts
+    ctx->crop_stream = st;
     MS_CUDA(cudaMemsetAsync(redo, 0, (size_t)crops_cap, st));
     MS_CUDA(cudaMemsetAsync(hist, 0, (size_t)n_buckets * sizeof(int32_t), st));
     MS_CUDA(cudaMemsetAsync(cnt, 0, 4 * sizeof(int32_t), st));
@@ -639,4 +685,17 @@ int msk_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_
         MS_LAUNCH_CHECK(ctx);
         return MS_OK;
     });
+}
+
+int msk_test_resize_tables(ms_ctx *ctx, int out_h, int out_w, const int32_t *wh, int64_t n_plans, int32_t *plans_out,
+                           const int32_t *axes, int64_t n_axes, int32_t *entries_out, cudaStream_t st)
+{
+    const int64_t n = n_plans > n_axes ? n_plans : n_axes;
+    if (n <= 0) return MS_OK;
+    int64_t grid = (n + 127) / 128;
+    if (grid > (int64_t)ctx->num_sms * 16) grid = (int64_t)ctx->num_sms * 16;
+    ms_launch(resize_tables_test_kernel, (int)grid, 128, 0, st, out_h, out_w, wh, n_plans, plans_out, axes, n_axes,
+              entries_out);
+    MS_LAUNCH_CHECK(ctx);
+    return MS_OK;
 }

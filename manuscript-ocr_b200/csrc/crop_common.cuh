@@ -331,6 +331,14 @@ __device__ __forceinline__ void plan_resize(int w, int h, int ih, int iw, Plan &
     }
 }
 
+// The part of Plan::fast that depends on the resize plan alone: INTER_AREA general with shrink factors below 3 (a
+// decimation window shorter than 3 source pixels touches at most 4 of them: every table entry has <= 4 taps), or the
+// exact 2 x 2 integer ratio, which has its own staged routine.
+__device__ __forceinline__ bool plan_fast_shape(const Plan &p)
+{
+    return (p.interp == 3 && p.scale_x < 2.999 && p.scale_y < 2.999) || (p.interp == 2 && p.isx == 2 && p.isy == 2);
+}
+
 // (float)(num / den) for 0 <= num <= den, given inv = 1.0 / den (correctly rounded): num * inv is within two double
 // ulps of the quotient, so it rounds to the same float unless it sits that close to the midpoint between two floats
 // (the 29 bits below float precision near 100...0) -- then, and for tiny values, the division itself is evaluated.

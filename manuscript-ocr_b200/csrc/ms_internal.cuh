@@ -108,6 +108,8 @@ struct ms_ctx {
     ms_graph_entry graphs[MS_GRAPH_SLOTS];
     const int32_t *quad_cnt;      // device counters of the last rotated-crop call (ms_quad_crop_last_counts)
     cudaStream_t quad_stream;
+    const int32_t *crop_cnt;      // device counters of the last axis-crop call (ms_crop_last_counts)
+    cudaStream_t crop_stream;
     int quad_no_stage;            // MS_B200_QUAD_NO_STAGE=1: rotated crops by the generic kernel only (A/B runs, tests)
     int ro_force_large;           // MS_B200_RO_FORCE_LARGE=1: every page takes the large-page reading-order kernel (tests)
     int busy;                     // 1 while a thread is inside an entry point (atomic test-and-set): a context owns ONE
@@ -255,6 +257,9 @@ int msk_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_
              const int32_t *n_crops, const int32_t *range, int64_t crops_cap, int out_h, int out_w, void *batch,
              int batch_dtype, uint8_t *canvas_u8, ms_bump bump, cudaStream_t st, const uint8_t *const *page_ptrs = nullptr,
              const int32_t *page_hw = nullptr);  // page_ptrs / page_hw (device): pages of their own sizes
+// test-only (ms_test_resize_tables_host): the resize plan and coefficient-table device functions on device buffers
+int msk_test_resize_tables(ms_ctx *ctx, int out_h, int out_w, const int32_t *wh, int64_t n_plans, int32_t *plans_out,
+                           const int32_t *axes, int64_t n_axes, int32_t *entries_out, cudaStream_t st);
 // tps.cu
 int msk_tps_rectify(ms_ctx *ctx, const float *input, const float *c_prime, const float *inv_delta_c, const float *p_hat_t,
                     int batch, int n_fid, int chans, int in_h, int in_w, int out_h, int out_w, float *out, cudaStream_t st);

@@ -88,7 +88,9 @@ SIGNATURES = {
     "ms_standard_nms_host": (_i, [_vp, _vp, _vp, _i64, _d, _vp, C.POINTER(_i64)]),
     "ms_polygon_iou_host": (_i, [_vp, _vp, _vp, _i64, _vp]),
     "ms_quad_crop_last_counts": (_i, [_vp, _vp]),
+    "ms_crop_last_counts": (_i, [_vp, _vp]),
     "ms_test_iou_proved_host": (_i, [_vp, _vp, _vp, _i64, _d, _vp]),
+    "ms_test_resize_tables_host": (_i, [_vp, _i, _i, _vp, _i64, _vp, _vp, _i64, _vp, _i64]),
     "ms_expand_boxes_host": (_i, [_vp, _vp, _i64, _d, _d, _vp]),
     "ms_east_boxes_host": (_i, [_vp, _vp, _i64, C.POINTER(EastParams), _i, _i, _vp, C.POINTER(_i64)]),
     "ms_word_rects_host": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp]),
