@@ -159,6 +159,14 @@ MS_API int ms_test_resize_tables_host(ms_ctx *ctx, int out_h, int out_w, const i
                                int32_t *plans_out, const int32_t *axes, int64_t n_axes, int32_t *entries_out,
                                int64_t entries_cap);
 
+/* TEST-ONLY (not a reference interface): the float32 sums behind the area-anomaly filter's mean and standard deviation
+ * (infer.py:222-224, numpy's pairwise summation), evaluated by the device functions east_finish_kernel uses, one CTA
+ * of its block size per vector.  Vector v is values[offsets[v] .. offsets[v] + lengths[v]), lengths[v] >= 1;
+ * out_serial[v] = the one-thread sum, out_cta[v] = the CTA's leaf-parallel sum (itself one thread beyond 1024
+ * leaves).  tests/ compare both with np.add.reduce bit for bit. */
+MS_API int ms_test_np_sum_host(ms_ctx *ctx, const float *values, const int64_t *offsets, const int32_t *lengths,
+                               int n_vec, float *out_serial, float *out_cta);
+
 /* replaces expand_boxes, detectors/_east/utils.py:384 (called infer.py:340). */
 MS_API int ms_expand_boxes_host(ms_ctx *ctx, const float *quads, int64_t n, double expand_w, double expand_h,
                          float *out);

@@ -1082,6 +1082,44 @@ extern "C" int ms_test_resize_tables_host(ms_ctx *ctx, int out_h, int out_w, con
     return MS_OK;
 }
 
+extern "C" int ms_test_np_sum_host(ms_ctx *ctx, const float *values, const int64_t *offsets, const int32_t *lengths,
+                                   int n_vec, float *out_serial, float *out_cta)
+{
+    MS_CTX(ctx);
+    if (n_vec < 0 || (n_vec > 0 && (!values || !offsets || !lengths || !out_serial || !out_cta))) {
+        ms_set_error("ms_test_np_sum_host: bad arguments");
+        return MS_ERR_INVALID;
+    }
+    // the values span [0, max(offsets[v] + lengths[v])); every vector holds at least one value
+    int64_t n_values = 0;
+    for (int v = 0; v < n_vec; v++) {
+        if (offsets[v] < 0 || lengths[v] <= 0) {
+            ms_set_error("ms_test_np_sum_host: vector %d at %lld has %d values", v, (long long)offsets[v], lengths[v]);
+            return MS_ERR_INVALID;
+        }
+        if (offsets[v] + lengths[v] > n_values) n_values = offsets[v] + lengths[v];
+    }
+    if (n_vec == 0) return MS_OK;
+    float *d_val, *d_out;
+    int64_t *d_off;
+    int32_t *d_len;
+    MS_TRY(stage_carve(ctx, "ms_test_np_sum_host", [&](ms_bump &sb) {
+        d_val = sb.take<float>((size_t)n_values);
+        d_off = sb.take<int64_t>((size_t)n_vec);
+        d_len = sb.take<int32_t>((size_t)n_vec);
+        d_out = sb.take<float>((size_t)n_vec * 2);
+    }));
+    cudaStream_t st = ctx->own_stream;
+    MS_CUDA(cudaMemcpyAsync(d_val, values, (size_t)n_values * 4, cudaMemcpyHostToDevice, st));
+    MS_CUDA(cudaMemcpyAsync(d_off, offsets, (size_t)n_vec * 8, cudaMemcpyHostToDevice, st));
+    MS_CUDA(cudaMemcpyAsync(d_len, lengths, (size_t)n_vec * 4, cudaMemcpyHostToDevice, st));
+    MS_TRY(msk_test_np_sum(ctx, d_val, d_off, d_len, n_vec, d_out, d_out + n_vec, st));
+    MS_CUDA(cudaMemcpyAsync(out_serial, d_out, (size_t)n_vec * 4, cudaMemcpyDeviceToHost, st));
+    MS_CUDA(cudaMemcpyAsync(out_cta, d_out + n_vec, (size_t)n_vec * 4, cudaMemcpyDeviceToHost, st));
+    MS_CUDA(cudaStreamSynchronize(st));
+    return MS_OK;
+}
+
 extern "C" int ms_expand_boxes_host(ms_ctx *ctx, const float *quads, int64_t n, double expand_w, double expand_h,
                                     float *out)
 {

@@ -240,6 +240,9 @@ int msk_east_boxes(ms_ctx *ctx, const float *quads, const int32_t *counts, int n
                    int32_t *counts_out, int32_t *flags, ms_bump bump, cudaStream_t st, int orig_h = 0,
                    int orig_w = 0);  // orig_hw == NULL: every page is (orig_h, orig_w), or target_size when <= 0
 size_t msk_east_boxes_scratch(int n_pages, int cap_per_page);
+// np_sum_test.cu, test-only (ms_test_np_sum_host): the numpy pairwise sums of east_finish_kernel, one CTA per vector
+int msk_test_np_sum(ms_ctx *ctx, const float *values, const int64_t *offsets, const int32_t *lengths, int n_vec,
+                    float *out_serial, float *out_cta, cudaStream_t st);
 int msk_word_rects(ms_ctx *ctx, const float *quads, const int32_t *counts, int n_pages, int cap_per_page,
                    const int32_t *img_hw, int img_h, int img_w, int min_text_size, int32_t *crops_out,
                    int64_t crops_cap, int32_t *n_crops, int page_base, int append, int32_t *range, ms_bump bump,

@@ -91,6 +91,7 @@ SIGNATURES = {
     "ms_crop_last_counts": (_i, [_vp, _vp]),
     "ms_test_iou_proved_host": (_i, [_vp, _vp, _vp, _i64, _d, _vp]),
     "ms_test_resize_tables_host": (_i, [_vp, _i, _i, _vp, _i64, _vp, _vp, _i64, _vp, _i64]),
+    "ms_test_np_sum_host": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp]),
     "ms_expand_boxes_host": (_i, [_vp, _vp, _i64, _d, _d, _vp]),
     "ms_east_boxes_host": (_i, [_vp, _vp, _i64, C.POINTER(EastParams), _i, _i, _vp, C.POINTER(_i64)]),
     "ms_word_rects_host": (_i, [_vp, _vp, _i64, _i, _i, _i, _vp, _vp]),
