@@ -197,7 +197,8 @@ MS_API int ms_reading_order_host(ms_ctx *ctx, const float *polys8, int64_t n, in
 MS_API int ms_crop_resize_pad_host(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, const int32_t *rects,
                             int64_t n, int out_h, int out_w, float *batch_f32, uint8_t *canvas_u8);
 
-/* DIAGNOSTIC (tests, bench): how the quads of this context's LAST ms_quad_crop_resize_pad* call were served --
+/* DIAGNOSTIC (tests, bench): how the quads of this context's LAST ms_quad_crop_resize_pad* call (or the crop stage of a
+ * quad page batch, ms_page_batch*_quads) were served --
  * counts[0] quads taken by the staged (TMA window) kernel, counts[1] quads served by the generic kernel (not
  * stageable, or handed back by the staged kernel).  Waits for the call's stream work. */
 MS_API int ms_quad_crop_last_counts(ms_ctx *ctx, int32_t *counts);
@@ -345,6 +346,29 @@ MS_API int ms_page_batch_ragged_ex(ms_ctx *ctx, const float *score, const float 
                             int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
                             int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
                             void *batch, int batch_dtype, uint8_t *canvas_u8, int32_t *flags, void *stream);
+
+/* EXTENSION -- not a reference behaviour (SURVEY 8f-4, reference todo.md:1): the page batch of ms_page_batch_ex with
+ * the rectified crops of ms_quad_crop_resize_pad as its crop stage.  Everything up to the final boxes is that of
+ * ms_page_batch_ex (boxes_out / box_counts / flags are the same bits).  Then crops_out gets, in (page, box) order, one
+ * row of 5 int32 [page, box, w, h, 0] per final quad that has a patch -- box is the quad's row in that page's boxes_out,
+ * (w, h) its patch size (no patch: a side below max(2, min_text_size) or above 32767, or a singular 4-point system) --
+ * and *n_crops (device int32) = min(listed, crops_cap); rows at or past crops_cap are not written.  Batch row i (and
+ * canvas i) is the crop of list row i; rows past *n_crops are not written.  border_mode / border_value as in
+ * ms_quad_crop_resize_pad.  Pages at most 32767 pixels on a side; an unknown dtype, a bad border or NULL buffers is
+ * MS_ERR_INVALID.  The crop mode and the border are part of the call's identity for the CUDA-graph cache. */
+MS_API int ms_page_batch_quads(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
+                               int map_h, int map_w, int img_h, int img_w, const ms_east_params *p, int min_text_size,
+                               int border_mode, int border_value, int out_h, int out_w, int cap_boxes, float *boxes_out,
+                               int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops, void *batch,
+                               int batch_dtype, uint8_t *canvas_u8, int32_t *flags, void *stream);
+/* EXTENSION -- not a reference behaviour: ms_page_batch_quads for page images of their own sizes (the tables of
+ * ms_page_batch_ragged).  The sizes are device data: the quads of a page above 32767 pixels on a side get no patch. */
+MS_API int ms_page_batch_ragged_quads(ms_ctx *ctx, const float *score, const float *geo,
+                                      const uint8_t *const *page_ptrs, const int32_t *page_hw, int n_pages, int map_h,
+                                      int map_w, const ms_east_params *p, int min_text_size, int border_mode,
+                                      int border_value, int out_h, int out_w, int cap_boxes, float *boxes_out,
+                                      int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
+                                      void *batch, int batch_dtype, uint8_t *canvas_u8, int32_t *flags, void *stream);
 
 /* Same path with HOST buffers (pinned or pageable; `score` / `geo` may also be DEVICE pointers of this context's
  * device -- maps a detector left on the GPU are used in place and only the page images cross PCIe): H2D of maps + pages, the batch, D2H of boxes,

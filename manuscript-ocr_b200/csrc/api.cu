@@ -568,11 +568,12 @@ static size_t front_scratch(int n_pages, int map_h, int map_w, int q, int cap_c,
     return al256(fixed + stage + 4096);
 }
 
-// ... and of the tail (crop rectangles, crops), which runs after the front stages and may reuse their bytes
-static size_t tail_scratch(int n_pages, int cap_c, int64_t crops_cap, int total_pages)
+// ... and of the tail (crop rectangles, crops; or the quad list, quad crops), which runs after the front stages and may
+// reuse their bytes
+static size_t tail_scratch(int n_pages, int cap_c, int64_t crops_cap, int total_pages, bool quads, int cap_boxes)
 {
-    size_t stage = word_rects_scratch_full(n_pages, cap_c);
-    const size_t s2 = msk_crop_scratch(crops_cap, total_pages);
+    size_t stage = quads ? msk_quad_list_scratch(n_pages, cap_boxes) : word_rects_scratch_full(n_pages, cap_c);
+    const size_t s2 = quads ? msk_quad_crop_scratch(crops_cap) : msk_crop_scratch(crops_cap, total_pages);
     if (s2 > stage) stage = s2;
     return al256(stage + 4096);
 }
@@ -676,7 +677,8 @@ static int page_batch_impl(ms_ctx *ctx, const pb_call &c, int page_base, int n_p
     const int nA = split ? n_pages / 2 : n_pages, nB = n_pages - nA;
     const size_t szA = front_scratch(nA, c.map_h, c.map_w, q, cap_c, ctx->edge_factor, c.cap_boxes);
     const size_t szB = split ? front_scratch(nB, c.map_h, c.map_w, q, cap_c, ctx->edge_factor, c.cap_boxes) : 0;
-    const size_t szT = tail_scratch(n_pages, cap_c, want_crops ? c.crops_cap : 0, c.n_pages);
+    const size_t szT = tail_scratch(n_pages, cap_c, want_crops ? c.crops_cap : 0, c.n_pages, c.crop_quads != 0,
+                                    c.cap_boxes);
     // (one sequence: the tail reuses the front stages' scratch; two halves: A | B | tail side by side)
     MS_TRY(ms_arena_reserve(ctx, split ? szA + szB + szT + 1024 : (szA > szT ? szA : szT) + 1024));
     ms_bump bumpA{ctx->arena, 0, split ? szA : ctx->arena_bytes};
@@ -705,7 +707,15 @@ static int page_batch_impl(ms_ctx *ctx, const pb_call &c, int page_base, int n_p
         ms_set_error("ms_page_batch: arena too small");
         return MS_ERR_CAPACITY;
     }
-    if (want_crops) {
+    if (want_crops && c.crop_quads) {  // (page_base == 0, append == 0: the device entry points)
+        MS_TRY(msk_quad_list(ctx, pg.boxes, pg.counts, n_pages, c.cap_boxes, c.pages, c.img_h, c.img_w, c.page_ptrs,
+                             c.page_hw, c.min_text_size, c.crops_out, c.crops_cap, c.n_crops, bumpT, st));
+        MS_TRY(timing_mark(ctx, 4, st));
+        if (c.batch || c.canvas_u8)
+            MS_TRY(msk_quad_crop_rows(ctx, pg.boxes, c.cap_boxes, n_pages, c.pages, c.img_h, c.img_w, c.page_ptrs,
+                                      c.page_hw, c.crops_out, c.n_crops, c.crops_cap, c.min_text_size, c.border_mode,
+                                      c.border_value, c.out_h, c.out_w, c.batch, c.batch_dtype, c.canvas_u8, bumpT, st));
+    } else if (want_crops) {
         MS_TRY(msk_word_rects(ctx, pg.boxes, pg.counts, n_pages, c.cap_boxes, pg.hw, c.img_h, c.img_w, c.min_text_size,
                               c.crops_out, c.crops_cap, c.n_crops, page_base, append, range, bumpT, st));
         MS_TRY(timing_mark(ctx, 4, st));
@@ -1303,6 +1313,74 @@ extern "C" int ms_page_batch_ragged(ms_ctx *ctx, const float *score, const float
     return ms_page_batch_ragged_ex(ctx, score, geo, page_ptrs, page_hw, n_pages, map_h, map_w, p, min_text_size, out_h,
                                    out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch_f32,
                                    MS_DTYPE_F32, canvas_u8, flags, stream);
+}
+
+// ---- EXTENSION -- not a reference behaviour: page batches whose crop stage is the rectified crop of every final quad --
+static int quad_batch_args_ok(int batch_dtype, int border_mode, int border_value, const char *who)
+{
+    MS_TRY(dtype_ok(batch_dtype, who));
+    if (border_mode < 0 || border_mode > 1 || border_value < 0 || border_value > 255) {
+        ms_set_error("%s: border_mode must be 0 (constant) or 1 (replicate), border_value 0..255", who);
+        return MS_ERR_INVALID;
+    }
+    return MS_OK;
+}
+
+extern "C" int ms_page_batch_quads(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
+                                   int map_h, int map_w, int img_h, int img_w, const ms_east_params *p,
+                                   int min_text_size, int border_mode, int border_value, int out_h, int out_w,
+                                   int cap_boxes, float *boxes_out, int32_t *box_counts, int32_t *crops_out,
+                                   int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype,
+                                   uint8_t *canvas_u8, int32_t *flags, void *stream)
+{
+    MS_CTX(ctx);
+    MS_TRY(quad_batch_args_ok(batch_dtype, border_mode, border_value, "ms_page_batch_quads"));
+    if (n_pages <= 0) return MS_OK;
+    if (!score || !geo || !p || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
+        ms_set_error("ms_page_batch_quads: bad arguments");
+        return MS_ERR_INVALID;
+    }
+    if (pages && (img_h <= 0 || img_w <= 0 || img_h > 32767 || img_w > 32767)) {
+        ms_set_error("ms_page_batch_quads: pages must be 1..32767 pixels on a side (16-bit remap coordinates), got %dx%d",
+                     img_h, img_w);
+        return MS_ERR_INVALID;
+    }
+    pb_call c;
+    pb_init(c, p);
+    c.score = score; c.geo = geo; c.pages = pages;
+    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w; c.img_h = img_h; c.img_w = img_w;
+    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
+    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
+    c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
+    c.crop_quads = 1; c.border_mode = border_mode; c.border_value = border_value;
+    return page_batch_cached(ctx, c, (cudaStream_t)stream);
+}
+
+extern "C" int ms_page_batch_ragged_quads(ms_ctx *ctx, const float *score, const float *geo,
+                                          const uint8_t *const *page_ptrs, const int32_t *page_hw, int n_pages,
+                                          int map_h, int map_w, const ms_east_params *p, int min_text_size,
+                                          int border_mode, int border_value, int out_h, int out_w, int cap_boxes,
+                                          float *boxes_out, int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
+                                          int32_t *n_crops, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                                          int32_t *flags, void *stream)
+{
+    MS_CTX(ctx);
+    MS_TRY(quad_batch_args_ok(batch_dtype, border_mode, border_value, "ms_page_batch_ragged_quads"));
+    if (n_pages <= 0) return MS_OK;
+    if (!score || !geo || !p || !page_ptrs || !page_hw || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
+        ms_set_error("ms_page_batch_ragged_quads: bad arguments");
+        return MS_ERR_INVALID;
+    }
+    // (the page sizes are device data: quads of a page above 32767 pixels on a side get no patch)
+    pb_call c;
+    pb_init(c, p);
+    c.score = score; c.geo = geo; c.page_ptrs = page_ptrs; c.page_hw = page_hw;
+    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w;
+    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
+    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
+    c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
+    c.crop_quads = 1; c.border_mode = border_mode; c.border_value = border_value;
+    return page_batch_cached(ctx, c, (cudaStream_t)stream);
 }
 
 // Read-back of a host page batch queued on the context's own stream, from device call d to the caller's buffers in h.

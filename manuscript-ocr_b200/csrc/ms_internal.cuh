@@ -31,6 +31,9 @@ struct pb_call {
     uint8_t *canvas_u8;
     int32_t *flags;
     int geo_compact;  // geo holds only the rows the decode reads, y % q == q / 2 (q = params.quantization)
+    // the crop stage: 0 = axis-aligned rectangles [page, x1, y1, x2, y2); 1 = rectified quads [page, box, w, h, 0]
+    // with the border of the perspective warp (0 = constant border_value, 1 = replicate)
+    int crop_quads, border_mode, border_value;
 };
 // A recorded ms_page_batch call and what its launches point into or were sized by; compared bytewise.
 struct ms_pb_key {
@@ -279,6 +282,20 @@ int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int
                   int border_value, int out_h, int out_w, void *batch, int batch_dtype, uint8_t *canvas_u8,
                   int32_t *sizes_out, ms_bump bump, cudaStream_t st);
 size_t msk_quad_crop_scratch(int64_t n);
+// the crop stage of a quad page batch over the final boxes (n_pages, cap_boxes, 9) / counts; pages (n_pages, img_h,
+// img_w, 3) or page_ptrs / page_hw.  msk_quad_list: crops_out rows [page, box, w, h, 0] of the boxes that have a
+// patch, in (page, box) order, and *n_crops = min(listed, crops_cap), all on the device.  msk_quad_crop_rows: the crop
+// of every listed row (batch row i = list row i; rows past *n_crops are not written).
+int msk_quad_list(ms_ctx *ctx, const float *boxes, const int32_t *counts, int n_pages, int cap_boxes,
+                  const uint8_t *pages, int img_h, int img_w, const uint8_t *const *page_ptrs, const int32_t *page_hw,
+                  int min_text_size, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops, ms_bump bump,
+                  cudaStream_t st);
+size_t msk_quad_list_scratch(int n_pages, int cap_boxes);
+int msk_quad_crop_rows(ms_ctx *ctx, const float *boxes, int cap_boxes, int n_pages, const uint8_t *pages, int img_h,
+                       int img_w, const uint8_t *const *page_ptrs, const int32_t *page_hw, const int32_t *crops,
+                       const int32_t *n_crops, int64_t crops_cap, int min_text_size, int border_mode, int border_value,
+                       int out_h, int out_w, void *batch, int batch_dtype, uint8_t *canvas_u8, ms_bump bump,
+                       cudaStream_t st);
 int msk_quad_warp(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, const float *quad_dev, int border_mode,
                   int border_value, uint8_t *patch_dev, size_t patch_cap, int *w, int *h, ms_bump bump, cudaStream_t st);
 

@@ -19,6 +19,9 @@
 // Kernels: quad_plan_kernel (thread per quad: size, homography, resize plan) and quad_crop_kernel (CTA per quad:
 // warp the patch into shared memory -- or evaluate it on the fly when it is larger than the stage -- then the same
 // per-pixel resampling as crop_generic_kernel).  HBM traffic per quad: the touched page pixels + 3*ih*iw*4 bytes out.
+// Every plan carries its own page (pointer and size): the quads come from one buffer of equally sized pages or from
+// page tables.  As the crop stage of a page batch (msk_quad_list + msk_quad_crop_rows) the quads are the batch's final
+// boxes, listed on the device by quad_list_mark_kernel / quad_list_write_kernel.
 #include "crop_common.cuh"
 
 namespace {
@@ -28,7 +31,9 @@ constexpr int kQcPatchBytes = 40 * 1024;  // shared-memory patch stage (e.g. 260
 constexpr int kQcMaxTab = 384;            // AxisEnt entries (nw + nh of a 64 x 256 canvas is 320)
 
 struct QuadPlan {
-    double m[9];  // patch (x, y, 1) -> page (X, Y, W)
+    double m[9];            // patch (x, y, 1) -> page (X, Y, W)
+    const uint8_t *px;      // the quad's page (img_h, img_w, 3), rows img_w * 3 bytes apart
+    int img_h, img_w;
     int page, w, h, bw0;
     int ok, staged;       // staged: taken by quad_crop_staged_kernel (source window copied into shared memory by TMA)
     int wx0, wy0, ww, wh;  // the window: columns [wx0, wx0 + ww), rows [wy0, wy0 + wh) of the page hold every tap
@@ -120,32 +125,80 @@ __device__ bool perspective_from_rect(const float *q, int w, int h, double *m)
     return true;
 }
 
-__global__ void __launch_bounds__(128) quad_plan_kernel(const float *__restrict__ quads, int quad_stride,
-                                                        const int32_t *__restrict__ page_of, int64_t n, int n_pages,
-                                                        int min_text_size, int ih, int iw, QuadPlan *__restrict__ qplans,
-                                                        Plan *__restrict__ plans, int32_t *__restrict__ sizes_out,
-                                                        const uint8_t *__restrict__ pages, int img_h, int img_w,
-                                                        int stage_ok, StageDesc *__restrict__ work,
-                                                        int32_t *__restrict__ n_work)
+// Where a crop call's quads and pages are.  Quads: an array of rows quad_stride floats apart with page_of (NULL: page
+// 0) -- quad i is batch row i -- or, for a page batch, the crop list `list` of *list_n rows [page, box, w, h, 0] over
+// the page-strided final boxes `quads` (n_pages, cap_boxes, quad_stride) -- list row i is batch row i.  Pages: one
+// buffer of equally sized pages (pages, img_h, img_w) or the device tables page_ptrs / page_hw of pages of their own
+// sizes.
+struct QuadSrc {
+    const float *quads;
+    int quad_stride, cap_boxes;
+    const int32_t *page_of, *list, *list_n;
+    const uint8_t *pages;
+    const uint8_t *const *page_ptrs;
+    const int32_t *page_hw;
+    int n_pages, img_h, img_w;
+};
+
+// page `page` of a call; false (no patch for its quads) when it is out of range, empty or larger than the 16-bit
+// coordinates of the remap allow
+__device__ __forceinline__ bool quad_page(const QuadSrc &s, int page, const uint8_t *&px, int &img_h, int &img_w)
+{
+    px = nullptr;
+    img_h = img_w = 0;
+    if (page < 0 || page >= s.n_pages) return false;
+    if (s.page_ptrs) {
+        px = s.page_ptrs[page];
+        img_h = s.page_hw[2 * page];
+        img_w = s.page_hw[2 * page + 1];
+    } else {
+        px = s.pages + (size_t)page * s.img_h * s.img_w * 3;
+        img_h = s.img_h;
+        img_w = s.img_w;
+    }
+    return px != nullptr && img_h > 0 && img_w > 0 && img_h <= 32767 && img_w <= 32767;
+}
+
+// a quad of a valid page has a patch: its size, at least min_text_size on a side (_pipeline.py:130-133 applied to the
+// patch), and a non-singular homography
+__device__ __forceinline__ bool quad_has_patch(const float *v, int min_text_size, int &w, int &h, double *m)
+{
+    bool ok = quad_patch_size(v, w, h);
+    ok = ok && w >= min_text_size && h >= min_text_size;
+    return ok && perspective_from_rect(v, w, h, m);
+}
+
+__global__ void __launch_bounds__(128) quad_plan_kernel(QuadSrc src, int64_t n, int min_text_size, int ih, int iw,
+                                                        QuadPlan *__restrict__ qplans, Plan *__restrict__ plans,
+                                                        int32_t *__restrict__ sizes_out, int stage_ok,
+                                                        StageDesc *__restrict__ work, int32_t *__restrict__ n_work)
 {
     ms_pdl_wait();
+    if (src.list_n) n = min(n, (int64_t)*src.list_n);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        const float *q = quads + i * quad_stride;
         QuadPlan qp;
         Plan p;
         plan_reset(p);
-        qp.page = page_of ? page_of[i] : 0;
+        int64_t qi = i;
+        if (src.list) {
+            qp.page = src.list[5 * i];
+            qi = (int64_t)qp.page * src.cap_boxes + src.list[5 * i + 1];
+        } else {
+            qp.page = src.page_of ? src.page_of[i] : 0;
+        }
         qp.ok = qp.staged = 0;
         qp.wx0 = qp.wy0 = qp.ww = qp.wh = qp.mis = qp.pad0 = 0;
         qp.bw0 = 1;
 #pragma unroll
         for (int k = 0; k < 9; k++) qp.m[k] = 0.0;
+        bool ok = quad_page(src, qp.page, qp.px, qp.img_h, qp.img_w);
         float v[8];
+        if (ok || !src.list) {  // (a list row names a box of a valid page)
+            const float *q = src.quads + qi * src.quad_stride;
 #pragma unroll
-        for (int k = 0; k < 8; k++) v[k] = q[k];
-        bool ok = qp.page >= 0 && qp.page < n_pages && quad_patch_size(v, qp.w, qp.h);
-        ok = ok && qp.w >= min_text_size && qp.h >= min_text_size;  // _pipeline.py:130-133 applied to the patch
-        ok = ok && perspective_from_rect(v, qp.w, qp.h, qp.m);
+            for (int k = 0; k < 8; k++) v[k] = q[k];
+        }
+        ok = ok && quad_has_patch(v, min_text_size, qp.w, qp.h, qp.m);
         if (ok) {
             // WarpPerspectiveInvoker's block width for a (w, h) destination
             const int bh0 = min(16, qp.h);
@@ -163,8 +216,12 @@ __global__ void __launch_bounds__(128) quad_plan_kernel(const float *__restrict_
             // every coordinate is finite, and the projective image of the patch rectangle is the convex hull of the
             // corner images -- and (v) the window that holds every tap (that hull, plus the bilinear neighbour and a
             // pixel of slack for the 1/32-pixel rounding and the float64 rounding of the per-pixel evaluation, both far
-            // below a pixel) is inside the page (no border handling) and fits the ring.
-            bool corners_ok = stage_ok && work && p.interp == 3 && p.scale_x < 2.999 && p.scale_y < 2.999 && qp.h >= 16 &&
+            // below a pixel) is inside the page (no border handling) and fits the ring.  The TMA bulk copies need the
+            // page's base address and row stride to be multiples of 16, and the window -- its last row rounded up to
+            // `pitch` -- inside the page's own bytes.
+            const size_t stride = (size_t)qp.img_w * 3;
+            bool corners_ok = stage_ok && work && (reinterpret_cast<uintptr_t>(qp.px) & 15) == 0 && stride % 16 == 0 &&
+                              p.interp == 3 && p.scale_x < 2.999 && p.scale_y < 2.999 && qp.h >= 16 &&
                               qp.w < 32768;
             double mnx = 1e300, mxx = -1e300, mny = 1e300, mxy = -1e300;
             if (corners_ok) {
@@ -185,14 +242,13 @@ __global__ void __launch_bounds__(128) quad_plan_kernel(const float *__restrict_
                 const int wx0 = (int)floor(mnx) - 1, wx1 = (int)floor(mxx) + 2;
                 const int wy0 = (int)floor(mny) - 1, wy1 = (int)floor(mxy) + 2;
                 const int band_rows = (int)ceil(kQsG * p.scale_y) + 2;
-                if (wx0 >= 0 && wy0 >= 0 && wx1 < img_w && wy1 < img_h &&
+                if (wx0 >= 0 && wy0 >= 0 && wx1 < qp.img_w && wy1 < qp.img_h &&
                     (size_t)band_rows * qp.w * 3 <= (size_t)kQsBandBytes) {
-                    const size_t stride = (size_t)img_w * 3;
-                    const uint8_t *first = pages + (size_t)qp.page * img_h * stride + (size_t)wy0 * stride + (size_t)wx0 * 3;
+                    const uint8_t *first = qp.px + (size_t)wy0 * stride + (size_t)wx0 * 3;
                     const int a = (int)(reinterpret_cast<uintptr_t>(first) & 15);
                     const int ww = wx1 - wx0 + 1, wh = wy1 - wy0 + 1;
                     const int pitch = (a + ww * 3 + 15) & ~15;
-                    const uint8_t *end = pages + (size_t)n_pages * img_h * stride;
+                    const uint8_t *end = qp.px + (size_t)qp.img_h * stride;
                     if ((size_t)pitch * wh + 16 <= (size_t)kQsWinMax &&
                         first - a + (size_t)(wh - 1) * stride + pitch <= end) {
                         qp.staged = 1;
@@ -349,8 +405,7 @@ struct WarpSrc {
 };
 
 template <class T, bool kWriteU8>
-__global__ void __launch_bounds__(kQcThreads, 4) quad_crop_kernel(const uint8_t *__restrict__ pages, int img_h,
-                                                                  int img_w, const QuadPlan *__restrict__ qplans,
+__global__ void __launch_bounds__(kQcThreads, 4) quad_crop_kernel(const QuadPlan *__restrict__ qplans,
                                                                   const Plan *__restrict__ plans, int64_t n,
                                                                   int replicate, int bval, int ih, int iw,
                                                                   T *__restrict__ batch,
@@ -391,7 +446,7 @@ __global__ void __launch_bounds__(kQcThreads, 4) quad_crop_kernel(const uint8_t 
         }
         const bool x3 = __syncthreads_and(x3_mine) != 0;  // also the barrier after the tables
         const QuadPlan &qp = s_qp;
-        const PageView pg{pages + (size_t)qp.page * img_h * (size_t)img_w * 3, img_h, img_w, replicate, bval};
+        const PageView pg{qp.px, qp.img_h, qp.img_w, replicate, bval};
         if (p.staged) {
             const size_t pitch = (size_t)qp.w * 3;
             warp_rows(qp, pg, qc_patch, pitch, warp, kQcThreads / 32, lane);
@@ -601,17 +656,18 @@ __global__ void __launch_bounds__(kQsThreads, 2)
 
 // quads for the generic kernel: not staged, or handed back
 __global__ void __launch_bounds__(256) quad_fallback_list_kernel(const QuadPlan *__restrict__ qplans, int64_t n,
+                                                                 const int32_t *__restrict__ n_dev,
                                                                  const uint8_t *__restrict__ redo,
                                                                  int32_t *__restrict__ list, int32_t *__restrict__ list_n)
 {
     ms_pdl_wait();
+    if (n_dev) n = min(n, (int64_t)*n_dev);  // a crop list: its rows on the device
     for (int64_t ci = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; ci < n; ci += (int64_t)gridDim.x * blockDim.x)
         if (!qplans[ci].staged || redo[ci]) list[atomicAdd(list_n, 1)] = (int32_t)ci;
 }
 
 // the patch alone (row-major h x w x 3), for one planned quad
-__global__ void __launch_bounds__(256) quad_warp_kernel(const uint8_t *__restrict__ page, int img_h, int img_w,
-                                                        const QuadPlan *__restrict__ qplan, int replicate, int bval,
+__global__ void __launch_bounds__(256) quad_warp_kernel(const QuadPlan *__restrict__ qplan, int replicate, int bval,
                                                         uint8_t *__restrict__ patch)
 {
     ms_pdl_wait();
@@ -620,7 +676,7 @@ __global__ void __launch_bounds__(256) quad_warp_kernel(const uint8_t *__restric
     __syncthreads();
     const QuadPlan &qp = s_qp;
     if (!qp.ok) return;
-    const PageView pg{page, img_h, img_w, replicate, bval};
+    const PageView pg{qp.px, qp.img_h, qp.img_w, replicate, bval};
     const int64_t npx = (int64_t)qp.w * qp.h;
     for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < npx; t += (int64_t)gridDim.x * blockDim.x) {
         const int y = (int)(t / qp.w), x = (int)(t - (int64_t)y * qp.w);
@@ -632,6 +688,98 @@ __global__ void __launch_bounds__(256) quad_warp_kernel(const uint8_t *__restric
     }
 }
 
+// ---- the crop list of a quad page batch ----------------------------------------------------------------------------
+// Pass 1, one CTA per page: the page's boxes that have a patch (quad_has_patch, the plan kernel's test) -- wh[box] =
+// w | h << 16, 0 for none -- and their number.  Pass 2, one CTA per page: the page's first row is the number of such
+// boxes on the pages before it; its rows [page, box, w, h, 0] follow in box order, those at or past crops_cap are not
+// written (the rule of word_rects), and the last page's CTA sets *n_crops = min(listed, crops_cap).
+constexpr int kQlThreads = 256;
+
+__device__ __forceinline__ int ql_block_sum(int v, int *s_warp)
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    v = __reduce_add_sync(0xffffffffu, v);
+    __syncthreads();  // s_warp is free
+    if (lane == 0) s_warp[warp] = v;
+    __syncthreads();
+    int t = 0;
+#pragma unroll
+    for (int k = 0; k < kQlThreads / 32; k++) t += s_warp[k];
+    return t;
+}
+
+__global__ void __launch_bounds__(kQlThreads) quad_list_mark_kernel(QuadSrc src, const int32_t *__restrict__ counts,
+                                                                    int min_text_size, int32_t *__restrict__ wh,
+                                                                    int32_t *__restrict__ page_n,
+                                                                    int32_t *__restrict__ page_nb)
+{
+    ms_pdl_wait();
+    __shared__ int s_warp[kQlThreads / 32];
+    const int page = blockIdx.x;
+    const uint8_t *px;
+    int img_h, img_w;
+    const int nb = quad_page(src, page, px, img_h, img_w) ? min(max(counts[page], 0), src.cap_boxes) : 0;
+    int mine = 0;
+    for (int b = threadIdx.x; b < nb; b += kQlThreads) {
+        const float *q = src.quads + ((size_t)page * src.cap_boxes + b) * src.quad_stride;
+        float v[8];
+#pragma unroll
+        for (int k = 0; k < 8; k++) v[k] = q[k];
+        int w, h;
+        double m[9];
+        const bool ok = quad_has_patch(v, min_text_size, w, h, m);
+        wh[(size_t)page * src.cap_boxes + b] = ok ? (w | (h << 16)) : 0;
+        mine += ok ? 1 : 0;
+    }
+    const int total = ql_block_sum(mine, s_warp);
+    if (threadIdx.x == 0) {
+        page_n[page] = total;
+        page_nb[page] = nb;
+    }
+}
+
+__global__ void __launch_bounds__(kQlThreads) quad_list_write_kernel(const int32_t *__restrict__ wh,
+                                                                     const int32_t *__restrict__ page_n,
+                                                                     const int32_t *__restrict__ page_nb, int n_pages,
+                                                                     int cap_boxes, int32_t *__restrict__ crops_out,
+                                                                     int64_t crops_cap, int32_t *__restrict__ n_crops)
+{
+    ms_pdl_wait();
+    __shared__ int s_warp[kQlThreads / 32];
+    const int page = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int before = 0;
+    for (int p = threadIdx.x; p < page; p += kQlThreads) before += page_n[p];
+    int64_t row = ql_block_sum(before, s_warp);
+    if (page == n_pages - 1 && threadIdx.x == 0) {
+        const int64_t listed = row + page_n[page];
+        *n_crops = (int32_t)(listed < crops_cap ? listed : crops_cap);
+    }
+    const int nb = page_nb[page];
+    for (int b0 = 0; b0 < nb && row < crops_cap; b0 += kQlThreads) {
+        const int b = b0 + threadIdx.x;
+        const int v = b < nb ? wh[(size_t)page * cap_boxes + b] : 0;
+        const unsigned bal = __ballot_sync(0xffffffffu, v != 0);
+        __syncthreads();  // s_warp is free
+        if (lane == 0) s_warp[warp] = __popc(bal);
+        __syncthreads();
+        int rank = __popc(bal & ((1u << lane) - 1u)), all = 0;
+#pragma unroll
+        for (int k = 0; k < kQlThreads / 32; k++) {
+            rank += k < warp ? s_warp[k] : 0;
+            all += s_warp[k];
+        }
+        if (v != 0 && row + rank < crops_cap) {
+            int32_t *r = crops_out + (row + rank) * 5;
+            r[0] = page;
+            r[1] = b;
+            r[2] = v & 0xffff;
+            r[3] = v >> 16;
+            r[4] = 0;
+        }
+        row += all;
+    }
+}
+
 }  // namespace
 
 size_t msk_quad_crop_scratch(int64_t n)
@@ -640,12 +788,8 @@ size_t msk_quad_crop_scratch(int64_t n)
     return k * (sizeof(QuadPlan) + sizeof(Plan) + sizeof(StageDesc) + 1 + sizeof(int32_t)) + 8192;
 }
 
-static int quad_args_ok(int n_pages, int img_h, int img_w, int border_mode, int border_value, const char *who)
+static int quad_border_ok(int border_mode, int border_value, const char *who)
 {
-    if (n_pages <= 0 || img_h <= 0 || img_w <= 0 || img_h > 32767 || img_w > 32767) {
-        ms_set_error("%s: pages must be 1..32767 pixels on a side (16-bit remap coordinates), got %dx%d", who, img_h, img_w);
-        return MS_ERR_INVALID;
-    }
     if (border_mode < 0 || border_mode > 1 || border_value < 0 || border_value > 255) {
         ms_set_error("%s: border_mode must be 0 (constant) or 1 (replicate), border_value 0..255", who);
         return MS_ERR_INVALID;
@@ -653,14 +797,21 @@ static int quad_args_ok(int n_pages, int img_h, int img_w, int border_mode, int 
     return MS_OK;
 }
 
-int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w, const float *quads,
-                  int quad_stride, const int32_t *page_of, int64_t n, int min_text_size, int border_mode,
-                  int border_value, int out_h, int out_w, void *batch, int batch_dtype, uint8_t *canvas_u8,
-                  int32_t *sizes_out, ms_bump bump, cudaStream_t st)
+static int quad_args_ok(int n_pages, int img_h, int img_w, int border_mode, int border_value, const char *who)
 {
-    if (n <= 0) return MS_OK;
-    MS_TRY(quad_args_ok(n_pages, img_h, img_w, border_mode, border_value, "quad_crop"));
-    if (out_h <= 0 || out_w <= 0 || quad_stride < 8 || (!batch && !canvas_u8) ||
+    if (n_pages <= 0 || img_h <= 0 || img_w <= 0 || img_h > 32767 || img_w > 32767) {
+        ms_set_error("%s: pages must be 1..32767 pixels on a side (16-bit remap coordinates), got %dx%d", who, img_h, img_w);
+        return MS_ERR_INVALID;
+    }
+    return quad_border_ok(border_mode, border_value, who);
+}
+
+// plan -> staged kernel -> fallback list -> generic kernel over the n quads (or up to n list rows) of `src`
+static int quad_crop_run(ms_ctx *ctx, const QuadSrc &src, int64_t n, int min_text_size, int border_mode,
+                         int border_value, int out_h, int out_w, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                         int32_t *sizes_out, ms_bump bump, cudaStream_t st)
+{
+    if (out_h <= 0 || out_w <= 0 || src.quad_stride < 8 || (!batch && !canvas_u8) ||
         (int64_t)out_h * out_w > (1 << 20)) {
         ms_set_error("quad_crop: bad arguments");
         return MS_ERR_INVALID;
@@ -675,21 +826,24 @@ int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int
         ms_set_error("quad_crop: scratch too small");
         return MS_ERR_CAPACITY;
     }
-    // The staged kernel needs 16-byte aligned page rows (TMA bulk copies) and 32-bit quad indices; MS_B200_QUAD_NO_STAGE=1
-    // sends every quad to the generic kernel (A/B runs and tests).
+    // The staged kernel needs 32-bit quad indices, and (decided per quad by the plan kernel) a 16-byte aligned page
+    // with 16-byte aligned rows (TMA bulk copies); MS_B200_QUAD_NO_STAGE=1 sends every quad to the generic kernel (A/B
+    // runs and tests).
     const int tab_bytes = area_tab_words(out_h, out_w) * (int)sizeof(uint32_t);
     const int smem_s = kQsRing + 64 + kQsCW * kQsBandPitch + kQsSlots * tab_bytes;
-    // (a 64 x 256 canvas' tables do not leave room for two CTAs per SM: generic kernel)
-    const int stage_ok = (reinterpret_cast<uintptr_t>(pages) & 15) == 0 && ((size_t)img_w * 3) % 16 == 0 &&
-                         n < ((int64_t)1 << 31) && !ctx->quad_no_stage && smem_s <= 112 * 1024;
+    // (a 64 x 256 canvas' tables do not leave room for two CTAs per SM: generic kernel).  Equally sized pages whose
+    // buffer or rows are not 16-byte aligned cannot have a staged quad: no staged launch.
+    const bool pages_may_stage = src.page_ptrs != nullptr || ((reinterpret_cast<uintptr_t>(src.pages) & 15) == 0 &&
+                                                              ((size_t)src.img_w * 3) % 16 == 0);
+    const int stage_ok = pages_may_stage && n < ((int64_t)1 << 31) && !ctx->quad_no_stage && smem_s <= 112 * 1024;
     MS_CUDA(cudaMemsetAsync(cnt, 0, 4 * sizeof(int32_t), st));
     ctx->quad_cnt = cnt;
     ctx->quad_stream = st;
     MS_CUDA(cudaMemsetAsync(redo, 0, (size_t)n, st));
     int64_t pg = (n + 127) / 128;
     if (pg > (int64_t)ctx->num_sms * 16) pg = (int64_t)ctx->num_sms * 16;
-    ms_launch(quad_plan_kernel, (int)pg, 128, 0, st, quads, quad_stride, page_of, n, n_pages, min_text_size, out_h, out_w,
-                                             qplans, plans, sizes_out, pages, img_h, img_w, stage_ok, work, cnt);
+    ms_launch(quad_plan_kernel, (int)pg, 128, 0, st, src, n, min_text_size, out_h, out_w, qplans, plans, sizes_out,
+              stage_ok, work, cnt);
     MS_LAUNCH_CHECK(ctx);
     const bool staged = stage_ok != 0;
     int64_t grid = (int64_t)ctx->num_sms * 4;  // 40 KB stage + 12 KB tables, 64 registers: four CTAs per SM
@@ -706,14 +860,94 @@ int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int
                       cnt + 1, out_h, out_w, out, canvas_u8, vec_ok, redo);
             MS_LAUNCH_CHECK(ctx);
         }
-        ms_launch(quad_fallback_list_kernel, (int)pg, 256, 0, st, qplans, n, redo, list, cnt + 2);
+        ms_launch(quad_fallback_list_kernel, (int)pg, 256, 0, st, qplans, n, src.list_n, redo, list, cnt + 2);
         MS_LAUNCH_CHECK(ctx);
         MS_TRY(ms_allow_smem(ctx, batch_slot<T, kU8>(MS_SMEM_QUAD_U8), quad_crop_kernel<T, kU8>, smem));
-        ms_launch(quad_crop_kernel<T, kU8>, (int)grid, kQcThreads, smem, st, pages, img_h, img_w, qplans, plans, n,
-                  border_mode, border_value, out_h, out_w, out, canvas_u8, vec_ok, list, cnt + 2);
+        ms_launch(quad_crop_kernel<T, kU8>, (int)grid, kQcThreads, smem, st, qplans, plans, n, border_mode, border_value,
+                  out_h, out_w, out, canvas_u8, vec_ok, list, cnt + 2);
         MS_LAUNCH_CHECK(ctx);
         return MS_OK;
     });
+}
+
+int msk_quad_crop(ms_ctx *ctx, const uint8_t *pages, int n_pages, int img_h, int img_w, const float *quads,
+                  int quad_stride, const int32_t *page_of, int64_t n, int min_text_size, int border_mode,
+                  int border_value, int out_h, int out_w, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                  int32_t *sizes_out, ms_bump bump, cudaStream_t st)
+{
+    if (n <= 0) return MS_OK;
+    MS_TRY(quad_args_ok(n_pages, img_h, img_w, border_mode, border_value, "quad_crop"));
+    QuadSrc src = {};
+    src.quads = quads;
+    src.quad_stride = quad_stride;
+    src.page_of = page_of;
+    src.pages = pages;
+    src.n_pages = n_pages;
+    src.img_h = img_h;
+    src.img_w = img_w;
+    return quad_crop_run(ctx, src, n, min_text_size, border_mode, border_value, out_h, out_w, batch, batch_dtype,
+                         canvas_u8, sizes_out, bump, st);
+}
+
+static QuadSrc quad_batch_src(const float *boxes, int cap_boxes, int n_pages, const uint8_t *pages, int img_h,
+                              int img_w, const uint8_t *const *page_ptrs, const int32_t *page_hw)
+{
+    QuadSrc src = {};
+    src.quads = boxes;
+    src.quad_stride = 9;
+    src.cap_boxes = cap_boxes;
+    src.n_pages = n_pages;
+    if (page_ptrs && page_hw) {
+        src.page_ptrs = page_ptrs;
+        src.page_hw = page_hw;
+    } else {
+        src.pages = pages;
+        src.img_h = img_h;
+        src.img_w = img_w;
+    }
+    return src;
+}
+
+size_t msk_quad_list_scratch(int n_pages, int cap_boxes)
+{
+    return (size_t)n_pages * cap_boxes * sizeof(int32_t) + 2 * (size_t)n_pages * sizeof(int32_t) + 4096;
+}
+
+int msk_quad_list(ms_ctx *ctx, const float *boxes, const int32_t *counts, int n_pages, int cap_boxes,
+                  const uint8_t *pages, int img_h, int img_w, const uint8_t *const *page_ptrs, const int32_t *page_hw,
+                  int min_text_size, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops, ms_bump bump,
+                  cudaStream_t st)
+{
+    if (n_pages <= 0) return MS_OK;
+    int32_t *wh = bump.take<int32_t>((size_t)n_pages * cap_boxes);
+    int32_t *page_n = bump.take<int32_t>((size_t)n_pages);
+    int32_t *page_nb = bump.take<int32_t>((size_t)n_pages);
+    if (!wh || !page_n || !page_nb) {
+        ms_set_error("quad_list: scratch too small");
+        return MS_ERR_CAPACITY;
+    }
+    const QuadSrc src = quad_batch_src(boxes, cap_boxes, n_pages, pages, img_h, img_w, page_ptrs, page_hw);
+    ms_launch(quad_list_mark_kernel, n_pages, kQlThreads, 0, st, src, counts, min_text_size, wh, page_n, page_nb);
+    MS_LAUNCH_CHECK(ctx);
+    ms_launch(quad_list_write_kernel, n_pages, kQlThreads, 0, st, wh, page_n, page_nb, n_pages, cap_boxes, crops_out,
+              crops_cap, n_crops);
+    MS_LAUNCH_CHECK(ctx);
+    return MS_OK;
+}
+
+int msk_quad_crop_rows(ms_ctx *ctx, const float *boxes, int cap_boxes, int n_pages, const uint8_t *pages, int img_h,
+                       int img_w, const uint8_t *const *page_ptrs, const int32_t *page_hw, const int32_t *crops,
+                       const int32_t *n_crops, int64_t crops_cap, int min_text_size, int border_mode, int border_value,
+                       int out_h, int out_w, void *batch, int batch_dtype, uint8_t *canvas_u8, ms_bump bump,
+                       cudaStream_t st)
+{
+    if (crops_cap <= 0 || n_pages <= 0) return MS_OK;
+    MS_TRY(quad_border_ok(border_mode, border_value, "quad_crop"));
+    QuadSrc src = quad_batch_src(boxes, cap_boxes, n_pages, pages, img_h, img_w, page_ptrs, page_hw);
+    src.list = crops;
+    src.list_n = n_crops;
+    return quad_crop_run(ctx, src, crops_cap, min_text_size, border_mode, border_value, out_h, out_w, batch,
+                         batch_dtype, canvas_u8, nullptr, bump, st);
 }
 
 // One quad's patch.  *w / *h receive the patch size (0, 0: no patch); the pixels are produced only when they fit
@@ -729,8 +963,14 @@ int msk_quad_warp(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, const 
         ms_set_error("quad_warp: scratch too small");
         return MS_ERR_CAPACITY;
     }
-    ms_launch(quad_plan_kernel, 1, 128, 0, st, quad_dev, 8, nullptr, 1, 1, 0, 32, 128, qplan, plan, size, nullptr, img_h, img_w, 0,
-                                        nullptr, nullptr);
+    QuadSrc src = {};
+    src.quads = quad_dev;
+    src.quad_stride = 8;
+    src.pages = page;
+    src.n_pages = 1;
+    src.img_h = img_h;
+    src.img_w = img_w;
+    ms_launch(quad_plan_kernel, 1, 128, 0, st, src, (int64_t)1, 0, 32, 128, qplan, plan, size, 0, nullptr, nullptr);
     MS_LAUNCH_CHECK(ctx);
     int32_t hs[2] = {0, 0};
     MS_CUDA(cudaMemcpyAsync(hs, size, sizeof(hs), cudaMemcpyDeviceToHost, st));
@@ -745,7 +985,7 @@ int msk_quad_warp(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, const 
     }
     int64_t grid = ((int64_t)hs[0] * hs[1] + 255) / 256;
     if (grid > (int64_t)ctx->num_sms * 8) grid = (int64_t)ctx->num_sms * 8;
-    ms_launch(quad_warp_kernel, (int)grid, 256, 0, st, page, img_h, img_w, qplan, border_mode, border_value, patch_dev);
+    ms_launch(quad_warp_kernel, (int)grid, 256, 0, st, qplan, border_mode, border_value, patch_dev);
     MS_LAUNCH_CHECK(ctx);
     return MS_OK;
 }

@@ -130,6 +130,12 @@ SIGNATURES = {
                                    _vp, _vp, _i64, _vp, _vp, _i, C.POINTER(_vp), _vp]),
     "ms_page_batch_ragged_host_ex": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i, _i,
                                           _vp, _vp, _vp, _i64, _vp, _vp, _i, C.POINTER(_vp), _vp]),
+    # EXTENSION: page batches whose crop stage is the rectified crop of every final quad (border_mode, border_value
+    # after min_text_size)
+    "ms_page_batch_quads": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i, _i, _i,
+                                 _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
+    "ms_page_batch_ragged_quads": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i, _i, _i,
+                                        _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
 }
 
 

@@ -38,7 +38,8 @@ class PageBatchResult:
     the same kind and page count: clone() what has to outlive it."""
     boxes: object        # (P, cap_boxes, 9) f32: rows [0, box_counts[p]) are page p's final boxes
     box_counts: object   # (P,) int32
-    crops: object        # (crops_cap, 5) int32 rows [page, x1, y1, x2, y2), first n_crops valid
+    crops: object        # (crops_cap, 5) int32 rows, first n_crops valid: [page, x1, y1, x2, y2) (crops="rects"), or
+                         # [page, box, w, h, 0] (crops="quads": box = the quad's row in boxes[page], (w, h) its patch)
     n_crops: object      # () / (1,) int32
     batch: object        # (crops_cap | n_crops, 3, h, w) CUDA tensor of the runner's batch_dtype (None if not requested)
     flags: object        # (P,) int32 MS_FLAG_* bits
@@ -90,10 +91,17 @@ class PageBatch:
 
     crops_cap: crop rows of the buffers (default n_pages * cap_boxes); it may be changed between calls, and the next
     call reallocates.  max_buffer_sets: keep the device buffers of at most this many page counts, dropping the least
-    recently used (default: one set per page count seen)."""
+    recently used (default: one set per page count seen).
+
+    crops: the crop stage of run / run_ragged.  "rects" (default) cuts the axis-aligned rectangle of every box (the
+    reference's crops).  "quads" (an EXTENSION, not a reference behaviour) cuts the rectified patch of every final quad,
+    cv2.warpPerspective with border_mode 0 (BORDER_CONSTANT, border_value on all channels) or 1 (BORDER_REPLICATE), as
+    ms_quad_crop_resize_pad does: the crop list then holds one row [page, box, w, h, 0] per quad that has a patch, in
+    (page, box) order, and batch row i is the crop of list row i.  The host entry points (run_host*) cut rectangles
+    only."""
 
     def __init__(self, device=0, params=None, min_text_size=5, out_hw=(32, 128), cap_boxes=4096, crops_cap=None,
-                 want_batch=True, batch_dtype=None, max_buffer_sets=None):
+                 want_batch=True, batch_dtype=None, max_buffer_sets=None, crops="rects", border_mode=0, border_value=0):
         import torch
 
         if not torch.cuda.is_available():
@@ -110,6 +118,10 @@ class PageBatch:
         self.batch_dtype = torch.float32 if batch_dtype is None else batch_dtype
         self._dtype_code = batch_dtype_code(self.batch_dtype)
         self.max_buffer_sets = max_buffer_sets
+        if crops not in ("rects", "quads"):
+            raise ValueError(f'crops must be "rects" or "quads", got {crops!r}')
+        self.crops = crops
+        self.border_mode, self.border_value = int(border_mode), int(border_value)
         self._bufs = {}
         self._host = {}
         self._ragged_tables = {}
@@ -172,13 +184,17 @@ class PageBatch:
         b = self._device_bufs(P)
         stream = torch.cuda.current_stream(self.device).cuda_stream
         lib = self.ctx.lib
+        head = (self.ctx.handle, score.data_ptr(), geo.data_ptr(), pages.data_ptr() if pages is not None else None,
+                P, H, W, img_h, img_w, C.byref(self.params), self.min_text_size)
+        tail = (self.out_h, self.out_w, self.cap_boxes, b["boxes"].data_ptr(), b["counts"].data_ptr(),
+                b["crops"].data_ptr(), b["cap"], b["n_crops"].data_ptr(),
+                b["batch"].data_ptr() if b["batch"] is not None else None, self._dtype_code, None, b["flags"].data_ptr(),
+                C.c_void_p(stream))
         with torch.cuda.device(self.device):
-            check(lib.ms_page_batch_ex(
-                self.ctx.handle, score.data_ptr(), geo.data_ptr(), pages.data_ptr() if pages is not None else None,
-                P, H, W, img_h, img_w, C.byref(self.params), self.min_text_size, self.out_h, self.out_w,
-                self.cap_boxes, b["boxes"].data_ptr(), b["counts"].data_ptr(), b["crops"].data_ptr(), b["cap"],
-                b["n_crops"].data_ptr(), b["batch"].data_ptr() if b["batch"] is not None else None, self._dtype_code,
-                None, b["flags"].data_ptr(), C.c_void_p(stream)))
+            if self.crops == "quads":
+                check(lib.ms_page_batch_quads(*head, self.border_mode, self.border_value, *tail))
+            else:
+                check(lib.ms_page_batch_ex(*head, *tail))
         return PageBatchResult(b["boxes"], b["counts"], b["crops"], b["n_crops"], b["batch"], b["flags"])
 
     def run_ragged(self, score, geo, pages, sync=False, allow_order_overflow=False):
@@ -217,13 +233,18 @@ class PageBatch:
         ptrs, hw = cached
         b = self._device_bufs(P)
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        with torch.cuda.device(self.device):
-            check(self.ctx.lib.ms_page_batch_ragged_ex(
-                self.ctx.handle, score.data_ptr(), geo.data_ptr(), ptrs.data_ptr(), hw.data_ptr(), P, H, W,
-                C.byref(self.params), self.min_text_size, self.out_h, self.out_w, self.cap_boxes, b["boxes"].data_ptr(),
-                b["counts"].data_ptr(), b["crops"].data_ptr(), b["cap"], b["n_crops"].data_ptr(),
+        lib = self.ctx.lib
+        head = (self.ctx.handle, score.data_ptr(), geo.data_ptr(), ptrs.data_ptr(), hw.data_ptr(), P, H, W,
+                C.byref(self.params), self.min_text_size)
+        tail = (self.out_h, self.out_w, self.cap_boxes, b["boxes"].data_ptr(), b["counts"].data_ptr(),
+                b["crops"].data_ptr(), b["cap"], b["n_crops"].data_ptr(),
                 b["batch"].data_ptr() if b["batch"] is not None else None, self._dtype_code, None, b["flags"].data_ptr(),
-                C.c_void_p(stream)))
+                C.c_void_p(stream))
+        with torch.cuda.device(self.device):
+            if self.crops == "quads":
+                check(lib.ms_page_batch_ragged_quads(*head, self.border_mode, self.border_value, *tail))
+            else:
+                check(lib.ms_page_batch_ragged_ex(*head, *tail))
         res = PageBatchResult(b["boxes"], b["counts"], b["crops"], b["n_crops"], b["batch"], b["flags"])
         res._keepalive = (keep, ptrs, hw)  # the kernels read them after this call returns
         return res

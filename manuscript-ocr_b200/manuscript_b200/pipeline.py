@@ -17,6 +17,10 @@ Three routes through predict(), all with the reference's results:
 process_batch on the fused route works on chunks of pages: one upload buffer, one detector-input launch, one network
 call and one ms_page_batch_ragged call per chunk, and recogniser batches that span pages ("fused_batch").
 
+rotated_crops=True (an extension) takes the same fused routes ("fused_rotated", "fused_batch_rotated") with
+ms_page_batch_ragged_quads: the crop stage is the rectified patch of every final quad, and the crop list rows
+[page, box, w, h, 0] name the words by their position in the page's reading order.
+
 With this package's TRBA, the device routes (and rotated_crops) write the recogniser batch in the TRBA's batch_dtype
 (float32 by default); a foreign recogniser still gets uint8 slices.
 """
@@ -81,6 +85,27 @@ def host_crop_rects(boxes, img_h, img_w, min_text_size):
     return np.stack([x1, y1, x2, y2], axis=1).astype(np.int32), valid
 
 
+def host_patch_sizes(boxes):
+    """The patch size of the rotated crop (quadcrop.cu quad_patch_size) for (K, >=8) float boxes: the longer of each
+    pair of opposite edges in float64 from the float32 vertices, rounded half to even.  Returns (w, h, ok): ok is
+    False where a coordinate is not finite, a side is above 32767 or below 2.  Used to check the device's quad crop
+    list against the word boxes."""
+    b = np.asarray(boxes, dtype=np.float32)
+    q = (b.reshape(len(b), -1)[:, :8] if len(b) else np.zeros((0, 8), np.float32)).astype(np.float64)
+    x, y = q[:, 0::2], q[:, 1::2]
+
+    def edge(a, c):
+        dx, dy = x[:, c] - x[:, a], y[:, c] - y[:, a]
+        return np.sqrt(dx * dx + dy * dy)
+
+    e01, e32, e03, e12 = edge(0, 1), edge(3, 2), edge(0, 3), edge(1, 2)
+    ew, eh = np.where(e32 > e01, e32, e01), np.where(e12 > e03, e12, e03)
+    ok = np.isfinite(e01) & np.isfinite(e32) & np.isfinite(e03) & np.isfinite(e12) & (ew <= 32767) & (eh <= 32767)
+    w = np.rint(np.where(ok, ew, 0)).astype(np.int64)
+    h = np.rint(np.where(ok, eh, 0)).astype(np.int64)
+    return w, h, ok & (w >= 2) & (h >= 2)
+
+
 _BATCH_CROPS_CAP0 = 8192  # first crop capacity of process_batch's page batch (grown to what a chunk needs)
 
 
@@ -95,23 +120,26 @@ class Pipeline:
         # cutting its bounding rectangle.  Off by default = the reference's behaviour.
         self.rotated_crops = bool(rotated_crops)
         self._runners = {}  # False: the one-page route's PageBatch, True: the batched route's, each with its key
-        # "fused" | "fused_batch" | "device_crops" | "host_crops" | "detect_only" (introspection for tests / bench)
+        # "fused" | "fused_batch" | "fused_rotated" | "fused_batch_rotated" | "device_crops" | "host_crops" |
+        # "rotated_crops" | "detect_only" (introspection for tests / bench)
         self.last_route = None
 
     # ---- route 1: everything between the image upload and the recogniser network on the device ---------------------
     def _fused_runner(self, batch=False):
         """The PageBatch of the one-page route, or (batch=True) of process_batch's: its crop buffer holds the chunk's
         crops (_BATCH_CROPS_CAP0 rows at first, grown to a power of two when a chunk needs more) instead of cap_boxes
-        per page, and it keeps the buffers of at most two chunk sizes (the full chunk and the last one)."""
+        per page, and it keeps the buffers of at most two chunk sizes (the full chunk and the last one).  With
+        rotated_crops its crop stage is the rectified quad crop, border constant 0 (the border of the per-image route)."""
         det, rec = self.detector, self.recognizer
-        key = (det.device, det.cap_boxes, rec.img_h, rec.img_w, int(self.min_text_size), rec.batch_dtype)
+        crops = "quads" if self.rotated_crops else "rects"
+        key = (det.device, det.cap_boxes, rec.img_h, rec.img_w, int(self.min_text_size), rec.batch_dtype, crops)
         entry = self._runners.get(batch)
         if entry is None or entry[0] != key:
             kw = dict(crops_cap=_BATCH_CROPS_CAP0, max_buffer_sets=2) if batch else {}
             entry = self._runners[batch] = (key, PageBatch(
                 device=det.device.index or 0, params=det._params(sort_reading_order=1),
                 min_text_size=int(self.min_text_size), out_hw=(rec.img_h, rec.img_w), cap_boxes=det.cap_boxes,
-                batch_dtype=rec.batch_dtype, **kw))
+                batch_dtype=rec.batch_dtype, crops=crops, border_mode=0, border_value=0, **kw))
         entry[1].params = det._params(sort_reading_order=1)
         return entry[1]
 
@@ -141,8 +169,11 @@ class Pipeline:
         while True:
             res = runner.run_ragged(score, geo, pages_dev, sync=True, allow_order_overflow=True)
             boxes = self._host_boxes(res, len(imgs))
-            need = sum(int(host_crop_rects(b, im.shape[0], im.shape[1], self.min_text_size)[1].sum())
-                       for b, im in zip(boxes, imgs))
+            if self.rotated_crops:  # a quad makes at most one crop (whether its system is singular is the device's call)
+                need = sum(len(b) for b in boxes)
+            else:
+                need = sum(int(host_crop_rects(b, im.shape[0], im.shape[1], self.min_text_size)[1].sum())
+                           for b, im in zip(boxes, imgs))
             if need <= runner.crops_cap:
                 break
             # the crop list stopped at crops_cap: run the chunk again with room for all of its crops
@@ -161,6 +192,17 @@ class Pipeline:
         words = words_from_boxes(boxes)                         # already in reading order (_pipeline.py:105-123)
         page = Page(blocks=[Block(words=words)])
         rects, valid = host_crop_rects(boxes, img.shape[0], img.shape[1], self.min_text_size)
+        if self.rotated_crops:
+            # rows [page, box, w, h, 0]: boxes in increasing order, each with the patch size the host computes for it
+            w, h, ok = host_patch_sizes(boxes)
+            ok &= (w >= self.min_text_size) & (h >= self.min_text_size)
+            b = crops[:, 1].astype(np.int64)
+            if len(b) and (b[0] < 0 or b[-1] >= len(boxes) or np.any(np.diff(b) <= 0) or not ok[b].all()
+                           or not np.array_equal(crops[:, 2], w[b]) or not np.array_equal(crops[:, 3], h[b])):
+                raise RuntimeError("quad crop list of the device and the word boxes disagree")
+            if not valid.any():  # the per-image route recognises nothing on a page without a crop rectangle
+                return page, None
+            return page, [words[j] for j in b.tolist()]
         if int(valid.sum()) != len(crops) or not np.array_equal(rects[valid], crops[:, 1:]):
             raise RuntimeError("crop list of the device and the word boxes disagree")
         return page, [words[j] for j in np.flatnonzero(valid).tolist()]
@@ -219,9 +261,10 @@ class Pipeline:
                     rects.append(rect)
         return words, (np.stack(rects).astype(np.int32) if rects else np.zeros((0, 4), np.int32))
 
-    def _recognise_rotated(self, image_array, words):
+    def _recognise_rotated(self, image_array, words, page_dev=None):
         """rotated_crops=True: one rectified patch per word quad; words without a patch (smaller than min_text_size on
-        a side, degenerate) are skipped like the reference skips small boxes.  Returns (kept words, results)."""
+        a side, degenerate) are skipped like the reference skips small boxes.  Returns (kept words, results).
+        page_dev: the page already on the device (RGB uint8), used instead of a second upload."""
         rec = self.recognizer
         rgb = TRBA._as_rgb(image_array)
         quads = np.array([w.polygon for w in words], dtype=np.float32).reshape(len(words), -1)[:, :8]
@@ -231,7 +274,8 @@ class Pipeline:
                     if p is not None and min(p.shape[:2]) >= self.min_text_size]
             return [words[i] for i in keep], rec.predict([patches[i] for i in keep])
         torch = rec.torch
-        page_dev = torch.from_numpy(np.ascontiguousarray(rgb)).to(rec.device)
+        if page_dev is None:
+            page_dev = torch.from_numpy(np.ascontiguousarray(rgb)).to(rec.device)
         quads_dev = torch.from_numpy(np.ascontiguousarray(quads)).to(rec.device)
         n = len(words)
         batch = torch.empty((n, 3, rec.img_h, rec.img_w), dtype=rec.batch_dtype, device=rec.device)
@@ -253,7 +297,12 @@ class Pipeline:
     def _finish_from_page(self, page, image_array, profile, page_dev=None):
         """Routes 2 / 3 from a detector's Page: reading order, crop rectangles, recognition, text written back."""
         words, rects = self._ordered_crop_rects(page, *image_array.shape[:2])
-        if words:
+        if words and self.rotated_crops:  # predict's rotated branch, cut from the uploaded page
+            words, results = self._recognise_rotated(image_array, [w for b in page.blocks for w in b.words],
+                                                     page_dev=page_dev)
+            for word, result in zip(words, results):
+                word.text, word.recognition_confidence = _text_and_confidence(result)
+        elif words:
             results = self._recognise(image_array, rects, page_dev=page_dev)
             for word, result in zip(words, results):
                 word.text, word.recognition_confidence = _text_and_confidence(result)
@@ -281,7 +330,7 @@ class Pipeline:
 
     # ---- the reference's public surface ---------------------------------------------------------------------------
     def _fused_ok(self, recognize_text):
-        return (recognize_text and not self.rotated_crops and isinstance(self.detector, EAST)
+        return (recognize_text and isinstance(self.detector, EAST)
                 and isinstance(self.recognizer, TRBA) and self.detector.model is not None
                 and self.recognizer.model is not None and self.detector.device == self.recognizer.device)
 
@@ -289,12 +338,17 @@ class Pipeline:
     def _is_rgb_u8(img):
         return isinstance(img, np.ndarray) and img.ndim == 3 and img.shape[2] == 3 and img.dtype == np.uint8
 
+    def _fused_image_ok(self, img):
+        """an image the fused route takes: uint8 RGB and, for rotated crops, at most 32767 pixels on a side (larger
+        pages keep the per-image route, which raises)"""
+        return self._is_rgb_u8(img) and (not self.rotated_crops or max(img.shape[:2]) <= 32767)
+
     def predict(self, image, recognize_text=True, vis=False, profile=False):
         t_start = time.time()
         if self._fused_ok(recognize_text):
             img = read_image(image)
-            if self._is_rgb_u8(img):
-                self.last_route = "fused"
+            if self._fused_image_ok(img):
+                self.last_route = "fused_rotated" if self.rotated_crops else "fused"
                 page = self._predict_fused(img, profile)
                 if profile:
                     print(f"Pipeline total: {time.time() - t_start:.3f}s")
@@ -340,7 +394,8 @@ class Pipeline:
         """_pipeline.py:178-191 (whose body calls a `self.process` that does not exist in the reference, so it can only
         raise AttributeError there): the evident intent, one predict per image, Pages only.
 
-        On the fused route (this package's EAST and TRBA, recognize_text, no rotated_crops) with every image an
+        On the fused route (this package's EAST and TRBA, recognize_text; "fused_batch_rotated" with rotated_crops,
+        whose images must also be at most 32767 pixels on a side) with every image an
         (H, W, 3) uint8 RGB array, the images are processed in chunks of at most `max_pages` (which bounds the memory of
         the (P, 3, T, T) network input): one upload buffer, one detector-input launch, one detector network call and one
         page batch per chunk, and recogniser batches of rec.batch_size crops that may span pages (last_route
@@ -358,7 +413,7 @@ class Pipeline:
         for i in range(0, len(images), max_pages):
             chunk = images[i:i + max_pages]
             imgs = [read_image(im) for im in chunk] if fused else None  # read chunk by chunk, not all at once
-            if fused and all(self._is_rgb_u8(im) for im in imgs):
+            if fused and all(self._fused_image_ok(im) for im in imgs):
                 results.extend(self._predict_fused_batch(imgs, profile))
                 routes.add("fused_batch")
                 continue
@@ -367,7 +422,7 @@ class Pipeline:
                 results.append(res[0] if vis else res)
                 routes.add(self.last_route)
         if routes == {"fused_batch"}:
-            self.last_route = "fused_batch"
+            self.last_route = "fused_batch_rotated" if self.rotated_crops else "fused_batch"
         return results
 
     def get_text(self, page):
