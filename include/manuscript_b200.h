@@ -407,6 +407,46 @@ MS_API int ms_page_batch_ragged_host_ex(ms_ctx *ctx, const float *score, const f
                                  int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
                                  void *batch_host, int batch_dtype, void **batch_dev_out, int32_t *flags);
 
+/* ---- baseline-JPEG decode on the device (an EXTENSION: the caller side of the path, like the detector input) ----
+ * The decoded page is cv2.cvtColor(cv2.imread(path), cv2.COLOR_BGR2RGB), equal in every byte: libjpeg-turbo's Huffman
+ * decode, ISLOW IDCT, fancy upsampling and YCbCr -> RGB restated in integer arithmetic (DESIGN 4.5).  The device takes
+ * SOF0 / SOF1 8-bit files with one scan holding every component, grayscale or YCbCr with chroma 1x1 and luma 1x1,
+ * 2x1, 1x2, 2x2 or 4x1, any restart interval, and no EXIF orientation other than 1.  Everything else is decoded by the
+ * caller on the host (reason codes below). */
+#define MS_JPEG_OK 0                 /* decoded on the device                                                  */
+#define MS_JPEG_NOT_JPEG 1           /* no SOI, a truncated or malformed header                                 */
+#define MS_JPEG_PROGRESSIVE 2        /* progressive coding                                                     */
+#define MS_JPEG_UNSUPPORTED_CODING 3 /* arithmetic, lossless or hierarchical coding, or not 8-bit              */
+#define MS_JPEG_COLOR 4              /* not 1 or 3 components, or 3 components that are not YCbCr (Adobe, RGB)  */
+#define MS_JPEG_SAMPLING 5           /* a sampling other than the supported ones                                */
+#define MS_JPEG_ORIENTATION 6        /* an EXIF orientation other than 1 (cv2.imread rotates the image)         */
+#define MS_JPEG_SCAN 7               /* a scan that does not hold every component, a missing table, DNL, > 256 MB */
+#define MS_JPEG_BAD_ENTROPY 16       /* ms_jpeg_decode_batch only: the entropy-coded data did not decode on the
+                                        device (truncated, an invalid code, a wrong restart marker, MCUs missing or
+                                        extra, a second scan); libjpeg's warnings-and-grey result is the host's */
+
+typedef struct ms_jpeg_info {
+    int32_t height, width;   /* the size cv2.imread returns (transposed for EXIF orientations 5..8) */
+    int32_t components;      /* of the frame header                                                 */
+    int32_t device;          /* 1: ms_jpeg_decode_batch decodes the file on the device              */
+    int32_t reason;          /* MS_JPEG_* (MS_JPEG_OK when device == 1)                            */
+    int32_t luma_h, luma_v;  /* sampling factors of the first component                           */
+    int32_t restart_interval; /* MCUs per restart interval, 0 = none                              */
+} ms_jpeg_info;
+
+/* Parses the markers of one file in host memory up to its first scan; needs no device.  MS_OK with out->device == 0 and
+ * a reason for a file that is not a JPEG the device takes; MS_ERR_INVALID only for NULL arguments. */
+MS_API int ms_jpeg_inspect_host(const uint8_t *data, int64_t size, ms_jpeg_info *out);
+
+/* Decodes n files (files[i]: size sizes[i] bytes of host memory) into out_pages[i], a device buffer of (h_i, w_i, 3) u8
+ * RGB of the size ms_jpeg_inspect_host reports.  The compressed bytes go to the device through one pinned staging
+ * buffer; scratch comes from the context's arena.  out_status[i] (host int32) is MS_JPEG_OK for a page decoded on the
+ * device, otherwise a reason code: the page is not written and the caller decodes the file on the host.  The call is
+ * stream-ordered: out_status is written by a copy ordered after the decode on `stream`, so synchronise the stream
+ * before reading it.  out_pages[i] may be NULL for a file the caller does not want decoded (status MS_JPEG_SCAN). */
+MS_API int ms_jpeg_decode_batch(ms_ctx *ctx, const uint8_t *const *files, const int64_t *sizes, int n,
+                                uint8_t *const *out_pages, int32_t *out_status, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

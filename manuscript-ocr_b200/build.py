@@ -14,7 +14,7 @@ CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 OUT = os.path.join(HERE, "manuscript_b200", "libmanuscript_b200.so")
 SOURCES = ["api.cu", "decode.cu", "sort.cu", "lanms.cu", "boxes.cu", "reading_order.cu", "crop.cu",
-           "quadcrop.cu", "tps.cu", "np_sum_test.cu"]
+           "quadcrop.cu", "tps.cu", "np_sum_test.cu", "jpeg.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

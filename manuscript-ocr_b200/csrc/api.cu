@@ -107,6 +107,8 @@ extern "C" int ms_create(int device, ms_ctx **out)
         rc = ms_check_cuda(cudaEventCreateWithFlags(&c->split_ev[i], cudaEventDisableTiming), "cudaEventCreate");
     for (int i = 0; i < 2 && rc == MS_OK; i++)
         rc = ms_check_cuda(cudaEventCreateWithFlags(&c->chunk_ev[i], cudaEventDisableTiming), "cudaEventCreate");
+    if (rc == MS_OK)
+        rc = ms_check_cuda(cudaEventCreateWithFlags(&c->jpeg_ev, cudaEventDisableTiming), "cudaEventCreate");
     if (rc == MS_OK) {
         c->pinned_bytes = 1 << 20;
         rc = ms_check_cuda(cudaMallocHost((void **)&c->pinned, c->pinned_bytes), "cudaMallocHost");
@@ -148,6 +150,11 @@ extern "C" void ms_destroy(ms_ctx *ctx)
     if (ctx->arena) cudaFree(ctx->arena);
     if (ctx->stage) cudaFree(ctx->stage);
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
+    if (ctx->jpeg_ev) {
+        cudaEventSynchronize(ctx->jpeg_ev);
+        cudaEventDestroy(ctx->jpeg_ev);
+    }
+    if (ctx->jpeg_pinned) cudaFreeHost(ctx->jpeg_pinned);
     delete ctx;
 }
 
@@ -1757,4 +1764,22 @@ extern "C" int ms_page_batch_ragged_host(ms_ctx *ctx, const float *score, const 
     return ms_page_batch_ragged_host_ex(ctx, score, geo, pages, page_hw, n_pages, map_h, map_w, p, min_text_size, out_h,
                                         out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops,
                                         batch_f32_host, MS_DTYPE_F32, reinterpret_cast<void **>(batch_dev_out), flags);
+}
+
+// ---- baseline-JPEG decode (jpeg.cu) ---------------------------------------------------------------------------------
+extern "C" int ms_jpeg_decode_batch(ms_ctx *ctx, const uint8_t *const *files, const int64_t *sizes, int n,
+                                    uint8_t *const *out_pages, int32_t *out_status, void *stream)
+{
+    MS_CTX(ctx);
+    if (n < 0 || (n > 0 && (!files || !sizes || !out_pages || !out_status))) {
+        ms_set_error("ms_jpeg_decode_batch: bad arguments");
+        return MS_ERR_INVALID;
+    }
+    if (n == 0) return MS_OK;
+    for (int i = 0; i < n; i++)
+        if (sizes[i] < 0) {
+            ms_set_error("ms_jpeg_decode_batch: negative size of file %d", i);
+            return MS_ERR_INVALID;
+        }
+    return ms_jpeg_decode_batch_impl(ctx, files, sizes, n, out_pages, out_status, (cudaStream_t)stream);
 }

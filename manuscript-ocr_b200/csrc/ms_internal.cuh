@@ -115,6 +115,10 @@ struct ms_ctx {
     cudaStream_t crop_stream;
     int quad_no_stage;            // MS_B200_QUAD_NO_STAGE=1: rotated crops by the generic kernel only (A/B runs, tests)
     int ro_force_large;           // MS_B200_RO_FORCE_LARGE=1: every page takes the large-page reading-order kernel (tests)
+    char *jpeg_pinned;            // pinned staging of ms_jpeg_decode_batch (descriptors + entropy-coded bytes), grown
+    size_t jpeg_pinned_bytes;     // on demand; jpeg_ev marks the end of the last copy out of it
+    cudaEvent_t jpeg_ev;
+    int jpeg_pending;
     int busy;                     // 1 while a thread is inside an entry point (atomic test-and-set): a context owns ONE
                                   // scratch arena, so a second thread entering gets MS_ERR_INVALID instead of corrupting it
 };
@@ -298,6 +302,10 @@ int msk_quad_crop_rows(ms_ctx *ctx, const float *boxes, int cap_boxes, int n_pag
                        cudaStream_t st);
 int msk_quad_warp(ms_ctx *ctx, const uint8_t *page, int img_h, int img_w, const float *quad_dev, int border_mode,
                   int border_value, uint8_t *patch_dev, size_t patch_cap, int *w, int *h, ms_bump bump, cudaStream_t st);
+
+// jpeg.cu: ms_jpeg_decode_batch without the entry guard
+int ms_jpeg_decode_batch_impl(ms_ctx *ctx, const uint8_t *const *files, const int64_t *sizes, int n,
+                              uint8_t *const *out_pages, int32_t *out_status, cudaStream_t st);
 
 // ---- device geometry: lanms.py:7-130 in float64, no fused multiply-add ------------------------------
 #define MS_MAXV 20  // lanms.py:34

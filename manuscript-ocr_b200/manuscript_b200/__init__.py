@@ -7,6 +7,10 @@ kernels through the C ABI.  There is no CPU fallback: importing works anywhere, 
 needs libmanuscript_b200.so and a B200.
 """
 from ._cabi import (  # noqa: F401
+    MS_JPEG_BAD_ENTROPY,
+    MS_JPEG_NOT_JPEG,
+    MS_JPEG_ORIENTATION,
+    MS_JPEG_PROGRESSIVE,
     CABIError,
     Context,
     EastParams,
@@ -30,7 +34,7 @@ from .ops import (  # noqa: F401
     word_rects,
 )
 from .batch import PageBatch, PageBatchResult, shard_pages  # noqa: F401
-from .east import EAST  # noqa: F401
+from .east import EAST, JpegInfo, jpeg_inspect  # noqa: F401
 from .imaging import read_image, visualize_page  # noqa: F401
 from .pipeline import Pipeline  # noqa: F401
 from .reading_order import (  # noqa: F401

@@ -22,6 +22,16 @@ MS_FLAG_INDEX_ERROR = 2
 MS_FLAG_EDGE_OVERFLOW = 4
 MS_FLAG_ORDER_OVERFLOW = 8
 
+MS_JPEG_OK = 0
+MS_JPEG_NOT_JPEG = 1
+MS_JPEG_PROGRESSIVE = 2
+MS_JPEG_UNSUPPORTED_CODING = 3
+MS_JPEG_COLOR = 4
+MS_JPEG_SAMPLING = 5
+MS_JPEG_ORIENTATION = 6
+MS_JPEG_SCAN = 7
+MS_JPEG_BAD_ENTROPY = 16
+
 MS_DTYPE_F32 = 0
 MS_DTYPE_F16 = 1
 MS_DTYPE_BF16 = 2
@@ -136,6 +146,9 @@ SIGNATURES = {
                                  _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
     "ms_page_batch_ragged_quads": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i, _i, _i,
                                         _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
+    # EXTENSION: baseline-JPEG decode on the device (ms_jpeg_info *, host files -> device pages)
+    "ms_jpeg_inspect_host": (_i, [_vp, _i64, _vp]),
+    "ms_jpeg_decode_batch": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp]),
 }
 
 

@@ -19,7 +19,7 @@ from pathlib import Path
 
 import numpy as np
 
-from ._cabi import MS_FLAG_EDGE_OVERFLOW, EastParams, batch_dtype_code, check
+from ._cabi import MS_FLAG_EDGE_OVERFLOW, EastParams, batch_dtype_code, check, load_library
 from .batch import PageBatch, _raise_for_flags
 from .imaging import read_image, visualize_page
 from .reading_order import reorder_words
@@ -29,6 +29,26 @@ DEFAULT_WEIGHTS = Path.home() / ".manuscript" / "east" / "east_quad_23_05.pth"  
 
 
 _WORD_FIELDS = frozenset(("polygon", "detection_confidence"))
+
+
+class JpegInfo(C.Structure):
+    """ms_jpeg_info: what ms_jpeg_inspect_host reads from a file's markers."""
+
+    _fields_ = [("height", C.c_int32), ("width", C.c_int32), ("components", C.c_int32), ("device", C.c_int32),
+                ("reason", C.c_int32), ("luma_h", C.c_int32), ("luma_v", C.c_int32),
+                ("restart_interval", C.c_int32)]
+
+
+def jpeg_inspect(data):
+    """bytes of a file -> JpegInfo (host only, no device needed): the size cv2.imread returns and whether
+    ms_jpeg_decode_batch decodes it on the device (reason: MS_JPEG_* code when not)."""
+    info = JpegInfo()
+    check(load_library().ms_jpeg_inspect_host(data, len(data), C.byref(info)))
+    return info
+
+
+def _is_path(source):
+    return isinstance(source, (str, Path))
 
 
 def words_from_boxes(boxes):
@@ -90,6 +110,7 @@ class EAST:
         self._batch_buf = {}  # tuple of image shapes -> (device buffer, page views): see upload_batch
         self._tables = {}     # page views -> their device pointer / size tables
         self._inputs_buf = None
+        self.device_decoded = []  # per page of the last upload / upload_batch: decoded from its JPEG on the device
 
     @classmethod
     def from_pretrained(cls, weights_path=None, **kwargs):
@@ -165,50 +186,101 @@ class EAST:
         return out[: int(m[2])].cpu().numpy()
 
     # ---- image -> device, device image -> network input -> maps (nothing returns to the host) --------------------
-    def upload(self, img):
-        """(H, W, 3) uint8 RGB host array -> the same image on the device, in a buffer this detector keeps per image
-        size.  This is the ONE host-to-device copy of pixels per page: the detector input and the word crops are both
-        made from it."""
+    def _sources(self, images):
+        """Host side of an upload: per source either ("jpeg", file bytes, (h, w, 3)) for a JPEG file the device decodes
+        (ms_jpeg_inspect_host) or ("array", contiguous (H, W, 3) uint8 RGB array, shape); other paths go through
+        read_image, as they always have."""
+        out = []
+        for src in images:
+            if _is_path(src):
+                data = Path(src).read_bytes() if Path(src).is_file() else b""
+                info = jpeg_inspect(data) if data else None
+                if info is not None and info.device:
+                    out.append(("jpeg", data, (int(info.height), int(info.width), 3)))
+                    continue
+                src = read_image(src)
+            a = np.asarray(src)
+            if a.ndim != 3 or a.shape[2] != 3 or a.dtype != np.uint8:
+                raise ValueError(f"EAST expects (H, W, 3) uint8 RGB images, got shape {a.shape} dtype {a.dtype}")
+            a = np.ascontiguousarray(a)
+            out.append(("array", a, a.shape))
+        return out
+
+    def _decode_jpegs(self, jobs):
+        """jobs: (file bytes, device view, path) -> every file decoded into its view (ms_jpeg_decode_batch, one call);
+        a file the device does not finish is read with read_image and copied.  Returns the per-job device mask."""
         torch = self.torch
-        a = np.asarray(img)
-        if a.ndim != 3 or a.shape[2] != 3 or a.dtype != np.uint8:
-            raise ValueError(f"EAST expects an (H, W, 3) uint8 RGB image, got shape {a.shape} dtype {a.dtype}")
-        a = np.ascontiguousarray(a)
-        buf = self._page_buf.get(a.shape[:2])
+        if not jobs:
+            return []
+        n = len(jobs)
+        keep = [C.c_char_p(d) for d, _, _ in jobs]
+        files = (C.c_void_p * n)(*[C.cast(k, C.c_void_p).value for k in keep])
+        sizes = (C.c_int64 * n)(*[len(d) for d, _, _ in jobs])
+        outs = (C.c_void_p * n)(*[v.data_ptr() for _, v, _ in jobs])
+        status = torch.empty((n,), dtype=torch.int32, pin_memory=True)
+        stream = torch.cuda.current_stream(self.device)
+        with torch.cuda.device(self.device):
+            check(self._runner.ctx.lib.ms_jpeg_decode_batch(self._runner.ctx.handle, files, sizes, n, outs,
+                                                            status.data_ptr(), C.c_void_p(stream.cuda_stream)))
+        stream.synchronize()  # the statuses
+        ok = (status.numpy() == 0).tolist()
+        for good, (_, v, path) in zip(ok, jobs):
+            if not good:  # the host decode: libjpeg's own result for data the device does not take
+                a = np.ascontiguousarray(read_image(path))
+                if a.shape != tuple(v.shape):
+                    raise ValueError(f"{path}: the decoded image is {a.shape}, its header says {tuple(v.shape)}")
+                v.copy_(torch.from_numpy(a), non_blocking=True)
+        return ok
+
+    def upload(self, img):
+        """(H, W, 3) uint8 RGB host array, or a path -> the same image on the device, in a buffer this detector keeps per
+        image size.  This is the ONE host-to-device copy of pixels per page: the detector input and the word crops are both
+        made from it.  A JPEG file the device takes (ms_jpeg_inspect_host) crosses PCIe compressed and is decoded there,
+        bit for bit what read_image gives; self.device_decoded is [True] then, [False] for any other source."""
+        torch = self.torch
+        (kind, a, shape), = self._sources([img])
+        buf = self._page_buf.get(shape[:2])
         if buf is None:
             if len(self._page_buf) >= 4:
                 self._page_buf.clear()
-            buf = self._page_buf[a.shape[:2]] = torch.empty(a.shape, dtype=torch.uint8, device=self.device)
-        buf.copy_(torch.from_numpy(a), non_blocking=True)
+            buf = self._page_buf[shape[:2]] = torch.empty(shape, dtype=torch.uint8, device=self.device)
+        if kind == "jpeg":
+            self.device_decoded = self._decode_jpegs([(a, buf, img)])
+        else:
+            buf.copy_(torch.from_numpy(a), non_blocking=True)
+            self.device_decoded = [False]
         return buf
 
     def upload_batch(self, images):
-        """List of (H_i, W_i, 3) uint8 RGB host arrays -> list of device views of the same images, one host-to-device copy
-        of pixels per page.  All pages live in one device buffer, each at a 16-byte-aligned offset (the crop kernels stage
-        such pages' rows by TMA); the buffer is kept per list of shapes, so a serving loop over batches of the same shapes
-        reuses the same addresses and the page batch replays its CUDA graph."""
+        """List of (H_i, W_i, 3) uint8 RGB host arrays or paths -> list of device views of the same images, one
+        host-to-device copy of pixels per page.  All pages live in one device buffer, each at a 16-byte-aligned offset (the
+        crop kernels stage such pages' rows by TMA); the buffer is kept per list of shapes, so a serving loop over batches
+        of the same shapes reuses the same addresses and the page batch replays its CUDA graph.  JPEG files the device
+        takes are decoded into their views by one ms_jpeg_decode_batch call (self.device_decoded: per page, True for
+        those); every other source is read with read_image and copied."""
         torch = self.torch
-        arrs = []
-        for img in images:
-            a = np.asarray(img)
-            if a.ndim != 3 or a.shape[2] != 3 or a.dtype != np.uint8:
-                raise ValueError(f"EAST expects (H, W, 3) uint8 RGB images, got shape {a.shape} dtype {a.dtype}")
-            arrs.append(np.ascontiguousarray(a))
-        key = tuple(a.shape[:2] for a in arrs)
+        srcs = self._sources(images)
+        key = tuple(shape[:2] for _, _, shape in srcs)
         entry = self._batch_buf.get(key)
         if entry is None:
             offs, total = [], 0
-            for a in arrs:
+            for _, _, shape in srcs:
                 offs.append(total)
-                total += (a.nbytes + 15) & ~15
+                total += (int(np.prod(shape)) + 15) & ~15
             if len(self._batch_buf) >= 4:
                 self._batch_buf.clear()
                 self._tables.clear()
             buf = torch.empty((max(total, 16),), dtype=torch.uint8, device=self.device)
-            views = [buf[o:o + a.nbytes].view(a.shape) for o, a in zip(offs, arrs)]
+            views = [buf[o:o + int(np.prod(shape))].view(shape) for o, (_, _, shape) in zip(offs, srcs)]
             entry = self._batch_buf[key] = (buf, views)
-        for v, a in zip(entry[1], arrs):
-            v.copy_(torch.from_numpy(a), non_blocking=True)
+        jobs, decoded = [], [False] * len(srcs)
+        for i, (v, (kind, a, _)) in enumerate(zip(entry[1], srcs)):
+            if kind == "jpeg":
+                jobs.append((a, v, images[i]))
+            else:
+                v.copy_(torch.from_numpy(a), non_blocking=True)
+        ok = iter(self._decode_jpegs(jobs))
+        self.device_decoded = [next(ok) if kind == "jpeg" else False for kind, _, _ in srcs]
         return list(entry[1])
 
     def _page_tables(self, pages_dev):
@@ -287,15 +359,21 @@ class EAST:
         return Page(blocks=[Block(words=words)])
 
     def predict(self, img_or_path, vis=False, profile=False, return_maps=False, sort_reading_order=False):
-        """Same contract as the reference's EAST.predict: dict with "page", "vis_image", "score_map", "geo_map"."""
-        img = read_image(img_or_path)
+        """Same contract as the reference's EAST.predict: dict with "page", "vis_image", "score_map", "geo_map".  A path
+        is decoded by upload (on the device for the JPEG files it takes); vis=True downloads that page to draw on."""
         t0 = time.time()
-        score, geo = self.maps_from_device_page(self.upload(img))
+        if _is_path(img_or_path):
+            page_dev = self.upload(img_or_path)
+            img = page_dev.cpu().numpy() if vis else page_dev
+        else:
+            img = read_image(img_or_path)
+            page_dev = self.upload(img)
+        score, geo = self.maps_from_device_page(page_dev)
         if profile:
             self.torch.cuda.synchronize()
             print(f"  Model inference: {time.time() - t0:.3f}s")
         t0 = time.time()
-        page = self.predict_from_maps(score, geo, img.shape[:2], sort_reading_order=sort_reading_order)
+        page = self.predict_from_maps(score, geo, tuple(img.shape[:2]), sort_reading_order=sort_reading_order)
         if profile:
             print(f"  Decode + NMS + box filters (device): {time.time() - t0:.3f}s")
             print(f"    Boxes after NMS: {sum(len(b.words) for b in page.blocks)}")

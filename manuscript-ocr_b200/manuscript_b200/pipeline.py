@@ -26,6 +26,7 @@ With this package's TRBA, the device routes (and rotated_crops) write the recogn
 """
 import ctypes as C
 import time
+from pathlib import Path
 
 import numpy as np
 
@@ -151,19 +152,23 @@ class Pipeline:
         boxes = res.boxes[:n_pages, :kmax].cpu().numpy()         # D2H: P x K_max x 36 bytes
         return [boxes[p, :int(counts[p])] for p in range(n_pages)]
 
-    def _predict_fused(self, img, profile):
+    def _predict_fused(self, img, profile, page_dev=None):
+        """img: the page array, or (a path's route) its device copy, of which only the shape is read"""
         t0 = time.time()
-        page_dev = self.detector.upload(img)                    # the one H2D copy of pixels
+        if page_dev is None:
+            page_dev = self.detector.upload(img)                # the one H2D copy of pixels
         score, geo = self.detector.maps_from_device_page(page_dev)  # network input + maps stay on the device
         res = self._fused_runner().run_ragged(score[None] if score.dim() == 2 else score, geo[None], [page_dev],
                                               sync=True, allow_order_overflow=True)
         return self._fused_pages(res, self._host_boxes(res, 1), [img], [page_dev], t0, profile)[0]
 
-    def _predict_fused_batch(self, imgs, profile):
+    def _predict_fused_batch(self, imgs, profile, pages_dev=None):
         """The fused route for a chunk of pages: one upload buffer, one detector-input launch, one network call, one
-        page batch, and recogniser batches cut from the one crop batch."""
+        page batch, and recogniser batches cut from the one crop batch.  imgs: page arrays, or where a page came from a
+        file, its device copy (pages_dev given: the chunk is uploaded already), of which only the shape is read."""
         t0 = time.time()
-        pages_dev = self.detector.upload_batch(imgs)            # one H2D copy of pixels per page
+        if pages_dev is None:
+            pages_dev = self.detector.upload_batch(imgs)        # one H2D copy of pixels per page
         score, geo = self.detector.maps_from_device_pages(pages_dev)
         runner = self._fused_runner(batch=True)
         while True:
@@ -266,7 +271,8 @@ class Pipeline:
         a side, degenerate) are skipped like the reference skips small boxes.  Returns (kept words, results).
         page_dev: the page already on the device (RGB uint8), used instead of a second upload."""
         rec = self.recognizer
-        rgb = TRBA._as_rgb(image_array)
+        # a page that came from a file exists only on the device (image_array is that copy): its shape is all that is read
+        rgb = image_array if (page_dev is not None and image_array is page_dev) else TRBA._as_rgb(image_array)
         quads = np.array([w.polygon for w in words], dtype=np.float32).reshape(len(words), -1)[:, :8]
         if not isinstance(rec, TRBA):
             patches = [ops.warp_quad(rgb, q) for q in quads]
@@ -343,9 +349,27 @@ class Pipeline:
         pages keep the per-image route, which raises)"""
         return self._is_rgb_u8(img) and (not self.rotated_crops or max(img.shape[:2]) <= 32767)
 
+    def _fused_size_ok(self, page_dev):
+        return not self.rotated_crops or max(page_dev.shape[:2]) <= 32767
+
+    @staticmethod
+    def _is_path(image):
+        return isinstance(image, (str, Path))
+
     def predict(self, image, recognize_text=True, vis=False, profile=False):
         t_start = time.time()
-        if self._fused_ok(recognize_text):
+        if self._fused_ok(recognize_text) and self._is_path(image):
+            # a file: decoded into the detector's page buffer (on the device for the JPEG files it takes); no host array
+            page_dev = self.detector.upload(image)
+            if self._fused_size_ok(page_dev):
+                self.last_route = "fused_rotated" if self.rotated_crops else "fused"
+                page = self._predict_fused(page_dev, profile, page_dev=page_dev)
+                if profile:
+                    print(f"Pipeline total: {time.time() - t_start:.3f}s")
+                if vis:  # _pipeline.py:166-174, drawn on the downloaded page
+                    return page, visualize_page(page_dev.cpu().numpy(), page, show_order=True)
+                return page
+        elif self._fused_ok(recognize_text):
             img = read_image(image)
             if self._fused_image_ok(img):
                 self.last_route = "fused_rotated" if self.rotated_crops else "fused"
@@ -412,6 +436,16 @@ class Pipeline:
         results, routes = [], set()
         for i in range(0, len(images), max_pages):
             chunk = images[i:i + max_pages]
+            if fused and any(self._is_path(im) for im in chunk):
+                # files are decoded into the chunk's page buffer (JPEG on the device); only the arrays live on the host
+                srcs = [im if self._is_path(im) else read_image(im) for im in chunk]
+                if all(self._is_path(im) or self._fused_image_ok(im) for im in srcs):
+                    pages_dev = self.detector.upload_batch(srcs)
+                    if all(self._fused_size_ok(pg) for pg in pages_dev):
+                        imgs = [pg if self._is_path(im) else im for im, pg in zip(srcs, pages_dev)]
+                        results.extend(self._predict_fused_batch(imgs, profile, pages_dev=pages_dev))
+                        routes.add("fused_batch")
+                        continue
             imgs = [read_image(im) for im in chunk] if fused else None  # read chunk by chunk, not all at once
             if fused and all(self._fused_image_ok(im) for im in imgs):
                 results.extend(self._predict_fused_batch(imgs, profile))
