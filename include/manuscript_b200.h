@@ -370,6 +370,54 @@ MS_API int ms_page_batch_ragged_quads(ms_ctx *ctx, const float *score, const flo
                                       int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
                                       void *batch, int batch_dtype, uint8_t *canvas_u8, int32_t *flags, void *stream);
 
+/* ---- detector maps as the network left them (an EXTENSION: the caller side of the path) --------------------------
+ * One descriptor for the two maps of a batch: both of one element type, each at its own element strides, so a 16-bit
+ * network output or a channels_last geometry (strides (8*H*W, 1, 8*W, 8)) is read in place.  Every value is widened to
+ * float32 at its load, which is exact: every result equals, bit for bit, that of the same call on the float32 dense
+ * copies of the maps (torch's .float().contiguous(), NaN payloads included).  Dense float32 maps are one case: the
+ * entry points without _maps take exactly that descriptor.  A NULL descriptor or map pointer, an unknown dtype or a
+ * negative stride is MS_ERR_INVALID. */
+typedef struct ms_maps {
+    const void *score;          /* (n_pages, map_h, map_w) */
+    const void *geo;            /* (n_pages, 8, map_h, map_w) */
+    int32_t dtype;              /* MS_DTYPE_F32 / MS_DTYPE_F16 / MS_DTYPE_BF16, both maps */
+    int64_t score_strides[3];   /* page, row, column -- in elements, >= 0 */
+    int64_t geo_strides[4];     /* page, channel, row, column -- in elements, >= 0 */
+} ms_maps;
+
+/* ms_decode_quads on the maps of *maps. */
+MS_API int ms_decode_quads_maps(ms_ctx *ctx, const ms_maps *maps, int n_pages, int map_h, int map_w,
+                                float score_thresh, double scale, int quantization, float *quads_out, int cap_per_page,
+                                int32_t *counts, int32_t *flags, void *stream);
+/* ms_page_batch_ex on the maps of *maps.  The map dtype and strides are part of the call's identity for the CUDA-graph
+ * cache; dense float32 maps give the call (and the graph) of ms_page_batch_ex. */
+MS_API int ms_page_batch_maps(ms_ctx *ctx, const ms_maps *maps, const uint8_t *pages, int n_pages, int map_h,
+                              int map_w, int img_h, int img_w, const ms_east_params *p, int min_text_size, int out_h,
+                              int out_w, int cap_boxes, float *boxes_out, int32_t *box_counts, int32_t *crops_out,
+                              int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                              int32_t *flags, void *stream);
+/* ms_page_batch_ragged_ex on the maps of *maps. */
+MS_API int ms_page_batch_ragged_maps(ms_ctx *ctx, const ms_maps *maps, const uint8_t *const *page_ptrs,
+                                     const int32_t *page_hw, int n_pages, int map_h, int map_w, const ms_east_params *p,
+                                     int min_text_size, int out_h, int out_w, int cap_boxes, float *boxes_out,
+                                     int32_t *box_counts, int32_t *crops_out, int64_t crops_cap, int32_t *n_crops,
+                                     void *batch, int batch_dtype, uint8_t *canvas_u8, int32_t *flags, void *stream);
+/* ms_page_batch_quads on the maps of *maps. */
+MS_API int ms_page_batch_quads_maps(ms_ctx *ctx, const ms_maps *maps, const uint8_t *pages, int n_pages, int map_h,
+                                    int map_w, int img_h, int img_w, const ms_east_params *p, int min_text_size,
+                                    int border_mode, int border_value, int out_h, int out_w, int cap_boxes,
+                                    float *boxes_out, int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
+                                    int32_t *n_crops, void *batch, int batch_dtype, uint8_t *canvas_u8, int32_t *flags,
+                                    void *stream);
+/* ms_page_batch_ragged_quads on the maps of *maps. */
+MS_API int ms_page_batch_ragged_quads_maps(ms_ctx *ctx, const ms_maps *maps, const uint8_t *const *page_ptrs,
+                                           const int32_t *page_hw, int n_pages, int map_h, int map_w,
+                                           const ms_east_params *p, int min_text_size, int border_mode,
+                                           int border_value, int out_h, int out_w, int cap_boxes, float *boxes_out,
+                                           int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
+                                           int32_t *n_crops, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                                           int32_t *flags, void *stream);
+
 /* Same path with HOST buffers (pinned or pageable; `score` / `geo` may also be DEVICE pointers of this context's
  * device -- maps a detector left on the GPU are used in place and only the page images cross PCIe): H2D of maps + pages, the batch, D2H of boxes,
  * counts, crop list and (optionally, if batch_f32_host != NULL) the crop batch.  Of boxes_out (n_pages*cap_boxes,9)

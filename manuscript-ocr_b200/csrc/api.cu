@@ -341,21 +341,56 @@ static int flags_to_rc(int32_t f, const char *where)
 // =========================================================================================================
 // device entry points
 // =========================================================================================================
-extern "C" int ms_decode_quads(ms_ctx *ctx, const float *score, const float *geo, int n_pages, int map_h, int map_w,
-                               float score_thresh, double scale, int quantization, float *quads_out, int cap_per_page,
-                               int32_t *counts, int32_t *flags, void *stream)
+// An ms_maps descriptor: what can be checked before the page count (a NULL descriptor, an unknown dtype, a negative
+// stride), then, for a call with pages, its map pointers.
+static int maps_desc_ok(const ms_maps *m, const char *who)
+{
+    if (!m) {
+        ms_set_error("%s: maps is NULL", who);
+        return MS_ERR_INVALID;
+    }
+    if (ms_dtype_bytes(m->dtype) == 0) {
+        ms_set_error("%s: unknown map dtype %d", who, (int)m->dtype);
+        return MS_ERR_INVALID;
+    }
+    for (int i = 0; i < 3; i++)
+        if (m->score_strides[i] < 0) {
+            ms_set_error("%s: negative score stride", who);
+            return MS_ERR_INVALID;
+        }
+    for (int i = 0; i < 4; i++)
+        if (m->geo_strides[i] < 0) {
+            ms_set_error("%s: negative geometry stride", who);
+            return MS_ERR_INVALID;
+        }
+    return MS_OK;
+}
+
+extern "C" int ms_decode_quads_maps(ms_ctx *ctx, const ms_maps *maps, int n_pages, int map_h, int map_w,
+                                    float score_thresh, double scale, int quantization, float *quads_out,
+                                    int cap_per_page, int32_t *counts, int32_t *flags, void *stream)
 {
     MS_CTX(ctx);
+    MS_TRY(maps_desc_ok(maps, "ms_decode_quads"));
     if (n_pages <= 0) return MS_OK;
-    if (!score || !geo || !quads_out || !counts || !flags) {
+    if (!maps->score || !maps->geo || !quads_out || !counts || !flags) {
         ms_set_error("ms_decode_quads: NULL pointer");
         return MS_ERR_INVALID;
     }
     if (quantization < 1) quantization = 1;  // utils.py:347 only quantises when > 1
     ms_bump bump;
     MS_TRY(arena_bump(ctx, msk_decode_scratch(n_pages, map_h, map_w, quantization), bump));
-    return msk_decode(ctx, score, geo, n_pages, map_h, map_w, score_thresh, scale, quantization, quads_out,
-                      cap_per_page, counts, flags, bump, (cudaStream_t)stream);
+    return msk_decode(ctx, *maps, n_pages, map_h, map_w, score_thresh, scale, quantization, quads_out, cap_per_page,
+                      counts, flags, bump, (cudaStream_t)stream);
+}
+
+extern "C" int ms_decode_quads(ms_ctx *ctx, const float *score, const float *geo, int n_pages, int map_h, int map_w,
+                               float score_thresh, double scale, int quantization, float *quads_out, int cap_per_page,
+                               int32_t *counts, int32_t *flags, void *stream)
+{
+    const ms_maps m = ms_dense_maps(score, geo, map_h, map_w, map_h, 8);
+    return ms_decode_quads_maps(ctx, &m, n_pages, map_h, map_w, score_thresh, scale, quantization, quads_out,
+                                cap_per_page, counts, flags, stream);
 }
 
 extern "C" int ms_decode_rbox(ms_ctx *ctx, const float *score, const float *geo5, int n_pages, int map_h, int map_w,
@@ -371,8 +406,8 @@ extern "C" int ms_decode_rbox(ms_ctx *ctx, const float *score, const float *geo5
     if (quantization < 1) quantization = 1;
     ms_bump bump;
     MS_TRY(arena_bump(ctx, msk_decode_scratch(n_pages, map_h, map_w, quantization), bump));
-    return msk_decode(ctx, score, geo5, n_pages, map_h, map_w, score_thresh, scale, quantization, quads_out, cap_per_page,
-                      counts, flags, bump, (cudaStream_t)stream, 0, 1);
+    return msk_decode(ctx, ms_dense_maps(score, geo5, map_h, map_w, map_h, 5), n_pages, map_h, map_w, score_thresh,
+                      scale, quantization, quads_out, cap_per_page, counts, flags, bump, (cudaStream_t)stream, 0, 1);
 }
 
 extern "C" int ms_lanms(ms_ctx *ctx, const float *quads, const int32_t *counts, int n_pages, int cap_per_page,
@@ -609,19 +644,31 @@ static void pb_init(pb_call &c, const ms_east_params *p)
     c.params.sort_reading_order = p->sort_reading_order;
 }
 
+// The maps of a call, field by field for the same reason.
+static void pb_set_maps(pb_call &c, const ms_maps *m)
+{
+    c.maps.score = m->score;
+    c.maps.geo = m->geo;
+    c.maps.dtype = m->dtype;
+    for (int i = 0; i < 3; i++) c.maps.score_strides[i] = m->score_strides[i];
+    for (int i = 0; i < 4; i++) c.maps.geo_strides[i] = m->geo_strides[i];
+}
+
 // the per-page arrays of a call from page `base` on
 struct pb_pages {
-    const float *score, *geo;
+    ms_maps maps;
     const int32_t *hw;
     float *boxes;
     int32_t *counts, *flags;
 };
 static pb_pages pb_at(const pb_call &c, int base)
 {
-    const size_t plane = (size_t)c.map_h * c.map_w;
-    const size_t gplane = c.geo_compact ? (size_t)(c.map_h / pb_quant(c)) * c.map_w : plane;
-    return {c.score + base * plane, c.geo + base * 8 * gplane, c.page_hw ? c.page_hw + 2 * (size_t)base : nullptr,
-            c.boxes_out + (size_t)base * c.cap_boxes * 9, c.box_counts + base, c.flags + base};
+    ms_maps m = c.maps;
+    const int64_t es = (int64_t)ms_dtype_bytes(m.dtype);
+    m.score = static_cast<const char *>(m.score) + base * m.score_strides[0] * es;
+    m.geo = static_cast<const char *>(m.geo) + base * m.geo_strides[0] * es;
+    return {m, c.page_hw ? c.page_hw + 2 * (size_t)base : nullptr, c.boxes_out + (size_t)base * c.cap_boxes * 9,
+            c.box_counts + base, c.flags + base};
 }
 
 // decode -> LANMS -> expand + EAST filters (-> reading order) of pages [base, base + n) of call c on stream st, boxes
@@ -640,8 +687,8 @@ static int front_half(ms_ctx *ctx, const pb_call &c, int base, int n, ms_bump bu
         ms_set_error("ms_page_batch: arena too small");
         return MS_ERR_CAPACITY;
     }
-    MS_TRY(msk_decode(ctx, pg.score, pg.geo, n, c.map_h, c.map_w, p->score_thresh, p->scale, q, qa, cap_c, ca, pg.flags,
-                      bump, st, c.geo_compact));
+    MS_TRY(msk_decode(ctx, pg.maps, n, c.map_h, c.map_w, p->score_thresh, p->scale, q, qa, cap_c, ca, pg.flags, bump,
+                      st, c.geo_compact));
     if (marks) MS_TRY(timing_mark(ctx, 1, st));
     MS_TRY(msk_lanms(ctx, qa, ca, n, cap_c, p->iou_threshold, qb, cb, pg.flags, bump, st));
     // expand + EAST filters; boxes are scaled to the page images' size (infer.py:134-147: the original image), or target_size
@@ -799,27 +846,41 @@ static int page_batch_cached(ms_ctx *ctx, const pb_call &c, cudaStream_t st)
     return rc;
 }
 
+extern "C" int ms_page_batch_maps(ms_ctx *ctx, const ms_maps *maps, const uint8_t *pages, int n_pages, int map_h,
+                                  int map_w, int img_h, int img_w, const ms_east_params *p, int min_text_size, int out_h,
+                                  int out_w, int cap_boxes, float *boxes_out, int32_t *box_counts, int32_t *crops_out,
+                                  int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                                  int32_t *flags, void *stream)
+{
+    MS_CTX(ctx);
+    MS_TRY(dtype_ok(batch_dtype, "ms_page_batch"));
+    MS_TRY(maps_desc_ok(maps, "ms_page_batch"));
+    if (n_pages <= 0) return MS_OK;
+    if (!maps->score || !maps->geo || !p || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
+        ms_set_error("ms_page_batch: bad arguments");
+        return MS_ERR_INVALID;
+    }
+    pb_call c;
+    pb_init(c, p);
+    pb_set_maps(c, maps);
+    c.pages = pages;
+    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w; c.img_h = img_h; c.img_w = img_w;
+    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
+    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
+    c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
+    return page_batch_cached(ctx, c, (cudaStream_t)stream);
+}
+
 extern "C" int ms_page_batch_ex(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
                                 int map_h, int map_w, int img_h, int img_w, const ms_east_params *p, int min_text_size,
                                 int out_h, int out_w, int cap_boxes, float *boxes_out, int32_t *box_counts,
                                 int32_t *crops_out, int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype,
                                 uint8_t *canvas_u8, int32_t *flags, void *stream)
 {
-    MS_CTX(ctx);
-    MS_TRY(dtype_ok(batch_dtype, "ms_page_batch"));
-    if (n_pages <= 0) return MS_OK;
-    if (!score || !geo || !p || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
-        ms_set_error("ms_page_batch: bad arguments");
-        return MS_ERR_INVALID;
-    }
-    pb_call c;
-    pb_init(c, p);
-    c.score = score; c.geo = geo; c.pages = pages;
-    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w; c.img_h = img_h; c.img_w = img_w;
-    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
-    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
-    c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
-    return page_batch_cached(ctx, c, (cudaStream_t)stream);
+    const ms_maps m = ms_dense_maps(score, geo, map_h, map_w, map_h, 8);
+    return ms_page_batch_maps(ctx, &m, pages, n_pages, map_h, map_w, img_h, img_w, p, min_text_size, out_h, out_w,
+                              cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch, batch_dtype,
+                              canvas_u8, flags, stream);
 }
 
 extern "C" int ms_page_batch(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
@@ -882,8 +943,8 @@ static int decode_host_impl(ms_ctx *ctx, const float *score, const float *geo, i
     MS_CUDA(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(int32_t), st));
     ms_bump bump;
     MS_TRY(arena_bump(ctx, msk_decode_scratch(1, map_h, map_w, quantization), bump));
-    MS_TRY(msk_decode(ctx, d_score, d_geo, 1, map_h, map_w, score_thresh, scale, quantization, d_out, capd, d_cnt,
-                      d_cnt + 1, bump, st, 0, rbox));
+    MS_TRY(msk_decode(ctx, ms_dense_maps(d_score, d_geo, map_h, map_w, map_h, planes), 1, map_h, map_w, score_thresh,
+                      scale, quantization, d_out, capd, d_cnt, d_cnt + 1, bump, st, 0, rbox));
     int32_t *h = reinterpret_cast<int32_t *>(ctx->pinned);
     MS_CUDA(cudaMemcpyAsync(h, d_cnt, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     MS_CUDA(cudaStreamSynchronize(st));
@@ -1287,6 +1348,33 @@ extern "C" int ms_crop_resize_pad_host(ms_ctx *ctx, const uint8_t *page, int img
     return MS_OK;
 }
 
+extern "C" int ms_page_batch_ragged_maps(ms_ctx *ctx, const ms_maps *maps, const uint8_t *const *page_ptrs,
+                                         const int32_t *page_hw, int n_pages, int map_h, int map_w,
+                                         const ms_east_params *p, int min_text_size, int out_h, int out_w, int cap_boxes,
+                                         float *boxes_out, int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
+                                         int32_t *n_crops, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                                         int32_t *flags, void *stream)
+{
+    MS_CTX(ctx);
+    MS_TRY(dtype_ok(batch_dtype, "ms_page_batch_ragged"));
+    MS_TRY(maps_desc_ok(maps, "ms_page_batch_ragged"));
+    if (n_pages <= 0) return MS_OK;
+    if (!maps->score || !maps->geo || !p || !page_ptrs || !page_hw || !boxes_out || !box_counts || !flags ||
+        cap_boxes <= 0) {
+        ms_set_error("ms_page_batch_ragged: bad arguments");
+        return MS_ERR_INVALID;
+    }
+    pb_call c;
+    pb_init(c, p);
+    pb_set_maps(c, maps);
+    c.page_ptrs = page_ptrs; c.page_hw = page_hw;
+    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w;
+    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
+    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
+    c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
+    return page_batch_cached(ctx, c, (cudaStream_t)stream);
+}
+
 extern "C" int ms_page_batch_ragged_ex(ms_ctx *ctx, const float *score, const float *geo,
                                        const uint8_t *const *page_ptrs, const int32_t *page_hw, int n_pages, int map_h,
                                        int map_w, const ms_east_params *p, int min_text_size, int out_h, int out_w,
@@ -1294,21 +1382,10 @@ extern "C" int ms_page_batch_ragged_ex(ms_ctx *ctx, const float *score, const fl
                                        int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype,
                                        uint8_t *canvas_u8, int32_t *flags, void *stream)
 {
-    MS_CTX(ctx);
-    MS_TRY(dtype_ok(batch_dtype, "ms_page_batch_ragged"));
-    if (n_pages <= 0) return MS_OK;
-    if (!score || !geo || !p || !page_ptrs || !page_hw || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
-        ms_set_error("ms_page_batch_ragged: bad arguments");
-        return MS_ERR_INVALID;
-    }
-    pb_call c;
-    pb_init(c, p);
-    c.score = score; c.geo = geo; c.page_ptrs = page_ptrs; c.page_hw = page_hw;
-    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w;
-    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
-    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
-    c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
-    return page_batch_cached(ctx, c, (cudaStream_t)stream);
+    const ms_maps m = ms_dense_maps(score, geo, map_h, map_w, map_h, 8);
+    return ms_page_batch_ragged_maps(ctx, &m, page_ptrs, page_hw, n_pages, map_h, map_w, p, min_text_size, out_h,
+                                     out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap, n_crops, batch,
+                                     batch_dtype, canvas_u8, flags, stream);
 }
 
 extern "C" int ms_page_batch_ragged(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *const *page_ptrs,
@@ -1333,17 +1410,18 @@ static int quad_batch_args_ok(int batch_dtype, int border_mode, int border_value
     return MS_OK;
 }
 
-extern "C" int ms_page_batch_quads(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
-                                   int map_h, int map_w, int img_h, int img_w, const ms_east_params *p,
-                                   int min_text_size, int border_mode, int border_value, int out_h, int out_w,
-                                   int cap_boxes, float *boxes_out, int32_t *box_counts, int32_t *crops_out,
-                                   int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype,
-                                   uint8_t *canvas_u8, int32_t *flags, void *stream)
+extern "C" int ms_page_batch_quads_maps(ms_ctx *ctx, const ms_maps *maps, const uint8_t *pages, int n_pages,
+                                        int map_h, int map_w, int img_h, int img_w, const ms_east_params *p,
+                                        int min_text_size, int border_mode, int border_value, int out_h, int out_w,
+                                        int cap_boxes, float *boxes_out, int32_t *box_counts, int32_t *crops_out,
+                                        int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype,
+                                        uint8_t *canvas_u8, int32_t *flags, void *stream)
 {
     MS_CTX(ctx);
     MS_TRY(quad_batch_args_ok(batch_dtype, border_mode, border_value, "ms_page_batch_quads"));
+    MS_TRY(maps_desc_ok(maps, "ms_page_batch_quads"));
     if (n_pages <= 0) return MS_OK;
-    if (!score || !geo || !p || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
+    if (!maps->score || !maps->geo || !p || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
         ms_set_error("ms_page_batch_quads: bad arguments");
         return MS_ERR_INVALID;
     }
@@ -1354,8 +1432,52 @@ extern "C" int ms_page_batch_quads(ms_ctx *ctx, const float *score, const float 
     }
     pb_call c;
     pb_init(c, p);
-    c.score = score; c.geo = geo; c.pages = pages;
+    pb_set_maps(c, maps);
+    c.pages = pages;
     c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w; c.img_h = img_h; c.img_w = img_w;
+    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
+    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
+    c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
+    c.crop_quads = 1; c.border_mode = border_mode; c.border_value = border_value;
+    return page_batch_cached(ctx, c, (cudaStream_t)stream);
+}
+
+extern "C" int ms_page_batch_quads(ms_ctx *ctx, const float *score, const float *geo, const uint8_t *pages, int n_pages,
+                                   int map_h, int map_w, int img_h, int img_w, const ms_east_params *p,
+                                   int min_text_size, int border_mode, int border_value, int out_h, int out_w,
+                                   int cap_boxes, float *boxes_out, int32_t *box_counts, int32_t *crops_out,
+                                   int64_t crops_cap, int32_t *n_crops, void *batch, int batch_dtype,
+                                   uint8_t *canvas_u8, int32_t *flags, void *stream)
+{
+    const ms_maps m = ms_dense_maps(score, geo, map_h, map_w, map_h, 8);
+    return ms_page_batch_quads_maps(ctx, &m, pages, n_pages, map_h, map_w, img_h, img_w, p, min_text_size, border_mode,
+                                    border_value, out_h, out_w, cap_boxes, boxes_out, box_counts, crops_out, crops_cap,
+                                    n_crops, batch, batch_dtype, canvas_u8, flags, stream);
+}
+
+extern "C" int ms_page_batch_ragged_quads_maps(ms_ctx *ctx, const ms_maps *maps, const uint8_t *const *page_ptrs,
+                                               const int32_t *page_hw, int n_pages, int map_h, int map_w,
+                                               const ms_east_params *p, int min_text_size, int border_mode,
+                                               int border_value, int out_h, int out_w, int cap_boxes, float *boxes_out,
+                                               int32_t *box_counts, int32_t *crops_out, int64_t crops_cap,
+                                               int32_t *n_crops, void *batch, int batch_dtype, uint8_t *canvas_u8,
+                                               int32_t *flags, void *stream)
+{
+    MS_CTX(ctx);
+    MS_TRY(quad_batch_args_ok(batch_dtype, border_mode, border_value, "ms_page_batch_ragged_quads"));
+    MS_TRY(maps_desc_ok(maps, "ms_page_batch_ragged_quads"));
+    if (n_pages <= 0) return MS_OK;
+    if (!maps->score || !maps->geo || !p || !page_ptrs || !page_hw || !boxes_out || !box_counts || !flags ||
+        cap_boxes <= 0) {
+        ms_set_error("ms_page_batch_ragged_quads: bad arguments");
+        return MS_ERR_INVALID;
+    }
+    // (the page sizes are device data: quads of a page above 32767 pixels on a side get no patch)
+    pb_call c;
+    pb_init(c, p);
+    pb_set_maps(c, maps);
+    c.page_ptrs = page_ptrs; c.page_hw = page_hw;
+    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w;
     c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
     c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
     c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
@@ -1371,23 +1493,10 @@ extern "C" int ms_page_batch_ragged_quads(ms_ctx *ctx, const float *score, const
                                           int32_t *n_crops, void *batch, int batch_dtype, uint8_t *canvas_u8,
                                           int32_t *flags, void *stream)
 {
-    MS_CTX(ctx);
-    MS_TRY(quad_batch_args_ok(batch_dtype, border_mode, border_value, "ms_page_batch_ragged_quads"));
-    if (n_pages <= 0) return MS_OK;
-    if (!score || !geo || !p || !page_ptrs || !page_hw || !boxes_out || !box_counts || !flags || cap_boxes <= 0) {
-        ms_set_error("ms_page_batch_ragged_quads: bad arguments");
-        return MS_ERR_INVALID;
-    }
-    // (the page sizes are device data: quads of a page above 32767 pixels on a side get no patch)
-    pb_call c;
-    pb_init(c, p);
-    c.score = score; c.geo = geo; c.page_ptrs = page_ptrs; c.page_hw = page_hw;
-    c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w;
-    c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
-    c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
-    c.batch = batch; c.batch_dtype = batch_dtype; c.canvas_u8 = canvas_u8; c.flags = flags;
-    c.crop_quads = 1; c.border_mode = border_mode; c.border_value = border_value;
-    return page_batch_cached(ctx, c, (cudaStream_t)stream);
+    const ms_maps m = ms_dense_maps(score, geo, map_h, map_w, map_h, 8);
+    return ms_page_batch_ragged_quads_maps(ctx, &m, page_ptrs, page_hw, n_pages, map_h, map_w, p, min_text_size,
+                                           border_mode, border_value, out_h, out_w, cap_boxes, boxes_out, box_counts,
+                                           crops_out, crops_cap, n_crops, batch, batch_dtype, canvas_u8, flags, stream);
 }
 
 // Read-back of a host page batch queued on the context's own stream, from device call d to the caller's buffers in h.
@@ -1447,7 +1556,7 @@ extern "C" int ms_page_batch_host_ex(ms_ctx *ctx, const float *score, const floa
     }
     pb_call c;  // the caller's buffers
     pb_init(c, p);
-    c.score = score; c.geo = geo; c.pages = pages;
+    c.pages = pages;
     c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w; c.img_h = img_h; c.img_w = img_w;
     c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
     c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
@@ -1497,8 +1606,7 @@ extern "C" int ms_page_batch_host_ex(ms_ctx *ctx, const float *score, const floa
         d.n_crops = want_crops ? sb.take<int32_t>(1) : nullptr;
         d.batch = !want_batch ? nullptr : caller_batch ? caller_batch : sb.take<char>((size_t)crops_cap * one_f);
     }));
-    d.score = d_score;
-    d.geo = geo_mapped ? geo_mapped : d_geo;
+    d.maps = ms_dense_maps(d_score, geo_mapped ? geo_mapped : d_geo, map_h, map_w, d.geo_compact ? map_h / q : map_h, 8);
     d.pages = d_pages;
     // Pipeline: pages are independent, so the batch is cut into chunks; the copy stream uploads chunk c+1 (maps +
     // page images) while the compute stream runs chunk c.  PCIe is the floor of this entry point: 22 MB per
@@ -1703,7 +1811,7 @@ extern "C" int ms_page_batch_ragged_host_ex(ms_ctx *ctx, const float *score, con
     }
     pb_call c;  // the caller's buffers
     pb_init(c, p);
-    c.score = score; c.geo = geo; c.page_ptrs = pages; c.page_hw = page_hw;
+    c.page_ptrs = pages; c.page_hw = page_hw;
     c.n_pages = n_pages; c.map_h = map_h; c.map_w = map_w;
     c.min_text_size = min_text_size; c.out_h = out_h; c.out_w = out_w; c.cap_boxes = cap_boxes; c.crops_cap = crops_cap;
     c.boxes_out = boxes_out; c.box_counts = box_counts; c.crops_out = crops_out; c.n_crops = n_crops;
@@ -1730,8 +1838,7 @@ extern "C" int ms_page_batch_ragged_host_ex(ms_ctx *ctx, const float *score, con
         d.batch = !want_batch ? nullptr : caller_batch ? caller_batch : sb.take<char>((size_t)crops_cap * one_f);
         d_img = sb.take<uint8_t>(img_total);
     }));
-    d.score = d_score;
-    d.geo = d_geo;
+    d.maps = ms_dense_maps(d_score, d_geo, map_h, map_w, map_h, 8);
     d.page_ptrs = d_ptrs;
     d.page_hw = d_hw;
     cudaStream_t st = ctx->own_stream;

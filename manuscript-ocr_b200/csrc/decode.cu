@@ -9,12 +9,19 @@
 //   * v = x*scale [f64] + f32(d*f32(scale)) -> f64 sum -> f32 (utils.py:368-381, NEP-50 promotion)
 //   * a centre outside the map raises IndexError in the reference -> MS_FLAG_INDEX_ERROR here
 //
-// Data layout: score (P,H,W) f32, geo (P,8,H,W) f32 planar, out page-strided (P*cap,9) f32.
-// HBM traffic (algorithmic): 4*H*W score read + 36*N gathered + 36*N written per page.
+// Data layout: score (P,H,W), geo (P,8,H,W) at any element strides (ms_maps), in float32, float16 or bfloat16; every
+// value is widened to float32 at its load (exact) and the arithmetic after it is the float32 path's.  Out page-strided
+// (P*cap,9) f32.
+// HBM traffic (algorithmic): H*W score elements read + 8*N gathered geometry elements + 36*N bytes written per page.
 //
 // Three launches: mark (ballot bitmasks + per-tile counts), scan (per page), emit (gather + staged,
 // coalesced row writes).  One cell per lane; a warp's 32 cells are 32 consecutive cells of a row, so
-// score loads are coalesced (float2 per lane for q=2).
+// score loads are coalesced (one 2-element vector per lane for q=2 where the layout allows it).
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
+#include <type_traits>
+
 #include "ms_internal.cuh"
 
 namespace {
@@ -46,19 +53,62 @@ __host__ __device__ inline DecodeGeom make_geom(int H, int W, int q)
     return g;
 }
 
-__device__ __forceinline__ bool cell_hit(const float *__restrict__ score, const DecodeGeom &g, int cell, float thr)
+// Element strides of the two maps (ms_maps) and the load paths the host chose from them and the pointers' alignment.
+struct MapLayout {
+    int64_t s_page, s_row, s_col;          // score
+    int64_t g_page, g_ch, g_row, g_col;    // geometry
+    int score_pairs;  // q = 2: the two pixels of a cell row are adjacent and 2-element aligned -> one vector load
+};
+
+// a map value widened to float32: the conversions torch's .float() makes on the device
+__device__ __forceinline__ float to_f32(float v) { return v; }
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+
+template <typename T>
+__device__ __forceinline__ float ld_map(const T *p)
+{
+    return to_f32(__ldg(p));
+}
+// two adjacent values, the first aligned to twice the element size: one 8-byte (float32) or 4-byte (16 bits) load
+__device__ __forceinline__ float2 ld_map2(const float *p) { return __ldg(reinterpret_cast<const float2 *>(p)); }
+template <typename T>
+__device__ __forceinline__ float2 ld_map2(const T *p)
+{
+    const unsigned int u = __ldg(reinterpret_cast<const unsigned int *>(p));
+    const T *v = reinterpret_cast<const T *>(&u);
+    return make_float2(to_f32(v[0]), to_f32(v[1]));
+}
+// the 8 geometry values of a pixel, adjacent and 16-byte aligned: two 16-byte loads (float32) or one (16 bits)
+__device__ __forceinline__ void ld_geo8(const float *p, float *d)
+{
+    const float4 a = __ldg(reinterpret_cast<const float4 *>(p)), b = __ldg(reinterpret_cast<const float4 *>(p) + 1);
+    d[0] = a.x, d[1] = a.y, d[2] = a.z, d[3] = a.w, d[4] = b.x, d[5] = b.y, d[6] = b.z, d[7] = b.w;
+}
+template <typename T>
+__device__ __forceinline__ void ld_geo8(const T *p, float *d)
+{
+    const uint4 u = __ldg(reinterpret_cast<const uint4 *>(p));
+    const T *v = reinterpret_cast<const T *>(&u);
+#pragma unroll
+    for (int i = 0; i < 8; i++) d[i] = to_f32(v[i]);
+}
+
+template <typename T>
+__device__ __forceinline__ bool cell_hit(const T *__restrict__ score, const DecodeGeom &g, const MapLayout &L, int cell,
+                                         float thr)
 {
     if (cell >= g.cells) return false;
     int cy = cell / g.CW, cx = cell - cy * g.CW;
-    if (g.q == 1) return __ldg(score + (size_t)cy * g.W + cx) > thr;
-    if (g.q == 2 && (g.W & 1) == 0) {
-        // both pixels of a row of the cell are in range when W is even
+    if (g.q == 1) return ld_map(score + cy * L.s_row + cx * L.s_col) > thr;
+    if (g.q == 2 && L.score_pairs) {
+        // both pixels of a row of the cell are in range when W is even (score_pairs implies it)
         int y = 2 * cy;
-        const float2 *r0 = reinterpret_cast<const float2 *>(score + (size_t)y * g.W) + cx;
-        float2 a = __ldg(r0);
+        const T *r0 = score + y * L.s_row + 2 * cx;
+        float2 a = ld_map2(r0);
         bool hit = a.x > thr || a.y > thr;
         if (y + 1 < g.H) {
-            float2 b = __ldg(reinterpret_cast<const float2 *>(score + (size_t)(y + 1) * g.W) + cx);
+            float2 b = ld_map2(r0 + L.s_row);
             hit = hit || b.x > thr || b.y > thr;
         }
         return hit;
@@ -70,14 +120,15 @@ __device__ __forceinline__ bool cell_hit(const float *__restrict__ score, const 
         for (int dx = 0; dx < g.q; dx++) {
             int x = cx * g.q + dx;
             if (x >= g.W) break;
-            hit = hit || (__ldg(score + (size_t)y * g.W + x) > thr);
+            hit = hit || (ld_map(score + y * L.s_row + x * L.s_col) > thr);
         }
     }
     return hit;
 }
 
 // mark: one lane per cell, ballot -> mask words + per-tile candidate counts
-__global__ void __launch_bounds__(kThreads) decode_mark_kernel(const float *__restrict__ score, DecodeGeom g,
+template <typename T>
+__global__ void __launch_bounds__(kThreads) decode_mark_kernel(const T *__restrict__ score, DecodeGeom g, MapLayout L,
                                                                float thr, uint32_t *__restrict__ masks,
                                                                int32_t *__restrict__ tile_counts,
                                                                int32_t *__restrict__ flags)
@@ -85,7 +136,7 @@ __global__ void __launch_bounds__(kThreads) decode_mark_kernel(const float *__re
     ms_pdl_wait();
     const int page = blockIdx.y, tile = blockIdx.x;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const float *sc = score + (size_t)page * g.H * g.W;
+    const T *sc = score + page * L.s_page;
     __shared__ int s_cnt[kWarps];
     int cnt = 0;
     bool bad = false;
@@ -93,7 +144,7 @@ __global__ void __launch_bounds__(kThreads) decode_mark_kernel(const float *__re
     for (int k = 0; k < kWordsPerWarp; k++) {
         int word = tile * kTileWords + warp * kWordsPerWarp + k;
         int cell = word * 32 + lane;
-        bool hit = word < g.words && cell_hit(sc, g, cell, thr);
+        bool hit = word < g.words && cell_hit(sc, g, L, cell, thr);
         if (hit && g.q > 1) {
             int cy = cell / g.CW, cx = cell - cy * g.CW;
             if (cy * g.q + g.q / 2 >= g.H || cx * g.q + g.q / 2 >= g.W) {  // utils.py:370 IndexError
@@ -188,11 +239,12 @@ __device__ __forceinline__ void rbox_to_quad(double ox, double oy, double dt, do
     }
 }
 
-// emit: rank candidates inside the tile, gather geometry at the cell centre, write rows in order
-template <bool kRbox>
-__global__ void __launch_bounds__(kThreads) decode_emit_kernel(const float *__restrict__ score,
-                                                               const float *__restrict__ geo, DecodeGeom g,
-                                                               double scale, const uint32_t *__restrict__ masks,
+// emit: rank candidates inside the tile, gather geometry at the cell centre, write rows in order.  kGeo8: a pixel's 8
+// QUAD geometry values are adjacent and 16-byte aligned (channels-last geometry), gathered by ld_geo8.
+template <typename T, bool kRbox, bool kGeo8>
+__global__ void __launch_bounds__(kThreads) decode_emit_kernel(const T *__restrict__ score, const T *__restrict__ geo,
+                                                               DecodeGeom g, MapLayout L, double scale,
+                                                               const uint32_t *__restrict__ masks,
                                                                const int32_t *__restrict__ tile_base, int cap,
                                                                float *__restrict__ out, int geo_compact)
 {
@@ -201,12 +253,8 @@ __global__ void __launch_bounds__(kThreads) decode_emit_kernel(const float *__re
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     __shared__ int s_word_base[kTileWords];
     __shared__ float s_rows[kWarps][32 * 9];
-    const size_t plane = (size_t)g.H * g.W;
-    // geo_compact: the geometry tensor holds only the rows a quantised read can touch (y % q == q / 2), i.e.
-    // (P, 8, H / q, W) -- what ms_page_batch_host uploads
-    const size_t gplane = geo_compact ? (size_t)(g.H / g.q) * g.W : plane;
-    const float *sc = score + (size_t)page * plane;
-    const float *ge = geo + (size_t)page * (kRbox ? 5 : 8) * gplane;
+    const T *sc = score + page * L.s_page;
+    const T *ge = geo + page * L.g_page;
     const uint32_t *mk = masks + (size_t)page * g.words;
 
     // exclusive prefix over the tile's 64 mask-word popcounts (two warps worth of data)
@@ -254,25 +302,34 @@ __global__ void __launch_bounds__(kThreads) decode_emit_kernel(const float *__re
             int cy = cell / g.CW, cx = cell - cy * g.CW;
             int y = g.q > 1 ? cy * g.q + g.q / 2 : cy;
             int x = g.q > 1 ? cx * g.q + g.q / 2 : cx;
-            const size_t pix = (size_t)y * g.W + x;
-            const size_t gpix = geo_compact ? (size_t)cy * g.W + x : pix;
+            // geo_compact: the geometry tensor holds only the rows a quantised read can touch (y % q == q / 2), i.e.
+            // (P, 8, H / q, W) -- what ms_page_batch_host uploads -- and L's geometry strides are that tensor's
+            const T *gp = ge + (geo_compact ? cy : y) * L.g_row + x * L.g_col;
+            // the score and geometry loads go out before the arithmetic that uses them: one memory latency per
+            // candidate instead of nine dependent ones
+            const float score_v = ld_map(sc + y * L.s_row + x * L.s_col);
             double xs = __dmul_rn((double)x, scale);
             double ys = __dmul_rn((double)y, scale);
             float *r = stage + rank * 9;
             if (kRbox) {
                 double d[5];
 #pragma unroll
-                for (int v = 0; v < 5; v++) d[v] = (double)__ldg(ge + (size_t)v * gplane + gpix);
+                for (int v = 0; v < 5; v++, gp += L.g_ch) d[v] = (double)ld_map(gp);
                 rbox_to_quad(xs, ys, d[0] * scale, d[1] * scale, d[2] * scale, d[3] * scale, d[4], r);
-            } else
+            } else {
+                float d[8];
+                if (kGeo8)
+                    ld_geo8(gp, d);
+                else
 #pragma unroll
-            for (int v = 0; v < 4; v++) {
-                float dx = __ldg(ge + (size_t)(2 * v) * gplane + gpix);
-                float dy = __ldg(ge + (size_t)(2 * v + 1) * gplane + gpix);
-                r[2 * v] = (float)__dadd_rn(xs, (double)__fmul_rn(dx, sc32));
-                r[2 * v + 1] = (float)__dadd_rn(ys, (double)__fmul_rn(dy, sc32));
+                    for (int v = 0; v < 8; v++, gp += L.g_ch) d[v] = ld_map(gp);
+#pragma unroll
+                for (int v = 0; v < 4; v++) {
+                    r[2 * v] = (float)__dadd_rn(xs, (double)__fmul_rn(d[2 * v], sc32));
+                    r[2 * v + 1] = (float)__dadd_rn(ys, (double)__fmul_rn(d[2 * v + 1], sc32));
+                }
             }
-            r[8] = __ldg(sc + pix);
+            r[8] = score_v;
         }
         __syncwarp();
         float *dst = out + ((size_t)page * cap + row0) * 9;
@@ -292,9 +349,39 @@ size_t msk_decode_scratch(int n_pages, int H, int W, int q)
     return b + 1024;
 }
 
-int msk_decode(ms_ctx *ctx, const float *score, const float *geo, int n_pages, int H, int W, float thr,
-               double scale, int q, float *quads_out, int cap_per_page, int32_t *counts, int32_t *flags,
-               ms_bump bump, cudaStream_t st, int geo_compact, int rbox)
+// the launches of one map element type
+template <typename T>
+static int decode_launch(ms_ctx *ctx, const T *score, const T *geo, const DecodeGeom &g, const MapLayout &L, bool geo8,
+                         float thr, double scale, float *quads_out, int cap_per_page, int32_t *counts, int32_t *flags,
+                         uint32_t *masks, int32_t *tile_counts, int32_t *tile_base, int n_pages, cudaStream_t st,
+                         int geo_compact, int rbox)
+{
+    dim3 grid(g.tiles, n_pages);
+    ms_launch(decode_mark_kernel<T>, grid, kThreads, 0, st, score, g, L, thr, masks, tile_counts, flags);
+    MS_LAUNCH_CHECK(ctx);
+    ms_launch(decode_scan_kernel, n_pages, 256, 0, st, tile_counts, g.tiles, cap_per_page, tile_base, counts, flags);
+    MS_LAUNCH_CHECK(ctx);
+    if constexpr (std::is_same<T, float>::value) {
+        if (rbox) {
+            ms_launch(decode_emit_kernel<float, true, false>, grid, kThreads, 0, st, score, geo, g, L, scale, masks,
+                      tile_base, cap_per_page, quads_out, geo_compact);
+            MS_LAUNCH_CHECK(ctx);
+            return MS_OK;
+        }
+    }
+    if (geo8)
+        ms_launch(decode_emit_kernel<T, false, true>, grid, kThreads, 0, st, score, geo, g, L, scale, masks, tile_base,
+                  cap_per_page, quads_out, geo_compact);
+    else
+        ms_launch(decode_emit_kernel<T, false, false>, grid, kThreads, 0, st, score, geo, g, L, scale, masks, tile_base,
+                  cap_per_page, quads_out, geo_compact);
+    MS_LAUNCH_CHECK(ctx);
+    return MS_OK;
+}
+
+int msk_decode(ms_ctx *ctx, const ms_maps &m, int n_pages, int H, int W, float thr, double scale, int q,
+               float *quads_out, int cap_per_page, int32_t *counts, int32_t *flags, ms_bump bump, cudaStream_t st,
+               int geo_compact, int rbox)
 {
     if (n_pages <= 0) return MS_OK;
     if (geo_compact && (q < 2 || H % q != 0)) {
@@ -305,6 +392,10 @@ int msk_decode(ms_ctx *ctx, const float *score, const float *geo, int n_pages, i
         ms_set_error("decode: bad shape H=%d W=%d q=%d cap=%d", H, W, q, cap_per_page);
         return MS_ERR_INVALID;
     }
+    if (rbox && m.dtype != MS_DTYPE_F32) {
+        ms_set_error("decode: RBOX maps are float32");
+        return MS_ERR_INVALID;
+    }
     DecodeGeom g = make_geom(H, W, q);
     uint32_t *masks = bump.take<uint32_t>((size_t)n_pages * g.words);
     int32_t *tile_counts = bump.take<int32_t>((size_t)n_pages * g.tiles);
@@ -313,17 +404,26 @@ int msk_decode(ms_ctx *ctx, const float *score, const float *geo, int n_pages, i
         ms_set_error("decode: scratch too small");
         return MS_ERR_CAPACITY;
     }
-    dim3 grid(g.tiles, n_pages);
-    ms_launch(decode_mark_kernel, grid, kThreads, 0, st, score, g, thr, masks, tile_counts, flags);
-    MS_LAUNCH_CHECK(ctx);
-    ms_launch(decode_scan_kernel, n_pages, 256, 0, st, tile_counts, g.tiles, cap_per_page, tile_base, counts, flags);
-    MS_LAUNCH_CHECK(ctx);
-    if (rbox)
-        ms_launch(decode_emit_kernel<true>, grid, kThreads, 0, st, score, geo, g, scale, masks, tile_base, cap_per_page,
-                                                            quads_out, geo_compact);
-    else
-        ms_launch(decode_emit_kernel<false>, grid, kThreads, 0, st, score, geo, g, scale, masks, tile_base, cap_per_page,
-                                                             quads_out, geo_compact);
-    MS_LAUNCH_CHECK(ctx);
-    return MS_OK;
+    // the vector loads: chosen from the strides and the pointers' alignment, else one load per element at the strides
+    const int64_t es = (int64_t)ms_dtype_bytes(m.dtype);
+    const int64_t *ss = m.score_strides, *gs = m.geo_strides;
+    MapLayout L = {ss[0], ss[1], ss[2], gs[0], gs[1], gs[2], gs[3], 0};
+    L.score_pairs = g.q == 2 && W % 2 == 0 && ss[2] == 1 && ss[1] % 2 == 0 && (n_pages == 1 || ss[0] % 2 == 0) &&
+                    (uintptr_t)m.score % (2 * es) == 0;
+    const bool geo8 = !rbox && gs[1] == 1 && gs[3] == 8 && (gs[2] * es) % 16 == 0 &&
+                      (n_pages == 1 || (gs[0] * es) % 16 == 0) && (uintptr_t)m.geo % 16 == 0;
+    switch (m.dtype) {
+    case MS_DTYPE_F32:
+        return decode_launch(ctx, (const float *)m.score, (const float *)m.geo, g, L, geo8, thr, scale, quads_out,
+                             cap_per_page, counts, flags, masks, tile_counts, tile_base, n_pages, st, geo_compact, rbox);
+    case MS_DTYPE_F16:
+        return decode_launch(ctx, (const __half *)m.score, (const __half *)m.geo, g, L, geo8, thr, scale, quads_out,
+                             cap_per_page, counts, flags, masks, tile_counts, tile_base, n_pages, st, geo_compact, rbox);
+    case MS_DTYPE_BF16:
+        return decode_launch(ctx, (const __nv_bfloat16 *)m.score, (const __nv_bfloat16 *)m.geo, g, L, geo8, thr, scale,
+                             quads_out, cap_per_page, counts, flags, masks, tile_counts, tile_base, n_pages, st,
+                             geo_compact, rbox);
+    }
+    ms_set_error("decode: unknown map dtype %d", m.dtype);
+    return MS_ERR_INVALID;
 }

@@ -6,18 +6,20 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
+#include <string.h>
 
 #include "../../include/manuscript_b200.h"
 
 #define MS_NUM_SMS_B200 148
 
 // Everything that defines one page-batch call (api.cu).  Per-page arrays point at the call's page 0 and are
-// page-strided: score (n_pages, map_h, map_w), geo (n_pages, 8, map_h / q or map_h, map_w), boxes_out (n_pages,
+// page-strided: the maps (n_pages, map_h, map_w) and (n_pages, 8, map_h / q or map_h, map_w) at their element strides
+// and element type, boxes_out (n_pages,
 // cap_boxes, 9), box_counts / flags (n_pages), page_hw (n_pages, 2).  pages (n_pages, img_h, img_w, 3) u8 or, for
 // images of their own sizes, page_ptrs + page_hw.  The host entry points describe the caller's host buffers in one
 // pb_call and the device staging in a copy of it.
 struct pb_call {
-    const float *score, *geo;
+    ms_maps maps;  // copied field by field (pb_set_maps): no padding bytes of the caller's struct
     const uint8_t *pages;
     const uint8_t *const *page_ptrs;
     const int32_t *page_hw;
@@ -221,9 +223,27 @@ inline void ms_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t sm
 // Every launcher takes its scratch as an ms_bump BY VALUE (stage-local; stages of one stream may
 // reuse the same bytes) sized by the matching msk_*_scratch().
 // decode.cu
-int msk_decode(ms_ctx *ctx, const float *score, const float *geo, int n_pages, int H, int W, float thr,
-               double scale, int q, float *quads_out, int cap_per_page, int32_t *counts, int32_t *flags,
-               ms_bump bump, cudaStream_t st, int geo_compact = 0, int rbox = 0);  // rbox: geo is (P,5,H,W)
+// Maps at their strides (geo_compact: the geometry strides are those of the compact (P, 8, H / q, W) tensor).
+int msk_decode(ms_ctx *ctx, const ms_maps &m, int n_pages, int H, int W, float thr, double scale, int q,
+               float *quads_out, int cap_per_page, int32_t *counts, int32_t *flags, ms_bump bump, cudaStream_t st,
+               int geo_compact = 0, int rbox = 0);  // rbox: geo is (P,5,H,W) float32
+// dense float32 maps: score (P, H, W), geo (P, chans, geo_rows, W)
+inline ms_maps ms_dense_maps(const float *score, const float *geo, int H, int W, int geo_rows, int chans)
+{
+    ms_maps m;
+    memset(&m, 0, sizeof(m));
+    m.score = score;
+    m.geo = geo;
+    m.dtype = MS_DTYPE_F32;
+    m.score_strides[0] = (int64_t)H * W;
+    m.score_strides[1] = W;
+    m.score_strides[2] = 1;
+    m.geo_strides[0] = (int64_t)chans * geo_rows * W;
+    m.geo_strides[1] = (int64_t)geo_rows * W;
+    m.geo_strides[2] = W;
+    m.geo_strides[3] = 1;
+    return m;
+}
 size_t msk_decode_scratch(int n_pages, int H, int W, int q);
 // sort.cu : stable LSD radix sort, per-page segments [page_off[p], page_off[p+1]) of (u32 key, u32 value), 4 passes
 int msk_sort_pages(ms_ctx *ctx, uint32_t *keys, uint32_t *vals, uint32_t *keys_tmp, uint32_t *vals_tmp,

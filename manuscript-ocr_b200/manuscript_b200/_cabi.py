@@ -72,6 +72,18 @@ class EastParams(C.Structure):
         return p
 
 
+class MsMaps(C.Structure):
+    """ms_maps: the score and geometry maps of a batch, one element type, each at its own element strides."""
+
+    _fields_ = [
+        ("score", C.c_void_p),
+        ("geo", C.c_void_p),
+        ("dtype", C.c_int32),
+        ("score_strides", C.c_int64 * 3),
+        ("geo_strides", C.c_int64 * 4),
+    ]
+
+
 _vp = C.c_void_p
 _i = C.c_int
 _i64 = C.c_int64
@@ -146,6 +158,16 @@ SIGNATURES = {
                                  _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
     "ms_page_batch_ragged_quads": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i, _i, _i,
                                         _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
+    # EXTENSION: the same entry points on an ms_maps descriptor (maps in float32 / float16 / bfloat16, any strides)
+    "ms_decode_quads_maps": (_i, [_vp, C.POINTER(MsMaps), _i, _i, _i, _f, _d, _i, _vp, _i, _vp, _vp, _vp]),
+    "ms_page_batch_maps": (_i, [_vp, C.POINTER(MsMaps), _vp, _i, _i, _i, _i, _i, C.POINTER(EastParams), _i, _i, _i,
+                                _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
+    "ms_page_batch_ragged_maps": (_i, [_vp, C.POINTER(MsMaps), _vp, _vp, _i, _i, _i, C.POINTER(EastParams), _i, _i,
+                                       _i, _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
+    "ms_page_batch_quads_maps": (_i, [_vp, C.POINTER(MsMaps), _vp, _i, _i, _i, _i, _i, C.POINTER(EastParams), _i,
+                                      _i, _i, _i, _i, _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
+    "ms_page_batch_ragged_quads_maps": (_i, [_vp, C.POINTER(MsMaps), _vp, _vp, _i, _i, _i, C.POINTER(EastParams), _i,
+                                             _i, _i, _i, _i, _i, _vp, _vp, _vp, _i64, _vp, _vp, _i, _vp, _vp, _vp]),
     # EXTENSION: baseline-JPEG decode on the device (ms_jpeg_info *, host files -> device pages)
     "ms_jpeg_inspect_host": (_i, [_vp, _i64, _vp]),
     "ms_jpeg_decode_batch": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp]),
@@ -161,6 +183,22 @@ def batch_dtype_code(dtype):
     if dtype not in codes:
         raise ValueError(f"the recogniser batch can be float32, float16 or bfloat16, not {dtype}")
     return codes[dtype]
+
+
+def maps_descriptor(score, geo):
+    """MsMaps of a (P, H, W) score and a (P, 8, H, W) geometry CUDA tensor, both float32, float16 or bfloat16, at the
+    strides they have.  The descriptor holds the tensors' addresses: the caller keeps them alive."""
+    import torch
+
+    codes = {torch.float32: MS_DTYPE_F32, torch.float16: MS_DTYPE_F16, torch.bfloat16: MS_DTYPE_BF16}
+    if score.dtype != geo.dtype or score.dtype not in codes:
+        raise ValueError(f"score and geometry maps must both be float32, float16 or bfloat16, got {score.dtype} and "
+                         f"{geo.dtype}")
+    if score.dim() != 3 or geo.dim() != 4:
+        raise ValueError(f"maps must be (P, H, W) and (P, 8, H, W), got {tuple(score.shape)} and {tuple(geo.shape)}")
+    return MsMaps(score.data_ptr(), geo.data_ptr(), codes[score.dtype], (C.c_int64 * 3)(*score.stride()),
+                  (C.c_int64 * 4)(*geo.stride()))
+
 
 _lib = None
 _lock = threading.Lock()

@@ -14,7 +14,7 @@ from dataclasses import dataclass
 import numpy as np
 
 from ._cabi import (MS_FLAG_CAND_OVERFLOW, MS_FLAG_EDGE_OVERFLOW, MS_FLAG_INDEX_ERROR, MS_FLAG_ORDER_OVERFLOW, CABIError,
-                    Context, EastParams, batch_dtype_code, check)
+                    Context, EastParams, batch_dtype_code, check, maps_descriptor)
 
 
 def shard_pages(n_pages, world_size, rank):
@@ -153,8 +153,11 @@ class PageBatch:
         return b
 
     def run(self, score, geo, pages=None, sync=False):
-        """score (P,H,W) or (P,1,H,W) f32, geo (P,8,H,W) f32, pages (P,IH,IW,3) u8 -- CUDA tensors on this
-        runner's device.  Enqueues the whole path on the current stream and returns device tensors.
+        """score (P,H,W) or (P,1,H,W), geo (P,8,H,W), pages (P,IH,IW,3) u8 -- CUDA tensors on this runner's device.
+        The maps are float32, float16 or bfloat16 (both the same) at whatever strides they have (a channels_last
+        geometry, a slice of a fused head): they are read in place, never copied, and every result equals that of the
+        same call on score.float().contiguous() and geo.float().contiguous().  Enqueues the whole path on the current
+        stream and returns device tensors.
 
         sync=False (default): nothing is read back; the results are valid only if `result.flags` is all zero --
         call result.raise_for_flags() (one small D2H copy) before trusting them.
@@ -173,9 +176,8 @@ class PageBatch:
             score = score[:, 0]
         P, H, W = score.shape
         assert geo.shape == (P, 8, H, W), geo.shape
-        assert score.is_cuda and geo.is_cuda and score.dtype == torch.float32 and geo.dtype == torch.float32
-        score = score.contiguous()
-        geo = geo.contiguous()
+        assert score.is_cuda and geo.is_cuda
+        maps = maps_descriptor(score, geo)
         img_h = img_w = 0
         if pages is not None:
             assert pages.is_cuda and pages.dtype == torch.uint8 and pages.shape[0] == P and pages.shape[3] == 3
@@ -184,23 +186,24 @@ class PageBatch:
         b = self._device_bufs(P)
         stream = torch.cuda.current_stream(self.device).cuda_stream
         lib = self.ctx.lib
-        head = (self.ctx.handle, score.data_ptr(), geo.data_ptr(), pages.data_ptr() if pages is not None else None,
-                P, H, W, img_h, img_w, C.byref(self.params), self.min_text_size)
+        head = (self.ctx.handle, C.byref(maps), pages.data_ptr() if pages is not None else None, P, H, W, img_h, img_w,
+                C.byref(self.params), self.min_text_size)
         tail = (self.out_h, self.out_w, self.cap_boxes, b["boxes"].data_ptr(), b["counts"].data_ptr(),
                 b["crops"].data_ptr(), b["cap"], b["n_crops"].data_ptr(),
                 b["batch"].data_ptr() if b["batch"] is not None else None, self._dtype_code, None, b["flags"].data_ptr(),
                 C.c_void_p(stream))
         with torch.cuda.device(self.device):
             if self.crops == "quads":
-                check(lib.ms_page_batch_quads(*head, self.border_mode, self.border_value, *tail))
+                check(lib.ms_page_batch_quads_maps(*head, self.border_mode, self.border_value, *tail))
             else:
-                check(lib.ms_page_batch_ex(*head, *tail))
+                check(lib.ms_page_batch_maps(*head, *tail))
         return PageBatchResult(b["boxes"], b["counts"], b["crops"], b["n_crops"], b["batch"], b["flags"])
 
     def run_ragged(self, score, geo, pages, sync=False, allow_order_overflow=False):
         """As run(), for page images of their own sizes: `pages` is a list of P CUDA uint8 tensors (H_i, W_i, 3) -- the
         original images, while the maps come from the detector's fixed target_size.  Boxes are scaled to each page's
-        size and crops are cut from its pixels (EAST.predict + Pipeline.predict semantics).  `sync` as in run()."""
+        size and crops are cut from its pixels (EAST.predict + Pipeline.predict semantics).  The maps are taken as by
+        run(): float32, float16 or bfloat16 at any strides, read in place.  `sync` as in run()."""
         if sync:
             while True:
                 res = self.run_ragged(score, geo, pages, sync=False)
@@ -214,8 +217,8 @@ class PageBatch:
             score = score[:, 0]
         P, H, W = score.shape
         assert geo.shape == (P, 8, H, W) and len(pages) == P
-        assert score.is_cuda and geo.is_cuda and score.dtype == torch.float32 and geo.dtype == torch.float32
-        score, geo = score.contiguous(), geo.contiguous()
+        assert score.is_cuda and geo.is_cuda
+        maps = maps_descriptor(score, geo)
         keep = []
         for pg in pages:
             assert pg.is_cuda and pg.dtype == torch.uint8 and pg.dim() == 3 and pg.shape[2] == 3
@@ -234,17 +237,17 @@ class PageBatch:
         b = self._device_bufs(P)
         stream = torch.cuda.current_stream(self.device).cuda_stream
         lib = self.ctx.lib
-        head = (self.ctx.handle, score.data_ptr(), geo.data_ptr(), ptrs.data_ptr(), hw.data_ptr(), P, H, W,
-                C.byref(self.params), self.min_text_size)
+        head = (self.ctx.handle, C.byref(maps), ptrs.data_ptr(), hw.data_ptr(), P, H, W, C.byref(self.params),
+                self.min_text_size)
         tail = (self.out_h, self.out_w, self.cap_boxes, b["boxes"].data_ptr(), b["counts"].data_ptr(),
                 b["crops"].data_ptr(), b["cap"], b["n_crops"].data_ptr(),
                 b["batch"].data_ptr() if b["batch"] is not None else None, self._dtype_code, None, b["flags"].data_ptr(),
                 C.c_void_p(stream))
         with torch.cuda.device(self.device):
             if self.crops == "quads":
-                check(lib.ms_page_batch_ragged_quads(*head, self.border_mode, self.border_value, *tail))
+                check(lib.ms_page_batch_ragged_quads_maps(*head, self.border_mode, self.border_value, *tail))
             else:
-                check(lib.ms_page_batch_ragged_ex(*head, *tail))
+                check(lib.ms_page_batch_ragged_maps(*head, *tail))
         res = PageBatchResult(b["boxes"], b["counts"], b["crops"], b["n_crops"], b["batch"], b["flags"])
         res._keepalive = (keep, ptrs, hw)  # the kernels read them after this call returns
         return res

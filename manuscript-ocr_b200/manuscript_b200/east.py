@@ -10,8 +10,9 @@ leave the device (the reference's `.cpu().numpy()` at infer.py:312-313 is gone).
 
 Many pages at once: upload_batch puts a list of images into one device buffer, and network_inputs makes all their
 network inputs with one ms_detector_input_batch launch.  input_dtype=torch.float16 / torch.bfloat16 (an extension) makes
-the network input 16-bit: exactly the float32 input cast with `.to(input_dtype)`.  The caller owns the network's dtype;
-maps that come back in another dtype are converted to float32 for the post-processing.
+the network input 16-bit: exactly the float32 input cast with `.to(input_dtype)`.  The caller owns the network's dtype
+and memory format: maps in float32, float16 or bfloat16, at any strides (a channels_last geometry), are read by the
+post-processing kernels as the network left them, with the results of their float32 dense copies.
 """
 import ctypes as C
 import time
@@ -19,7 +20,7 @@ from pathlib import Path
 
 import numpy as np
 
-from ._cabi import MS_FLAG_EDGE_OVERFLOW, EastParams, batch_dtype_code, check, load_library
+from ._cabi import MS_FLAG_EDGE_OVERFLOW, EastParams, batch_dtype_code, check, load_library, maps_descriptor
 from .batch import PageBatch, _raise_for_flags
 from .imaging import read_image, visualize_page
 from .reading_order import reorder_words
@@ -29,6 +30,7 @@ DEFAULT_WEIGHTS = Path.home() / ".manuscript" / "east" / "east_quad_23_05.pth"  
 
 
 _WORD_FIELDS = frozenset(("polygon", "detection_confidence"))
+_FLOAT32 = "float32"  # the default `dtype` of maps_from_device_page(s): torch.float32 (torch is imported lazily)
 
 
 class JpegInfo(C.Structure):
@@ -45,6 +47,16 @@ def jpeg_inspect(data):
     info = JpegInfo()
     check(load_library().ms_jpeg_inspect_host(data, len(data), C.byref(info)))
     return info
+
+
+def kernel_maps(score, geo):
+    """The maps as the post-processing kernels read them: the tensors themselves when both are float32, float16 or
+    bfloat16 of one dtype (at any strides), float32 copies otherwise."""
+    import torch
+
+    if score.dtype == geo.dtype and score.dtype in (torch.float32, torch.float16, torch.bfloat16):
+        return score, geo
+    return score.float(), geo.float()
 
 
 def _is_path(source):
@@ -142,17 +154,21 @@ class EAST:
     # ---- the hot path: maps (device or host) -> final boxes (K,9) float32 on the host -----------------------------
     def boxes_from_maps(self, score_map, geo_map, orig_hw):
         """score (H,W) / (1,H,W), geo (8,H,W) torch CUDA tensors or numpy arrays; orig_hw = (h, w) of the image
-        the boxes are scaled back to (infer.py:346-348).  Runs infer.py:319-356 on the device."""
+        the boxes are scaled back to (infer.py:346-348).  Runs infer.py:319-356 on the device.  CUDA tensors of this
+        device in float32, float16 or bfloat16 (both the same) are read in place at their strides; anything else is
+        converted to float32 first."""
         torch = self.torch
-        s = torch.as_tensor(score_map, dtype=torch.float32, device=self.device)
-        g = torch.as_tensor(geo_map, dtype=torch.float32, device=self.device)
+        if all(isinstance(t, torch.Tensor) and t.device == self.device for t in (score_map, geo_map)):
+            s, g = kernel_maps(score_map, geo_map)
+        else:
+            s = torch.as_tensor(score_map, dtype=torch.float32, device=self.device)
+            g = torch.as_tensor(geo_map, dtype=torch.float32, device=self.device)
         if s.dim() == 3:
             s = s[0]
         H, W = s.shape
         if g.shape != (8, H, W):
             raise ValueError(f"geo_map must be (8,{H},{W}), got {tuple(g.shape)}")
-        s = s.contiguous()
-        g = g.contiguous()
+        maps = maps_descriptor(s[None], g[None])
         r = self._runner
         r.params = self._params()
         ctx, lib = r.ctx, r.ctx.lib
@@ -170,9 +186,9 @@ class EAST:
         while True:
             meta[:4] = 0
             with torch.cuda.device(self.device):
-                check(lib.ms_decode_quads(ctx.handle, s.data_ptr(), g.data_ptr(), 1, H, W, p.score_thresh, p.scale,
-                                          p.quantization, cand.data_ptr(), cap, meta[0:].data_ptr(),
-                                          meta[3:].data_ptr(), C.c_void_p(stream)))
+                check(lib.ms_decode_quads_maps(ctx.handle, C.byref(maps), 1, H, W, p.score_thresh, p.scale,
+                                               p.quantization, cand.data_ptr(), cap, meta[0:].data_ptr(),
+                                               meta[3:].data_ptr(), C.c_void_p(stream)))
                 check(lib.ms_lanms(ctx.handle, cand.data_ptr(), meta[0:].data_ptr(), 1, cap, p.iou_threshold,
                                    kept.data_ptr(), meta[1:].data_ptr(), meta[3:].data_ptr(), C.c_void_p(stream)))
                 check(lib.ms_east_boxes(ctx.handle, kept.data_ptr(), meta[1:].data_ptr(), 1, cap, C.byref(p),
@@ -334,23 +350,31 @@ class EAST:
                                               C.c_void_p(stream)))
         return self._input_buf
 
-    def maps_from_device_page(self, page_dev):
-        """Device image -> (score (1,H',W'), geometry (8,H',W')) CUDA tensors (infer.py:301-313 without the host)."""
+    def _maps_as(self, score, geo, dtype):
+        if dtype is None:
+            return score, geo
+        dtype = self.torch.float32 if dtype is _FLOAT32 else dtype
+        return score.to(dtype), geo.to(dtype)
+
+    def maps_from_device_page(self, page_dev, dtype=_FLOAT32):
+        """Device image -> (score (1,H',W'), geometry (8,H',W')) CUDA tensors (infer.py:301-313 without the host), in
+        float32 by default; dtype=None returns the network's own tensors as they are (their dtype and strides)."""
         if self.model is None:
             raise RuntimeError("EAST(model=...) is required for predict(): the detector network is outside this "
                                "package (use boxes_from_maps / predict_from_maps when the maps already exist)")
         with self.torch.no_grad():
             out = self.model(self.network_input(page_dev))
-        return out["score"][0].float(), out["geometry"][0].float()
+        return self._maps_as(out["score"][0], out["geometry"][0], dtype)
 
-    def maps_from_device_pages(self, pages_dev):
-        """List of P device images -> (score (P,1,H',W'), geometry (P,8,H',W')) float32 CUDA tensors: one
-        network_inputs launch and one call of the network on the (P, 3, T, T) input."""
+    def maps_from_device_pages(self, pages_dev, dtype=_FLOAT32):
+        """List of P device images -> (score (P,1,H',W'), geometry (P,8,H',W')) CUDA tensors, float32 by default
+        (dtype=None: the network's own tensors as they are): one network_inputs launch and one call of the network on
+        the (P, 3, T, T) input."""
         if self.model is None:
             raise RuntimeError("EAST(model=...) is required for predict()")
         with self.torch.no_grad():
             out = self.model(self.network_inputs(pages_dev))
-        return out["score"].float(), out["geometry"].float()
+        return self._maps_as(out["score"], out["geometry"], dtype)
 
     def predict_from_maps(self, score_map, geo_map, orig_hw, sort_reading_order=False):
         words = words_from_boxes(self.boxes_from_maps(score_map, geo_map, orig_hw))
@@ -368,7 +392,7 @@ class EAST:
         else:
             img = read_image(img_or_path)
             page_dev = self.upload(img)
-        score, geo = self.maps_from_device_page(page_dev)
+        score, geo = self.maps_from_device_page(page_dev, dtype=None)  # read in place by the post-processing
         if profile:
             self.torch.cuda.synchronize()
             print(f"  Model inference: {time.time() - t0:.3f}s")
@@ -380,6 +404,6 @@ class EAST:
         return {
             "page": page,
             "vis_image": visualize_page(img, page, show_order=False) if vis else None,  # infer.py:390
-            "score_map": score[0].cpu().numpy() if return_maps else None,
-            "geo_map": geo.cpu().numpy() if return_maps else None,
+            "score_map": score[0].float().cpu().numpy() if return_maps else None,
+            "geo_map": geo.float().cpu().numpy() if return_maps else None,
         }

@@ -6,9 +6,9 @@
 Three routes through predict(), all with the reference's results:
 
 * FUSED -- detector is this package's EAST and recogniser its TRBA: the page image is uploaded ONCE; the network
-  input is made from it on the device, the maps stay on the device, and one ms_page_batch_ragged call (decode, LANMS,
-  box filters, reading order, crop rectangles, resize-and-pad) writes the recogniser's batch, which the recogniser
-  network reads in place.  Device -> host: the final boxes and the crop list (a few tens of kB), never pixels.
+  input is made from it on the device, the maps stay on the device as the network returned them (float32, float16 or
+  bfloat16, any strides), and one ms_page_batch_ragged_maps call (decode, LANMS, box filters, reading order, crop
+  rectangles, resize-and-pad) writes the recogniser's batch, which the recogniser network reads in place.  Device -> host: the final boxes and the crop list (a few tens of kB), never pixels.
 * DEVICE CROPS -- any detector, this package's TRBA: the page is uploaded once, reading order + crop rectangles + the
   crop batch are computed on the device from the detector's polygons.
 * HOST CROPS -- a foreign recogniser gets the list of uint8 crops it expects (plain slices of the page image), in the
@@ -33,7 +33,7 @@ import numpy as np
 from . import ops
 from ._cabi import batch_dtype_code, check
 from .batch import PageBatch
-from .east import EAST, words_from_boxes
+from .east import EAST, kernel_maps, words_from_boxes
 from .imaging import read_image, visualize_page
 from .reading_order import reorder_words
 from .trba import TRBA
@@ -157,7 +157,8 @@ class Pipeline:
         t0 = time.time()
         if page_dev is None:
             page_dev = self.detector.upload(img)                # the one H2D copy of pixels
-        score, geo = self.detector.maps_from_device_page(page_dev)  # network input + maps stay on the device
+        # network input + maps stay on the device, in the network's own dtype and layout
+        score, geo = kernel_maps(*self.detector.maps_from_device_page(page_dev, dtype=None))
         res = self._fused_runner().run_ragged(score[None] if score.dim() == 2 else score, geo[None], [page_dev],
                                               sync=True, allow_order_overflow=True)
         return self._fused_pages(res, self._host_boxes(res, 1), [img], [page_dev], t0, profile)[0]
@@ -169,7 +170,7 @@ class Pipeline:
         t0 = time.time()
         if pages_dev is None:
             pages_dev = self.detector.upload_batch(imgs)        # one H2D copy of pixels per page
-        score, geo = self.detector.maps_from_device_pages(pages_dev)
+        score, geo = kernel_maps(*self.detector.maps_from_device_pages(pages_dev, dtype=None))
         runner = self._fused_runner(batch=True)
         while True:
             res = runner.run_ragged(score, geo, pages_dev, sync=True, allow_order_overflow=True)
